@@ -2,7 +2,7 @@
 """Benchmark of the cascaded-PSD hot path (BASELINE.json metric: sustained MS/s through the full
 PSD cascade; % of HBM roofline).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 Workload (config.workload): BASELINE.json configs[1] -- default PsdCascade (N=4096 Hann, 50 % overlap,
 divide-by-8 half-band cascade per stage) over one second of a 200 MS/s synthetic raw f32 stream.
@@ -19,6 +19,11 @@ so nothing is served from cache between steps); `e2e` is the same metric through
 call with the samples in pinned HOST memory (H2D inside the timed region) and the spectra read back.
 `--impl reference` times the CPU restatement of the reference (oracle/, kind "port": the Rust
 reference cannot be built offline) on the box's host cores.
+
+`--dump-outputs DIR` writes, after all timed runs, the psd() readout that ends the headline loop as
+the caller receives it, per channel c: `psd_ch<c>.npy` (float32 spectrum) and `breaks_ch<c>.npy`
+(float64, one row per stage, columns BREAK_FIELDS).  The input is seeded, so two builds run with
+the same arguments can be compared output for output.  The benchmark writes nothing into the tree.
 """
 import argparse
 import json
@@ -29,6 +34,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the tree may be read-only; leave no __pycache__ in it either
 
 N_FFT = 4096
 SAMPLES_PER_STEP = 200_000_000
@@ -323,14 +329,13 @@ def run_ours(args):
         if world > 1:
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
         prof, launches = ch.c.profile_read()
-        p, b = res[0] if rank == 0 else (None, None)
-        return float(ms.item()), prof, launches, clocks, p, b
+        return float(ms.item()), prof, launches, clocks, res
 
-    ms_rs, _, _, _, _, _ = device_run(True)
-    ms, _, launches, clocks, p, b = device_run(False)
+    ms_rs, _, _, _, _ = device_run(True)
+    ms, _, launches, clocks, readout = device_run(False)
     # the same loop once more with every kernel launch bracketed by CUDA events (per-kernel times for the roofline;
     # the event records cost a few percent, so the headline comes from the unprofiled run above)
-    ms_prof, prof, _, _, _, _ = device_run(False, profile=True)
+    ms_prof, prof, _, _, _ = device_run(False, profile=True)
     value = world * SAMPLES_PER_STEP * args.steps / (ms * 1e-3) / 1e6
     value_rs = world * SAMPLES_PER_STEP * args.steps / (ms_rs * 1e-3) / 1e6
 
@@ -391,7 +396,7 @@ def run_ours(args):
             "share_of_step": k_ms / ms_prof, "profiled_ms_per_step": ms_prof / args.steps,
             "other_kernels_ms": {k: v[0] for k, v in prof.items() if k != "psd_stage0"},
             "whole_step_frac": BYTES_PER_SAMPLE * SAMPLES_PER_STEP * args.steps / (ms * 1e-3) / 1e9 / peak}
-    d2h = sum(len(k.bins) for k in b if k.include) * 4
+    d2h = sum(len(k.bins) for k in readout[0][1] if k.include) * 4
     out = {"metric": "sustained MS/s through full PSD cascade", "value": value, "unit": "MS/s", "n_gpus": world,
            "steps": args.steps, "warmup": args.warmup, "ms_per_step": ms / args.steps, "higher_is_better": True,
            "scaling": "weak", "vs_baseline": None, "dtype": "f32", "data": "synthetic",
@@ -412,9 +417,26 @@ def run_ours(args):
         out["cpu_baseline_n512"] = n512
         out["e2e_small_calls"] = small_calls()
         out["e2e_frames"] = e2e_frames(local)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, readout)
     emit(out)
     if world > 1:
         dist.destroy_process_group()
+
+
+BREAK_FIELDS = ("start", "include", "count", "avg", "bins_start", "bins_end", "fft_size", "decimation", "pending",
+                "processed")
+
+
+def dump_outputs(d, readout):
+    """readout: psd_all()'s [(spectrum, breaks)] per channel; at most 16 stages x (N/2 + 1) bins per channel"""
+    import numpy as np
+    os.makedirs(d, exist_ok=True)
+    for c, (p, breaks) in enumerate(readout):
+        rows = [(k.start, k.include, k.count, k.avg, k.bins.start, k.bins.stop, k.fft_size, k.decimation, k.pending,
+                 k.processed) for k in breaks]
+        np.save(os.path.join(d, "psd_ch%d.npy" % c), np.asarray(p, np.float32))
+        np.save(os.path.join(d, "breaks_ch%d.npy" % c), np.array(rows, np.float64).reshape(-1, len(BREAK_FIELDS)))
 
 
 def timechunk_record(new_group, barrier, rank, world, dist, dev):
@@ -556,7 +578,12 @@ def main():
     ap.add_argument("--steps", type=int, default=10)
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the headline loop's final psd() readout as .npy files")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -6,11 +6,14 @@ import this module.  The product package (stabilizer_stream_b200) never does.
 The shared object is built on demand with `make -C oracle` into a directory keyed on the host
 CPU's feature flags, because it is compiled with -march=native (mirroring the reference's
 `-C target-cpu=native`, .cargo/config.toml:1-2) and the repo snapshot travels between hosts.
+When the tree is read-only and holds no build for this host, it is built into a per-user
+temporary directory instead.
 """
 import ctypes as C
 import hashlib
 import os
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -40,14 +43,18 @@ def _host_key():
 
 
 def lib_path():
-    return os.path.join(_HERE, "_build", _host_key(), "libsspsd_oracle.so")
+    key = _host_key()
+    out = os.path.join(_HERE, "_build", key, "libsspsd_oracle.so")
+    build_dir = os.path.join(_HERE, "_build")
+    if os.path.exists(out) or os.access(build_dir if os.path.isdir(build_dir) else _HERE, os.W_OK):
+        return out
+    return os.path.join(tempfile.gettempdir(), "sspsd_oracle_%d" % os.getuid(), key, "libsspsd_oracle.so")
 
 
 def build(verbose=False):
     out = lib_path()
     if not os.path.exists(out):
-        rel = os.path.relpath(out, _HERE)
-        r = subprocess.run(["make", "-C", _HERE, "OUT=" + rel], capture_output=True, text=True)
+        r = subprocess.run(["make", "-C", _HERE, "OUT=" + out], capture_output=True, text=True)
         if r.returncode != 0:
             raise RuntimeError("oracle build failed:\n" + r.stdout + r.stderr)
         if verbose:

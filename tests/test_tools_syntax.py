@@ -43,3 +43,34 @@ def test_reference_arm_runs_and_matches_the_gpu_arms_config():
     assert out["e2e"]["h2d_bytes_per_step"] == 0 and "parity_note" in out
     for key in ("sustained_2s", "timechunk", "e2e_small_calls", "e2e_frames", "cpu_baseline_n512", "value_readout_every_step"):
         assert '"%s"' % key in open(os.path.join(ROOT, "bench.py")).read()
+
+
+def test_bench_dump_outputs_layout(tmp_path):
+    """--dump-outputs: one float32 spectrum and one float64 break table per channel of the readout"""
+    import sys
+
+    import numpy as np
+    sys.path.insert(0, ROOT)
+    import bench
+    from stabilizer_stream_b200 import Break
+    breaks = [Break(0, False, 0, 0, range(0, 0), 4096, 64, 10, 0),
+              Break(0, True, 3, 0xFFFFFFFF, range(0, 1639), 4096, 8, 7, 1 << 40),
+              Break(1639, True, 97655, 0xFFFFFFFF, range(205, 2049), 4096, 1, 2048, 200_000_000)]
+    p = np.linspace(1, 2, 1639 + 1844, dtype=np.float32)
+    bench.dump_outputs(str(tmp_path / "out"), [(p, breaks), (np.zeros(0, np.float32), [])])
+    assert sorted(os.listdir(tmp_path / "out")) == ["breaks_ch0.npy", "breaks_ch1.npy", "psd_ch0.npy", "psd_ch1.npy"]
+    got = np.load(tmp_path / "out" / "psd_ch0.npy")
+    assert got.dtype == np.float32 and np.array_equal(got, p)
+    b = np.load(tmp_path / "out" / "breaks_ch0.npy")
+    assert b.dtype == np.float64 and b.shape == (3, len(bench.BREAK_FIELDS))
+    assert b[1, -1] == 1 << 40
+    assert b[2].tolist() == [1639, 1, 97655, 0xFFFFFFFF, 205, 2049, 4096, 1, 2048, 200_000_000]
+    assert np.load(tmp_path / "out" / "breaks_ch1.npy").shape == (0, len(bench.BREAK_FIELDS))
+
+
+def test_bench_rejects_bad_arguments():
+    import subprocess
+    import sys
+    for argv in (["--steps", "0"], ["--warmup", "-1"], ["--impl", "reference", "--dump-outputs", "x"]):
+        r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + argv, capture_output=True, text=True, timeout=120)
+        assert r.returncode == 2 and not r.stdout, (argv, r.stderr[-500:])
