@@ -166,6 +166,38 @@ int32_t sspsd_cascade_flush(sspsd_cascade *h);
 /* flush + wait for the handle's stream */
 int32_t sspsd_cascade_sync(sspsd_cascade *h);
 
+/* ---------------------------------------------------------------------------------------------
+ * Cross-spectral density of two streams (no reference analogue: the reference's Psd::process with |c|^2
+ * replaced by conj(cx) cy, see DESIGN.md).  Traces that belong together -- ADC0/DAC0 of a dual-IIR
+ * channel, BI/BQ of a lock-in, ADC0/ADC1 -- are fed pairwise; x and y go through the same cascade
+ * (segments, window, detrend, half-band decimators, EWMA weights), and every stage accumulates
+ *   Sxx = sum w |X|^2,  Syy = sum w |Y|^2,  Sxy = sum w conj(X) Y   (scipy.signal.csd's convention)
+ * so for y = h * x the transfer function is H = pxy / pxx and the coherence |pxy|^2 / (pxx pyy).  The
+ * readout has the breaks of sspsd_cascade_psd and the same 1/(gain_i 8^i) scale on every row: pxx is what
+ * a cascade fed x alone returns.  n_fft = 64 .. 4096 (8192 returns SSPSD_EINVAL: the two-for-one transform
+ * is an N-point complex FFT).  SSPSD_MEM_DEVICE input follows the rule of sspsd_cascade_process_f32 for
+ * BOTH x and y, on the handle's stream (sspsd_csd_stream).  Multi-GPU groups are not supported.
+ * --------------------------------------------------------------------------------------------- */
+typedef struct sspsd_csd sspsd_csd;
+int32_t sspsd_csd_create(const sspsd_config *cfg, sspsd_csd **out);
+void sspsd_csd_destroy(sspsd_csd *h);
+/* deep copy of all per-stage state of both channels */
+int32_t sspsd_csd_clone(sspsd_csd *h, sspsd_csd **out);
+int32_t sspsd_csd_reset(sspsd_csd *h);
+/* the next n samples of both streams (x and y in the same memory kind); any n including 0; results do not
+ * depend on how the streams are split over calls */
+int32_t sspsd_csd_process_f32(sspsd_csd *h, const float *x, const float *y, size_t n, int32_t mem);
+int32_t sspsd_csd_set_avg(sspsd_csd *h, sspsd_avg_opts avg);
+int32_t sspsd_csd_set_detrend(sspsd_csd *h, int32_t detrend);
+int32_t sspsd_csd_rbw(const sspsd_csd *h, float *rbw);
+/* pxx, pyy: *p_len floats; pxy: 2 * *p_len floats, (re, im) interleaved; breaks as sspsd_cascade_psd */
+int32_t sspsd_csd_read(sspsd_csd *h, const sspsd_merge_opts *opts, float *pxx, float *pyy, float *pxy,
+                       size_t *p_len, sspsd_break *b, size_t *b_len);
+int32_t sspsd_csd_num_stages(sspsd_csd *h, uint32_t *n);
+int32_t sspsd_csd_stream(const sspsd_csd *h, void **stream);
+int32_t sspsd_csd_flush(sspsd_csd *h);
+int32_t sspsd_csd_sync(sspsd_csd *h);
+
 /* Break::frequencies(&[Break]) -> Vec<f32>, src/psd.rs:315-327 (pure host helper) */
 int32_t sspsd_break_frequencies(const sspsd_break *b, size_t n_breaks, float *f, size_t *f_len);
 

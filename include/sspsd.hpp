@@ -142,6 +142,92 @@ private:
     sspsd_cascade* h_ = nullptr;
 };
 
+/// Cascaded cross-spectral density of two streams (sspsd_csd_* in sspsd.h), N = 64 .. 4096.  pxx and pyy are what a
+/// PsdCascade<N> fed x or y alone returns; pxy accumulates conj(X) Y, so pxy / pxx is the transfer function x -> y.
+template <size_t N>
+class CsdCascade {
+public:
+    struct Spectra {
+        std::vector<float> pxx, pyy;
+        std::vector<std::pair<float, float>> pxy;  // (re, im)
+        std::vector<Break> breaks;
+    };
+    explicit CsdCascade(int device = 0, void* stream = nullptr, int32_t hbf = SSPSD_HBF_140, Window w = Window::Hann)
+    {
+        sspsd_config cfg;
+        check(sspsd_config_default((uint32_t)N, &cfg));
+        cfg.device = device;
+        cfg.stream = stream;
+        cfg.hbf = hbf;
+        cfg.window = (int32_t)w;
+        check(sspsd_csd_create(&cfg, &h_));
+    }
+    CsdCascade(const CsdCascade& o) { check(sspsd_csd_clone(o.h_, &h_)); }
+    CsdCascade& operator=(const CsdCascade& o)
+    {
+        if (this != &o) {
+            sspsd_csd* n = nullptr;
+            check(sspsd_csd_clone(o.h_, &n));
+            sspsd_csd_destroy(h_);
+            h_ = n;
+        }
+        return *this;
+    }
+    CsdCascade(CsdCascade&& o) noexcept : h_(o.h_) { o.h_ = nullptr; }
+    ~CsdCascade() { sspsd_csd_destroy(h_); }
+
+    float rbw() const
+    {
+        float r;
+        check(sspsd_csd_rbw(h_, &r));
+        return r;
+    }
+    void set_avg(AvgOpts a) { check(sspsd_csd_set_avg(h_, sspsd_avg_opts{a.limit, a.count})); }
+    void set_detrend(Detrend d) { check(sspsd_csd_set_detrend(h_, (int32_t)d)); }
+    void process(const float* x, const float* y, size_t n, Mem mem = Mem::Host)
+    {
+        check(sspsd_csd_process_f32(h_, x, y, n, (int32_t)mem));
+    }
+    void process(const std::vector<float>& x, const std::vector<float>& y)
+    {
+        if (x.size() != y.size()) throw Error(SSPSD_EINVAL, "x and y must have the same length");
+        process(x.data(), y.data(), x.size());
+    }
+    Spectra csd(const MergeOpts& o = MergeOpts()) const
+    {
+        sspsd_merge_opts mo{o.keep_overlap, o.min_count, o.keep_transition_band};
+        Spectra s;
+        const size_t cap = SSPSD_MAX_STAGES * (N / 2 + 1);
+        s.pxx.resize(cap);
+        s.pyy.resize(cap);
+        std::vector<float> xy(2 * cap);
+        sspsd_break cb[SSPSD_MAX_STAGES];
+        size_t pl = cap, bl = SSPSD_MAX_STAGES;
+        check(sspsd_csd_read(h_, &mo, s.pxx.data(), s.pyy.data(), xy.data(), &pl, cb, &bl));
+        s.pxx.resize(pl);
+        s.pyy.resize(pl);
+        for (size_t k = 0; k < pl; ++k) s.pxy.emplace_back(xy[2 * k], xy[2 * k + 1]);
+        for (size_t i = 0; i < bl; ++i)
+            s.breaks.push_back(Break{(size_t)cb[i].start, cb[i].include != 0, cb[i].count, cb[i].avg,
+                                     {(size_t)cb[i].bins_start, (size_t)cb[i].bins_end}, (size_t)cb[i].fft_size,
+                                     (size_t)cb[i].decimation, (size_t)cb[i].pending, (size_t)cb[i].processed});
+        return s;
+    }
+    uint32_t num_stages() const
+    {
+        uint32_t n;
+        check(sspsd_csd_num_stages(h_, &n));
+        return n;
+    }
+    void reset() { check(sspsd_csd_reset(h_)); }
+    void flush() { check(sspsd_csd_flush(h_)); }
+    void sync() { check(sspsd_csd_sync(h_)); }
+    sspsd_csd* handle() const { return h_; }
+
+private:
+    sspsd_csd* h_ = nullptr;
+};
+
 /// Psd<N> + trait PsdStage, src/psd.rs:119-288
 template <size_t N>
 class Psd {

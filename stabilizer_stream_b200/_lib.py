@@ -100,6 +100,19 @@ PROTOTYPES = {
     "sspsd_cascade_flush": (_i32, [_vp]),
     "sspsd_cascade_sync": (_i32, [_vp]),
     "sspsd_break_frequencies": (_i32, [C.POINTER(BreakC), _sz, _vp, _psz]),
+    "sspsd_csd_create": (_i32, [C.POINTER(Config), C.POINTER(_vp)]),
+    "sspsd_csd_destroy": (None, [_vp]),
+    "sspsd_csd_clone": (_i32, [_vp, C.POINTER(_vp)]),
+    "sspsd_csd_reset": (_i32, [_vp]),
+    "sspsd_csd_process_f32": (_i32, [_vp, _vp, _vp, _sz, _i32]),
+    "sspsd_csd_set_avg": (_i32, [_vp, AvgOptsC]),
+    "sspsd_csd_set_detrend": (_i32, [_vp, _i32]),
+    "sspsd_csd_rbw": (_i32, [_vp, C.POINTER(C.c_float)]),
+    "sspsd_csd_read": (_i32, [_vp, C.POINTER(MergeOptsC), _vp, _vp, _vp, _psz, C.POINTER(BreakC), _psz]),
+    "sspsd_csd_num_stages": (_i32, [_vp, C.POINTER(C.c_uint32)]),
+    "sspsd_csd_stream": (_i32, [_vp, C.POINTER(_vp)]),
+    "sspsd_csd_flush": (_i32, [_vp]),
+    "sspsd_csd_sync": (_i32, [_vp]),
     "sspsd_cascade_partials": (_i32, [_vp, C.POINTER(PartialsC)]),
     "sspsd_cascade_set_counts": (_i32, [_vp, C.POINTER(C.c_uint64), C.c_uint32]),
     "sspsd_cascade_seek": (_i32, [_vp, C.c_uint64]),

@@ -385,7 +385,7 @@ int Cascade::init(const sspsd_config& cfg, uint32_t max_stages)
     // readout joins the streams, so nothing changes for a caller that reads out after every batch).
     const char* ov = getenv("SSPSD_OVERLAP");
     deep_from_ = ov ? (size_t)atoi(ov) : 1;
-    if (max_stages_ > 1 && deep_from_ > 0) {
+    if (max_stages_ > 1 && deep_from_ > 0 && !one_stream_) {
         // high priority: the small deep-stage grids should be scheduled ahead of the remaining stage-0 CTAs
         int lo_prio = 0, hi_prio = 0;
         SSPSD_CUDA(cudaDeviceGetStreamPriorityRange(&lo_prio, &hi_prio));
@@ -529,6 +529,7 @@ int Cascade::ensure_fresh(StageState& st, size_t need, size_t reserve)
 
 int Cascade::launch_psd(size_t i, const StreamSrc& src, uint64_t k0, uint64_t nseg, int jb, float g_first, float g_s)
 {
+    if (hook_) return hook_->stage_psd(*this, i, src, k0, nseg, jb, g_first, g_s);
     StageParams p{};
     p.src = src;
     p.k0 = (long long)k0;
@@ -1348,11 +1349,11 @@ int Cascade::reset()
     return SSPSD_OK;
 }
 
-int Cascade::clone_from(Cascade& o)
+int Cascade::clone_from(Cascade& o, const sspsd_config* cfg)
 {
     int rc = o.sync();
     if (rc) return rc;
-    rc = init(o.cfg_, o.max_stages_);
+    rc = init(cfg ? *cfg : o.cfg_, o.max_stages_);
     if (rc) return rc;
     DeviceGuard g(cfg_.device);
     if (!g.ok) return SSPSD_ECUDA;

@@ -75,12 +75,22 @@ struct StageState {
     cudaEvent_t ev_psd[2] = {nullptr, nullptr};   // PSD stream: the PSD kernel has finished reading fresh[b] + carry
 };
 
+class Cascade;
+// Two-channel mode (XCascade): a stage's PSD launch is handed to the hook instead, with the launch's segment
+// range and EWMA weights; the EWMA pre-scale of the cascade's own rows still runs and is unused.
+struct StageHook {
+    virtual int stage_psd(Cascade& c, size_t i, const StreamSrc& src, uint64_t k0, uint64_t nseg, int jb, float g_first,
+                          float g_s) = 0;
+};
+
 class Cascade {
+    friend class XCascade;
+
 public:
     Cascade() = default;
     ~Cascade();
     int init(const sspsd_config& cfg, uint32_t max_stages);
-    int clone_from(Cascade& o);
+    int clone_from(Cascade& o, const sspsd_config* cfg = nullptr);  // cfg: configuration of the copy (default o's)
     int reset();
 
     int process(const float* x, size_t n, int mem);
@@ -168,6 +178,8 @@ private:
     uint64_t next_valid_from(uint64_t valid) const;
     uint64_t own_offset(size_t i) const;  // stage-0 position of sample 0 of stage i
 
+    StageHook* hook_ = nullptr;
+    bool one_stream_ = false;  // set before init(): every stage and PSD launch on stream_ (no side streams)
     sspsd_config cfg_{};
     uint32_t n_ = 0, log2n_ = 0, hop_ = 0, max_stages_ = SSPSD_MAX_STAGES;
     WindowInfo win_{};

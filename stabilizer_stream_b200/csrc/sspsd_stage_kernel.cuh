@@ -55,8 +55,8 @@ __device__ __forceinline__ AccSink acc_sink(const float* /*unused*/, float* acc,
     return AccSink{acc, part ? part + (size_t)row_index * part_stride : nullptr};
 }
 
-// acc[k] += sum over rows (in row order, f64) of part[r][k]
-__global__ void reduce_partials_kernel(float* __restrict__ acc, const float* __restrict__ part, int nrows, int stride, int nbins)
+// acc[k] += sum over rows (in row order, f64) of part[r][k]  (internal linkage: included by more than one unit)
+static __global__ void reduce_partials_kernel(float* __restrict__ acc, const float* __restrict__ part, int nrows, int stride, int nbins)
 {
     const int k = blockIdx.x * blockDim.x + threadIdx.x;
     if (k >= nbins) return;

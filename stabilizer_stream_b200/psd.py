@@ -325,6 +325,110 @@ class PsdCascade(_StreamOrdered):
             self._h = None
 
 
+class CsdCascade(_StreamOrdered):
+    """Cascaded cross-spectral density of two streams x and y (include/sspsd.h, sspsd_csd_*).  Both go through the
+    same cascade as PsdCascade; every stage accumulates |X|^2, |Y|^2 and conj(X) Y (scipy.signal.csd's convention),
+    so for y = h * x, pxy / pxx is the transfer function H and pxx is what a PsdCascade fed x alone returns.
+    n = 64 .. 4096."""
+
+    def __init__(self, n=512, window=Window.HANN, device=0, hbf=Hbf.TAPS_140, stream=None, max_batch=0, host_stage=0,
+                 deep_defer=0, deterministic=False, _handle=None):
+        self.n = n
+        self.device = int(device)
+        if _handle is not None:
+            self._h = _handle
+            return
+        cfg = _config(n, window, hbf, device, stream, max_batch, host_stage, deep_defer, deterministic)
+        h = C.c_void_p()
+        L.check(L.lib().sspsd_csd_create(C.byref(cfg), C.byref(h)))
+        self._h = h
+
+    def clone(self):
+        h = C.c_void_p()
+        L.check(L.lib().sspsd_csd_clone(self._h, C.byref(h)))
+        return CsdCascade(self.n, device=self.device, _handle=h)
+
+    def _stream_ptr(self):
+        s = C.c_void_p()
+        L.check(L.lib().sspsd_csd_stream(self._h, C.byref(s)))
+        return s.value or 0
+
+    def reset(self):
+        L.check(L.lib().sspsd_csd_reset(self._h))
+
+    def rbw(self):
+        r = C.c_float()
+        L.check(L.lib().sspsd_csd_rbw(self._h, C.byref(r)))
+        return r.value
+
+    def set_avg(self, avg: AvgOpts):
+        L.check(L.lib().sspsd_csd_set_avg(self._h, L.AvgOptsC(avg.limit, avg.count)))
+
+    def set_detrend(self, d: Detrend):
+        L.check(L.lib().sspsd_csd_set_detrend(self._h, int(d)))
+
+    def process(self, x, y):
+        """the next samples of both streams: equal-length float32 numpy arrays, or CUDA tensors (both)"""
+        px, n, mem, kx = _as_buffer(x)
+        py, ny, memy, ky = _as_buffer(y)
+        if n != ny:
+            raise ValueError("x and y must have the same length (%d != %d)" % (n, ny))
+        if mem != memy:
+            raise ValueError("x and y must both be host arrays or both be CUDA tensors")
+        if mem == L.MEM_DEVICE:
+            self._order_device_input(kx)
+            self._order_device_input(ky)
+        L.check(L.lib().sspsd_csd_process_f32(self._h, px, py, n, mem))
+        if mem == L.MEM_DEVICE:
+            self._release_device_input(kx)
+        del kx, ky
+
+    def flush(self):
+        L.check(L.lib().sspsd_csd_flush(self._h))
+
+    def sync(self):
+        L.check(L.lib().sspsd_csd_sync(self._h))
+
+    def num_stages(self):
+        n = C.c_uint32()
+        L.check(L.lib().sspsd_csd_num_stages(self._h, C.byref(n)))
+        return n.value
+
+    def csd(self, opts: MergeOpts = None):
+        """-> (pxx, pyy, pxy (complex64), breaks), merged like PsdCascade.psd"""
+        opts = opts or MergeOpts()
+        o = L.MergeOptsC(int(opts.keep_overlap), opts.min_count, int(opts.keep_transition_band))
+        cap = L.MAX_STAGES * (self.n // 2 + 1)
+        pxx, pyy = np.zeros(cap, np.float32), np.zeros(cap, np.float32)
+        pxy = np.zeros(2 * cap, np.float32)
+        b = (L.BreakC * L.MAX_STAGES)()
+        pl, bl = C.c_size_t(cap), C.c_size_t(L.MAX_STAGES)
+        L.check(L.lib().sspsd_csd_read(self._h, C.byref(o), pxx.ctypes.data, pyy.ctypes.data, pxy.ctypes.data,
+                                       C.byref(pl), b, C.byref(bl)))
+        n = pl.value
+        return (pxx[:n].copy(), pyy[:n].copy(), pxy[:2 * n].view(np.complex64).copy(),
+                [Break._from_c(b[i]) for i in range(bl.value)])
+
+    @staticmethod
+    def coherence(pxx, pyy, pxy):
+        """magnitude-squared coherence |pxy|^2 / (pxx pyy) per bin (0 where a power is 0)"""
+        pxx, pyy = np.asarray(pxx, np.float64), np.asarray(pyy, np.float64)
+        den = pxx * pyy
+        return np.divide(np.abs(np.asarray(pxy, np.complex128)) ** 2, den, out=np.zeros_like(den), where=den > 0)
+
+    @staticmethod
+    def transfer(pxx, pxy):
+        """transfer function estimate H = pxy / pxx per bin (0 where pxx is 0)"""
+        pxx = np.asarray(pxx, np.float64)
+        return np.divide(np.asarray(pxy, np.complex128), pxx, out=np.zeros(pxx.shape, np.complex128), where=pxx > 0)
+
+    def __del__(self):
+        h = getattr(self, "_h", None)
+        if h and L is not None and getattr(L, "_lib", None) is not None:
+            L._lib.sspsd_csd_destroy(h)
+            self._h = None
+
+
 class Psd(_StreamOrdered):
     """Psd<N> + trait PsdStage, src/psd.rs:119-288 (one stage, decimated output exposed)."""
 
