@@ -198,6 +198,37 @@ int32_t sspsd_csd_stream(const sspsd_csd *h, void **stream);
 int32_t sspsd_csd_flush(sspsd_csd *h);
 int32_t sspsd_csd_sync(sspsd_csd *h);
 
+/* ---------------------------------------------------------------------------------------------
+ * Cross-spectral matrix of k = 2, 3 or 4 streams (a Stabilizer stream's traces: ADC0, ADC1, DAC0, DAC1 of
+ * AdcDac, ...).  All k go through one cascade, and every stage accumulates the Hermitian matrix
+ *   S_ij = sum w conj(X_i) X_j
+ * (sspsd_csd_*'s convention: S[0,1] is pxy of a sspsd_csd fed (x0, x1)), with sspsd_csd_*'s limits
+ * (n_fft = 64 .. 4096, Hann or rectangular, Linear detrend SSPSD_EUNIMPLEMENTED).  Every transform is
+ * shared by all pairs, so the matrix costs k decimations and k FFTs per segment, where k (k - 1) / 2
+ * sspsd_csd handles cost k (k - 1) of each.  k = 2 computes exactly what sspsd_csd_* computes.
+ * --------------------------------------------------------------------------------------------- */
+typedef struct sspsd_csm sspsd_csm;
+/* k not in {2, 3, 4}: SSPSD_EINVAL */
+int32_t sspsd_csm_create(const sspsd_config *cfg, int32_t k, sspsd_csm **out);
+void sspsd_csm_destroy(sspsd_csm *h);
+int32_t sspsd_csm_clone(sspsd_csm *h, sspsd_csm **out);
+int32_t sspsd_csm_channels(const sspsd_csm *h, int32_t *k);
+int32_t sspsd_csm_reset(sspsd_csm *h);
+/* x: k pointers to the next n samples of each stream (all in the same memory kind); any n including 0 */
+int32_t sspsd_csm_process_f32(sspsd_csm *h, const float *const *x, size_t n, int32_t mem);
+int32_t sspsd_csm_set_avg(sspsd_csm *h, sspsd_avg_opts avg);
+int32_t sspsd_csm_set_detrend(sspsd_csm *h, int32_t detrend);
+int32_t sspsd_csm_rbw(const sspsd_csm *h, float *rbw);
+/* s: 2 k k *p_len floats, S_ij[b] at s[2 ((i k + j) *p_len + b) + {0, 1}] (re, im) with *p_len the merged
+ * length on return; the diagonal is real (imaginary part exactly 0) and S_ji = conj(S_ij) exactly.  On input
+ * *p_len is the capacity per (i, j); too small: SSPSD_ESHORT with the lengths needed, as sspsd_csd_read */
+int32_t sspsd_csm_read(sspsd_csm *h, const sspsd_merge_opts *opts, float *s, size_t *p_len, sspsd_break *b,
+                       size_t *b_len);
+int32_t sspsd_csm_num_stages(sspsd_csm *h, uint32_t *n);
+int32_t sspsd_csm_stream(const sspsd_csm *h, void **stream);
+int32_t sspsd_csm_flush(sspsd_csm *h);
+int32_t sspsd_csm_sync(sspsd_csm *h);
+
 /* Break::frequencies(&[Break]) -> Vec<f32>, src/psd.rs:315-327 (pure host helper) */
 int32_t sspsd_break_frequencies(const sspsd_break *b, size_t n_breaks, float *f, size_t *f_len);
 

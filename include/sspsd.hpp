@@ -228,6 +228,102 @@ private:
     sspsd_csd* h_ = nullptr;
 };
 
+/// Cascaded cross-spectral matrix of K = 2 .. 4 streams (sspsd_csm_* in sspsd.h), N = 64 .. 4096.  s(i, j) accumulates
+/// conj(X_i) X_j: s(0, 1) is CsdCascade's pxy of (x0, x1), and s(i, i) what a PsdCascade<N> fed x_i alone returns.
+template <size_t N>
+class CsmCascade {
+public:
+    struct Matrix {
+        size_t k = 0, bins = 0;
+        std::vector<std::pair<float, float>> s;  // (re, im) of S_ij[b] at (i k + j) bins + b
+        std::vector<Break> breaks;
+        std::pair<float, float> operator()(size_t i, size_t j, size_t b) const { return s[(i * k + j) * bins + b]; }
+    };
+    explicit CsmCascade(int k, int device = 0, void* stream = nullptr, int32_t hbf = SSPSD_HBF_140,
+                        Window w = Window::Hann)
+    {
+        sspsd_config cfg;
+        check(sspsd_config_default((uint32_t)N, &cfg));
+        cfg.device = device;
+        cfg.stream = stream;
+        cfg.hbf = hbf;
+        cfg.window = (int32_t)w;
+        check(sspsd_csm_create(&cfg, k, &h_));
+        k_ = k;
+    }
+    CsmCascade(const CsmCascade& o) : k_(o.k_) { check(sspsd_csm_clone(o.h_, &h_)); }
+    CsmCascade& operator=(const CsmCascade& o)
+    {
+        if (this != &o) {
+            sspsd_csm* n = nullptr;
+            check(sspsd_csm_clone(o.h_, &n));
+            sspsd_csm_destroy(h_);
+            h_ = n;
+            k_ = o.k_;
+        }
+        return *this;
+    }
+    CsmCascade(CsmCascade&& o) noexcept : h_(o.h_), k_(o.k_) { o.h_ = nullptr; }
+    ~CsmCascade() { sspsd_csm_destroy(h_); }
+
+    int channels() const { return k_; }
+    float rbw() const
+    {
+        float r;
+        check(sspsd_csm_rbw(h_, &r));
+        return r;
+    }
+    void set_avg(AvgOpts a) { check(sspsd_csm_set_avg(h_, sspsd_avg_opts{a.limit, a.count})); }
+    void set_detrend(Detrend d) { check(sspsd_csm_set_detrend(h_, (int32_t)d)); }
+    /// x: channels() pointers to n samples each
+    void process(const float* const* x, size_t n, Mem mem = Mem::Host)
+    {
+        check(sspsd_csm_process_f32(h_, x, n, (int32_t)mem));
+    }
+    void process(const std::vector<std::vector<float>>& x)
+    {
+        if ((int)x.size() != k_) throw Error(SSPSD_EINVAL, "one vector per channel");
+        const float* p[4];
+        for (int c = 0; c < k_; ++c) {
+            if (x[c].size() != x[0].size()) throw Error(SSPSD_EINVAL, "channels must have the same length");
+            p[c] = x[c].data();
+        }
+        process(p, x[0].size());
+    }
+    Matrix csm(const MergeOpts& o = MergeOpts()) const
+    {
+        sspsd_merge_opts mo{o.keep_overlap, o.min_count, o.keep_transition_band};
+        const size_t cap = SSPSD_MAX_STAGES * (N / 2 + 1);
+        std::vector<float> s(2 * (size_t)k_ * k_ * cap);
+        sspsd_break cb[SSPSD_MAX_STAGES];
+        size_t pl = cap, bl = SSPSD_MAX_STAGES;
+        check(sspsd_csm_read(h_, &mo, s.data(), &pl, cb, &bl));
+        Matrix m;
+        m.k = (size_t)k_;
+        m.bins = pl;
+        for (size_t r = 0; r < m.k * m.k * pl; ++r) m.s.emplace_back(s[2 * r], s[2 * r + 1]);
+        for (size_t i = 0; i < bl; ++i)
+            m.breaks.push_back(Break{(size_t)cb[i].start, cb[i].include != 0, cb[i].count, cb[i].avg,
+                                     {(size_t)cb[i].bins_start, (size_t)cb[i].bins_end}, (size_t)cb[i].fft_size,
+                                     (size_t)cb[i].decimation, (size_t)cb[i].pending, (size_t)cb[i].processed});
+        return m;
+    }
+    uint32_t num_stages() const
+    {
+        uint32_t n;
+        check(sspsd_csm_num_stages(h_, &n));
+        return n;
+    }
+    void reset() { check(sspsd_csm_reset(h_)); }
+    void flush() { check(sspsd_csm_flush(h_)); }
+    void sync() { check(sspsd_csm_sync(h_)); }
+    sspsd_csm* handle() const { return h_; }
+
+private:
+    sspsd_csm* h_ = nullptr;
+    int k_ = 0;
+};
+
 /// Psd<N> + trait PsdStage, src/psd.rs:119-288
 template <size_t N>
 class Psd {

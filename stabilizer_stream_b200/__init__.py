@@ -4,10 +4,10 @@ Host-side mirror of the reference API (src/psd.rs, src/de, src/loss.rs, src/var.
 C ABI in include/sspsd.h.  The CUDA library is the only implementation: importing `psd` symbols
 works without a GPU, creating any handle does not.
 """
-from .psd import (DEPTH, HBF_PASSBAND, AvgOpts, Break, CsdCascade, DecodeError, Detrend, Format, FrameDecoder, Hbf, Loss,
+from .psd import (DEPTH, HBF_PASSBAND, AvgOpts, Break, CsdCascade, CsmCascade, DecodeError, Detrend, Format, FrameDecoder, Hbf, Loss,
                   MergeOpts, Psd, PsdCascade, Receiver, ShardMode, Source, SourceKind, TimeChunk, Trace, Var, Window,
                   Group, time_plan)
 
-__all__ = ["DEPTH", "HBF_PASSBAND", "AvgOpts", "Break", "CsdCascade", "DecodeError", "Detrend", "Format", "FrameDecoder", "Hbf",
+__all__ = ["DEPTH", "HBF_PASSBAND", "AvgOpts", "Break", "CsdCascade", "CsmCascade", "DecodeError", "Detrend", "Format", "FrameDecoder", "Hbf",
            "Loss", "MergeOpts", "Psd", "PsdCascade", "Receiver", "ShardMode", "Source", "SourceKind", "TimeChunk", "Trace",
            "Var", "Window", "Group", "time_plan"]

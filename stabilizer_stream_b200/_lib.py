@@ -113,6 +113,20 @@ PROTOTYPES = {
     "sspsd_csd_stream": (_i32, [_vp, C.POINTER(_vp)]),
     "sspsd_csd_flush": (_i32, [_vp]),
     "sspsd_csd_sync": (_i32, [_vp]),
+    "sspsd_csm_create": (_i32, [C.POINTER(Config), _i32, C.POINTER(_vp)]),
+    "sspsd_csm_destroy": (None, [_vp]),
+    "sspsd_csm_clone": (_i32, [_vp, C.POINTER(_vp)]),
+    "sspsd_csm_channels": (_i32, [_vp, C.POINTER(_i32)]),
+    "sspsd_csm_reset": (_i32, [_vp]),
+    "sspsd_csm_process_f32": (_i32, [_vp, _vp, _sz, _i32]),
+    "sspsd_csm_set_avg": (_i32, [_vp, AvgOptsC]),
+    "sspsd_csm_set_detrend": (_i32, [_vp, _i32]),
+    "sspsd_csm_rbw": (_i32, [_vp, C.POINTER(C.c_float)]),
+    "sspsd_csm_read": (_i32, [_vp, C.POINTER(MergeOptsC), _vp, _psz, C.POINTER(BreakC), _psz]),
+    "sspsd_csm_num_stages": (_i32, [_vp, C.POINTER(C.c_uint32)]),
+    "sspsd_csm_stream": (_i32, [_vp, C.POINTER(_vp)]),
+    "sspsd_csm_flush": (_i32, [_vp]),
+    "sspsd_csm_sync": (_i32, [_vp]),
     "sspsd_cascade_partials": (_i32, [_vp, C.POINTER(PartialsC)]),
     "sspsd_cascade_set_counts": (_i32, [_vp, C.POINTER(C.c_uint64), C.c_uint32]),
     "sspsd_cascade_seek": (_i32, [_vp, C.c_uint64]),

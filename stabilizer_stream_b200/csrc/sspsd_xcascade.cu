@@ -1,14 +1,20 @@
 // sspsd_xcascade.cu -- XCascade: the cascaded cross-spectral density of two streams (sspsd_csd_* of
-// include/sspsd.h).
+// include/sspsd.h) and the cross-spectral matrix of K = 2 .. 4 streams (sspsd_csm_*).
 //
-// Two Cascades, one per channel, are driven in lockstep.  Their bookkeeping (segments, decimation, deferral,
-// EWMA counts) does not depend on the data, so both run exactly the same stages over the same segment ranges;
-// their own PSD launches are replaced by a hook (Cascade::hook_).  Channel y runs a chunk first and leaves, per
-// stage, the StreamSrc its PSD kernel would have read; channel x then runs the same chunk and, where its PSD
-// kernel would go, launches csd_stage_kernel over both sources.  Both cascades order all their work on ONE
-// stream (no deep / PSD side streams), so stream order alone makes every CSD launch follow both channels'
-// decimators and precede any later overwrite of the buffers it reads; between two lockstep steps each stage
-// runs at most once, so the source y left for a stage is the one x's launch needs.
+// K Cascades, one per channel, are driven in lockstep.  Their bookkeeping (segments, decimation, deferral,
+// EWMA counts) does not depend on the data, so all run exactly the same stages over the same segment ranges;
+// their own PSD launches are replaced by a hook (Cascade::hook_).  Channels K-1 .. 1 run a chunk first and
+// leave, per stage, the StreamSrc their PSD kernel would have read; channel 0 then runs the same chunk and,
+// where its PSD kernel would go, launches the block kernels over all sources.  All cascades order all their
+// work on ONE stream (no deep / PSD side streams), so stream order alone makes every launch follow all
+// channels' decimators and precede any later overwrite of the buffers it reads; between two lockstep steps each
+// stage runs at most once, so the source a channel left for a stage is the one channel 0's launch needs.
+//
+// Block decomposition (DESIGN.md 3b): channels pair up as (0, 1) and (2, 3).  The diagonal block of each pair
+// is csd_stage_kernel's four rows; the off-diagonal block (K >= 3) is csm_cross_kernel's eight.  A stage's
+// accumulator block is [pair (0,1): Sxx Syy ReSxy ImSxy][pair (2,3): the same][cross: 8 rows], so K = 2 (the
+// CSD) has exactly the first four rows.  K = 3 runs pair (2,3)'s csd_stage_kernel with channel 2 in both slots:
+// its rows 1..3 are S22 again and are never read.
 #include "sspsd_cascade.cuh"
 
 #include <algorithm>
@@ -17,7 +23,7 @@
 #include <new>
 #include <vector>
 
-#include "sspsd_csd_kernel.cuh"
+#include "sspsd_csm_kernel.cuh"
 
 namespace sspsd {
 
@@ -46,6 +52,31 @@ int launch_csd_t(const CsdParams& p, int grid, cudaStream_t s)
 {
     csd_stage_kernel<LOG2N><<<grid, Plan<LOG2N + 1>::NT, csd_smem_bytes<LOG2N>(p.T, p.hop), s>>>(p);
     return cuda_ok(cudaGetLastError(), "csd_stage_kernel launch") ? SSPSD_OK : SSPSD_ECUDA;
+}
+
+template <int LOG2N>
+int prepare_csm_t(int hop, int* tmax)
+{
+    using PL = Plan<LOG2N + 1>;
+    // two CTAs per SM up to 256 threads (2 x (110 KB + 1 KB reserved) of the SM's 228 KB), one above
+    const long long budget = PL::NT <= 256 ? 110 * 1024 : 220 * 1024;
+    int t = 256;
+    while (t > 1 && (long long)csm_smem_bytes<LOG2N>(t, hop) > budget) --t;
+    if ((long long)csm_smem_bytes<LOG2N>(t, hop) > budget) {
+        set_error("FFT size does not fit in shared memory");
+        return SSPSD_EINVAL;
+    }
+    *tmax = t;
+    SSPSD_CUDA(cudaFuncSetAttribute(csm_cross_kernel<LOG2N>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                    (int)csm_smem_bytes<LOG2N>(t, hop)));
+    return SSPSD_OK;
+}
+
+template <int LOG2N>
+int launch_csm_t(const CsmParams& p, int grid, cudaStream_t s)
+{
+    csm_cross_kernel<LOG2N><<<grid, Plan<LOG2N + 1>::NT, csm_smem_bytes<LOG2N>(p.T, p.hop), s>>>(p);
+    return cuda_ok(cudaGetLastError(), "csm_cross_kernel launch") ? SSPSD_OK : SSPSD_ECUDA;
 }
 
 #define SSPSD_CSD_SIZES(X) X(6) X(7) X(8) X(9) X(10) X(11) X(12)
@@ -77,34 +108,83 @@ int launch_csd(int log2n, const CsdParams& p, int grid, cudaStream_t s)
     }
 }
 
+int prepare_csm(int log2n, int hop, int* tmax)
+{
+    switch (log2n) {
+#define X(L) \
+    case L:  \
+        return prepare_csm_t<L>(hop, tmax);
+        SSPSD_CSD_SIZES(X)
+#undef X
+    default:
+        return SSPSD_EINVAL;
+    }
+}
+
+int launch_csm(int log2n, const CsmParams& p, int grid, cudaStream_t s)
+{
+    switch (log2n) {
+#define X(L) \
+    case L:  \
+        return launch_csm_t<L>(p, grid, s);
+        SSPSD_CSD_SIZES(X)
+#undef X
+    default:
+        return SSPSD_EINVAL;
+    }
+}
+
+// persistent tiled launch as psd_stage_kernel's: tiles as large as shared memory allows once there is enough
+// work, about two CTAs per SM walking contiguous ranges of tiles
+struct TiledLaunch {
+    int T, tile_cap, tpc, grid;
+};
+TiledLaunch tiled_launch(uint64_t nseg, int groups, int tmax, int hop, int n, int num_sms)
+{
+    TiledLaunch l;
+    const long long t = ((long long)nseg + 2ll * num_sms - 1) / (2ll * num_sms);
+    l.T = (int)std::max<long long>(std::min<long long>(groups, (long long)nseg), std::min<long long>(t, tmax));
+    l.T = std::min(l.T, tmax);
+    l.tile_cap = (l.T - 1) * hop + n;
+    const long long ntiles = ((long long)nseg + l.T - 1) / l.T;
+    l.tpc = (int)std::max<long long>(1, (ntiles + 2ll * num_sms - 1) / (2ll * num_sms));
+    l.grid = (int)((ntiles + l.tpc - 1) / l.tpc);
+    return l;
+}
+
 }  // namespace
 
 class XCascade : public StageHook {
 public:
     XCascade() = default;
     ~XCascade();
-    int init(const sspsd_config& cfg);
+    int init(const sspsd_config& cfg, int k);
     int clone_from(XCascade& o);
     int reset();
-    int process(const float* x, const float* y, size_t n, int mem);
+    int process(const float* const* x, size_t n, int mem);
     int set_avg(sspsd_avg_opts a);
     int set_detrend(int d);
     int flush();
     int sync();
     int read(const sspsd_merge_opts& o, float* pxx, float* pyy, float* pxy, size_t* p_len, sspsd_break* b,
              size_t* b_len);
+    int read_matrix(const sspsd_merge_opts& o, float* s, size_t* p_len, sspsd_break* b, size_t* b_len);
     int num_stages(uint32_t* n);
-    float rbw() const { return x_.rbw(); }
+    int channels() const { return k_; }
+    float rbw() const { return ch_[0].rbw(); }
     cudaStream_t stream() const { return stream_; }
     int stage_psd(Cascade& c, size_t i, const StreamSrc& src, uint64_t k0, uint64_t nseg, int jb, float g_first,
                   float g_s) override;
 
 private:
-    int setup(const sspsd_config& cfg);
+    int setup(const sspsd_config& cfg, int k);
     sspsd_config channel_cfg() const;
-    int feed_chunk(const float* x, const float* y, size_t n, bool device);
+    int feed_chunk(const float* const* x, size_t n, bool device);
     int flush_staged();
     int flush_all();
+    size_t block_rows() const { return k_ == 2 ? CSD_ROWS : 2 * CSD_ROWS + CSM_XROWS; }
+    size_t acc_floats() const { return (size_t)SSPSD_MAX_STAGES * block_rows() * stride_; }
+    int ensure_part(float** part, size_t* cap, size_t need);
 
     // destroyed after the channels, whose destructors still synchronise the stream
     struct OwnedStream {
@@ -117,23 +197,26 @@ private:
             cudaStreamDestroy(s);
         }
     } own_;
-    Cascade x_, y_;
+    Cascade ch_[4];  // channel 0 launches the block kernels; 1 .. k_-1 leave their sources
+    int k_ = 2;
     sspsd_config cfg_{};
     cudaStream_t stream_ = nullptr;
     uint32_t n_ = 0, log2n_ = 0;
-    int num_sms_ = 148, tmax_ = 1, groups_ = 1;
-    uint32_t stride_ = 0;  // floats per row; a stage's block is CSD_ROWS rows
+    int num_sms_ = 148, tmax_ = 1, groups_ = 1, xtmax_ = 1;
+    uint32_t stride_ = 0;  // floats per row; a stage's block is block_rows() rows
     float* d_win_ = nullptr;
     float2* d_tw_ = nullptr;
-    float* d_acc_ = nullptr;  // [SSPSD_MAX_STAGES][CSD_ROWS][stride_]
+    float* d_acc_ = nullptr;  // [SSPSD_MAX_STAGES][block_rows()][stride_]
     float* h_acc_ = nullptr;
-    float* d_part_ = nullptr;
+    float* d_part_ = nullptr;   // deterministic mode: csd_stage_kernel's partial blocks
     size_t part_cap_ = 0;
-    struct YSource {
+    float* d_xpart_ = nullptr;  // and csm_cross_kernel's (another row layout: its padding must stay zero too)
+    size_t xpart_cap_ = 0;
+    struct Source {
         StreamSrc src;
         uint64_t k0, nseg;
         bool valid;
-    } ysrc_[SSPSD_MAX_STAGES] = {};
+    } srcs_[4][SSPSD_MAX_STAGES] = {};
 };
 
 XCascade::~XCascade()
@@ -145,6 +228,7 @@ XCascade::~XCascade()
     cudaFree(d_tw_);
     cudaFree(d_acc_);
     cudaFree(d_part_);
+    cudaFree(d_xpart_);
     if (h_acc_) cudaFreeHost(h_acc_);
 }
 
@@ -155,9 +239,13 @@ sspsd_config XCascade::channel_cfg() const
     return c;
 }
 
-// everything but the two channels: the stream, the window and twiddle tables, the accumulator blocks
-int XCascade::setup(const sspsd_config& cfg)
+// everything but the channels: the stream, the window and twiddle tables, the accumulator blocks
+int XCascade::setup(const sspsd_config& cfg, int k)
 {
+    if (k < 2 || k > 4) {
+        set_error("CsmCascade supports 2 .. 4 channels");
+        return SSPSD_EINVAL;
+    }
     const uint32_t n = cfg.n_fft;
     if (n < 64 || n > 4096 || (n & (n - 1))) {
         set_error("CsdCascade supports n_fft = 64 .. 4096 (the two-for-one transform is an N-point complex FFT)");
@@ -179,6 +267,7 @@ int XCascade::setup(const sspsd_config& cfg)
     DeviceGuard g(cfg.device);
     if (!g.ok) return SSPSD_ECUDA;
     cfg_ = cfg;
+    k_ = k;
     if (cfg.stream) {
         stream_ = (cudaStream_t)cfg.stream;
     } else {
@@ -191,6 +280,10 @@ int XCascade::setup(const sspsd_config& cfg)
     const int hop = cfg.window == SSPSD_WINDOW_HANN ? (int)n / 2 : (int)n;
     int rc = prepare_csd((int)log2n_, hop, &tmax_, &groups_);
     if (rc) return rc;
+    if (k_ > 2) {
+        rc = prepare_csm((int)log2n_, hop, &xtmax_);
+        if (rc) return rc;
+    }
 
     // Window::hann / ::rectangular with the PSD path's f32 expression; twiddles exp(-2 pi i q / N)
     std::vector<float> win(n, 1.0f);
@@ -208,7 +301,7 @@ int XCascade::setup(const sspsd_config& cfg)
         tw[q] = make_float2((float)std::cos(a), (float)std::sin(a));
     }
     stride_ = (n / 2 + 1 + 63) & ~63u;
-    const size_t acc_bytes = (size_t)SSPSD_MAX_STAGES * CSD_ROWS * stride_ * sizeof(float);
+    const size_t acc_bytes = acc_floats() * sizeof(float);
     SSPSD_CUDA(cudaMalloc(&d_win_, n * sizeof(float)));
     SSPSD_CUDA(cudaMalloc(&d_tw_, n * sizeof(float2)));
     SSPSD_CUDA(cudaMalloc(&d_acc_, acc_bytes));
@@ -217,39 +310,40 @@ int XCascade::setup(const sspsd_config& cfg)
     SSPSD_CUDA(cudaMemcpyAsync(d_tw_, tw.data(), n * sizeof(float2), cudaMemcpyHostToDevice, stream_));
     SSPSD_CUDA(cudaMemsetAsync(d_acc_, 0, acc_bytes, stream_));
     SSPSD_CUDA(cudaStreamSynchronize(stream_));  // the host vectors above go out of scope
-    for (Cascade* c : {&x_, &y_}) {
-        c->one_stream_ = true;
-        c->hook_ = this;
+    for (int c = 0; c < k_; ++c) {
+        ch_[c].one_stream_ = true;
+        ch_[c].hook_ = this;
     }
     n_ = n;
     return SSPSD_OK;
 }
 
-int XCascade::init(const sspsd_config& cfg)
+int XCascade::init(const sspsd_config& cfg, int k)
 {
-    int rc = setup(cfg);
+    int rc = setup(cfg, k);
     if (rc) return rc;
     const sspsd_config c = channel_cfg();
-    rc = x_.init(c, SSPSD_MAX_STAGES);
-    if (rc) return rc;
-    return y_.init(c, SSPSD_MAX_STAGES);
+    for (int i = 0; i < k_; ++i) {
+        rc = ch_[i].init(c, SSPSD_MAX_STAGES);
+        if (rc) return rc;
+    }
+    return SSPSD_OK;
 }
 
 int XCascade::clone_from(XCascade& o)
 {
     int rc = o.sync();
     if (rc) return rc;
-    rc = setup(o.cfg_);  // the caller's stream (cfg.stream) is shared by the copy, a private one is not
+    rc = setup(o.cfg_, o.k_);  // the caller's stream (cfg.stream) is shared by the copy, a private one is not
     if (rc) return rc;
     const sspsd_config c = channel_cfg();
-    rc = x_.clone_from(o.x_, &c);
-    if (rc) return rc;
-    rc = y_.clone_from(o.y_, &c);
-    if (rc) return rc;
+    for (int i = 0; i < k_; ++i) {
+        rc = ch_[i].clone_from(o.ch_[i], &c);
+        if (rc) return rc;
+    }
     DeviceGuard g(cfg_.device);
     if (!g.ok) return SSPSD_ECUDA;
-    SSPSD_CUDA(cudaMemcpyAsync(d_acc_, o.d_acc_, (size_t)SSPSD_MAX_STAGES * CSD_ROWS * stride_ * sizeof(float),
-                               cudaMemcpyDeviceToDevice, stream_));
+    SSPSD_CUDA(cudaMemcpyAsync(d_acc_, o.d_acc_, acc_floats() * sizeof(float), cudaMemcpyDeviceToDevice, stream_));
     SSPSD_CUDA(cudaStreamSynchronize(stream_));
     return SSPSD_OK;
 }
@@ -258,31 +352,53 @@ int XCascade::reset()
 {
     DeviceGuard g(cfg_.device);
     if (!g.ok) return SSPSD_ECUDA;
-    int rc = x_.reset();
-    if (rc) return rc;
-    rc = y_.reset();
-    if (rc) return rc;
-    for (auto& s : ysrc_) s.valid = false;
-    SSPSD_CUDA(cudaMemsetAsync(d_acc_, 0, (size_t)SSPSD_MAX_STAGES * CSD_ROWS * stride_ * sizeof(float), stream_));
+    for (int i = 0; i < k_; ++i) {
+        int rc = ch_[i].reset();
+        if (rc) return rc;
+    }
+    for (auto& row : srcs_)
+        for (auto& s : row) s.valid = false;
+    SSPSD_CUDA(cudaMemsetAsync(d_acc_, 0, acc_floats() * sizeof(float), stream_));
     return SSPSD_OK;
 }
 
-// Channel y's PSD launch leaves its source; channel x's launches the CSD kernel over both.
+int XCascade::ensure_part(float** part, size_t* cap, size_t need)
+{
+    if (need <= *cap) return SSPSD_OK;
+    SSPSD_CUDA(cudaStreamSynchronize(stream_));
+    if (*part) SSPSD_CUDA(cudaFree(*part));
+    *part = nullptr;
+    SSPSD_CUDA(cudaMalloc(part, need * sizeof(float)));
+    // the row padding is never written: keep it zero so that the reduction adds nothing there
+    SSPSD_CUDA(cudaMemsetAsync(*part, 0, need * sizeof(float), stream_));
+    *cap = need;
+    return SSPSD_OK;
+}
+
+// Channels 1 .. k_-1 leave their sources; channel 0's launches the block kernels over all of them.
 int XCascade::stage_psd(Cascade& c, size_t i, const StreamSrc& src, uint64_t k0, uint64_t nseg, int jb, float g_first,
                         float g_s)
 {
-    YSource& ys = ysrc_[i];
-    if (&c == &y_) {
-        ys = YSource{src, k0, nseg, true};
-        return SSPSD_OK;
+    for (int ci = 1; ci < k_; ++ci) {
+        if (&c == &ch_[ci]) {
+            srcs_[ci][i] = Source{src, k0, nseg, true};
+            return SSPSD_OK;
+        }
     }
-    if (!ys.valid || ys.k0 != k0 || ys.nseg != nseg) {
-        set_error("internal: channels out of lockstep");
-        return SSPSD_EINVAL;
+    for (int ci = 1; ci < k_; ++ci) {
+        Source& s = srcs_[ci][i];
+        if (!s.valid || s.k0 != k0 || s.nseg != nseg) {
+            set_error("internal: channels out of lockstep");
+            return SSPSD_EINVAL;
+        }
+        s.valid = false;
     }
-    ys.valid = false;
-    float* acc = d_acc_ + i * CSD_ROWS * stride_;
-    const int nblock = (int)(CSD_ROWS * stride_);
+    StreamSrc all[4] = {src, srcs_[1][i].src, src, src};
+    for (int ci = 2; ci < k_; ++ci) all[ci] = srcs_[ci][i].src;
+    if (k_ == 3) all[3] = all[2];  // pair (2, 3)'s diagonal block: channel 2 in both slots, rows 1..3 unused
+
+    float* acc = d_acc_ + i * block_rows() * stride_;
+    const int nblock = (int)(block_rows() * stride_);
     if ((uint64_t)jb < nseg) {
         // the EWMA pre-scale of the running sums before this batch (Cascade::run_stage, ewma_plan: same f32 factor)
         double t = (double)g_first;
@@ -294,78 +410,111 @@ int XCascade::stage_psd(Cascade& c, size_t i, const StreamSrc& src, uint64_t k0,
             SSPSD_CUDA(cudaGetLastError());
         }
     }
-    CsdParams p{};
-    p.src[0] = src;
-    p.src[1] = ys.src;
+    const int hop = (int)ch_[0].hop_;
+    const bool det = (cfg_.flags & SSPSD_FLAG_DETERMINISTIC) != 0;
+
+    // diagonal blocks: csd_stage_kernel over pair (0, 1), then (2, 3)
+    const TiledLaunch l = tiled_launch(nseg, groups_, tmax_, hop, (int)n_, num_sms_);
+    const int cblock = (int)(CSD_ROWS * stride_);
+    for (int pr = 0; 2 * pr < k_; ++pr) {
+        CsdParams p{};
+        p.src[0] = all[2 * pr];
+        p.src[1] = all[2 * pr + 1];
+        p.k0 = (long long)k0;
+        p.nseg = (int)nseg;
+        p.hop = hop;
+        p.detrend = ch_[0].detrend_;
+        p.win = d_win_;
+        p.tw = d_tw_;
+        p.acc = acc + (size_t)pr * cblock;
+        p.stride = (int)stride_;
+        p.jb = jb;
+        p.g_first = g_first;
+        p.g_s = g_s;
+        p.T = l.T;
+        p.tile_cap = l.tile_cap;
+        p.tpc = l.tpc;
+        const int rows = l.grid * groups_;
+        if (det) {
+            // one partial block per (CTA, group), summed in row order by reduce_partials_kernel
+            int rc = ensure_part(&d_part_, &part_cap_, (size_t)rows * cblock);
+            if (rc) return rc;
+            p.part = d_part_;
+            p.part_stride = cblock;
+        }
+        int rc = launch_csd((int)log2n_, p, l.grid, stream_);
+        if (rc) return rc;
+        if (p.part) {
+            reduce_partials_kernel<<<(cblock + 127) / 128, 128, 0, stream_>>>(p.acc, p.part, rows, cblock, cblock);
+            SSPSD_CUDA(cudaGetLastError());
+        }
+    }
+    if (k_ == 2) return SSPSD_OK;
+
+    // off-diagonal block: csm_cross_kernel over all channels
+    const TiledLaunch x = tiled_launch(nseg, groups_, xtmax_, hop, (int)n_, num_sms_);
+    const int xblock = (int)(CSM_XROWS * stride_);
+    CsmParams p{};
+    for (int ci = 0; ci < 4; ++ci) p.src[ci] = all[ci];
+    p.nch = k_;
     p.k0 = (long long)k0;
     p.nseg = (int)nseg;
-    p.hop = (int)x_.hop_;
-    p.detrend = x_.detrend_;
+    p.T = x.T;
+    p.tpc = x.tpc;
+    p.hop = hop;
+    p.detrend = ch_[0].detrend_;
+    p.tile_cap = x.tile_cap;
     p.win = d_win_;
     p.tw = d_tw_;
-    p.acc = acc;
+    p.acc = acc + 2 * (size_t)cblock;
     p.stride = (int)stride_;
     p.jb = jb;
     p.g_first = g_first;
     p.g_s = g_s;
-    // persistent tiled launch as psd_stage_kernel's: tiles as large as shared memory allows once there is enough
-    // work, about two CTAs per SM walking contiguous ranges of tiles
-    const long long t = ((long long)nseg + 2ll * num_sms_ - 1) / (2ll * num_sms_);
-    p.T = (int)std::max<long long>(std::min<long long>(groups_, (long long)nseg), std::min<long long>(t, tmax_));
-    p.T = std::min(p.T, tmax_);
-    p.tile_cap = (p.T - 1) * p.hop + (int)n_;
-    const long long ntiles = ((long long)nseg + p.T - 1) / p.T;
-    p.tpc = (int)std::max<long long>(1, (ntiles + 2ll * num_sms_ - 1) / (2ll * num_sms_));
-    const int grid = (int)((ntiles + p.tpc - 1) / p.tpc);
-    const int rows = grid * groups_;
-    if (cfg_.flags & SSPSD_FLAG_DETERMINISTIC) {
-        // one partial block per (CTA, group), summed in row order by reduce_partials_kernel
-        const size_t need = (size_t)rows * nblock;
-        if (need > part_cap_) {
-            SSPSD_CUDA(cudaStreamSynchronize(stream_));
-            if (d_part_) SSPSD_CUDA(cudaFree(d_part_));
-            d_part_ = nullptr;
-            SSPSD_CUDA(cudaMalloc(&d_part_, need * sizeof(float)));
-            // the row padding is never written: keep it zero so that the reduction adds nothing there
-            SSPSD_CUDA(cudaMemsetAsync(d_part_, 0, need * sizeof(float), stream_));
-            part_cap_ = need;
-        }
-        p.part = d_part_;
-        p.part_stride = nblock;
+    const int rows = x.grid * groups_;
+    if (det) {
+        int rc = ensure_part(&d_xpart_, &xpart_cap_, (size_t)rows * xblock);
+        if (rc) return rc;
+        p.part = d_xpart_;
+        p.part_stride = xblock;
     }
-    int rc = launch_csd((int)log2n_, p, grid, stream_);
+    int rc = launch_csm((int)log2n_, p, x.grid, stream_);
     if (rc) return rc;
     if (p.part) {
-        reduce_partials_kernel<<<(nblock + 127) / 128, 128, 0, stream_>>>(acc, p.part, rows, nblock, nblock);
+        reduce_partials_kernel<<<(xblock + 127) / 128, 128, 0, stream_>>>(p.acc, p.part, rows, xblock, xblock);
         SSPSD_CUDA(cudaGetLastError());
     }
     return SSPSD_OK;
 }
 
-// one lockstep step: the same chunk through y's stages, then through x's (which launch the CSD kernels)
-int XCascade::feed_chunk(const float* x, const float* y, size_t n, bool device)
+// one lockstep step: the same chunk through channels k_-1 .. 1, then through channel 0 (which launches the kernels)
+int XCascade::feed_chunk(const float* const* x, size_t n, bool device)
 {
-    int rc = device ? y_.feed_device_chunk(y, n) : y_.feed_host_chunk(y, n);
-    if (rc) return rc;
-    rc = device ? x_.feed_device_chunk(x, n) : x_.feed_host_chunk(x, n);
-    if (rc) return rc;
-    // y's input buffer of this chunk was read by the CSD kernels queued just now: its next refill waits for them
-    SSPSD_CUDA(cudaEventRecord(y_.ev_free_[y_.in_buf_ ^ 1], stream_));
+    for (int c = k_ - 1; c >= 0; --c) {
+        int rc = device ? ch_[c].feed_device_chunk(x[c], n) : ch_[c].feed_host_chunk(x[c], n);
+        if (rc) return rc;
+    }
+    // the other channels' input buffers of this chunk were read by the kernels queued just now: their next
+    // refill waits for them
+    for (int c = 1; c < k_; ++c) SSPSD_CUDA(cudaEventRecord(ch_[c].ev_free_[ch_[c].in_buf_ ^ 1], stream_));
     return SSPSD_OK;
 }
 
-// Cascade::flush_staged for both channels, chunk by chunk in lockstep
+// Cascade::flush_staged for all channels, chunk by chunk in lockstep
 int XCascade::flush_staged()
 {
-    const size_t staged = x_.staged_;
+    const size_t staged = ch_[0].staged_;
     if (staged == 0) return SSPSD_OK;
-    const int hb = x_.stage_buf_;
-    const size_t chunk = (size_t)std::min<uint64_t>(Cascade::host_chunk(), x_.cfg_.max_batch);
+    const int hb = ch_[0].stage_buf_;
+    const size_t chunk = (size_t)std::min<uint64_t>(Cascade::host_chunk(), ch_[0].cfg_.max_batch);
     for (size_t pos = 0; pos < staged; pos += chunk) {
-        int rc = feed_chunk(x_.h_stage_[hb] + pos, y_.h_stage_[hb] + pos, std::min(chunk, staged - pos), false);
+        const float* xs[4];
+        for (int c = 0; c < k_; ++c) xs[c] = ch_[c].h_stage_[hb] + pos;
+        int rc = feed_chunk(xs, std::min(chunk, staged - pos), false);
         if (rc) return rc;
     }
-    for (Cascade* c : {&x_, &y_}) {
+    for (int i = 0; i < k_; ++i) {
+        Cascade* c = &ch_[i];
         SSPSD_CUDA(cudaEventRecord(c->ev_stage_[hb], c->copy_stream_));
         c->stage_pending_[hb] = true;
         c->staged_ = 0;
@@ -383,21 +532,27 @@ int XCascade::flush_all()
 {
     int rc = flush_staged();
     if (rc) return rc;
-    for (size_t j = 1; j < x_.stages_.size(); ++j) {
-        rc = y_.run_pending(j);
-        if (rc) return rc;
-        rc = x_.run_pending(j);
-        if (rc) return rc;
+    for (size_t j = 1; j < ch_[0].stages_.size(); ++j) {
+        for (int c = k_ - 1; c >= 0; --c) {
+            rc = ch_[c].run_pending(j);
+            if (rc) return rc;
+        }
     }
     return SSPSD_OK;
 }
 
-int XCascade::process(const float* x, const float* y, size_t n, int mem)
+int XCascade::process(const float* const* x, size_t n, int mem)
 {
     if (n == 0) return SSPSD_OK;
-    if (!x || !y) {
+    if (!x) {
         set_error("null input");
         return SSPSD_EINVAL;
+    }
+    for (int c = 0; c < k_; ++c) {
+        if (!x[c]) {
+            set_error("null input");
+            return SSPSD_EINVAL;
+        }
     }
     if (mem != SSPSD_MEM_HOST && mem != SSPSD_MEM_DEVICE) {
         set_error("bad mem kind");
@@ -406,39 +561,42 @@ int XCascade::process(const float* x, const float* y, size_t n, int mem)
     DeviceGuard g(cfg_.device);
     if (!g.ok) return SSPSD_ECUDA;
     int rc;
-    const uint64_t max_batch = x_.cfg_.max_batch;
+    const float* xs[4];
+    const uint64_t max_batch = ch_[0].cfg_.max_batch;
     if (mem == SSPSD_MEM_DEVICE) {
         rc = flush_staged();
         if (rc) return rc;
-        // Cascade::process_device's chunks: at most max_batch, boundaries 16-byte aligned relative to x and y
+        // Cascade::process_device's chunks: at most max_batch, boundaries 16-byte aligned relative to every input
         const size_t nchunks = (n + max_batch - 1) / max_batch;
         size_t per = (n + nchunks - 1) / nchunks;
         per = (per + 4095) & ~(size_t)4095;
         for (size_t pos = 0; pos < n; pos += per) {
-            rc = feed_chunk(x + pos, y + pos, std::min<size_t>(n - pos, per), true);
+            for (int c = 0; c < k_; ++c) xs[c] = x[c] + pos;
+            rc = feed_chunk(xs, std::min<size_t>(n - pos, per), true);
             if (rc) return rc;
         }
         return SSPSD_OK;
     }
-    const uint64_t hs = x_.cfg_.host_stage;
+    const uint64_t hs = ch_[0].cfg_.host_stage;
     if (n < hs) {
         // small calls are collected in the channels' pinned staging buffers (Cascade::process_host)
-        for (Cascade* c : {&x_, &y_}) {
+        for (int i = 0; i < k_; ++i) {
+            Cascade* c = &ch_[i];
             if (!c->h_stage_[0]) {
                 SSPSD_CUDA(cudaMallocHost(&c->h_stage_[0], hs * sizeof(float)));
                 SSPSD_CUDA(cudaMallocHost(&c->h_stage_[1], hs * sizeof(float)));
             }
         }
-        while (n) {
-            const size_t take = std::min<size_t>(n, hs - x_.staged_);
-            std::memcpy(x_.h_stage_[x_.stage_buf_] + x_.staged_, x, take * sizeof(float));
-            std::memcpy(y_.h_stage_[y_.stage_buf_] + y_.staged_, y, take * sizeof(float));
-            x_.staged_ += take;
-            y_.staged_ += take;
-            x += take;
-            y += take;
-            n -= take;
-            if (x_.staged_ == hs) {
+        size_t pos = 0;
+        while (pos < n) {
+            const size_t take = std::min<size_t>(n - pos, hs - ch_[0].staged_);
+            for (int i = 0; i < k_; ++i) {
+                Cascade* c = &ch_[i];
+                std::memcpy(c->h_stage_[c->stage_buf_] + c->staged_, x[i] + pos, take * sizeof(float));
+                c->staged_ += take;
+            }
+            pos += take;
+            if (ch_[0].staged_ == hs) {
                 rc = flush_staged();
                 if (rc) return rc;
             }
@@ -448,14 +606,17 @@ int XCascade::process(const float* x, const float* y, size_t n, int mem)
     rc = flush_staged();
     if (rc) return rc;
     const size_t chunk = (size_t)std::min<uint64_t>(Cascade::host_chunk(), max_batch);
-    x_.last_copy_ = y_.last_copy_ = -1;
+    for (int c = 0; c < k_; ++c) ch_[c].last_copy_ = -1;
     for (size_t pos = 0; pos < n; pos += chunk) {
-        rc = feed_chunk(x + pos, y + pos, std::min(chunk, n - pos), false);
+        for (int c = 0; c < k_; ++c) xs[c] = x[c] + pos;
+        rc = feed_chunk(xs, std::min(chunk, n - pos), false);
         if (rc) return rc;
     }
     // the caller's buffers are borrowed for the call only: wait for the last H2D copies
-    for (Cascade* c : {&x_, &y_})
+    for (int i = 0; i < k_; ++i) {
+        Cascade* c = &ch_[i];
         if (c->last_copy_ >= 0) SSPSD_CUDA(cudaEventSynchronize(c->ev_copied_[c->last_copy_]));
+    }
     return SSPSD_OK;
 }
 
@@ -465,9 +626,11 @@ int XCascade::set_avg(sspsd_avg_opts a)
     if (!g.ok) return SSPSD_ECUDA;
     int rc = flush_all();  // options apply to segments completed after the call
     if (rc) return rc;
-    rc = x_.set_avg(a);
-    if (rc) return rc;
-    return y_.set_avg(a);
+    for (int c = 0; c < k_; ++c) {
+        rc = ch_[c].set_avg(a);
+        if (rc) return rc;
+    }
+    return SSPSD_OK;
 }
 
 int XCascade::set_detrend(int d)
@@ -476,9 +639,11 @@ int XCascade::set_detrend(int d)
     if (!g.ok) return SSPSD_ECUDA;
     int rc = flush_all();
     if (rc) return rc;
-    rc = x_.set_detrend(d);  // validates d (Linear: SSPSD_EUNIMPLEMENTED)
-    if (rc) return rc;
-    return y_.set_detrend(d);
+    for (int c = 0; c < k_; ++c) {
+        rc = ch_[c].set_detrend(d);  // validates d (Linear: SSPSD_EUNIMPLEMENTED)
+        if (rc) return rc;
+    }
+    return SSPSD_OK;
 }
 
 int XCascade::flush()
@@ -502,7 +667,7 @@ int XCascade::num_stages(uint32_t* n)
 {
     int rc = flush();
     if (rc) return rc;
-    *n = x_.n_stages();
+    *n = ch_[0].n_stages();
     return SSPSD_OK;
 }
 
@@ -518,11 +683,11 @@ int XCascade::read(const sspsd_merge_opts& o, float* pxx, float* pyy, float* pxy
     if (!g.ok) return SSPSD_ECUDA;
     int rc = flush_all();
     if (rc) return rc;
-    const size_t ns = x_.stages_.size();
+    const size_t ns = ch_[0].stages_.size();
     uint64_t book[4 * SSPSD_MAX_STAGES + 2];
-    x_.export_book(book);
+    ch_[0].export_book(book);
     size_t pl = 0, bl = 0;
-    Cascade::merge_host(x_.cfg_, book, nullptr, 0, o, nullptr, &pl, nullptr, &bl);
+    Cascade::merge_host(ch_[0].cfg_, book, nullptr, 0, o, nullptr, &pl, nullptr, &bl);
     const bool fits = (pl <= *p_len) && (ns <= *b_len) && (pl == 0 || (pxx && pyy && pxy)) && (ns == 0 || b);
     if (!fits || ns == 0) {
         *p_len = pl;
@@ -533,19 +698,97 @@ int XCascade::read(const sspsd_merge_opts& o, float* pxx, float* pyy, float* pxy
         }
         return SSPSD_OK;
     }
-    const size_t block = (size_t)CSD_ROWS * stride_;
+    const size_t block = block_rows() * stride_;
     SSPSD_CUDA(cudaMemcpyAsync(h_acc_, d_acc_, ns * block * sizeof(float), cudaMemcpyDeviceToHost, stream_));
     SSPSD_CUDA(cudaStreamSynchronize(stream_));
     std::vector<float> re(pl), im(pl);
     float* outs[CSD_ROWS] = {pxx, pyy, re.data(), im.data()};
     for (int r = 0; r < CSD_ROWS; ++r) {
         size_t pr = pl, br = ns;
-        rc = Cascade::merge_host(x_.cfg_, book, h_acc_ + (size_t)r * stride_, block, o, outs[r], &pr, b, &br);
+        rc = Cascade::merge_host(ch_[0].cfg_, book, h_acc_ + (size_t)r * stride_, block, o, outs[r], &pr, b, &br);
         if (rc) return rc;
     }
     for (size_t k = 0; k < pl; ++k) {
         pxy[2 * k] = re[k];
         pxy[2 * k + 1] = im[k];
+    }
+    *p_len = pl;
+    *b_len = ns;
+    return SSPSD_OK;
+}
+
+// The whole K x K matrix, s[2 ((i K + j) p_len + k) + {0, 1}]: every stored row merged as read() merges its rows,
+// the diagonal real (imaginary part 0), the lower triangle the conjugate of the upper.
+int XCascade::read_matrix(const sspsd_merge_opts& o, float* s, size_t* p_len, sspsd_break* b, size_t* b_len)
+{
+    if (!p_len || !b_len) {
+        set_error("null length pointer");
+        return SSPSD_EINVAL;
+    }
+    DeviceGuard g(cfg_.device);
+    if (!g.ok) return SSPSD_ECUDA;
+    int rc = flush_all();
+    if (rc) return rc;
+    const size_t ns = ch_[0].stages_.size();
+    uint64_t book[4 * SSPSD_MAX_STAGES + 2];
+    ch_[0].export_book(book);
+    size_t pl = 0, bl = 0;
+    Cascade::merge_host(ch_[0].cfg_, book, nullptr, 0, o, nullptr, &pl, nullptr, &bl);
+    const bool fits = (pl <= *p_len) && (ns <= *b_len) && (pl == 0 || s) && (ns == 0 || b);
+    if (!fits || ns == 0) {
+        *p_len = pl;
+        *b_len = ns;
+        if (!fits) {
+            set_error("output capacity too small");
+            return SSPSD_ESHORT;
+        }
+        return SSPSD_OK;
+    }
+    const size_t block = block_rows() * stride_;
+    SSPSD_CUDA(cudaMemcpyAsync(h_acc_, d_acc_, ns * block * sizeof(float), cudaMemcpyDeviceToHost, stream_));
+    SSPSD_CUDA(cudaStreamSynchronize(stream_));
+    // stored rows of the upper triangle: (i, j) -> (row of Re, row of Im); the diagonal has no Im row
+    int re_row[4][4], im_row[4][4];
+    for (int a = 0; 2 * a < k_; ++a) {
+        const int i = 2 * a, r = a * CSD_ROWS;
+        re_row[i][i] = r;
+        re_row[i + 1][i + 1] = r + 1;
+        re_row[i][i + 1] = r + 2;
+        im_row[i][i + 1] = r + 3;
+    }
+    for (int i = 0; i < 2; ++i)
+        for (int j = 2; j < 4; ++j) {
+            const int r = 2 * CSD_ROWS + 2 * (2 * i + (j - 2));  // S02, S03, S12, S13
+            re_row[i][j] = r;
+            im_row[i][j] = r + 1;
+        }
+    std::vector<float> re(pl), im(pl);
+    auto merged = [&](int row, float* out) {
+        size_t pr = pl, br = ns;
+        return Cascade::merge_host(ch_[0].cfg_, book, h_acc_ + (size_t)row * stride_, block, o, out, &pr, b, &br);
+    };
+    for (int i = 0; i < k_; ++i) {
+        for (int j = i; j < k_; ++j) {
+            float* up = s + 2 * ((size_t)(i * k_ + j) * pl);
+            float* lo = s + 2 * ((size_t)(j * k_ + i) * pl);
+            rc = merged(re_row[i][j], re.data());
+            if (rc) return rc;
+            if (i == j) {
+                for (size_t k = 0; k < pl; ++k) {
+                    up[2 * k] = re[k];
+                    up[2 * k + 1] = 0.0f;
+                }
+                continue;
+            }
+            rc = merged(im_row[i][j], im.data());
+            if (rc) return rc;
+            for (size_t k = 0; k < pl; ++k) {
+                up[2 * k] = re[k];
+                up[2 * k + 1] = im[k];
+                lo[2 * k] = re[k];
+                lo[2 * k + 1] = -im[k];
+            }
+        }
     }
     *p_len = pl;
     *b_len = ns;
@@ -569,7 +812,7 @@ int32_t sspsd_csd_create(const sspsd_config* cfg, sspsd_csd** out)
     *out = nullptr;
     sspsd_csd* h = new (std::nothrow) sspsd_csd();
     if (!h) return SSPSD_ENOMEM;
-    int rc = h->c.init(*cfg);
+    int rc = h->c.init(*cfg, 2);
     if (rc) {
         delete h;
         return rc;
@@ -603,7 +846,12 @@ int32_t sspsd_csd_reset(sspsd_csd* h) { return h ? h->c.reset() : SSPSD_EINVAL; 
 int32_t sspsd_csd_process_f32(sspsd_csd* h, const float* x, const float* y, size_t n, int32_t mem)
 {
     if (!h) return SSPSD_EINVAL;
-    return h->c.process(x, y, n, mem);
+    if (n && (!x || !y)) {
+        set_error("null input");
+        return SSPSD_EINVAL;
+    }
+    const float* xs[2] = {x, y};
+    return h->c.process(xs, n, mem);
 }
 
 int32_t sspsd_csd_set_avg(sspsd_csd* h, sspsd_avg_opts avg) { return h ? h->c.set_avg(avg) : SSPSD_EINVAL; }
@@ -641,3 +889,96 @@ int32_t sspsd_csd_stream(const sspsd_csd* h, void** stream)
 
 int32_t sspsd_csd_flush(sspsd_csd* h) { return h ? h->c.flush() : SSPSD_EINVAL; }
 int32_t sspsd_csd_sync(sspsd_csd* h) { return h ? h->c.sync() : SSPSD_EINVAL; }
+
+struct sspsd_csm {
+    sspsd::XCascade c;
+};
+
+int32_t sspsd_csm_create(const sspsd_config* cfg, int32_t k, sspsd_csm** out)
+{
+    if (!cfg || !out) {
+        set_error("null argument");
+        return SSPSD_EINVAL;
+    }
+    *out = nullptr;
+    sspsd_csm* h = new (std::nothrow) sspsd_csm();
+    if (!h) return SSPSD_ENOMEM;
+    int rc = h->c.init(*cfg, k);
+    if (rc) {
+        delete h;
+        return rc;
+    }
+    *out = h;
+    return SSPSD_OK;
+}
+
+void sspsd_csm_destroy(sspsd_csm* h) { delete h; }
+
+int32_t sspsd_csm_clone(sspsd_csm* h, sspsd_csm** out)
+{
+    if (!h || !out) {
+        set_error("null argument");
+        return SSPSD_EINVAL;
+    }
+    *out = nullptr;
+    sspsd_csm* n = new (std::nothrow) sspsd_csm();
+    if (!n) return SSPSD_ENOMEM;
+    int rc = n->c.clone_from(h->c);
+    if (rc) {
+        delete n;
+        return rc;
+    }
+    *out = n;
+    return SSPSD_OK;
+}
+
+int32_t sspsd_csm_channels(const sspsd_csm* h, int32_t* k)
+{
+    if (!h || !k) return SSPSD_EINVAL;
+    *k = h->c.channels();
+    return SSPSD_OK;
+}
+
+int32_t sspsd_csm_reset(sspsd_csm* h) { return h ? h->c.reset() : SSPSD_EINVAL; }
+
+int32_t sspsd_csm_process_f32(sspsd_csm* h, const float* const* x, size_t n, int32_t mem)
+{
+    if (!h) return SSPSD_EINVAL;
+    return h->c.process(x, n, mem);
+}
+
+int32_t sspsd_csm_set_avg(sspsd_csm* h, sspsd_avg_opts avg) { return h ? h->c.set_avg(avg) : SSPSD_EINVAL; }
+
+int32_t sspsd_csm_set_detrend(sspsd_csm* h, int32_t d) { return h ? h->c.set_detrend(d) : SSPSD_EINVAL; }
+
+int32_t sspsd_csm_rbw(const sspsd_csm* h, float* rbw)
+{
+    if (!h || !rbw) return SSPSD_EINVAL;
+    *rbw = h->c.rbw();
+    return SSPSD_OK;
+}
+
+int32_t sspsd_csm_read(sspsd_csm* h, const sspsd_merge_opts* opts, float* s, size_t* p_len, sspsd_break* b,
+                       size_t* b_len)
+{
+    if (!h) return SSPSD_EINVAL;
+    sspsd_merge_opts o{0, 1, 0};  // MergeOpts::default(), psd.rs:350-358
+    if (opts) o = *opts;
+    return h->c.read_matrix(o, s, p_len, b, b_len);
+}
+
+int32_t sspsd_csm_num_stages(sspsd_csm* h, uint32_t* n)
+{
+    if (!h || !n) return SSPSD_EINVAL;
+    return h->c.num_stages(n);
+}
+
+int32_t sspsd_csm_stream(const sspsd_csm* h, void** stream)
+{
+    if (!h || !stream) return SSPSD_EINVAL;
+    *stream = (void*)h->c.stream();
+    return SSPSD_OK;
+}
+
+int32_t sspsd_csm_flush(sspsd_csm* h) { return h ? h->c.flush() : SSPSD_EINVAL; }
+int32_t sspsd_csm_sync(sspsd_csm* h) { return h ? h->c.sync() : SSPSD_EINVAL; }

@@ -429,6 +429,127 @@ class CsdCascade(_StreamOrdered):
             self._h = None
 
 
+class CsmCascade(_StreamOrdered):
+    """Cascaded cross-spectral matrix of K = 2, 3 or 4 streams (include/sspsd.h, sspsd_csm_*).  All go through one
+    cascade and every stage accumulates S_ij = sum w conj(X_i) X_j, CsdCascade's convention: S[0, 1] is pxy of
+    CsdCascade(x0, x1) and S[i, i] what a PsdCascade fed x_i alone returns.  Every transform is shared by all
+    pairs: the matrix of K streams costs K FFTs and K decimations per segment.  n = 64 .. 4096."""
+
+    def __init__(self, n=512, channels=4, window=Window.HANN, device=0, hbf=Hbf.TAPS_140, stream=None, max_batch=0,
+                 host_stage=0, deep_defer=0, deterministic=False, _handle=None):
+        self.n = n
+        self.channels = int(channels)
+        self.device = int(device)
+        if _handle is not None:
+            self._h = _handle
+            return
+        cfg = _config(n, window, hbf, device, stream, max_batch, host_stage, deep_defer, deterministic)
+        h = C.c_void_p()
+        L.check(L.lib().sspsd_csm_create(C.byref(cfg), self.channels, C.byref(h)))
+        self._h = h
+
+    def clone(self):
+        h = C.c_void_p()
+        L.check(L.lib().sspsd_csm_clone(self._h, C.byref(h)))
+        return CsmCascade(self.n, self.channels, device=self.device, _handle=h)
+
+    def _stream_ptr(self):
+        s = C.c_void_p()
+        L.check(L.lib().sspsd_csm_stream(self._h, C.byref(s)))
+        return s.value or 0
+
+    def reset(self):
+        L.check(L.lib().sspsd_csm_reset(self._h))
+
+    def rbw(self):
+        r = C.c_float()
+        L.check(L.lib().sspsd_csm_rbw(self._h, C.byref(r)))
+        return r.value
+
+    def set_avg(self, avg: AvgOpts):
+        L.check(L.lib().sspsd_csm_set_avg(self._h, L.AvgOptsC(avg.limit, avg.count)))
+
+    def set_detrend(self, d: Detrend):
+        L.check(L.lib().sspsd_csm_set_detrend(self._h, int(d)))
+
+    def process(self, xs):
+        """the next samples of every stream: K equal-length float32 numpy arrays or CUDA tensors, or one (K, n)
+        array or tensor"""
+        if len(xs) != self.channels:
+            raise ValueError("expected %d channels, got %d" % (self.channels, len(xs)))
+        bufs = [_as_buffer(x) for x in xs]
+        n, mem = bufs[0][1], bufs[0][2]
+        if any(b[1] != n for b in bufs):
+            raise ValueError("all channels must have the same length (%s)" % [b[1] for b in bufs])
+        if any(b[2] != mem for b in bufs):
+            raise ValueError("channels must all be host arrays or all be CUDA tensors")
+        ptrs = (C.c_void_p * self.channels)(*[b[0] for b in bufs])
+        if mem == L.MEM_DEVICE:
+            for b in bufs:
+                self._order_device_input(b[3])
+        L.check(L.lib().sspsd_csm_process_f32(self._h, ptrs, n, mem))
+        if mem == L.MEM_DEVICE:
+            self._release_device_input(bufs[0][3])
+        del bufs
+
+    def flush(self):
+        L.check(L.lib().sspsd_csm_flush(self._h))
+
+    def sync(self):
+        L.check(L.lib().sspsd_csm_sync(self._h))
+
+    def num_stages(self):
+        n = C.c_uint32()
+        L.check(L.lib().sspsd_csm_num_stages(self._h, C.byref(n)))
+        return n.value
+
+    def csm(self, opts: MergeOpts = None):
+        """-> (S complex64 [K, K, bins], breaks), every entry merged like PsdCascade.psd"""
+        opts = opts or MergeOpts()
+        o = L.MergeOptsC(int(opts.keep_overlap), opts.min_count, int(opts.keep_transition_band))
+        k = self.channels
+        cap = L.MAX_STAGES * (self.n // 2 + 1)
+        s = np.zeros(2 * k * k * cap, np.float32)
+        b = (L.BreakC * L.MAX_STAGES)()
+        pl, bl = C.c_size_t(cap), C.c_size_t(L.MAX_STAGES)
+        L.check(L.lib().sspsd_csm_read(self._h, C.byref(o), s.ctypes.data, C.byref(pl), b, C.byref(bl)))
+        n = pl.value
+        m = s[:2 * k * k * n].view(np.complex64).reshape(k, k, n).copy()
+        return m, [Break._from_c(b[i]) for i in range(bl.value)]
+
+    @staticmethod
+    def coherence(S):
+        """magnitude-squared coherence |S_ij|^2 / (S_ii S_jj) per bin, [K, K, bins] (0 where a power is 0)"""
+        S = np.asarray(S, np.complex128)
+        d = np.real(np.einsum("iib->ib", S))
+        den = d[:, None, :] * d[None, :, :]
+        return np.divide(np.abs(S) ** 2, den, out=np.zeros(den.shape), where=den > 0)
+
+    @staticmethod
+    def transfer(S, inputs, outputs):
+        """MIMO transfer function estimate H [len(outputs), len(inputs), bins] with y_o = sum_i H[o, i] u_i:
+        H = (S_uu^-1 S_uy)^T per bin, S_uu the inputs' block and S_uy the inputs-by-outputs block of S.  0 where
+        S_uu is singular (det 0, or below 1e-12 of the product of its diagonal).  With one input this is
+        CsdCascade.transfer."""
+        S = np.asarray(S, np.complex128)
+        inputs, outputs = list(inputs), list(outputs)
+        suu = np.moveaxis(S[np.ix_(inputs, inputs)], -1, 0)    # [bins, ni, ni]
+        suy = np.moveaxis(S[np.ix_(inputs, outputs)], -1, 0)   # [bins, ni, no]
+        diag = np.prod(np.real(np.einsum("bii->bi", suu)), axis=1)
+        det = np.linalg.det(suu)
+        ok = (diag > 0) & (np.abs(det) > 1e-12 * np.where(diag > 0, diag, 0))
+        h = np.zeros((S.shape[-1], len(inputs), len(outputs)), np.complex128)
+        if np.any(ok):
+            h[ok] = np.linalg.solve(suu[ok], suy[ok])
+        return np.transpose(h, (2, 1, 0))
+
+    def __del__(self):
+        h = getattr(self, "_h", None)
+        if h and L is not None and getattr(L, "_lib", None) is not None:
+            L._lib.sspsd_csm_destroy(h)
+            self._h = None
+
+
 class Psd(_StreamOrdered):
     """Psd<N> + trait PsdStage, src/psd.rs:119-288 (one stage, decimated output exposed)."""
 
