@@ -228,15 +228,6 @@ int upload_taps_once(int device)
     return SSPSD_OK;
 }
 
-// EWMA bookkeeping for a batch of S segments, psd.rs:215-225
-struct EwmaPlan {
-    int jb;         // first segment of the batch whose factor differs from 1 (>= S: pure boxcar)
-    float g_first;  // factor applied at segment jb
-    float g_s;      // factor applied at every later segment: avg / (avg + 1)
-    float total;    // product of all factors (scales the running sum before the batch)
-    uint32_t count_after;
-};
-
 EwmaPlan ewma_plan(uint32_t count, uint32_t avg, uint64_t S)
 {
     EwmaPlan e{};
@@ -527,9 +518,17 @@ int Cascade::ensure_fresh(StageState& st, size_t need, size_t reserve)
     return SSPSD_OK;
 }
 
-int Cascade::launch_psd(size_t i, const StreamSrc& src, uint64_t k0, uint64_t nseg, int jb, float g_first, float g_s)
+// stage i's PSD kernel over segments [k0, k0 + nseg), after the EWMA pre-scale of the stage's running sum
+int Cascade::launch_psd(size_t i, const StreamSrc& src, uint64_t k0, uint64_t nseg, const EwmaPlan& e)
 {
-    if (hook_) return hook_->stage_psd(*this, i, src, k0, nseg, jb, g_first, g_s);
+    if (hook_) return hook_->stage_psd(*this, i, src, k0, nseg, e);
+    if (e.total != 1.0f) {
+        int nb = (int)(n_ / 2 + 1);
+        prof_begin(SSPSD_PROF_OTHER, 0, psd_stream(i));
+        scale_kernel<<<(nb + 255) / 256, 256, 0, psd_stream(i)>>>(d_acc_ + i * acc_stride_, nb, e.total);
+        prof_end(psd_stream(i));
+        SSPSD_CUDA(cudaGetLastError());
+    }
     StageParams p{};
     p.src = src;
     p.k0 = (long long)k0;
@@ -545,9 +544,9 @@ int Cascade::launch_psd(size_t i, const StreamSrc& src, uint64_t k0, uint64_t ns
         p.twM = d_twM_;
         p.twN = d_twN_;
         p.acc = d_acc_ + i * acc_stride_;
-        p.jb = jb;
-        p.g_first = g_first;
-        p.g_s = g_s;
+        p.jb = e.jb;
+        p.g_first = e.g_first;
+        p.g_s = e.g_s;
         int grid = (int)((nseg + p.T - 1) / p.T);
         int rcp = prepare_partials(i, grid * W16::SPI, &p);
         if (rcp) return rcp;
@@ -571,9 +570,9 @@ int Cascade::launch_psd(size_t i, const StreamSrc& src, uint64_t k0, uint64_t ns
         p.twM = d_twM_;
         p.twN = d_twN_;
         p.acc = d_acc_ + i * acc_stride_;
-        p.jb = jb;
-        p.g_first = g_first;
-        p.g_s = g_s;
+        p.jb = e.jb;
+        p.g_first = e.g_first;
+        p.g_s = e.g_s;
         int grid = (int)((nseg + p.T - 1) / p.T);
         int rcp = prepare_partials(i, grid, &p);
         if (rcp) return rcp;
@@ -599,9 +598,9 @@ int Cascade::launch_psd(size_t i, const StreamSrc& src, uint64_t k0, uint64_t ns
         p.twM = d_twM_;
         p.twN = d_twN_;
         p.acc = d_acc_ + i * acc_stride_;
-        p.jb = jb;
-        p.g_first = g_first;
-        p.g_s = g_s;
+        p.jb = e.jb;
+        p.g_first = e.g_first;
+        p.g_s = e.g_s;
         int grid = (int)((nseg + p.T - 1) / p.T);
         int rcp = prepare_partials(i, grid * R16::G, &p);
         if (rcp) return rcp;
@@ -628,9 +627,9 @@ int Cascade::launch_psd(size_t i, const StreamSrc& src, uint64_t k0, uint64_t ns
     p.twM = d_twM_;
     p.twN = d_twN_;
     p.acc = d_acc_ + i * acc_stride_;
-    p.jb = jb;
-    p.g_first = g_first;
-    p.g_s = g_s;
+    p.jb = e.jb;
+    p.g_first = e.g_first;
+    p.g_s = e.g_s;
     long long ntiles = ((long long)nseg + p.T - 1) / p.T;
     p.tpc = tiled_r16 ? 1 : (int)std::max<long long>(1, (ntiles + 2ll * num_sms_ - 1) / (2ll * num_sms_));
     int grid = (int)((ntiles + p.tpc - 1) / p.tpc);
@@ -763,21 +762,13 @@ int Cascade::run_stage(size_t i, const float* fresh, long long split, uint64_t n
         uint64_t a = std::max(craw0, klo), b = std::min(craw1, khi);
         if (b > a) {
             if (st.avg == 0xffffffffu) {
-                rc = launch_psd(i, src, a, b - a, (int)(b - a), 1.0f, 1.0f);
+                rc = launch_psd(i, src, a, b - a, EwmaPlan{(int)(b - a), 1.0f, 1.0f, 1.0f, 0});  // boxcar
             } else {
                 // EWMA follows the global segment order: before global segment a the reference's count
                 // is min(a, avg + 1) (psd.rs:218-225).  The row ends up normalised "as if the stream ended
                 // at b"; the caller multiplies it by g^(segments scaled after b) before the reduction.
                 const uint32_t cnt = (uint32_t)std::min<uint64_t>(a, (uint64_t)st.avg + 1);
-                EwmaPlan e = ewma_plan(cnt, st.avg, b - a);
-                if (e.total != 1.0f) {
-                    int nb = (int)(n_ / 2 + 1);
-                    prof_begin(SSPSD_PROF_OTHER, 0, ps);
-                    scale_kernel<<<(nb + 255) / 256, 256, 0, ps>>>(d_acc_ + i * acc_stride_, nb, e.total);
-                    prof_end(ps);
-                    SSPSD_CUDA(cudaGetLastError());
-                }
-                rc = launch_psd(i, src, a, b - a, e.jb, e.g_first, e.g_s);
+                rc = launch_psd(i, src, a, b - a, ewma_plan(cnt, st.avg, b - a));
             }
             if (rc) return rc;
             psd_launched = true;
@@ -785,15 +776,8 @@ int Cascade::run_stage(size_t i, const float* fresh, long long split, uint64_t n
         }
     } else if (craw1 > craw0) {
         const uint64_t S = craw1 - craw0;
-        EwmaPlan e = ewma_plan(st.count, st.avg, S);
-        if (e.total != 1.0f) {
-            int nb = (int)(n_ / 2 + 1);
-            prof_begin(SSPSD_PROF_OTHER, 0, ps);
-            scale_kernel<<<(nb + 255) / 256, 256, 0, ps>>>(d_acc_ + i * acc_stride_, nb, e.total);
-            prof_end(ps);
-            SSPSD_CUDA(cudaGetLastError());
-        }
-        rc = launch_psd(i, src, craw0, S, e.jb, e.g_first, e.g_s);
+        const EwmaPlan e = ewma_plan(st.count, st.avg, S);
+        rc = launch_psd(i, src, craw0, S, e);
         if (rc) return rc;
         st.count = e.count_after;
         psd_launched = true;

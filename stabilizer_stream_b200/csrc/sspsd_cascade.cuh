@@ -75,12 +75,20 @@ struct StageState {
     cudaEvent_t ev_psd[2] = {nullptr, nullptr};   // PSD stream: the PSD kernel has finished reading fresh[b] + carry
 };
 
+// EWMA bookkeeping for a batch of S segments, psd.rs:215-225
+struct EwmaPlan {
+    int jb;         // first segment of the batch whose factor differs from 1 (>= S: pure boxcar)
+    float g_first;  // factor applied at segment jb
+    float g_s;      // factor applied at every later segment: avg / (avg + 1)
+    float total;    // product of all factors (scales the running sum before the batch)
+    uint32_t count_after;
+};
+
 class Cascade;
-// Two-channel mode (XCascade): a stage's PSD launch is handed to the hook instead, with the launch's segment
-// range and EWMA weights; the EWMA pre-scale of the cascade's own rows still runs and is unused.
+// Multi-channel mode (XCascade): a stage's PSD launch, EWMA pre-scale included, is handed to the hook instead, with
+// the launch's segment range and EWMA plan; the cascade's own accumulator rows are then never touched.
 struct StageHook {
-    virtual int stage_psd(Cascade& c, size_t i, const StreamSrc& src, uint64_t k0, uint64_t nseg, int jb, float g_first,
-                          float g_s) = 0;
+    virtual int stage_psd(Cascade& c, size_t i, const StreamSrc& src, uint64_t k0, uint64_t nseg, const EwmaPlan& e) = 0;
 };
 
 class Cascade {
@@ -133,7 +141,7 @@ private:
     int add_stage();
     void free_stages(bool keep_buffers);
     int run_stage(size_t i, const float* fresh, long long split, uint64_t n_new);
-    int launch_psd(size_t i, const StreamSrc& src, uint64_t k0, uint64_t nseg, int jb, float g_first, float g_s);
+    int launch_psd(size_t i, const StreamSrc& src, uint64_t k0, uint64_t nseg, const EwmaPlan& e);
     int launch_decim(size_t i, const StreamSrc& src, uint64_t m0, uint64_t m1, float* out_fresh,
                      long long out_split, long long out_cap);
     int prepare_partials(size_t i, int rows, struct StageParams* p);

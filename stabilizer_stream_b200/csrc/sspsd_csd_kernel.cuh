@@ -21,13 +21,15 @@ namespace sspsd {
 // rows of one stage's accumulator block (each acc_stride floats): Sxx, Syy, Re Sxy, Im Sxy
 enum { CSD_ROWS = 4 };
 
-struct CsdParams {
-    StreamSrc src[2];  // channel x, channel y: same bookkeeping, own buffers
+// Parameters of both block kernels of a stage (csd_stage_kernel reads src[0..1], csm_cross_kernel src[0..nch-1]).
+struct XStageParams {
+    StreamSrc src[4];  // channels: same bookkeeping, own buffers
+    int nch;           // csm_cross_kernel: 3 or 4 (src[3] unused when 3)
     long long k0;
     int nseg, T, tpc, hop, detrend, tile_cap;
     const float* win;   // N window values
     const float2* tw;   // N entries: exp(-2 pi i q / N)
-    float* acc;         // CSD_ROWS rows of `stride` floats
+    float* acc;         // the kernel's rows of `stride` floats
     int stride;
     float* part;        // deterministic mode: per-(CTA, group) partial blocks of part_stride floats
     int part_stride;
@@ -53,9 +55,123 @@ struct CsdPlan {
     static constexpr int RED = PL::TPS > 32 ? PL::TPS / 32 : 1;  // mean-detrend partial sums per group and channel
 };
 
+// read-at-each-use operand of pair_pass0: v[t] = p[(first + t) * stride], through the read-only data cache
+template <class T>
+struct LdgStrided {
+    const T* p;
+    int first, stride;
+    __device__ __forceinline__ T operator[](int t) const { return __ldg(p + (first + t) * stride); }
+};
+
+// pass 0 of one pair: z[n] = x[n] + i y[n], each channel detrended on its own, windowed (wv[t]: window value of the
+// thread's point t), radix-8 butterfly, twiddled (tw0[t - 1] = W_N^(j t), t = 1 .. 7), stored to the pair's work
+// planes.  red: this pair's mean-detrend partial sums.  wv and tw0 are arrays held in registers (csd_stage_kernel) or
+// LdgStrided views read at each use (csm_cross_kernel's register budget, DESIGN.md 3b).
+template <int LOG2N, class WV, class TW>
+__device__ __forceinline__ void pair_pass0(const float* sx, const float* sy, int detrend, const WV& wv, const TW& tw0,
+                                           float* red, float* wre, float* wim, int tid, int j, int group)
+{
+    using PL = Plan<LOG2N + 1>;
+    constexpr int N = PL::M, TPS = PL::TPS, NT = PL::NT;
+    constexpr int WPG = CsdPlan<LOG2N>::RED;
+    float2 v[8];
+#pragma unroll
+    for (int t = 0; t < 8; ++t) v[t] = make_float2(sx[j + t * TPS], sy[j + t * TPS]);
+
+    if (detrend == 1) {  // Midpoint
+        const float2 off = make_float2(-sx[N / 2], -sy[N / 2]);
+#pragma unroll
+        for (int t = 0; t < 8; ++t) v[t] = __fadd2_rn(v[t], off);
+    } else if (detrend == 2) {  // Span
+        const float2 x0 = make_float2(sx[0], sy[0]);
+        const float2 slope = make_float2((sx[N - 1] - x0.x) / (float)(N - 1), (sy[N - 1] - x0.y) / (float)(N - 1));
+#pragma unroll
+        for (int t = 0; t < 8; ++t) {
+            const float n0 = (float)(j + t * TPS);
+            v[t].x -= fmaf(slope.x, n0, x0.x);
+            v[t].y -= fmaf(slope.y, n0, x0.y);
+        }
+    } else if (detrend == 3) {  // Mean
+        float2 sum = make_float2(0.f, 0.f);
+#pragma unroll
+        for (int t = 0; t < 8; ++t) sum = __fadd2_rn(sum, v[t]);
+        if constexpr (TPS <= 32) {
+#pragma unroll
+            for (int m = TPS / 2; m > 0; m >>= 1) {
+                sum.x += __shfl_xor_sync(0xffffffffu, sum.x, m);
+                sum.y += __shfl_xor_sync(0xffffffffu, sum.y, m);
+            }
+        } else {
+#pragma unroll
+            for (int m = 16; m > 0; m >>= 1) {
+                sum.x += __shfl_xor_sync(0xffffffffu, sum.x, m);
+                sum.y += __shfl_xor_sync(0xffffffffu, sum.y, m);
+            }
+            if ((tid & 31) == 0) {
+                red[2 * (group * WPG + (j >> 5))] = sum.x;
+                red[2 * (group * WPG + (j >> 5)) + 1] = sum.y;
+            }
+            group_sync<TPS, NT>(group);
+            sum = make_float2(0.f, 0.f);
+#pragma unroll
+            for (int w = 0; w < WPG; ++w) {
+                sum.x += red[2 * (group * WPG + w)];
+                sum.y += red[2 * (group * WPG + w) + 1];
+            }
+        }
+        const float2 off = make_float2(-sum.x * (1.0f / (float)N), -sum.y * (1.0f / (float)N));
+#pragma unroll
+        for (int t = 0; t < 8; ++t) v[t] = __fadd2_rn(v[t], off);
+    }
+#pragma unroll
+    for (int t = 0; t < 8; ++t) {
+        const float w = wv[t];
+        v[t] = __fmul2_rn(v[t], make_float2(w, w));
+    }
+
+    butterfly<8>(v);
+    const int a0 = ws_pos(j);
+#pragma unroll
+    for (int t = 0; t < 8; ++t) {
+        const int a = a0 + t * TPS + 4 * ((t * TPS) >> 5);
+        const float2 y = t ? cmul(v[t], tw0[t - 1]) : v[0];
+        wre[a] = y.x;
+        wim[a] = y.y;
+    }
+}
+
+// The bins a thread owns under the last-pass map (butterflies qA and qB, whose outputs pair up as (k, N - k)):
+// j != 0: kA, kA + K, 2K - kA, K - kA (and -1: none);  j == 0: 0, K, 2K = N/2, K/2, 3K/2.
+template <int LOG2N>
+__device__ __forceinline__ void owned_bins(int j, int kA, int (&bins)[5])
+{
+    constexpr int K = Plan<LOG2N + 1>::K;
+    if (j != 0) {
+        bins[0] = kA; bins[1] = kA + K; bins[2] = 2 * K - kA; bins[3] = K - kA; bins[4] = -1;
+    } else {
+        bins[0] = 0; bins[1] = K; bins[2] = 2 * K; bins[3] = K / 2; bins[4] = 3 * K / 2;
+    }
+}
+
+// flush of a thread's accumulators acc[owned bin][row]: one atomic (or partial-row store) per owned value, row r
+// at r * stride
+template <int LOG2N, int ROWS>
+__device__ __forceinline__ void pair_flush(const float (&acc)[5][ROWS], int j, int kA, const AccSink& sink, int stride)
+{
+    int bins[5];
+    owned_bins<LOG2N>(j, kA, bins);
+#pragma unroll
+    for (int b = 0; b < 5; ++b) {
+        if (bins[b] < 0) continue;
+        SSPSD_ASSERT(bins[b] <= Plan<LOG2N + 1>::M / 2);
+#pragma unroll
+        for (int r = 0; r < ROWS; ++r) sink.add(r * stride + bins[b], acc[b][r]);
+    }
+}
+
 template <int LOG2N>
 __global__ void __launch_bounds__(Plan<LOG2N + 1>::NT, Plan<LOG2N + 1>::NT <= 256 ? 2 : 1)
-csd_stage_kernel(const CsdParams p)
+csd_stage_kernel(const XStageParams p)
 {
     using PL = Plan<LOG2N + 1>;
     constexpr int N = PL::M, TPS = PL::TPS, NT = PL::NT, G = PL::G, K = PL::K, WS = PL::WS;
@@ -110,8 +226,7 @@ csd_stage_kernel(const CsdParams p)
 
     float* wre = wsb + group * 2 * WS;
     float* wim = wre + WS;
-    // owned bins: j != 0: kA, kA + K, 2K - kA, K - kA;  j == 0: 0, K, 2K, K/2, 3K/2
-    float acc[5][4];
+    float acc[5][4];  // [owned_bins][Sxx, Syy, Re Sxy, Im Sxy]
 #pragma unroll
     for (int b = 0; b < 5; ++b)
 #pragma unroll
@@ -123,16 +238,7 @@ csd_stage_kernel(const CsdParams p)
     const int ns = min(p.T, p.nseg - seg0);
     const float* tile_x = tiles + (2 * buf) * p.tile_cap;
     const float* tile_y = tile_x + p.tile_cap;
-    for (int i = tid; i < ns; i += NT) {
-        int jj = seg0 + i;
-        int n_s = p.nseg - 1 - max(jj, p.jb);
-        double w = 1.0;
-        if (n_s > 0)
-            w = pow((double)p.g_s, (double)n_s);
-        if (jj < p.jb && p.jb < p.nseg)
-            w *= (double)p.g_first;
-        wgt[i] = (float)(0.25 * w);
-    }
+    for (int i = tid; i < ns; i += NT) wgt[i] = ewma_weight(p, seg0 + i);
     mbar_wait(&bars[buf], (uint32_t)((tl - tile0) >> 1) & 1u);
     __syncthreads();
 
@@ -145,70 +251,7 @@ csd_stage_kernel(const CsdParams p)
         const float* sy = tile_y + sc * hop;
         const float wseg = valid ? wgt[sc] : 0.f;
 
-        // ---- pass 0: z[n] = x[n] + i y[n], each channel detrended on its own, windowed ----
-        float2 v[8];
-#pragma unroll
-        for (int t = 0; t < 8; ++t) v[t] = make_float2(sx[j + t * TPS], sy[j + t * TPS]);
-
-        if (p.detrend == 1) {  // Midpoint
-            const float2 off = make_float2(-sx[N / 2], -sy[N / 2]);
-#pragma unroll
-            for (int t = 0; t < 8; ++t) v[t] = __fadd2_rn(v[t], off);
-        } else if (p.detrend == 2) {  // Span
-            const float2 x0 = make_float2(sx[0], sy[0]);
-            const float2 slope = make_float2((sx[N - 1] - x0.x) / (float)(N - 1), (sy[N - 1] - x0.y) / (float)(N - 1));
-#pragma unroll
-            for (int t = 0; t < 8; ++t) {
-                const float n0 = (float)(j + t * TPS);
-                v[t].x -= fmaf(slope.x, n0, x0.x);
-                v[t].y -= fmaf(slope.y, n0, x0.y);
-            }
-        } else if (p.detrend == 3) {  // Mean
-            float2 sum = make_float2(0.f, 0.f);
-#pragma unroll
-            for (int t = 0; t < 8; ++t) sum = __fadd2_rn(sum, v[t]);
-            if constexpr (TPS <= 32) {
-#pragma unroll
-                for (int m = TPS / 2; m > 0; m >>= 1) {
-                    sum.x += __shfl_xor_sync(0xffffffffu, sum.x, m);
-                    sum.y += __shfl_xor_sync(0xffffffffu, sum.y, m);
-                }
-            } else {
-#pragma unroll
-                for (int m = 16; m > 0; m >>= 1) {
-                    sum.x += __shfl_xor_sync(0xffffffffu, sum.x, m);
-                    sum.y += __shfl_xor_sync(0xffffffffu, sum.y, m);
-                }
-                if ((tid & 31) == 0) {
-                    red[2 * (group * WPG + (j >> 5))] = sum.x;
-                    red[2 * (group * WPG + (j >> 5)) + 1] = sum.y;
-                }
-                group_sync<TPS, NT>(group);
-                sum = make_float2(0.f, 0.f);
-#pragma unroll
-                for (int w = 0; w < WPG; ++w) {
-                    sum.x += red[2 * (group * WPG + w)];
-                    sum.y += red[2 * (group * WPG + w) + 1];
-                }
-            }
-            const float2 off = make_float2(-sum.x * (1.0f / (float)N), -sum.y * (1.0f / (float)N));
-#pragma unroll
-            for (int t = 0; t < 8; ++t) v[t] = __fadd2_rn(v[t], off);
-        }
-#pragma unroll
-        for (int t = 0; t < 8; ++t) v[t] = __fmul2_rn(v[t], make_float2(wv[t], wv[t]));
-
-        butterfly<8>(v);
-        {
-            const int a0 = ws_pos(j);
-#pragma unroll
-            for (int t = 0; t < 8; ++t) {
-                int a = a0 + t * TPS + 4 * ((t * TPS) >> 5);
-                float2 y = t ? cmul(v[t], tw[0][t - 1]) : v[0];
-                wre[a] = y.x;
-                wim[a] = y.y;
-            }
-        }
+        pair_pass0<LOG2N>(sx, sy, p.detrend, wv, tw[0], red, wre, wim, tid, j, group);
         group_sync<TPS, NT>(group);
 
         mid_passes<LOG2N + 1, 1>(wre, wim, j, group, tw);
@@ -242,34 +285,7 @@ csd_stage_kernel(const CsdParams p)
     if (tid == 0 && tl + 2 < tile1) issue_tile(tl + 2);
     }  // tiles
 
-    // ---- flush: one atomic (or partial-row store) per owned value ----
-    int bins[5];
-    if (j != 0) {
-        bins[0] = kA; bins[1] = kA + K; bins[2] = 2 * K - kA; bins[3] = K - kA; bins[4] = -1;
-    } else {
-        bins[0] = 0; bins[1] = K; bins[2] = 2 * K; bins[3] = K / 2; bins[4] = 3 * K / 2;
-    }
-    float* row = p.part ? p.part + (size_t)(blockIdx.x * G + group) * p.part_stride : nullptr;
-#pragma unroll
-    for (int b = 0; b < 5; ++b) {
-        if (bins[b] < 0) continue;
-#pragma unroll
-        for (int r = 0; r < 4; ++r) {
-            SSPSD_ASSERT(bins[b] <= N / 2);
-            const int k = r * p.stride + bins[b];
-            if (row)
-                row[k] = acc[b][r];
-            else
-                atomicAdd(&p.acc[k], acc[b][r]);
-        }
-    }
-}
-
-// EWMA pre-scale of a stage's accumulator block (scale_kernel of the PSD path, which lives in another unit)
-__global__ void csd_scale_kernel(float* __restrict__ acc, int n, float s)
-{
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n) acc[i] *= s;
+    pair_flush<LOG2N>(acc, j, kA, acc_sink(nullptr, p.acc, p.part, p.part_stride, blockIdx.x * G + group), p.stride);
 }
 
 // shared memory (bytes) of csd_stage_kernel<LOG2N> for tiles of T segments

@@ -25,27 +25,6 @@ namespace sspsd {
 // rows of the cross block: Re/Im of S02, S03, S12, S13
 enum { CSM_XROWS = 8 };
 
-struct CsmParams {
-    StreamSrc src[4];  // channels 0 .. 3 (src[3] unused when nch == 3)
-    int nch;           // 3 or 4
-    long long k0;
-    int nseg, T, tpc, hop, detrend, tile_cap;
-    const float* win;  // N window values
-    const float2* tw;  // N entries: exp(-2 pi i q / N)
-    float* acc;        // CSM_XROWS rows of `stride` floats
-    int stride;
-    float* part;       // deterministic mode: per-(CTA, group) partial blocks of part_stride floats
-    int part_stride;
-    int jb;
-    float g_first, g_s;
-};
-
-template <int LOG2N>
-struct CsmPlan {
-    using PL = Plan<LOG2N + 1>;
-    static constexpr int RED = CsdPlan<LOG2N>::RED;
-};
-
 // one owned bin of both pairs: (Z_A[k], Z_A[N-k]) and (Z_B[k], Z_B[N-k]) -> the 8 row increments (0.25 w in wseg)
 __device__ __forceinline__ void csm_bin(float2 pk, float2 pm, float2 qk, float2 qm, float wseg, float (&a8)[8])
 {
@@ -62,83 +41,6 @@ __device__ __forceinline__ void csm_bin(float2 pk, float2 pm, float2 qk, float2 
     a8[5] = fmaf(wseg, fmaf(dA.x, aB.x, dA.y * aB.y), a8[5]);   // Im i conj(dA) aB = Re conj(dA) aB
     a8[6] = fmaf(wseg, fmaf(dA.x, dB.x, dA.y * dB.y), a8[6]);   // Re conj(dA) dB
     a8[7] = fmaf(wseg, fmaf(dA.x, dB.y, -dA.y * dB.x), a8[7]);  // Im conj(dA) dB
-}
-
-// pass 0 of one pair (csd_stage_kernel's): z[n] = x[n] + i y[n], each channel detrended on its own, windowed,
-// radix-8 butterfly, twiddled, stored to the pair's work planes.  red: this pair's mean-detrend partial sums.
-template <int LOG2N>
-__device__ __forceinline__ void csm_pass0(const float* sx, const float* sy, int detrend, const float* win,
-                                          const float2* __restrict__ twg, float* red, float* wre, float* wim, int tid,
-                                          int j, int group)
-{
-    using PL = Plan<LOG2N + 1>;
-    constexpr int N = PL::M, TPS = PL::TPS, NT = PL::NT;
-    constexpr int WPG = CsmPlan<LOG2N>::RED;
-    float2 v[8];
-#pragma unroll
-    for (int t = 0; t < 8; ++t) v[t] = make_float2(sx[j + t * TPS], sy[j + t * TPS]);
-
-    if (detrend == 1) {  // Midpoint
-        const float2 off = make_float2(-sx[N / 2], -sy[N / 2]);
-#pragma unroll
-        for (int t = 0; t < 8; ++t) v[t] = __fadd2_rn(v[t], off);
-    } else if (detrend == 2) {  // Span
-        const float2 x0 = make_float2(sx[0], sy[0]);
-        const float2 slope = make_float2((sx[N - 1] - x0.x) / (float)(N - 1), (sy[N - 1] - x0.y) / (float)(N - 1));
-#pragma unroll
-        for (int t = 0; t < 8; ++t) {
-            const float n0 = (float)(j + t * TPS);
-            v[t].x -= fmaf(slope.x, n0, x0.x);
-            v[t].y -= fmaf(slope.y, n0, x0.y);
-        }
-    } else if (detrend == 3) {  // Mean
-        float2 sum = make_float2(0.f, 0.f);
-#pragma unroll
-        for (int t = 0; t < 8; ++t) sum = __fadd2_rn(sum, v[t]);
-        if constexpr (TPS <= 32) {
-#pragma unroll
-            for (int m = TPS / 2; m > 0; m >>= 1) {
-                sum.x += __shfl_xor_sync(0xffffffffu, sum.x, m);
-                sum.y += __shfl_xor_sync(0xffffffffu, sum.y, m);
-            }
-        } else {
-#pragma unroll
-            for (int m = 16; m > 0; m >>= 1) {
-                sum.x += __shfl_xor_sync(0xffffffffu, sum.x, m);
-                sum.y += __shfl_xor_sync(0xffffffffu, sum.y, m);
-            }
-            if ((tid & 31) == 0) {
-                red[2 * (group * WPG + (j >> 5))] = sum.x;
-                red[2 * (group * WPG + (j >> 5)) + 1] = sum.y;
-            }
-            group_sync<TPS, NT>(group);
-            sum = make_float2(0.f, 0.f);
-#pragma unroll
-            for (int w = 0; w < WPG; ++w) {
-                sum.x += red[2 * (group * WPG + w)];
-                sum.y += red[2 * (group * WPG + w) + 1];
-            }
-        }
-        const float2 off = make_float2(-sum.x * (1.0f / (float)N), -sum.y * (1.0f / (float)N));
-#pragma unroll
-        for (int t = 0; t < 8; ++t) v[t] = __fadd2_rn(v[t], off);
-    }
-#pragma unroll
-    for (int t = 0; t < 8; ++t) {
-        const float w = __ldg(win + j + t * TPS);
-        v[t] = __fmul2_rn(v[t], make_float2(w, w));
-    }
-
-    butterfly<8>(v);
-    constexpr int LR = PL::log2radix(0), LS = PL::log2stride(0);
-    const int a0 = ws_pos(j);
-#pragma unroll
-    for (int t = 0; t < 8; ++t) {
-        const int a = a0 + t * TPS + 4 * ((t * TPS) >> 5);
-        const float2 y = t ? cmul(v[t], __ldg(&twg[(j * t) << (PL::LOG2M - LR - LS)])) : v[0];
-        wre[a] = y.x;
-        wim[a] = y.y;
-    }
 }
 
 // passes 1 .. P-2 over both pairs' planes (mid_passes with the twiddles read at each use), one barrier per pass
@@ -183,11 +85,11 @@ __device__ __forceinline__ void csm_mid_passes(float* __restrict__ ws, int j, in
 
 template <int LOG2N>
 __global__ void __launch_bounds__(Plan<LOG2N + 1>::NT, Plan<LOG2N + 1>::NT <= 256 ? 2 : 1)
-csm_cross_kernel(const CsmParams p)
+csm_cross_kernel(const XStageParams p)
 {
     using PL = Plan<LOG2N + 1>;
     constexpr int N = PL::M, TPS = PL::TPS, NT = PL::NT, G = PL::G, K = PL::K, WS = PL::WS;
-    constexpr int WPG = CsmPlan<LOG2N>::RED;
+    constexpr int WPG = CsdPlan<LOG2N>::RED;
     extern __shared__ __align__(16) float smem[];
     float* tiles = smem;                    // [buffer][channel] tile_cap floats
     float* wsb = smem + 8 * p.tile_cap;     // [group][pair][re, im] WS floats
@@ -238,8 +140,7 @@ csm_cross_kernel(const CsmParams p)
     const int posA = ws_pos(4 * qA), posB = ws_pos(4 * qB);
 
     float* ws = wsb + group * 4 * WS;
-    // owned bins: j != 0: kA, kA + K, 2K - kA, K - kA;  j == 0: 0, K, 2K, K/2, 3K/2
-    float acc[5][8];
+    float acc[5][8];  // [owned_bins][Re/Im of S02, S03, S12, S13]
 #pragma unroll
     for (int b = 0; b < 5; ++b)
 #pragma unroll
@@ -250,16 +151,7 @@ csm_cross_kernel(const CsmParams p)
     const int seg0 = tl * p.T;
     const int ns = min(p.T, p.nseg - seg0);
     const float* tile = tiles + (4 * buf) * p.tile_cap;
-    for (int i = tid; i < ns; i += NT) {
-        int jj = seg0 + i;
-        int n_s = p.nseg - 1 - max(jj, p.jb);
-        double w = 1.0;
-        if (n_s > 0)
-            w = pow((double)p.g_s, (double)n_s);
-        if (jj < p.jb && p.jb < p.nseg)
-            w *= (double)p.g_first;
-        wgt[i] = (float)(0.25 * w);
-    }
+    for (int i = tid; i < ns; i += NT) wgt[i] = ewma_weight(p, seg0 + i);
     mbar_wait(&bars[buf], (uint32_t)((tl - tile0) >> 1) & 1u);
     __syncthreads();
 
@@ -271,11 +163,12 @@ csm_cross_kernel(const CsmParams p)
         const float* s0 = tile + sc * hop;
         const float wseg = valid ? wgt[sc] : 0.f;
 
-        // ---- pass 0 of both pairs, each into its own work planes ----
+        // ---- pass 0 of both pairs, each into its own work planes; window and twiddles read at each use ----
 #pragma unroll
         for (int pr = 0; pr < 2; ++pr)
-            csm_pass0<LOG2N>(s0 + (2 * pr) * p.tile_cap, s0 + (2 * pr + 1) * p.tile_cap, p.detrend, p.win, p.tw,
-                             red + pr * 2 * G * WPG, ws + pr * 2 * WS, ws + pr * 2 * WS + WS, tid, j, group);
+            pair_pass0<LOG2N>(s0 + (2 * pr) * p.tile_cap, s0 + (2 * pr + 1) * p.tile_cap, p.detrend,
+                              LdgStrided<float>{p.win + j, 0, TPS}, LdgStrided<float2>{p.tw, 1, j},
+                              red + pr * 2 * G * WPG, ws + pr * 2 * WS, ws + pr * 2 * WS + WS, tid, j, group);
         group_sync<TPS, NT>(group);
 
         csm_mid_passes<LOG2N, 1>(ws, j, group, p.tw);
@@ -313,27 +206,7 @@ csm_cross_kernel(const CsmParams p)
     if (tid == 0 && tl + 2 < tile1) issue_tile(tl + 2);
     }  // tiles
 
-    // ---- flush: one atomic (or partial-row store) per owned value ----
-    int bins[5];
-    if (j != 0) {
-        bins[0] = kA; bins[1] = kA + K; bins[2] = 2 * K - kA; bins[3] = K - kA; bins[4] = -1;
-    } else {
-        bins[0] = 0; bins[1] = K; bins[2] = 2 * K; bins[3] = K / 2; bins[4] = 3 * K / 2;
-    }
-    float* row = p.part ? p.part + (size_t)(blockIdx.x * G + group) * p.part_stride : nullptr;
-#pragma unroll
-    for (int b = 0; b < 5; ++b) {
-        if (bins[b] < 0) continue;
-#pragma unroll
-        for (int r = 0; r < 8; ++r) {
-            SSPSD_ASSERT(bins[b] <= N / 2);
-            const int k = r * p.stride + bins[b];
-            if (row)
-                row[k] = acc[b][r];
-            else
-                atomicAdd(&p.acc[k], acc[b][r]);
-        }
-    }
+    pair_flush<LOG2N>(acc, j, kA, acc_sink(nullptr, p.acc, p.part, p.part_stride, blockIdx.x * G + group), p.stride);
 }
 
 // shared memory (bytes) of csm_cross_kernel<LOG2N> for tiles of T segments
@@ -342,7 +215,7 @@ inline size_t csm_smem_bytes(int T, int hop)
 {
     using PL = Plan<LOG2N + 1>;
     size_t tile = (size_t)(T - 1) * hop + PL::M;
-    size_t redn = ((size_t)4 * PL::G * CsmPlan<LOG2N>::RED + 1) & ~(size_t)1;
+    size_t redn = ((size_t)4 * PL::G * CsdPlan<LOG2N>::RED + 1) & ~(size_t)1;
     size_t fl = 8 * tile + (size_t)PL::G * 4 * PL::WS + ((T + 3) & ~3) + redn;
     return fl * sizeof(float) + 2 * sizeof(uint64_t);
 }

@@ -500,12 +500,4 @@ __global__ void carry_copy_kernel(StreamSrc src, long long g0, int n, float* __r
     carry_job(src, CarryJob{g0, n, head_n, dst, head_dst, dst_cap});
 }
 
-// acc[i] *= s (EWMA rescale of the running average before a batch, psd.rs:218-232)
-__global__ void scale_kernel(float* __restrict__ acc, int n, float s)
-{
-    int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n)
-        acc[i] *= s;
-}
-
 }  // namespace sspsd

@@ -65,6 +65,20 @@ __device__ __forceinline__ float ld_stream1(const StreamSrc& s, long long g)
     return 0.f;
 }
 
+// EWMA weight of segment j of a launch of p.nseg segments (psd.rs:218-233), the product of the factors applied after
+// it: g_s^(nseg-1-max(j,jb)) * (j < jb && jb < nseg ? g_first : 1), in f64; boxcar: jb >= nseg.  The 0.25 folds the
+// /2 of the real-input (or two-for-one) split.  p: any stage kernel's parameters; its fields are read where they are
+// used (pow is a call: a value read before it would be held across it).
+template <class P>
+__device__ __forceinline__ float ewma_weight(const P& p, int j)
+{
+    const int n_s = p.nseg - 1 - max(j, p.jb);
+    double w = 1.0;
+    if (n_s > 0) w = pow((double)p.g_s, (double)n_s);
+    if (j < p.jb && p.jb < p.nseg) w *= (double)p.g_first;
+    return (float)(0.25 * w);
+}
+
 // ---------------------------------------------------------------------------------------------
 // TMA bulk copies (cp.async.bulk, SASS UBLKCP) completing on an mbarrier
 // ---------------------------------------------------------------------------------------------

@@ -65,6 +65,14 @@ static __global__ void reduce_partials_kernel(float* __restrict__ acc, const flo
     acc[k] = (float)((double)acc[k] + s);
 }
 
+// acc[i] *= s (EWMA rescale of the running average before a batch, psd.rs:218-232; internal linkage as above)
+static __global__ void scale_kernel(float* __restrict__ acc, int n, float s)
+{
+    int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n)
+        acc[i] *= s;
+}
+
 template <int TPS, int NT>
 __device__ __forceinline__ void group_sync(int group)
 {
@@ -251,17 +259,8 @@ psd_stage_kernel(const StageParams p)
     const int seg0 = tl * p.T;
     const int ns = min(p.T, p.nseg - seg0);
     const float* tile = tiles + buf * p.tile_cap;
-    // per-segment averaging weights of this tile (0.25 folds the /2 of the real-input split)
-    for (int i = tid; i < ns; i += NT) {
-        int jj = seg0 + i;
-        int n_s = p.nseg - 1 - max(jj, p.jb);
-        double w = 1.0;
-        if (n_s > 0)
-            w = pow((double)p.g_s, (double)n_s);
-        if (jj < p.jb && p.jb < p.nseg)
-            w *= (double)p.g_first;
-        wgt[i] = (float)(0.25 * w);
-    }
+    // per-segment averaging weights of this tile
+    for (int i = tid; i < ns; i += NT) wgt[i] = ewma_weight(p, seg0 + i);
     mbar_wait(&bars[buf], (uint32_t)((tl - tile0) >> 1) & 1u);
     __syncthreads();
 

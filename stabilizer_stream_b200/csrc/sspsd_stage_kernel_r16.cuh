@@ -113,14 +113,7 @@ __global__ void __launch_bounds__(R16::NT, 2) psd_stage_kernel_r16(const StagePa
     for (int v = tid; v < tile_len / 4; v += NT)
         reinterpret_cast<float4*>(tile)[v] = ld_stream4(p.src, g0 + 4ll * v);
 
-    if (tid < ns) {
-        int jj = seg0 + tid;
-        int n_s = p.nseg - 1 - max(jj, p.jb);
-        double w = 1.0;
-        if (n_s > 0) w = pow((double)p.g_s, (double)n_s);
-        if (jj < p.jb && p.jb < p.nseg) w *= (double)p.g_first;
-        wgt[tid] = (float)(0.25 * w);
-    }
+    if (tid < ns) wgt[tid] = ewma_weight(p, seg0 + tid);
 
     // ---- segment-invariant per-thread constants ----
     // the window is re-read through L1 for every segment (16 LDG.64): with the arithmetic on aligned

@@ -60,14 +60,7 @@ __device__ __forceinline__ void psd_stage_ring_body(const StageParams& p)
         for (int h = 0; h < pre; ++h) ring_issue(p.src, g0 + (long long)h * HOP, HOP, ring + h * HOP, &bars[h]);
     }
 
-    for (int i = tid; i < ns; i += NT) {
-        int jj = c0 + i;
-        int n_s = p.nseg - 1 - max(jj, p.jb);
-        double w = 1.0;
-        if (n_s > 0) w = pow((double)p.g_s, (double)n_s);
-        if (jj < p.jb && p.jb < p.nseg) w *= (double)p.g_first;
-        wgt[i] = (float)(0.25 * w);
-    }
+    for (int i = tid; i < ns; i += NT) wgt[i] = ewma_weight(p, c0 + i);
 
     // ---- segment-invariant per-thread constants (as in the tiled radix-16 kernel) ----
     // the window lives in shared memory (one LDS.64 per point and segment): the packed arithmetic needs

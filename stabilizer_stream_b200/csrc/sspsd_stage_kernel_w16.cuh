@@ -63,14 +63,7 @@ __global__ void __launch_bounds__(W16::NT, 2) psd_stage_kernel_w16(const StagePa
     if (tid == 0)
         for (int c = 0; c < min(nchunks, RING); ++c) issue(c);
 
-    for (int i = tid; i < ns; i += NT) {
-        int jj = c0 + i;
-        int n_s = p.nseg - 1 - max(jj, p.jb);
-        double w = 1.0;
-        if (n_s > 0) w = pow((double)p.g_s, (double)n_s);
-        if (jj < p.jb && p.jb < p.nseg) w *= (double)p.g_first;
-        wgt[i] = (float)(0.25 * w);
-    }
+    for (int i = tid; i < ns; i += NT) wgt[i] = ewma_weight(p, c0 + i);
     for (int i = tid; i < M; i += NT) wtab[i] = __ldg(reinterpret_cast<const float2*>(p.win) + i);
 
     // ---- segment-invariant per-lane constants ----

@@ -29,65 +29,43 @@ namespace sspsd {
 
 namespace {
 
+// One of the two block kernels at one N, its rows and its shared-memory budget per CTA
+struct BlockKernel {
+    void (*fn)(XStageParams);
+    size_t (*smem)(int T, int hop);  // bytes for tiles of T segments
+    long long budget;
+    int rows;
+    const char* what;
+};
+enum { DIAG = 0, CROSS = 1 };
+struct BlockKernels {
+    BlockKernel k[2];  // [DIAG]: csd_stage_kernel, [CROSS]: csm_cross_kernel
+    int nt, groups;    // threads per CTA, segments in flight per CTA (both kernels)
+};
+
 template <int LOG2N>
-int prepare_csd_t(int hop, int* tmax, int* groups)
+BlockKernels block_kernels_t()
 {
     using PL = Plan<LOG2N + 1>;
-    const long long budget = PL::NT <= 256 ? 100 * 1024 : 200 * 1024;
-    int t = 256;
-    while (t > 1 && (long long)csd_smem_bytes<LOG2N>(t, hop) > budget) --t;
-    if ((long long)csd_smem_bytes<LOG2N>(t, hop) > budget) {
-        set_error("FFT size does not fit in shared memory");
-        return SSPSD_EINVAL;
-    }
-    *tmax = t;
-    *groups = PL::G;
-    SSPSD_CUDA(cudaFuncSetAttribute(csd_stage_kernel<LOG2N>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                    (int)csd_smem_bytes<LOG2N>(t, hop)));
-    return SSPSD_OK;
+    // two CTAs per SM up to 256 threads, one above; the cross kernel's 110 KB: 2 x (110 KB + 1 KB reserved) of the
+    // SM's 228 KB
+    const bool two = PL::NT <= 256;
+    return {{{csd_stage_kernel<LOG2N>, csd_smem_bytes<LOG2N>, two ? 100 * 1024 : 200 * 1024, CSD_ROWS,
+              "csd_stage_kernel launch"},
+             {csm_cross_kernel<LOG2N>, csm_smem_bytes<LOG2N>, two ? 110 * 1024 : 220 * 1024, CSM_XROWS,
+              "csm_cross_kernel launch"}},
+            PL::NT,
+            PL::G};
 }
 
-template <int LOG2N>
-int launch_csd_t(const CsdParams& p, int grid, cudaStream_t s)
-{
-    csd_stage_kernel<LOG2N><<<grid, Plan<LOG2N + 1>::NT, csd_smem_bytes<LOG2N>(p.T, p.hop), s>>>(p);
-    return cuda_ok(cudaGetLastError(), "csd_stage_kernel launch") ? SSPSD_OK : SSPSD_ECUDA;
-}
-
-template <int LOG2N>
-int prepare_csm_t(int hop, int* tmax)
-{
-    using PL = Plan<LOG2N + 1>;
-    // two CTAs per SM up to 256 threads (2 x (110 KB + 1 KB reserved) of the SM's 228 KB), one above
-    const long long budget = PL::NT <= 256 ? 110 * 1024 : 220 * 1024;
-    int t = 256;
-    while (t > 1 && (long long)csm_smem_bytes<LOG2N>(t, hop) > budget) --t;
-    if ((long long)csm_smem_bytes<LOG2N>(t, hop) > budget) {
-        set_error("FFT size does not fit in shared memory");
-        return SSPSD_EINVAL;
-    }
-    *tmax = t;
-    SSPSD_CUDA(cudaFuncSetAttribute(csm_cross_kernel<LOG2N>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                    (int)csm_smem_bytes<LOG2N>(t, hop)));
-    return SSPSD_OK;
-}
-
-template <int LOG2N>
-int launch_csm_t(const CsmParams& p, int grid, cudaStream_t s)
-{
-    csm_cross_kernel<LOG2N><<<grid, Plan<LOG2N + 1>::NT, csm_smem_bytes<LOG2N>(p.T, p.hop), s>>>(p);
-    return cuda_ok(cudaGetLastError(), "csm_cross_kernel launch") ? SSPSD_OK : SSPSD_ECUDA;
-}
-
-#define SSPSD_CSD_SIZES(X) X(6) X(7) X(8) X(9) X(10) X(11) X(12)
-
-int prepare_csd(int log2n, int hop, int* tmax, int* groups)
+int block_kernels(int log2n, BlockKernels* out)
 {
     switch (log2n) {
-#define X(L) \
-    case L:  \
-        return prepare_csd_t<L>(hop, tmax, groups);
-        SSPSD_CSD_SIZES(X)
+#define X(L)                          \
+    case L:                           \
+        *out = block_kernels_t<L>();  \
+        return SSPSD_OK;
+        X(6) X(7) X(8) X(9) X(10) X(11) X(12)
 #undef X
     default:
         set_error("CsdCascade supports n_fft = 64 .. 4096 (the two-for-one transform is an N-point complex FFT)");
@@ -95,43 +73,18 @@ int prepare_csd(int log2n, int hop, int* tmax, int* groups)
     }
 }
 
-int launch_csd(int log2n, const CsdParams& p, int grid, cudaStream_t s)
+// the largest tile (segments) that fits the kernel's budget; raises its dynamic shared-memory limit to that
+int prepare_block(const BlockKernel& k, int hop, int* tmax)
 {
-    switch (log2n) {
-#define X(L) \
-    case L:  \
-        return launch_csd_t<L>(p, grid, s);
-        SSPSD_CSD_SIZES(X)
-#undef X
-    default:
+    int t = 256;
+    while (t > 1 && (long long)k.smem(t, hop) > k.budget) --t;
+    if ((long long)k.smem(t, hop) > k.budget) {
+        set_error("FFT size does not fit in shared memory");
         return SSPSD_EINVAL;
     }
-}
-
-int prepare_csm(int log2n, int hop, int* tmax)
-{
-    switch (log2n) {
-#define X(L) \
-    case L:  \
-        return prepare_csm_t<L>(hop, tmax);
-        SSPSD_CSD_SIZES(X)
-#undef X
-    default:
-        return SSPSD_EINVAL;
-    }
-}
-
-int launch_csm(int log2n, const CsmParams& p, int grid, cudaStream_t s)
-{
-    switch (log2n) {
-#define X(L) \
-    case L:  \
-        return launch_csm_t<L>(p, grid, s);
-        SSPSD_CSD_SIZES(X)
-#undef X
-    default:
-        return SSPSD_EINVAL;
-    }
+    *tmax = t;
+    SSPSD_CUDA(cudaFuncSetAttribute(k.fn, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)k.smem(t, hop)));
+    return SSPSD_OK;
 }
 
 // persistent tiled launch as psd_stage_kernel's: tiles as large as shared memory allows once there is enough
@@ -173,8 +126,7 @@ public:
     int channels() const { return k_; }
     float rbw() const { return ch_[0].rbw(); }
     cudaStream_t stream() const { return stream_; }
-    int stage_psd(Cascade& c, size_t i, const StreamSrc& src, uint64_t k0, uint64_t nseg, int jb, float g_first,
-                  float g_s) override;
+    int stage_psd(Cascade& c, size_t i, const StreamSrc& src, uint64_t k0, uint64_t nseg, const EwmaPlan& e) override;
 
 private:
     int setup(const sspsd_config& cfg, int k);
@@ -185,6 +137,9 @@ private:
     size_t block_rows() const { return k_ == 2 ? CSD_ROWS : 2 * CSD_ROWS + CSM_XROWS; }
     size_t acc_floats() const { return (size_t)SSPSD_MAX_STAGES * block_rows() * stride_; }
     int ensure_part(float** part, size_t* cap, size_t need);
+    int launch_block(int kind, XStageParams p, uint64_t nseg, float* acc, float** part, size_t* part_cap);
+    int read_rows(const sspsd_merge_opts& o, bool outs, size_t* p_len, sspsd_break* b, size_t* b_len,
+                  uint64_t (&book)[4 * SSPSD_MAX_STAGES + 2], size_t* pl, size_t* ns);
 
     // destroyed after the channels, whose destructors still synchronise the stream
     struct OwnedStream {
@@ -202,7 +157,9 @@ private:
     sspsd_config cfg_{};
     cudaStream_t stream_ = nullptr;
     uint32_t n_ = 0, log2n_ = 0;
-    int num_sms_ = 148, tmax_ = 1, groups_ = 1, xtmax_ = 1;
+    int num_sms_ = 148;
+    BlockKernels kern_{};
+    int tmax_[2] = {1, 1};  // largest tile of each block kernel
     uint32_t stride_ = 0;  // floats per row; a stage's block is block_rows() rows
     float* d_win_ = nullptr;
     float2* d_tw_ = nullptr;
@@ -278,10 +235,10 @@ int XCascade::setup(const sspsd_config& cfg, int k)
     while ((1u << log2n_) < n) ++log2n_;
     SSPSD_CUDA(cudaDeviceGetAttribute(&num_sms_, cudaDevAttrMultiProcessorCount, cfg.device));
     const int hop = cfg.window == SSPSD_WINDOW_HANN ? (int)n / 2 : (int)n;
-    int rc = prepare_csd((int)log2n_, hop, &tmax_, &groups_);
+    int rc = block_kernels((int)log2n_, &kern_);
     if (rc) return rc;
-    if (k_ > 2) {
-        rc = prepare_csm((int)log2n_, hop, &xtmax_);
+    for (int kind = DIAG; kind <= (k_ > 2 ? CROSS : DIAG); ++kind) {
+        rc = prepare_block(kern_.k[kind], hop, &tmax_[kind]);
         if (rc) return rc;
     }
 
@@ -375,9 +332,35 @@ int XCascade::ensure_part(float** part, size_t* cap, size_t need)
     return SSPSD_OK;
 }
 
+// One block kernel over a stage's segments, its rows at acc: tiles, the partial buffer in deterministic mode (one
+// partial block per (CTA, group), summed in row order by reduce_partials_kernel), the launch and the reduction.
+int XCascade::launch_block(int kind, XStageParams p, uint64_t nseg, float* acc, float** part, size_t* part_cap)
+{
+    const BlockKernel& k = kern_.k[kind];
+    const int block = (int)(k.rows * stride_);
+    const TiledLaunch l = tiled_launch(nseg, kern_.groups, tmax_[kind], p.hop, (int)n_, num_sms_);
+    p.T = l.T;
+    p.tile_cap = l.tile_cap;
+    p.tpc = l.tpc;
+    p.acc = acc;
+    const int rows = l.grid * kern_.groups;
+    if (cfg_.flags & SSPSD_FLAG_DETERMINISTIC) {
+        int rc = ensure_part(part, part_cap, (size_t)rows * block);
+        if (rc) return rc;
+        p.part = *part;
+        p.part_stride = block;
+    }
+    k.fn<<<l.grid, kern_.nt, k.smem(p.T, p.hop), stream_>>>(p);
+    if (!cuda_ok(cudaGetLastError(), k.what)) return SSPSD_ECUDA;
+    if (p.part) {
+        reduce_partials_kernel<<<(block + 127) / 128, 128, 0, stream_>>>(p.acc, p.part, rows, block, block);
+        SSPSD_CUDA(cudaGetLastError());
+    }
+    return SSPSD_OK;
+}
+
 // Channels 1 .. k_-1 leave their sources; channel 0's launches the block kernels over all of them.
-int XCascade::stage_psd(Cascade& c, size_t i, const StreamSrc& src, uint64_t k0, uint64_t nseg, int jb, float g_first,
-                        float g_s)
+int XCascade::stage_psd(Cascade& c, size_t i, const StreamSrc& src, uint64_t k0, uint64_t nseg, const EwmaPlan& e)
 {
     for (int ci = 1; ci < k_; ++ci) {
         if (&c == &ch_[ci]) {
@@ -393,98 +376,39 @@ int XCascade::stage_psd(Cascade& c, size_t i, const StreamSrc& src, uint64_t k0,
         }
         s.valid = false;
     }
-    StreamSrc all[4] = {src, srcs_[1][i].src, src, src};
-    for (int ci = 2; ci < k_; ++ci) all[ci] = srcs_[ci][i].src;
-    if (k_ == 3) all[3] = all[2];  // pair (2, 3)'s diagonal block: channel 2 in both slots, rows 1..3 unused
-
-    float* acc = d_acc_ + i * block_rows() * stride_;
-    const int nblock = (int)(block_rows() * stride_);
-    if ((uint64_t)jb < nseg) {
-        // the EWMA pre-scale of the running sums before this batch (Cascade::run_stage, ewma_plan: same f32 factor)
-        double t = (double)g_first;
-        const uint64_t n_s = nseg - 1 - (uint64_t)jb;
-        if (n_s > 0) t *= std::pow((double)g_s, (double)n_s);
-        const float total = (float)t;
-        if (total != 1.0f) {
-            csd_scale_kernel<<<(nblock + 255) / 256, 256, 0, stream_>>>(acc, nblock, total);
-            SSPSD_CUDA(cudaGetLastError());
-        }
-    }
-    const int hop = (int)ch_[0].hop_;
-    const bool det = (cfg_.flags & SSPSD_FLAG_DETERMINISTIC) != 0;
-
-    // diagonal blocks: csd_stage_kernel over pair (0, 1), then (2, 3)
-    const TiledLaunch l = tiled_launch(nseg, groups_, tmax_, hop, (int)n_, num_sms_);
-    const int cblock = (int)(CSD_ROWS * stride_);
-    for (int pr = 0; 2 * pr < k_; ++pr) {
-        CsdParams p{};
-        p.src[0] = all[2 * pr];
-        p.src[1] = all[2 * pr + 1];
-        p.k0 = (long long)k0;
-        p.nseg = (int)nseg;
-        p.hop = hop;
-        p.detrend = ch_[0].detrend_;
-        p.win = d_win_;
-        p.tw = d_tw_;
-        p.acc = acc + (size_t)pr * cblock;
-        p.stride = (int)stride_;
-        p.jb = jb;
-        p.g_first = g_first;
-        p.g_s = g_s;
-        p.T = l.T;
-        p.tile_cap = l.tile_cap;
-        p.tpc = l.tpc;
-        const int rows = l.grid * groups_;
-        if (det) {
-            // one partial block per (CTA, group), summed in row order by reduce_partials_kernel
-            int rc = ensure_part(&d_part_, &part_cap_, (size_t)rows * cblock);
-            if (rc) return rc;
-            p.part = d_part_;
-            p.part_stride = cblock;
-        }
-        int rc = launch_csd((int)log2n_, p, l.grid, stream_);
-        if (rc) return rc;
-        if (p.part) {
-            reduce_partials_kernel<<<(cblock + 127) / 128, 128, 0, stream_>>>(p.acc, p.part, rows, cblock, cblock);
-            SSPSD_CUDA(cudaGetLastError());
-        }
-    }
-    if (k_ == 2) return SSPSD_OK;
-
-    // off-diagonal block: csm_cross_kernel over all channels
-    const TiledLaunch x = tiled_launch(nseg, groups_, xtmax_, hop, (int)n_, num_sms_);
-    const int xblock = (int)(CSM_XROWS * stride_);
-    CsmParams p{};
-    for (int ci = 0; ci < 4; ++ci) p.src[ci] = all[ci];
+    XStageParams p{};
+    p.src[0] = src;
+    for (int ci = 1; ci < k_; ++ci) p.src[ci] = srcs_[ci][i].src;
+    if (k_ == 3) p.src[3] = p.src[2];  // pair (2, 3)'s diagonal block: channel 2 in both slots, rows 1..3 unused
     p.nch = k_;
     p.k0 = (long long)k0;
     p.nseg = (int)nseg;
-    p.T = x.T;
-    p.tpc = x.tpc;
-    p.hop = hop;
+    p.hop = (int)ch_[0].hop_;
     p.detrend = ch_[0].detrend_;
-    p.tile_cap = x.tile_cap;
     p.win = d_win_;
     p.tw = d_tw_;
-    p.acc = acc + 2 * (size_t)cblock;
     p.stride = (int)stride_;
-    p.jb = jb;
-    p.g_first = g_first;
-    p.g_s = g_s;
-    const int rows = x.grid * groups_;
-    if (det) {
-        int rc = ensure_part(&d_xpart_, &xpart_cap_, (size_t)rows * xblock);
-        if (rc) return rc;
-        p.part = d_xpart_;
-        p.part_stride = xblock;
-    }
-    int rc = launch_csm((int)log2n_, p, x.grid, stream_);
-    if (rc) return rc;
-    if (p.part) {
-        reduce_partials_kernel<<<(xblock + 127) / 128, 128, 0, stream_>>>(p.acc, p.part, rows, xblock, xblock);
+    p.jb = e.jb;
+    p.g_first = e.g_first;
+    p.g_s = e.g_s;
+
+    float* acc = d_acc_ + i * block_rows() * stride_;
+    if (e.total != 1.0f) {
+        // the EWMA pre-scale of the running sums before this batch, over the stage's whole block
+        const int nblock = (int)(block_rows() * stride_);
+        scale_kernel<<<(nblock + 255) / 256, 256, 0, stream_>>>(acc, nblock, e.total);
         SSPSD_CUDA(cudaGetLastError());
     }
-    return SSPSD_OK;
+    // diagonal blocks: csd_stage_kernel over pair (0, 1), then (2, 3)
+    int rc = launch_block(DIAG, p, nseg, acc, &d_part_, &part_cap_);
+    if (rc || k_ == 2) return rc;
+    XStageParams q = p;
+    q.src[0] = p.src[2];
+    q.src[1] = p.src[3];
+    rc = launch_block(DIAG, q, nseg, acc + CSD_ROWS * stride_, &d_part_, &part_cap_);
+    if (rc) return rc;
+    // off-diagonal block: csm_cross_kernel over all channels
+    return launch_block(CROSS, p, nseg, acc + 2 * CSD_ROWS * stride_, &d_xpart_, &xpart_cap_);
 }
 
 // one lockstep step: the same chunk through channels k_-1 .. 1, then through channel 0 (which launches the kernels)
@@ -671,10 +595,13 @@ int XCascade::num_stages(uint32_t* n)
     return SSPSD_OK;
 }
 
-// PsdCascade::psd's merge (Cascade::merge_host) applied to each row: same breaks, same 1/(gain_i 8^i) per stage
-int XCascade::read(const sspsd_merge_opts& o, float* pxx, float* pyy, float* pxy, size_t* p_len, sspsd_break* b,
-                   size_t* b_len)
+// The common start of read() and read_matrix(): flush, export the book, size the readout (*pl bins, *ns breaks) and
+// check the caller's capacity (outs: the output pointers are non-null), then copy every stage's block to h_acc_.
+// With nothing to merge (*ns == 0) or too little room, *p_len and *b_len are set here and the caller returns rc.
+int XCascade::read_rows(const sspsd_merge_opts& o, bool outs, size_t* p_len, sspsd_break* b, size_t* b_len,
+                        uint64_t (&book)[4 * SSPSD_MAX_STAGES + 2], size_t* pl, size_t* ns)
 {
+    *ns = 0;
     if (!p_len || !b_len) {
         set_error("null length pointer");
         return SSPSD_EINVAL;
@@ -683,24 +610,37 @@ int XCascade::read(const sspsd_merge_opts& o, float* pxx, float* pyy, float* pxy
     if (!g.ok) return SSPSD_ECUDA;
     int rc = flush_all();
     if (rc) return rc;
-    const size_t ns = ch_[0].stages_.size();
-    uint64_t book[4 * SSPSD_MAX_STAGES + 2];
+    const size_t n_st = ch_[0].stages_.size();
     ch_[0].export_book(book);
-    size_t pl = 0, bl = 0;
-    Cascade::merge_host(ch_[0].cfg_, book, nullptr, 0, o, nullptr, &pl, nullptr, &bl);
-    const bool fits = (pl <= *p_len) && (ns <= *b_len) && (pl == 0 || (pxx && pyy && pxy)) && (ns == 0 || b);
-    if (!fits || ns == 0) {
-        *p_len = pl;
-        *b_len = ns;
+    size_t bl = 0;
+    *pl = 0;
+    Cascade::merge_host(ch_[0].cfg_, book, nullptr, 0, o, nullptr, pl, nullptr, &bl);
+    const bool fits = (*pl <= *p_len) && (n_st <= *b_len) && (*pl == 0 || outs) && (n_st == 0 || b);
+    if (!fits || n_st == 0) {
+        *p_len = *pl;
+        *b_len = n_st;
         if (!fits) {
             set_error("output capacity too small");
             return SSPSD_ESHORT;
         }
         return SSPSD_OK;
     }
-    const size_t block = block_rows() * stride_;
-    SSPSD_CUDA(cudaMemcpyAsync(h_acc_, d_acc_, ns * block * sizeof(float), cudaMemcpyDeviceToHost, stream_));
+    *ns = n_st;
+    SSPSD_CUDA(cudaMemcpyAsync(h_acc_, d_acc_, n_st * block_rows() * stride_ * sizeof(float), cudaMemcpyDeviceToHost,
+                               stream_));
     SSPSD_CUDA(cudaStreamSynchronize(stream_));
+    return SSPSD_OK;
+}
+
+// PsdCascade::psd's merge (Cascade::merge_host) applied to each row: same breaks, same 1/(gain_i 8^i) per stage
+int XCascade::read(const sspsd_merge_opts& o, float* pxx, float* pyy, float* pxy, size_t* p_len, sspsd_break* b,
+                   size_t* b_len)
+{
+    uint64_t book[4 * SSPSD_MAX_STAGES + 2];
+    size_t pl, ns;
+    int rc = read_rows(o, pxx && pyy && pxy, p_len, b, b_len, book, &pl, &ns);
+    if (rc || ns == 0) return rc;
+    const size_t block = block_rows() * stride_;
     std::vector<float> re(pl), im(pl);
     float* outs[CSD_ROWS] = {pxx, pyy, re.data(), im.data()};
     for (int r = 0; r < CSD_ROWS; ++r) {
@@ -721,32 +661,11 @@ int XCascade::read(const sspsd_merge_opts& o, float* pxx, float* pyy, float* pxy
 // the diagonal real (imaginary part 0), the lower triangle the conjugate of the upper.
 int XCascade::read_matrix(const sspsd_merge_opts& o, float* s, size_t* p_len, sspsd_break* b, size_t* b_len)
 {
-    if (!p_len || !b_len) {
-        set_error("null length pointer");
-        return SSPSD_EINVAL;
-    }
-    DeviceGuard g(cfg_.device);
-    if (!g.ok) return SSPSD_ECUDA;
-    int rc = flush_all();
-    if (rc) return rc;
-    const size_t ns = ch_[0].stages_.size();
     uint64_t book[4 * SSPSD_MAX_STAGES + 2];
-    ch_[0].export_book(book);
-    size_t pl = 0, bl = 0;
-    Cascade::merge_host(ch_[0].cfg_, book, nullptr, 0, o, nullptr, &pl, nullptr, &bl);
-    const bool fits = (pl <= *p_len) && (ns <= *b_len) && (pl == 0 || s) && (ns == 0 || b);
-    if (!fits || ns == 0) {
-        *p_len = pl;
-        *b_len = ns;
-        if (!fits) {
-            set_error("output capacity too small");
-            return SSPSD_ESHORT;
-        }
-        return SSPSD_OK;
-    }
+    size_t pl, ns;
+    int rc = read_rows(o, s != nullptr, p_len, b, b_len, book, &pl, &ns);
+    if (rc || ns == 0) return rc;
     const size_t block = block_rows() * stride_;
-    SSPSD_CUDA(cudaMemcpyAsync(h_acc_, d_acc_, ns * block * sizeof(float), cudaMemcpyDeviceToHost, stream_));
-    SSPSD_CUDA(cudaStreamSynchronize(stream_));
     // stored rows of the upper triangle: (i, j) -> (row of Re, row of Im); the diagonal has no Im row
     int re_row[4][4], im_row[4][4];
     for (int a = 0; 2 * a < k_; ++a) {
@@ -801,18 +720,26 @@ struct sspsd_csd {
     sspsd::XCascade c;
 };
 
+struct sspsd_csm {
+    sspsd::XCascade c;
+};
+
 using sspsd::set_error;
 
-int32_t sspsd_csd_create(const sspsd_config* cfg, sspsd_csd** out)
+namespace {
+
+// create / clone of either handle (sspsd_csd: k = 2)
+template <class H>
+int32_t x_create(const sspsd_config* cfg, int k, H** out)
 {
     if (!cfg || !out) {
         set_error("null argument");
         return SSPSD_EINVAL;
     }
     *out = nullptr;
-    sspsd_csd* h = new (std::nothrow) sspsd_csd();
+    H* h = new (std::nothrow) H();
     if (!h) return SSPSD_ENOMEM;
-    int rc = h->c.init(*cfg, 2);
+    int rc = h->c.init(*cfg, k);
     if (rc) {
         delete h;
         return rc;
@@ -821,16 +748,15 @@ int32_t sspsd_csd_create(const sspsd_config* cfg, sspsd_csd** out)
     return SSPSD_OK;
 }
 
-void sspsd_csd_destroy(sspsd_csd* h) { delete h; }
-
-int32_t sspsd_csd_clone(sspsd_csd* h, sspsd_csd** out)
+template <class H>
+int32_t x_clone(H* h, H** out)
 {
     if (!h || !out) {
         set_error("null argument");
         return SSPSD_EINVAL;
     }
     *out = nullptr;
-    sspsd_csd* n = new (std::nothrow) sspsd_csd();
+    H* n = new (std::nothrow) H();
     if (!n) return SSPSD_ENOMEM;
     int rc = n->c.clone_from(h->c);
     if (rc) {
@@ -840,6 +766,14 @@ int32_t sspsd_csd_clone(sspsd_csd* h, sspsd_csd** out)
     *out = n;
     return SSPSD_OK;
 }
+
+}  // namespace
+
+int32_t sspsd_csd_create(const sspsd_config* cfg, sspsd_csd** out) { return x_create(cfg, 2, out); }
+
+void sspsd_csd_destroy(sspsd_csd* h) { delete h; }
+
+int32_t sspsd_csd_clone(sspsd_csd* h, sspsd_csd** out) { return x_clone(h, out); }
 
 int32_t sspsd_csd_reset(sspsd_csd* h) { return h ? h->c.reset() : SSPSD_EINVAL; }
 
@@ -890,47 +824,11 @@ int32_t sspsd_csd_stream(const sspsd_csd* h, void** stream)
 int32_t sspsd_csd_flush(sspsd_csd* h) { return h ? h->c.flush() : SSPSD_EINVAL; }
 int32_t sspsd_csd_sync(sspsd_csd* h) { return h ? h->c.sync() : SSPSD_EINVAL; }
 
-struct sspsd_csm {
-    sspsd::XCascade c;
-};
-
-int32_t sspsd_csm_create(const sspsd_config* cfg, int32_t k, sspsd_csm** out)
-{
-    if (!cfg || !out) {
-        set_error("null argument");
-        return SSPSD_EINVAL;
-    }
-    *out = nullptr;
-    sspsd_csm* h = new (std::nothrow) sspsd_csm();
-    if (!h) return SSPSD_ENOMEM;
-    int rc = h->c.init(*cfg, k);
-    if (rc) {
-        delete h;
-        return rc;
-    }
-    *out = h;
-    return SSPSD_OK;
-}
+int32_t sspsd_csm_create(const sspsd_config* cfg, int32_t k, sspsd_csm** out) { return x_create(cfg, k, out); }
 
 void sspsd_csm_destroy(sspsd_csm* h) { delete h; }
 
-int32_t sspsd_csm_clone(sspsd_csm* h, sspsd_csm** out)
-{
-    if (!h || !out) {
-        set_error("null argument");
-        return SSPSD_EINVAL;
-    }
-    *out = nullptr;
-    sspsd_csm* n = new (std::nothrow) sspsd_csm();
-    if (!n) return SSPSD_ENOMEM;
-    int rc = n->c.clone_from(h->c);
-    if (rc) {
-        delete n;
-        return rc;
-    }
-    *out = n;
-    return SSPSD_OK;
-}
+int32_t sspsd_csm_clone(sspsd_csm* h, sspsd_csm** out) { return x_clone(h, out); }
 
 int32_t sspsd_csm_channels(const sspsd_csm* h, int32_t* k)
 {
