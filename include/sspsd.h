@@ -454,6 +454,21 @@ int32_t sspsd_cascade_process_frames(sspsd_decoder *d, sspsd_cascade *const *cas
                                      size_t frame_stride, int32_t frames_mem, sspsd_loss *loss,
                                      sspsd_decode_info *info);
 
+/* Fused decode -> cross-spectral matrix: channel i of `m` is fed trace traces[i] of every frame (traces == NULL:
+ * channel i <- trace i), all K channels in lockstep on the handle's stream.  Host / device frames, loss accounting,
+ * malformed frames (the good prefix before one is consumed by all K channels) and `info` exactly as
+ * sspsd_cascade_process_frames.  An index may repeat (the matrix of repeated channels).  SSPSD_EINVAL, with nothing
+ * consumed and `loss` unchanged: a NULL handle, an index >= 4, an index at or above the trace count of the frames'
+ * format (Mpll has 3; checked against frame 0 before anything is queued), decoder and handle on different devices.
+ * `traces` holds one index per channel (sspsd_csm_channels). */
+int32_t sspsd_csm_process_frames(sspsd_decoder *d, sspsd_csm *m, const uint32_t *traces, const uint8_t *frames,
+                                 size_t n_frames, size_t frame_len, size_t frame_stride, int32_t frames_mem,
+                                 sspsd_loss *loss, sspsd_decode_info *info);
+/* the same into a cross-spectral density: x <- trace trace_x, y <- trace trace_y */
+int32_t sspsd_csd_process_frames(sspsd_decoder *d, sspsd_csd *c, uint32_t trace_x, uint32_t trace_y,
+                                 const uint8_t *frames, size_t n_frames, size_t frame_len, size_t frame_stride,
+                                 int32_t frames_mem, sspsd_loss *loss, sspsd_decode_info *info);
+
 /* Loss::update on one header (host helper, bit-exact u64/u32 wrapping arithmetic), src/loss.rs:11-26 */
 void sspsd_loss_update(sspsd_loss *loss, uint32_t seq, uint8_t batches);
 /* the ratio logged by Loss::analyze, src/loss.rs:28-30 */
@@ -516,6 +531,12 @@ int32_t sspsd_receiver_recv(sspsd_receiver *r, uint32_t max_frames, int32_t time
 /* recv + sspsd_cascade_process_frames in one call (info->frames_ok == 0 on timeout) */
 int32_t sspsd_receiver_pump(sspsd_receiver *r, sspsd_decoder *d, sspsd_cascade *const *cascades, uint32_t n_cascades,
                             uint32_t max_frames, int32_t timeout_ms, sspsd_loss *loss, sspsd_decode_info *info);
+/* recv + sspsd_csm_process_frames / sspsd_csd_process_frames.  NULL handles and indices >= 4 are refused before a
+ * datagram is taken; a trace map the frames' format cannot serve refuses (and drops) that run. */
+int32_t sspsd_receiver_pump_csm(sspsd_receiver *r, sspsd_decoder *d, sspsd_csm *m, const uint32_t *traces,
+                                uint32_t max_frames, int32_t timeout_ms, sspsd_loss *loss, sspsd_decode_info *info);
+int32_t sspsd_receiver_pump_csd(sspsd_receiver *r, sspsd_decoder *d, sspsd_csd *c, uint32_t trace_x, uint32_t trace_y,
+                                uint32_t max_frames, int32_t timeout_ms, sspsd_loss *loss, sspsd_decode_info *info);
 
 /* ---------------------------------------------------------------------------------------------
  * Var::eval (AVAR/MVAR/FVAR from a phase PSD), src/var.rs:26-45 -- host helper on psd() output

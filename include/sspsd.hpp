@@ -433,6 +433,47 @@ public:
         check(st);
         return info;
     }
+    /// fused decode -> cross-spectral density: x <- trace trace_x, y <- trace trace_y of every frame
+    template <size_t N>
+    sspsd_decode_info process_frames(CsdCascade<N>& c, uint32_t trace_x, uint32_t trace_y, const uint8_t* frames,
+                                     size_t n_frames, size_t frame_len, Loss* loss, Mem mem = Mem::Host,
+                                     size_t frame_stride = 0)
+    {
+        sspsd_decode_info info{};
+        int32_t st = sspsd_csd_process_frames(d_, c.handle(), trace_x, trace_y, frames, n_frames, frame_len,
+                                              frame_stride ? frame_stride : frame_len, (int32_t)mem,
+                                              loss ? &loss->c : nullptr, &info);
+        return finish(st, info);
+    }
+    /// fused decode -> cross-spectral matrix: channel i <- trace traces[i] (one index per channel; empty: 0 .. K-1)
+    template <size_t N>
+    sspsd_decode_info process_frames(CsmCascade<N>& m, const std::vector<uint32_t>& traces, const uint8_t* frames,
+                                     size_t n_frames, size_t frame_len, Loss* loss, Mem mem = Mem::Host,
+                                     size_t frame_stride = 0)
+    {
+        sspsd_decode_info info{};
+        int32_t st = sspsd_csm_process_frames(d_, m.handle(), trace_map(m, traces), frames, n_frames, frame_len,
+                                              frame_stride ? frame_stride : frame_len, (int32_t)mem,
+                                              loss ? &loss->c : nullptr, &info);
+        return finish(st, info);
+    }
+    sspsd_decoder* handle() const { return d_; }
+
+    /// the C ABI's view of a CsmCascade trace map (NULL for the identity); throws unless one index per channel
+    template <size_t N>
+    static const uint32_t* trace_map(const CsmCascade<N>& m, const std::vector<uint32_t>& traces)
+    {
+        if (traces.empty()) return nullptr;
+        if (traces.size() != (size_t)m.channels()) throw Error(SSPSD_EINVAL, "one trace index per channel");
+        return traces.data();
+    }
+    /// the result of a fused call: a malformed frame throws DecodeError, any other failure Error
+    static sspsd_decode_info finish(int32_t st, const sspsd_decode_info& info)
+    {
+        if (st >= SSPSD_EHEADER && st <= SSPSD_ESHORT) throw DecodeError(st, info.frames_ok);
+        check(st);
+        return info;
+    }
 
 private:
     sspsd_decoder* d_ = nullptr;
@@ -507,6 +548,26 @@ public:
         Run r{};
         check(sspsd_receiver_recv(h_, max_frames, timeout_ms, &r.frames, &r.n_frames, &r.frame_len));
         return r;
+    }
+    /// recv + FrameDecoder::process_frames into a CsdCascade (info.frames_ok == 0 on timeout)
+    template <size_t N>
+    sspsd_decode_info pump(FrameDecoder& d, CsdCascade<N>& c, uint32_t trace_x, uint32_t trace_y, Loss* loss,
+                           uint32_t max_frames = 1024, int32_t timeout_ms = 1000)
+    {
+        sspsd_decode_info info{};
+        int32_t st = sspsd_receiver_pump_csd(h_, d.handle(), c.handle(), trace_x, trace_y, max_frames, timeout_ms,
+                                             loss ? &loss->c : nullptr, &info);
+        return FrameDecoder::finish(st, info);
+    }
+    /// recv + FrameDecoder::process_frames into a CsmCascade (info.frames_ok == 0 on timeout)
+    template <size_t N>
+    sspsd_decode_info pump(FrameDecoder& d, CsmCascade<N>& m, const std::vector<uint32_t>& traces, Loss* loss,
+                           uint32_t max_frames = 1024, int32_t timeout_ms = 1000)
+    {
+        sspsd_decode_info info{};
+        int32_t st = sspsd_receiver_pump_csm(h_, d.handle(), m.handle(), FrameDecoder::trace_map(m, traces), max_frames,
+                                             timeout_ms, loss ? &loss->c : nullptr, &info);
+        return FrameDecoder::finish(st, info);
     }
     sspsd_receiver* handle() const { return h_; }
 

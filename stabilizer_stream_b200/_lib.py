@@ -153,6 +153,10 @@ PROTOTYPES = {
                                    C.POINTER(DecodeInfoC)]),
     "sspsd_cascade_process_frames": (_i32, [_vp, C.POINTER(_vp), C.c_uint32, _vp, _sz, _sz, _sz, _i32,
                                             C.POINTER(LossC), C.POINTER(DecodeInfoC)]),
+    "sspsd_csm_process_frames": (_i32, [_vp, _vp, C.POINTER(C.c_uint32), _vp, _sz, _sz, _sz, _i32, C.POINTER(LossC),
+                                        C.POINTER(DecodeInfoC)]),
+    "sspsd_csd_process_frames": (_i32, [_vp, _vp, C.c_uint32, C.c_uint32, _vp, _sz, _sz, _sz, _i32, C.POINTER(LossC),
+                                        C.POINTER(DecodeInfoC)]),
     "sspsd_loss_update": (None, [C.POINTER(LossC), C.c_uint32, C.c_uint8]),
     "sspsd_loss_ratio": (C.c_float, [C.POINTER(LossC)]),
     "sspsd_var_eval": (C.c_float, [C.POINTER(VarC), _vp, _vp, _sz, C.c_float]),
@@ -192,6 +196,10 @@ PROTOTYPES = {
     "sspsd_receiver_recv": (_i32, [_vp, C.c_uint32, _i32, C.POINTER(_vp), _psz, _psz]),
     "sspsd_receiver_pump": (_i32, [_vp, _vp, C.POINTER(_vp), C.c_uint32, C.c_uint32, _i32, C.POINTER(LossC),
                                    C.POINTER(DecodeInfoC)]),
+    "sspsd_receiver_pump_csm": (_i32, [_vp, _vp, _vp, C.POINTER(C.c_uint32), C.c_uint32, _i32, C.POINTER(LossC),
+                                       C.POINTER(DecodeInfoC)]),
+    "sspsd_receiver_pump_csd": (_i32, [_vp, _vp, _vp, C.c_uint32, C.c_uint32, C.c_uint32, _i32, C.POINTER(LossC),
+                                       C.POINTER(DecodeInfoC)]),
 }
 
 _lib = None

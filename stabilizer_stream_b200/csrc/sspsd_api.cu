@@ -460,9 +460,11 @@ int queue_decode(sspsd_decoder* d, const uint8_t* dfr, size_t n_frames, size_t s
 }
 
 // Runs scan + loss + payload decode on d->stream.  dst[t] are device pointers (aligned if `aligned`).
-// On return (stream synchronised) d->h_res[0] holds the batch result.
+// On return (stream synchronised) d->h_res[0] holds the batch result.  `sink` (if any) is shown the format byte
+// before the decode is queued and may refuse it.
 int decode_on_device(sspsd_decoder* d, const uint8_t* frames, size_t n_frames, size_t frame_len, size_t frame_stride,
-                     int frames_mem, const sspsd_loss* loss, float* const* dst, bool dst_aligned, size_t dst_cap)
+                     int frames_mem, const sspsd_loss* loss, float* const* dst, bool dst_aligned, size_t dst_cap,
+                     sspsd::FrameSink* sink = nullptr)
 {
     const size_t n_bytes = n_frames ? (n_frames - 1) * frame_stride + frame_len : 0;
     const uint8_t* dfr = frames;
@@ -486,6 +488,10 @@ int decode_on_device(sspsd_decoder* d, const uint8_t* frames, size_t n_frames, s
             SSPSD_CUDA(cudaMemcpyAsync(hdr, dfr, 4, cudaMemcpyDeviceToHost, d->stream));
             SSPSD_CUDA(cudaStreamSynchronize(d->stream));
         }
+    }
+    if (sink) {
+        rc = sink->accept(hdr[2]);
+        if (rc) return rc;
     }
     rc = queue_decode(d, dfr, n_frames, 0, frame_len, frame_stride, loss, dst, dst_aligned, dst_cap, hdr[2], 0);
     if (rc) return rc;
@@ -603,28 +609,36 @@ int32_t sspsd_decode_frames(sspsd_decoder* d, const uint8_t* frames, size_t n_fr
     return SSPSD_OK;
 }
 
-int32_t sspsd_cascade_process_frames(sspsd_decoder* d, sspsd_cascade* const* cascades, uint32_t n_cascades,
-                                     const uint8_t* frames, size_t n_frames, size_t frame_len, size_t frame_stride,
-                                     int32_t frames_mem, sspsd_loss* loss, sspsd_decode_info* info)
+}  // extern "C"
+
+namespace sspsd {
+
+int trace_consumed(sspsd_decoder* d, int t, cudaStream_t s)
 {
-    if (!d || (n_frames && !frames) || frame_stride < frame_len || n_cascades > SSPSD_MAX_TRACES ||
-        (n_cascades && !cascades)) {
-        set_error("bad argument");
-        return SSPSD_EINVAL;
-    }
+    SSPSD_CUDA(cudaEventRecord(d->ev_consumed[t], s));
+    d->consumed_pending[t] = true;
+    return SSPSD_OK;
+}
+
+// The frame pipeline of sspsd_cascade_process_frames and sspsd_csd / sspsd_csm_process_frames: header scan, copies,
+// decode, loss cross-check; what the decoded traces feed is the sink's business.
+int process_frames(sspsd_decoder* d, FrameSink& sink, const uint8_t* frames, size_t n_frames, size_t frame_len,
+                   size_t frame_stride, int frames_mem, sspsd_loss* loss, sspsd_decode_info* info)
+{
     if (info) std::memset(info, 0, sizeof(*info));
     if (n_frames == 0) return SSPSD_OK;
     if (frame_len < SSPSD_HEADER_SIZE) {
         set_error("frame shorter than its header");
         return SSPSD_ESHORT;
     }
-    for (uint32_t t = 0; t < n_cascades; ++t)
-        if (cascades[t] && cascades[t]->c.device() != d->device) {
-            set_error("cascade and decoder live on different devices");
-            return SSPSD_EINVAL;
-        }
+    int rc = sink.check_device(d->device);
+    if (rc) return rc;
     DevGuard g(d->device);
     if (!g.ok) return SSPSD_ECUDA;
+    if (frames_mem == SSPSD_MEM_HOST) {
+        rc = sink.accept(frames[2]);
+        if (rc) return rc;
+    }
     const size_t payload = frame_len - SSPSD_HEADER_SIZE;
     const size_t worst = n_frames * std::max<size_t>(payload / 64 * 8, payload / 24);
     // (the previous batch's traces may still be read by the cascades' streams: decode_on_device makes the decode
@@ -645,14 +659,14 @@ int32_t sspsd_cascade_process_frames(sspsd_decoder* d, sspsd_cascade* const* cas
         // frame_status() the scan kernel runs, one cache line per frame, prefetched ahead) and applies Loss::update to
         // them, so the number of good frames, the format, the batch count and the sequence state the NEXT sub-chunk starts
         // from are known without a device round trip; scan / loss / payload decode of sub-chunk k are queued behind its
-        // copy and the cascades behind its decode, so they run while sub-chunk k + 1 is still being copied.  The one
+        // copy and the sink's work behind its decode, so they run while sub-chunk k + 1 is still being copied.  The one
         // wait is at the end (the caller's buffer is borrowed for the call only, and the loss counters the device
         // computed are the ones returned: the host's serve as a cross-check).
         static const bool trace = getenv("SSPSD_FRAMES_TRACE") != nullptr;
         using clk = std::chrono::steady_clock;
         const auto t0 = clk::now();
         const size_t n_bytes = (n_frames - 1) * frame_stride + frame_len;
-        int rc = frames_reserve(d, n_bytes);
+        rc = frames_reserve(d, n_bytes);
         if (rc) return rc;
         rc = status_reserve(d, n_frames);
         if (rc) return rc;
@@ -707,15 +721,8 @@ int32_t sspsd_cascade_process_frames(sspsd_decoder* d, sspsd_cascade* const* cas
                                   dst, off % 4 == 0, d->traces_cap - off, fmt0, (int)k);
                 if (rc) return rc;
                 SSPSD_CUDA(cudaEventRecord(d->ev_decoded, d->stream));
-                const size_t ns = nk * batches * div;
-                for (uint32_t t = 0; t < n_cascades && t < ntr; ++t) {
-                    if (!cascades[t]) continue;
-                    SSPSD_CUDA(cudaStreamWaitEvent(cascades[t]->c.stream(), d->ev_decoded, 0));
-                    rc = cascades[t]->c.process(dst[t], ns, SSPSD_MEM_DEVICE);
-                    if (rc) return rc;
-                    SSPSD_CUDA(cudaEventRecord(d->ev_consumed[t], cascades[t]->c.stream()));
-                    d->consumed_pending[t] = true;
-                }
+                rc = sink.consume(d, dst, ntr, nk * batches * div, d->ev_decoded);
+                if (rc) return rc;
                 queued = k + 1;
             }
             if (trace) {
@@ -763,7 +770,8 @@ int32_t sspsd_cascade_process_frames(sspsd_decoder* d, sspsd_cascade* const* cas
         }
         return SSPSD_OK;
     }
-    int rc = decode_on_device(d, frames, n_frames, frame_len, frame_stride, frames_mem, loss, d->d_traces, true, d->traces_cap);
+    rc = decode_on_device(d, frames, n_frames, frame_len, frame_stride, frames_mem, loss, d->d_traces, true, d->traces_cap,
+                          &sink);
     if (rc) return rc;
     const sspsd::DecodeResult r = *d->h_res;
     const unsigned int div = r.format == SSPSD_FORMAT_ADCDAC ? 8 : 1;
@@ -771,20 +779,65 @@ int32_t sspsd_cascade_process_frames(sspsd_decoder* d, sspsd_cascade* const* cas
     if (r.first_bad > 0) {
         const size_t ns = (size_t)r.first_bad * r.batches * div;
         const uint32_t ntr = r.format == SSPSD_FORMAT_MPLL ? 3 : 4;
-        for (uint32_t t = 0; t < n_cascades && t < ntr; ++t) {
-            if (!cascades[t]) continue;
-            // decode_on_device synchronised d->stream, so the traces are complete for any stream
-            rc = cascades[t]->c.process(d->d_traces[t], ns, SSPSD_MEM_DEVICE);
-            if (rc) return rc;
-            SSPSD_CUDA(cudaEventRecord(d->ev_consumed[t], cascades[t]->c.stream()));
-            d->consumed_pending[t] = true;
-        }
+        // decode_on_device synchronised d->stream, so the traces are complete for any stream
+        rc = sink.consume(d, d->d_traces, ntr, ns, nullptr);
+        if (rc) return rc;
     }
     if (r.first_bad < n_frames) {
         set_error("malformed frame");
         return (int32_t)r.status;
     }
     return SSPSD_OK;
+}
+
+}  // namespace sspsd
+
+namespace {
+
+// sspsd_cascade_process_frames: trace t -> cascades[t], each on its own stream
+struct CascadeSink : sspsd::FrameSink {
+    sspsd_cascade* const* c;
+    uint32_t n;
+    CascadeSink(sspsd_cascade* const* c_, uint32_t n_) : c(c_), n(n_) {}
+    int check_device(int device) override
+    {
+        for (uint32_t t = 0; t < n; ++t)
+            if (c[t] && c[t]->c.device() != device) {
+                set_error("cascade and decoder live on different devices");
+                return SSPSD_EINVAL;
+            }
+        return SSPSD_OK;
+    }
+    int accept(unsigned int) override { return SSPSD_OK; }  // cascades past the format's traces get nothing
+    int consume(sspsd_decoder* d, float* const* tr, uint32_t n_traces, size_t ns, cudaEvent_t ready) override
+    {
+        for (uint32_t t = 0; t < n && t < n_traces; ++t) {
+            if (!c[t]) continue;
+            if (ready) SSPSD_CUDA(cudaStreamWaitEvent(c[t]->c.stream(), ready, 0));
+            int rc = c[t]->c.process(tr[t], ns, SSPSD_MEM_DEVICE);
+            if (rc) return rc;
+            rc = sspsd::trace_consumed(d, (int)t, c[t]->c.stream());
+            if (rc) return rc;
+        }
+        return SSPSD_OK;
+    }
+};
+
+}  // namespace
+
+extern "C" {
+
+int32_t sspsd_cascade_process_frames(sspsd_decoder* d, sspsd_cascade* const* cascades, uint32_t n_cascades,
+                                     const uint8_t* frames, size_t n_frames, size_t frame_len, size_t frame_stride,
+                                     int32_t frames_mem, sspsd_loss* loss, sspsd_decode_info* info)
+{
+    if (!d || (n_frames && !frames) || frame_stride < frame_len || n_cascades > SSPSD_MAX_TRACES ||
+        (n_cascades && !cascades)) {
+        set_error("bad argument");
+        return SSPSD_EINVAL;
+    }
+    CascadeSink sink(cascades, n_cascades);
+    return sspsd::process_frames(d, sink, frames, n_frames, frame_len, frame_stride, frames_mem, loss, info);
 }
 
 void sspsd_loss_update(sspsd_loss* l, uint32_t seq, uint8_t batches)

@@ -240,6 +240,22 @@ private:
     size_t sink_cap_ = 0, sink_len_ = 0;
 };
 
+// What a frame batch is decoded into (sspsd_api.cu's frame pipeline): the PsdCascades of
+// sspsd_cascade_process_frames, or one CsdCascade / CsmCascade and its trace map.
+struct FrameSink {
+    // before anything is queued: handles on the decoder's device
+    virtual int check_device(int device) = 0;
+    // the batch's format byte (frame 0), once known and before anything is queued: can the sink take its traces
+    virtual int accept(unsigned int fmt) = 0;
+    // one decoded sub-chunk: trace t at tr[t] (t < n_traces), ns samples each, complete once `ready` has fired
+    // (nullptr: already complete).  Every trace read is reported with trace_consumed() on the stream that reads it.
+    virtual int consume(sspsd_decoder* d, float* const* tr, uint32_t n_traces, size_t ns, cudaEvent_t ready) = 0;
+};
+int process_frames(sspsd_decoder* d, FrameSink& sink, const uint8_t* frames, size_t n_frames, size_t frame_len,
+                   size_t frame_stride, int frames_mem, sspsd_loss* loss, sspsd_decode_info* info);
+// the decoder's trace buffer t is read by work queued on s so far: the next decode into it waits for that
+int trace_consumed(sspsd_decoder* d, int t, cudaStream_t s);
+
 }  // namespace sspsd
 
 // the opaque handles of include/sspsd.h

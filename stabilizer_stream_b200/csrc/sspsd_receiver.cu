@@ -210,4 +210,35 @@ int32_t sspsd_receiver_pump(sspsd_receiver* h, sspsd_decoder* d, sspsd_cascade* 
                                         info);
 }
 
+// The handles and the trace map are checked (an empty batch) before a run is taken from the ring, so that a bad
+// argument drops no datagram.
+int32_t sspsd_receiver_pump_csm(sspsd_receiver* h, sspsd_decoder* d, sspsd_csm* m, const uint32_t* traces,
+                                uint32_t max_frames, int32_t timeout_ms, sspsd_loss* loss, sspsd_decode_info* info)
+{
+    if (!h) return SSPSD_EINVAL;
+    if (info) std::memset(info, 0, sizeof(*info));
+    int rc = sspsd_csm_process_frames(d, m, traces, nullptr, 0, 0, 0, SSPSD_MEM_HOST, nullptr, nullptr);
+    if (rc) return rc;
+    const uint8_t* frames = nullptr;
+    size_t n = 0, len = 0;
+    rc = h->r.recv(max_frames, timeout_ms, &frames, &n, &len);
+    if (rc || n == 0) return rc;
+    return sspsd_csm_process_frames(d, m, traces, frames, n, len, h->r.slot_bytes(), SSPSD_MEM_HOST, loss, info);
+}
+
+int32_t sspsd_receiver_pump_csd(sspsd_receiver* h, sspsd_decoder* d, sspsd_csd* c, uint32_t trace_x, uint32_t trace_y,
+                                uint32_t max_frames, int32_t timeout_ms, sspsd_loss* loss, sspsd_decode_info* info)
+{
+    if (!h) return SSPSD_EINVAL;
+    if (info) std::memset(info, 0, sizeof(*info));
+    int rc = sspsd_csd_process_frames(d, c, trace_x, trace_y, nullptr, 0, 0, 0, SSPSD_MEM_HOST, nullptr, nullptr);
+    if (rc) return rc;
+    const uint8_t* frames = nullptr;
+    size_t n = 0, len = 0;
+    rc = h->r.recv(max_frames, timeout_ms, &frames, &n, &len);
+    if (rc || n == 0) return rc;
+    return sspsd_csd_process_frames(d, c, trace_x, trace_y, frames, n, len, h->r.slot_bytes(), SSPSD_MEM_HOST, loss,
+                                    info);
+}
+
 }  // extern "C"

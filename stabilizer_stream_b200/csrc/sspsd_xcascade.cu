@@ -124,6 +124,7 @@ public:
     int read_matrix(const sspsd_merge_opts& o, float* s, size_t* p_len, sspsd_break* b, size_t* b_len);
     int num_stages(uint32_t* n);
     int channels() const { return k_; }
+    int device() const { return cfg_.device; }
     float rbw() const { return ch_[0].rbw(); }
     cudaStream_t stream() const { return stream_; }
     int stage_psd(Cascade& c, size_t i, const StreamSrc& src, uint64_t k0, uint64_t nseg, const EwmaPlan& e) override;
@@ -767,6 +768,71 @@ int32_t x_clone(H* h, H** out)
     return SSPSD_OK;
 }
 
+// Channel i <- trace map[i] of every decoded sub-chunk: one XCascade::process on the handle's one stream.  All
+// channels sit at one stream position and the decoder's trace buffers share one alignment, so either every channel
+// reads its sub-chunk in place or every channel takes the realigning copy.
+struct XSink : sspsd::FrameSink {
+    sspsd::XCascade& x;
+    const uint32_t* map;
+    XSink(sspsd::XCascade& x_, const uint32_t* map_) : x(x_), map(map_) {}
+    int check_device(int device) override
+    {
+        if (x.device() != device) {
+            set_error("cross-spectral handle and decoder live on different devices");
+            return SSPSD_EINVAL;
+        }
+        return SSPSD_OK;
+    }
+    int accept(unsigned int fmt) override
+    {
+        const uint32_t ntr = fmt == SSPSD_FORMAT_MPLL ? 3 : 4;
+        for (int i = 0; i < x.channels(); ++i)
+            if (map[i] >= ntr) {
+                set_error("trace index " + std::to_string(map[i]) + " past the " + std::to_string(ntr) +
+                          " traces of the frames' format");
+                return SSPSD_EINVAL;
+            }
+        return SSPSD_OK;
+    }
+    int consume(sspsd_decoder* d, float* const* tr, uint32_t, size_t ns, cudaEvent_t ready) override
+    {
+        const float* xs[4];
+        for (int i = 0; i < x.channels(); ++i) xs[i] = tr[map[i]];
+        if (ready) SSPSD_CUDA(cudaStreamWaitEvent(x.stream(), ready, 0));
+        int rc = x.process(xs, ns, SSPSD_MEM_DEVICE);
+        if (rc) return rc;
+        for (int i = 0; i < x.channels(); ++i) {
+            rc = sspsd::trace_consumed(d, (int)map[i], x.stream());
+            if (rc) return rc;
+        }
+        return SSPSD_OK;
+    }
+};
+
+// sspsd_csd / sspsd_csm_process_frames; traces: one index per channel, NULL for 0 .. K-1
+template <class H>
+int32_t x_process_frames(sspsd_decoder* d, H* h, const uint32_t* traces, const uint8_t* frames, size_t n_frames,
+                         size_t frame_len, size_t frame_stride, int32_t frames_mem, sspsd_loss* loss,
+                         sspsd_decode_info* info)
+{
+    if (!d || !h || (n_frames && !frames) || frame_stride < frame_len) {
+        set_error("bad argument");
+        return SSPSD_EINVAL;
+    }
+    uint32_t map[4] = {0, 1, 2, 3};
+    if (traces) {
+        for (int i = 0; i < h->c.channels(); ++i) {
+            if (traces[i] >= SSPSD_MAX_TRACES) {
+                set_error("trace index " + std::to_string(traces[i]) + " out of range (frames carry at most 4 traces)");
+                return SSPSD_EINVAL;
+            }
+            map[i] = traces[i];
+        }
+    }
+    XSink sink(h->c, map);
+    return sspsd::process_frames(d, sink, frames, n_frames, frame_len, frame_stride, frames_mem, loss, info);
+}
+
 }  // namespace
 
 int32_t sspsd_csd_create(const sspsd_config* cfg, sspsd_csd** out) { return x_create(cfg, 2, out); }
@@ -786,6 +852,14 @@ int32_t sspsd_csd_process_f32(sspsd_csd* h, const float* x, const float* y, size
     }
     const float* xs[2] = {x, y};
     return h->c.process(xs, n, mem);
+}
+
+int32_t sspsd_csd_process_frames(sspsd_decoder* d, sspsd_csd* c, uint32_t trace_x, uint32_t trace_y,
+                                 const uint8_t* frames, size_t n_frames, size_t frame_len, size_t frame_stride,
+                                 int32_t frames_mem, sspsd_loss* loss, sspsd_decode_info* info)
+{
+    const uint32_t traces[2] = {trace_x, trace_y};
+    return x_process_frames(d, c, traces, frames, n_frames, frame_len, frame_stride, frames_mem, loss, info);
 }
 
 int32_t sspsd_csd_set_avg(sspsd_csd* h, sspsd_avg_opts avg) { return h ? h->c.set_avg(avg) : SSPSD_EINVAL; }
@@ -843,6 +917,13 @@ int32_t sspsd_csm_process_f32(sspsd_csm* h, const float* const* x, size_t n, int
 {
     if (!h) return SSPSD_EINVAL;
     return h->c.process(x, n, mem);
+}
+
+int32_t sspsd_csm_process_frames(sspsd_decoder* d, sspsd_csm* m, const uint32_t* traces, const uint8_t* frames,
+                                 size_t n_frames, size_t frame_len, size_t frame_stride, int32_t frames_mem,
+                                 sspsd_loss* loss, sspsd_decode_info* info)
+{
+    return x_process_frames(d, m, traces, frames, n_frames, frame_len, frame_stride, frames_mem, loss, info);
 }
 
 int32_t sspsd_csm_set_avg(sspsd_csm* h, sspsd_avg_opts avg) { return h ? h->c.set_avg(avg) : SSPSD_EINVAL; }

@@ -661,6 +661,20 @@ class Loss:
         return L.lib().sspsd_loss_ratio(C.byref(self.c))
 
 
+def _trace_map(target, traces):
+    """The trace indices a CsdCascade / CsmCascade target of process_frames / pump reads, one per channel (default
+    0 .. K-1); None for a list of PsdCascades, which take trace t into target[t]."""
+    if not isinstance(target, (CsdCascade, CsmCascade)):
+        if traces is not None:
+            raise ValueError("traces= applies to a CsdCascade or CsmCascade target")
+        return None
+    k = 2 if isinstance(target, CsdCascade) else target.channels
+    tmap = list(range(k)) if traces is None else [int(t) for t in traces]
+    if len(tmap) != k:
+        raise ValueError("expected %d trace indices (one per channel), got %d" % (k, len(tmap)))
+    return tmap
+
+
 class FrameDecoder(_StreamOrdered):
     """Batched Frame::from_bytes + Loss::update + Payload::traces (src/de/frame.rs:49-60,
     src/loss.rs:11-26, src/de/data.rs)."""
@@ -736,17 +750,29 @@ class FrameDecoder(_StreamOrdered):
         L.check(st)
         return info
 
-    def process_frames(self, cascades, frames, frame_len, loss: Loss = None, frame_stride=None, n_frames=None):
-        """Fused decode -> one PsdCascade per trace (src/bin/psd.rs:174-182)."""
+    def process_frames(self, target, frames, frame_len, loss: Loss = None, frame_stride=None, n_frames=None,
+                       traces=None):
+        """Fused decode -> spectra.  `target` is a list of PsdCascades (trace t -> target[t], None drops a trace;
+        src/bin/psd.rs:174-182), a CsdCascade (x, y <- traces, default (0, 1)) or a CsmCascade (channel i <-
+        traces[i], default range(K)).  Raises DecodeError on a malformed frame after having consumed the frames
+        before it."""
+        tmap = _trace_map(target, traces)
         frame_stride = frame_stride or frame_len
         ptr, nbytes, mem, keep = self._frames(frames, frame_len, frame_stride)
         if n_frames is None:
             n_frames = 0 if nbytes < frame_len else 1 + (nbytes - frame_len) // frame_stride
-        hs = (C.c_void_p * len(cascades))(*[(c._h if c is not None else None) for c in cascades])
         info = L.DecodeInfoC()
-        st = L.lib().sspsd_cascade_process_frames(self._h, hs, len(cascades), ptr, n_frames, frame_len,
-                                                  frame_stride, mem, C.byref(loss.c) if loss is not None else None,
-                                                  C.byref(info))
+        lp = C.byref(loss.c) if loss is not None else None
+        if isinstance(target, CsmCascade):
+            st = L.lib().sspsd_csm_process_frames(self._h, target._h, (C.c_uint32 * len(tmap))(*tmap), ptr, n_frames,
+                                                  frame_len, frame_stride, mem, lp, C.byref(info))
+        elif isinstance(target, CsdCascade):
+            st = L.lib().sspsd_csd_process_frames(self._h, target._h, tmap[0], tmap[1], ptr, n_frames, frame_len,
+                                                  frame_stride, mem, lp, C.byref(info))
+        else:
+            hs = (C.c_void_p * len(target))(*[(c._h if c is not None else None) for c in target])
+            st = L.lib().sspsd_cascade_process_frames(self._h, hs, len(target), ptr, n_frames, frame_len,
+                                                      frame_stride, mem, lp, C.byref(info))
         del keep
         if st in (L.EHEADER, L.EFORMAT, L.ESIZE, L.EBATCHES, L.ESHORT) and info.frames_ok < n_frames:
             raise DecodeError(st, info.frames_ok)
@@ -896,15 +922,24 @@ class Receiver:
         buf = (C.c_uint8 * (n.value * slot)).from_address(ptr.value)
         return np.frombuffer(buf, np.uint8).reshape(n.value, slot), ln.value
 
-    def pump(self, decoder, cascades, loss: "Loss" = None, max_frames=1024, timeout_ms=1000):
-        """recv + FrameDecoder.process_frames in one call; returns the decode info (frames_ok == 0 on
-        timeout).  Malformed datagrams raise DecodeError like process_frames."""
-        hs = (C.c_void_p * L.MAX_TRACES)()
-        for t, c in enumerate(cascades[:L.MAX_TRACES]):
-            hs[t] = c._h if c is not None else None
+    def pump(self, decoder, target, loss: "Loss" = None, max_frames=1024, timeout_ms=1000, traces=None):
+        """recv + FrameDecoder.process_frames in one call (`target` and `traces` as there); returns the decode info
+        (frames_ok == 0 on timeout).  Malformed datagrams raise DecodeError like process_frames."""
+        tmap = _trace_map(target, traces)
         info = L.DecodeInfoC()
-        st = L.lib().sspsd_receiver_pump(self._h, decoder._h, hs, min(len(cascades), L.MAX_TRACES), max_frames,
-                                         timeout_ms, C.byref(loss.c) if loss is not None else None, C.byref(info))
+        lp = C.byref(loss.c) if loss is not None else None
+        if isinstance(target, CsmCascade):
+            st = L.lib().sspsd_receiver_pump_csm(self._h, decoder._h, target._h, (C.c_uint32 * len(tmap))(*tmap),
+                                                 max_frames, timeout_ms, lp, C.byref(info))
+        elif isinstance(target, CsdCascade):
+            st = L.lib().sspsd_receiver_pump_csd(self._h, decoder._h, target._h, tmap[0], tmap[1], max_frames,
+                                                 timeout_ms, lp, C.byref(info))
+        else:
+            hs = (C.c_void_p * L.MAX_TRACES)()
+            for t, c in enumerate(target[:L.MAX_TRACES]):
+                hs[t] = c._h if c is not None else None
+            st = L.lib().sspsd_receiver_pump(self._h, decoder._h, hs, min(len(target), L.MAX_TRACES), max_frames,
+                                             timeout_ms, lp, C.byref(info))
         if L.EHEADER <= st <= L.ESHORT:
             raise DecodeError(st, info.frames_ok)
         L.check(st)

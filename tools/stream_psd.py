@@ -12,6 +12,10 @@ Sources (reference src/source.rs:16-48, 102-167):
   --dsm FTW           MASH-1-1-1 modulated sine marker generated on the device (source.rs:119-130)
 --repeat wraps files around; the run ends after --samples items per trace (files: at EOF without --repeat).
 Host reads go through a pinned double buffer, so the H2D copy of block b+1 overlaps the kernels of block b.
+
+--csm TRACES (with --file or --udp), e.g. 0,2 or 0,1,2,3: feed the listed traces of the frames to one CsmCascade
+instead of one PsdCascade per trace, and report the diagonal PSD of --trace (one of TRACES, default the first) plus
+the median coherence of every pair; --save FILE.npz writes the matrix S [K, K, bins], the frequencies and the breaks.
 """
 import argparse
 import json
@@ -23,8 +27,37 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
-from stabilizer_stream_b200 import (Break, Detrend, FrameDecoder, Loss, MergeOpts, PsdCascade, Receiver, Source,
-                                    Var)  # noqa: E402
+from stabilizer_stream_b200 import (Break, CsmCascade, Detrend, FrameDecoder, Loss, MergeOpts, PsdCascade, Receiver,
+                                    Source, Var)  # noqa: E402
+
+BREAK_FIELDS = ("start", "include", "count", "avg", "bins_start", "bins_end", "fft_size", "decimation", "pending",
+                "processed")
+
+
+def break_row(k):
+    return [k.start, k.include, k.count, k.avg, k.bins.start, k.bins.stop, k.fft_size, k.decimation, k.pending,
+            k.processed]
+
+
+def parse_csm(ap, a):
+    """--csm / --trace / --save checks, before any device work: -> the trace list or None"""
+    if a.csm is None:
+        if a.save:
+            ap.error("--save needs --csm")
+        return None
+    try:
+        traces = [int(t) for t in a.csm.split(",")]
+    except ValueError:
+        ap.error("--csm takes comma-separated trace indices, e.g. 0,2")
+    if not 2 <= len(traces) <= 4:
+        ap.error("--csm takes 2 to 4 trace indices (a CsmCascade has at most 4 channels)")
+    if any(not 0 <= t < 4 for t in traces):
+        ap.error("--csm trace indices are 0 .. 3")
+    if not (a.file or a.udp):
+        ap.error("--csm needs --file or --udp (frames carry the traces)")
+    if a.trace is not None and a.trace not in traces:
+        ap.error("--trace must be one of the --csm traces")
+    return traces
 
 
 def main():
@@ -39,10 +72,15 @@ def main():
     ap.add_argument("--samples", type=float, default=0, help="stop after this many items per trace (0: until EOF)")
     ap.add_argument("--fft", type=int, default=512, help="FFT size N (the reference binaries use 512)")
     ap.add_argument("--detrend", default="midpoint", choices=["none", "midpoint", "span", "mean"])
-    ap.add_argument("--trace", type=int, default=0)
+    ap.add_argument("--trace", type=int, default=None, help="trace to report (default 0; with --csm the first of TRACES)")
+    ap.add_argument("--csm", metavar="TRACES", help="comma-separated traces (2 to 4) into one CsmCascade")
+    ap.add_argument("--save", metavar="FILE.npz", help="with --csm: write S, the frequencies and the breaks")
     ap.add_argument("--block", type=int, default=1 << 24, help="items (or frames*64) read per block")
     ap.add_argument("--json", action="store_true")
     a = ap.parse_args()
+    csm_traces = parse_csm(ap, a)
+    if a.trace is None:
+        a.trace = csm_traces[0] if csm_traces else 0
     dev = torch.device("cuda", 0)
     det = Detrend[a.detrend.upper()]
     limit = int(a.samples)
@@ -51,10 +89,19 @@ def main():
     t0 = time.perf_counter()
 
     def cascades(n):
+        if csm_traces:
+            if not cas:
+                m = CsmCascade(a.fft, len(csm_traces))
+                m.set_detrend(det)
+                cas.append(m)
+            return
         while len(cas) < n:
             c = PsdCascade(a.fft)
             c.set_detrend(det)
             cas.append(c)
+
+    def target():
+        return cas[0] if csm_traces else cas
 
     if a.noise is not None or a.dsm is not None:
         cascades(1)
@@ -101,7 +148,7 @@ def main():
                         continue
                     break
                 cascades(4)
-                info = dec.process_frames(cas, data[:nfr * a.frame_size], a.frame_size, loss)
+                info = dec.process_frames(target(), data[:nfr * a.frame_size], a.frame_size, loss, traces=csm_traces)
                 if not names:
                     from stabilizer_stream_b200.psd import TRACE_NAMES, Format
                     names = list(TRACE_NAMES[Format(info.format)])
@@ -114,7 +161,7 @@ def main():
         dec = FrameDecoder()
         cascades(4)
         while True:
-            info = rx.pump(dec, cas, loss, max_frames=1024, timeout_ms=1000)
+            info = rx.pump(dec, target(), loss, max_frames=1024, timeout_ms=1000, traces=csm_traces)
             if info.frames_ok == 0:
                 break
             if not names:
@@ -126,9 +173,25 @@ def main():
     else:
         ap.error("one of --raw, --file, --udp, --noise, --dsm is required")
 
-    c = cas[min(a.trace, len(cas) - 1)]
-    y, b = c.psd(MergeOpts())
-    dt = time.perf_counter() - t0
+    coherence = []
+    if csm_traces:
+        S, b = cas[0].csm(MergeOpts())
+        dt = time.perf_counter() - t0
+        y = np.real(S[csm_traces.index(a.trace), csm_traces.index(a.trace)]).astype(np.float32)
+        coh = CsmCascade.coherence(S)
+        k = len(csm_traces)
+        for i in range(k):
+            for j in range(i + 1, k):
+                coherence.append({"traces": [csm_traces[i], csm_traces[j]],
+                                  "median": float(np.median(coh[i, j])) if coh.shape[-1] else None})
+        if a.save:
+            np.savez(a.save, S=S, frequencies=Break.frequencies(b), traces=np.array(csm_traces),
+                     breaks=np.array([break_row(k_) for k_ in b], np.uint64).reshape(-1, len(BREAK_FIELDS)),
+                     break_fields=np.array(BREAK_FIELDS))
+    else:
+        c = cas[min(a.trace, len(cas) - 1)]
+        y, b = c.psd(MergeOpts())
+        dt = time.perf_counter() - t0
     f = Break.frequencies(b)
     fdev = []
     if b:
@@ -138,17 +201,23 @@ def main():
             fdev.append((tau, float(np.sqrt(max(var.eval(y, f, tau), 0.0)))))
             tau *= 2.0
     out = {"trace": names[min(a.trace, len(names) - 1)] if names else None, "items_per_trace": int(total),
-           "traces": len(cas), "seconds": dt, "MSps_per_trace": total / dt / 1e6,
+           "traces": len(csm_traces) if csm_traces else len(cas), "seconds": dt, "MSps_per_trace": total / dt / 1e6,
            "breaks": [{"start": k.start, "count": k.count, "bins": [k.bins.start, k.bins.stop], "decimation": k.decimation,
                        "pending": k.pending, "processed": k.processed, "include": k.include} for k in b],
            "psd_bins": int(y.size), "psd_median": float(np.median(y)) if y.size else None,
            "fdev": fdev[:8], "loss": {"received": loss.received, "dropped": loss.dropped}}
+    if csm_traces:
+        out["csm"] = {"traces": csm_traces, "coherence": coherence}
     if a.json:
         print(json.dumps(out))
     else:
         print("breaks:", out["breaks"])
         print("psd: %d bins, median %.6g" % (out["psd_bins"], out["psd_median"] or 0))
         print("fdev:", out["fdev"])
+        for c_ in coherence:
+            i, j = c_["traces"]
+            print("coherence %s / %s: median %.4g over %d bins" % (names[i] if names else i, names[j] if names else j,
+                                                                 c_["median"] or 0, y.size))
         if loss.received:
             print("Loss: %g %% (%d of %d)" % (100 * loss.ratio(), loss.dropped, loss.received + loss.dropped))
         print("%.1f MS/s per trace over %.2f s" % (out["MSps_per_trace"], dt))
