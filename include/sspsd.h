@@ -229,6 +229,54 @@ int32_t sspsd_csm_stream(const sspsd_csm *h, void **stream);
 int32_t sspsd_csm_flush(sspsd_csm *h);
 int32_t sspsd_csm_sync(sspsd_csm *h);
 
+/* ---------------------------------------------------------------------------------------------
+ * Two-sided spectrum of a complex stream z (DESIGN.md 3c), in one of two modes fixed at creation:
+ *   SSPSD_ZOOM_IQ          z[n] = i[n] + i q[n] of two real streams (a lock-in's BI / BQ); ftw must be 0
+ *   SSPSD_ZOOM_HETERODYNE  z[n] = x[n] exp(-2 pi i phi_n / 2^32), phi_n = (n ftw) mod 2^32, of one real stream:
+ *                          x mixed down by the carrier f0 = ftw / 2^32 (in units of the sample rate; the DDS /
+ *                          lock-in convention of sspsd_source's dsm), n the absolute sample index since create or
+ *                          reset (integer arithmetic: exact over any stream length, independent of the call split)
+ * z goes through the cascade of sspsd_cascade_* with its real and imaginary parts in lockstep (same segments,
+ * window, EWMA weights, detrend of each part, half-band decimators), and every stage accumulates
+ *   P+[k] = sum w |Z[k]|^2,  P-[k] = sum w |Z[N-k]|^2,  k = 0 .. N/2   (P-[0] = P+[0], P-[N/2] = P+[N/2]).
+ * The readout has the breaks of sspsd_cascade_psd with the same options; each row is scaled by
+ * 1 / (2 gain_i 8^i), the two-sided density: a real x fed as (x, 0) reads back about psd(x) / 2 on each side.
+ * p_pos[j] is the density at f0 + f_j and p_neg[j] at f0 - f_j, f_j of sspsd_break_frequencies (f0 = 0 in I/Q
+ * mode).  Limits as sspsd_csd_*: n_fft = 64 .. 4096 (else SSPSD_EINVAL), Hann or rectangular window, Linear
+ * detrend SSPSD_EUNIMPLEMENTED.  SSPSD_MEM_DEVICE input follows the rule of sspsd_cascade_process_f32, on the
+ * handle's stream (sspsd_zoom_stream).
+ * --------------------------------------------------------------------------------------------- */
+typedef struct sspsd_zoom sspsd_zoom;
+enum { SSPSD_ZOOM_IQ = 0, SSPSD_ZOOM_HETERODYNE = 1 };
+/* an unknown mode, or ftw != 0 in I/Q mode: SSPSD_EINVAL */
+int32_t sspsd_zoom_create(const sspsd_config *cfg, int32_t mode, uint32_t ftw, sspsd_zoom **out);
+void sspsd_zoom_destroy(sspsd_zoom *h);
+/* deep copy, the mixer's sample position included */
+int32_t sspsd_zoom_clone(sspsd_zoom *h, sspsd_zoom **out);
+/* back to no samples: the mixer's position restarts at 0, the carrier is kept */
+int32_t sspsd_zoom_reset(sspsd_zoom *h);
+/* the next n samples of i and q (I/Q mode; in heterodyne mode SSPSD_EINVAL with nothing consumed) */
+int32_t sspsd_zoom_process_iq_f32(sspsd_zoom *h, const float *i, const float *q, size_t n, int32_t mem);
+/* the next n samples of x (heterodyne mode; in I/Q mode SSPSD_EINVAL with nothing consumed) */
+int32_t sspsd_zoom_process_f32(sspsd_zoom *h, const float *x, size_t n, int32_t mem);
+int32_t sspsd_zoom_set_avg(sspsd_zoom *h, sspsd_avg_opts avg);
+int32_t sspsd_zoom_set_detrend(sspsd_zoom *h, int32_t detrend);
+int32_t sspsd_zoom_rbw(const sspsd_zoom *h, float *rbw);
+/* p_pos, p_neg: *p_len floats each; capacity and SSPSD_ESHORT as sspsd_csd_read */
+int32_t sspsd_zoom_read(sspsd_zoom *h, const sspsd_merge_opts *opts, float *p_pos, float *p_neg, size_t *p_len,
+                        sspsd_break *b, size_t *b_len);
+int32_t sspsd_zoom_carrier(const sspsd_zoom *h, int32_t *mode, uint32_t *ftw);
+int32_t sspsd_zoom_num_stages(sspsd_zoom *h, uint32_t *n);
+int32_t sspsd_zoom_stream(const sspsd_zoom *h, void **stream);
+int32_t sspsd_zoom_flush(sspsd_zoom *h);
+int32_t sspsd_zoom_sync(sspsd_zoom *h);
+/* The mixer of heterodyne mode on its own, asynchronously on `stream`, all pointers device memory:
+ *   i_out[k] = x[k] cos(2 pi phi / 2^32),  q_out[k] = -x[k] sin(2 pi phi / 2^32),  phi = ((pos0 + k) ftw) mod 2^32.
+ * Every output is within 2^-23 |x[k]| of the float64 product; at multiples of a quarter turn the factors are
+ * exactly 0 and +-1. */
+int32_t sspsd_heterodyne_f32(void *stream, const float *x, size_t n, uint64_t pos0, uint32_t ftw, float *i_out,
+                             float *q_out);
+
 /* Break::frequencies(&[Break]) -> Vec<f32>, src/psd.rs:315-327 (pure host helper) */
 int32_t sspsd_break_frequencies(const sspsd_break *b, size_t n_breaks, float *f, size_t *f_len);
 
@@ -464,6 +512,11 @@ int32_t sspsd_cascade_process_frames(sspsd_decoder *d, sspsd_cascade *const *cas
 int32_t sspsd_csm_process_frames(sspsd_decoder *d, sspsd_csm *m, const uint32_t *traces, const uint8_t *frames,
                                  size_t n_frames, size_t frame_len, size_t frame_stride, int32_t frames_mem,
                                  sspsd_loss *loss, sspsd_decode_info *info);
+/* the same into a zoom handle: I/Q mode i <- traces[0], q <- traces[1] (Fls: BI, BQ are traces 2, 3); heterodyne
+ * mode x <- traces[0], mixed on the device before it is fed.  traces == NULL: 0 (and 1). */
+int32_t sspsd_zoom_process_frames(sspsd_decoder *d, sspsd_zoom *z, const uint32_t *traces, const uint8_t *frames,
+                                  size_t n_frames, size_t frame_len, size_t frame_stride, int32_t frames_mem,
+                                  sspsd_loss *loss, sspsd_decode_info *info);
 /* the same into a cross-spectral density: x <- trace trace_x, y <- trace trace_y */
 int32_t sspsd_csd_process_frames(sspsd_decoder *d, sspsd_csd *c, uint32_t trace_x, uint32_t trace_y,
                                  const uint8_t *frames, size_t n_frames, size_t frame_len, size_t frame_stride,
@@ -537,6 +590,9 @@ int32_t sspsd_receiver_pump_csm(sspsd_receiver *r, sspsd_decoder *d, sspsd_csm *
                                 uint32_t max_frames, int32_t timeout_ms, sspsd_loss *loss, sspsd_decode_info *info);
 int32_t sspsd_receiver_pump_csd(sspsd_receiver *r, sspsd_decoder *d, sspsd_csd *c, uint32_t trace_x, uint32_t trace_y,
                                 uint32_t max_frames, int32_t timeout_ms, sspsd_loss *loss, sspsd_decode_info *info);
+/* recv + sspsd_zoom_process_frames, with the checks of sspsd_receiver_pump_csm */
+int32_t sspsd_receiver_pump_zoom(sspsd_receiver *r, sspsd_decoder *d, sspsd_zoom *z, const uint32_t *traces,
+                                 uint32_t max_frames, int32_t timeout_ms, sspsd_loss *loss, sspsd_decode_info *info);
 
 /* ---------------------------------------------------------------------------------------------
  * Var::eval (AVAR/MVAR/FVAR from a phase PSD), src/var.rs:26-45 -- host helper on psd() output

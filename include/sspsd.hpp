@@ -228,6 +228,114 @@ private:
     sspsd_csd* h_ = nullptr;
 };
 
+/// Two-sided cascaded spectrum of a complex stream (sspsd_zoom_* in sspsd.h), N = 64 .. 4096: I/Q streams as they are
+/// (ZoomCascade::iq()), or one real stream mixed down by the carrier ftw / 2^32 (ZoomCascade::heterodyne(ftw)).
+/// p_pos[j] is the density at f0 + f_j and p_neg[j] at f0 - f_j, f_j of Break::frequencies.
+template <size_t N>
+class ZoomCascade {
+public:
+    struct Spectra {
+        std::vector<float> p_pos, p_neg;
+        std::vector<Break> breaks;
+    };
+    static ZoomCascade iq(int device = 0, void* stream = nullptr, int32_t hbf = SSPSD_HBF_140, Window w = Window::Hann)
+    {
+        return ZoomCascade(SSPSD_ZOOM_IQ, 0, device, stream, hbf, w);
+    }
+    static ZoomCascade heterodyne(uint32_t ftw, int device = 0, void* stream = nullptr, int32_t hbf = SSPSD_HBF_140,
+                                  Window w = Window::Hann)
+    {
+        return ZoomCascade(SSPSD_ZOOM_HETERODYNE, ftw, device, stream, hbf, w);
+    }
+    ZoomCascade(int32_t mode, uint32_t ftw, int device = 0, void* stream = nullptr, int32_t hbf = SSPSD_HBF_140,
+                Window w = Window::Hann)
+    {
+        sspsd_config cfg;
+        check(sspsd_config_default((uint32_t)N, &cfg));
+        cfg.device = device;
+        cfg.stream = stream;
+        cfg.hbf = hbf;
+        cfg.window = (int32_t)w;
+        check(sspsd_zoom_create(&cfg, mode, ftw, &h_));
+    }
+    ZoomCascade(const ZoomCascade& o) { check(sspsd_zoom_clone(o.h_, &h_)); }
+    ZoomCascade& operator=(const ZoomCascade& o)
+    {
+        if (this != &o) {
+            sspsd_zoom* n = nullptr;
+            check(sspsd_zoom_clone(o.h_, &n));
+            sspsd_zoom_destroy(h_);
+            h_ = n;
+        }
+        return *this;
+    }
+    ZoomCascade(ZoomCascade&& o) noexcept : h_(o.h_) { o.h_ = nullptr; }
+    ~ZoomCascade() { sspsd_zoom_destroy(h_); }
+
+    float rbw() const
+    {
+        float r;
+        check(sspsd_zoom_rbw(h_, &r));
+        return r;
+    }
+    /// (mode, ftw)
+    std::pair<int32_t, uint32_t> carrier() const
+    {
+        int32_t m;
+        uint32_t f;
+        check(sspsd_zoom_carrier(h_, &m, &f));
+        return {m, f};
+    }
+    void set_avg(AvgOpts a) { check(sspsd_zoom_set_avg(h_, sspsd_avg_opts{a.limit, a.count})); }
+    void set_detrend(Detrend d) { check(sspsd_zoom_set_detrend(h_, (int32_t)d)); }
+    /// I/Q mode
+    void process(const float* i, const float* q, size_t n, Mem mem = Mem::Host)
+    {
+        check(sspsd_zoom_process_iq_f32(h_, i, q, n, (int32_t)mem));
+    }
+    void process(const std::vector<float>& i, const std::vector<float>& q)
+    {
+        if (i.size() != q.size()) throw Error(SSPSD_EINVAL, "i and q must have the same length");
+        process(i.data(), q.data(), i.size());
+    }
+    /// heterodyne mode
+    void process(const float* x, size_t n, Mem mem = Mem::Host) { check(sspsd_zoom_process_f32(h_, x, n, (int32_t)mem)); }
+    void process(const std::vector<float>& x) { process(x.data(), x.size()); }
+    Spectra spectrum(const MergeOpts& o = MergeOpts()) const
+    {
+        sspsd_merge_opts mo{o.keep_overlap, o.min_count, o.keep_transition_band};
+        Spectra s;
+        const size_t cap = SSPSD_MAX_STAGES * (N / 2 + 1);
+        s.p_pos.resize(cap);
+        s.p_neg.resize(cap);
+        sspsd_break cb[SSPSD_MAX_STAGES];
+        size_t pl = cap, bl = SSPSD_MAX_STAGES;
+        check(sspsd_zoom_read(h_, &mo, s.p_pos.data(), s.p_neg.data(), &pl, cb, &bl));
+        s.p_pos.resize(pl);
+        s.p_neg.resize(pl);
+        for (size_t i = 0; i < bl; ++i)
+            s.breaks.push_back(Break{(size_t)cb[i].start, cb[i].include != 0, cb[i].count, cb[i].avg,
+                                     {(size_t)cb[i].bins_start, (size_t)cb[i].bins_end}, (size_t)cb[i].fft_size,
+                                     (size_t)cb[i].decimation, (size_t)cb[i].pending, (size_t)cb[i].processed});
+        return s;
+    }
+    uint32_t num_stages() const
+    {
+        uint32_t n;
+        check(sspsd_zoom_num_stages(h_, &n));
+        return n;
+    }
+    /// traces the frame entry points read: two in I/Q mode, one in heterodyne mode
+    int traces() const { return carrier().first == SSPSD_ZOOM_IQ ? 2 : 1; }
+    void reset() { check(sspsd_zoom_reset(h_)); }
+    void flush() { check(sspsd_zoom_flush(h_)); }
+    void sync() { check(sspsd_zoom_sync(h_)); }
+    sspsd_zoom* handle() const { return h_; }
+
+private:
+    sspsd_zoom* h_ = nullptr;
+};
+
 /// Cascaded cross-spectral matrix of K = 2 .. 4 streams (sspsd_csm_* in sspsd.h), N = 64 .. 4096.  s(i, j) accumulates
 /// conj(X_i) X_j: s(0, 1) is CsdCascade's pxy of (x0, x1), and s(i, i) what a PsdCascade<N> fed x_i alone returns.
 template <size_t N>
@@ -457,8 +565,29 @@ public:
                                               loss ? &loss->c : nullptr, &info);
         return finish(st, info);
     }
+    /// fused decode -> two-sided spectrum: I/Q mode i, q <- traces[0], traces[1]; heterodyne mode x <- traces[0],
+    /// mixed on the device (empty: 0 .. 1 / 0)
+    template <size_t N>
+    sspsd_decode_info process_frames(ZoomCascade<N>& z, const std::vector<uint32_t>& traces, const uint8_t* frames,
+                                     size_t n_frames, size_t frame_len, Loss* loss, Mem mem = Mem::Host,
+                                     size_t frame_stride = 0)
+    {
+        sspsd_decode_info info{};
+        int32_t st = sspsd_zoom_process_frames(d_, z.handle(), trace_map(z, traces), frames, n_frames, frame_len,
+                                               frame_stride ? frame_stride : frame_len, (int32_t)mem,
+                                               loss ? &loss->c : nullptr, &info);
+        return finish(st, info);
+    }
     sspsd_decoder* handle() const { return d_; }
 
+    /// the C ABI's view of a ZoomCascade trace map (NULL for the identity); throws unless one index per trace read
+    template <size_t N>
+    static const uint32_t* trace_map(const ZoomCascade<N>& z, const std::vector<uint32_t>& traces)
+    {
+        if (traces.empty()) return nullptr;
+        if (traces.size() != (size_t)z.traces()) throw Error(SSPSD_EINVAL, "one trace index per stream of the mode");
+        return traces.data();
+    }
     /// the C ABI's view of a CsmCascade trace map (NULL for the identity); throws unless one index per channel
     template <size_t N>
     static const uint32_t* trace_map(const CsmCascade<N>& m, const std::vector<uint32_t>& traces)
@@ -567,6 +696,16 @@ public:
         sspsd_decode_info info{};
         int32_t st = sspsd_receiver_pump_csm(h_, d.handle(), m.handle(), FrameDecoder::trace_map(m, traces), max_frames,
                                              timeout_ms, loss ? &loss->c : nullptr, &info);
+        return FrameDecoder::finish(st, info);
+    }
+    /// recv + FrameDecoder::process_frames into a ZoomCascade (info.frames_ok == 0 on timeout)
+    template <size_t N>
+    sspsd_decode_info pump(FrameDecoder& d, ZoomCascade<N>& z, const std::vector<uint32_t>& traces, Loss* loss,
+                           uint32_t max_frames = 1024, int32_t timeout_ms = 1000)
+    {
+        sspsd_decode_info info{};
+        int32_t st = sspsd_receiver_pump_zoom(h_, d.handle(), z.handle(), FrameDecoder::trace_map(z, traces),
+                                              max_frames, timeout_ms, loss ? &loss->c : nullptr, &info);
         return FrameDecoder::finish(st, info);
     }
     sspsd_receiver* handle() const { return h_; }

@@ -13,6 +13,7 @@ LIB_PATH = os.environ.get("SSPSD_LIB") or os.path.join(_HERE, "libsspsd.so")
 
 OK, EINVAL, EUNIMPLEMENTED, ECUDA, ENOMEM, EHEADER, EFORMAT, ESIZE, EBATCHES, ESHORT, ENCCL, EIO = range(12)
 MEM_HOST, MEM_DEVICE = 0, 1
+ZOOM_IQ, ZOOM_HETERODYNE = 0, 1
 FLAG_DETERMINISTIC = 1
 MAX_STAGES = 16
 MAX_TRACES = 4
@@ -127,6 +128,22 @@ PROTOTYPES = {
     "sspsd_csm_stream": (_i32, [_vp, C.POINTER(_vp)]),
     "sspsd_csm_flush": (_i32, [_vp]),
     "sspsd_csm_sync": (_i32, [_vp]),
+    "sspsd_zoom_create": (_i32, [C.POINTER(Config), _i32, C.c_uint32, C.POINTER(_vp)]),
+    "sspsd_zoom_destroy": (None, [_vp]),
+    "sspsd_zoom_clone": (_i32, [_vp, C.POINTER(_vp)]),
+    "sspsd_zoom_reset": (_i32, [_vp]),
+    "sspsd_zoom_process_iq_f32": (_i32, [_vp, _vp, _vp, _sz, _i32]),
+    "sspsd_zoom_process_f32": (_i32, [_vp, _vp, _sz, _i32]),
+    "sspsd_zoom_set_avg": (_i32, [_vp, AvgOptsC]),
+    "sspsd_zoom_set_detrend": (_i32, [_vp, _i32]),
+    "sspsd_zoom_rbw": (_i32, [_vp, C.POINTER(C.c_float)]),
+    "sspsd_zoom_read": (_i32, [_vp, C.POINTER(MergeOptsC), _vp, _vp, _psz, C.POINTER(BreakC), _psz]),
+    "sspsd_zoom_carrier": (_i32, [_vp, C.POINTER(_i32), C.POINTER(C.c_uint32)]),
+    "sspsd_zoom_num_stages": (_i32, [_vp, C.POINTER(C.c_uint32)]),
+    "sspsd_zoom_stream": (_i32, [_vp, C.POINTER(_vp)]),
+    "sspsd_zoom_flush": (_i32, [_vp]),
+    "sspsd_zoom_sync": (_i32, [_vp]),
+    "sspsd_heterodyne_f32": (_i32, [_vp, _vp, _sz, C.c_uint64, C.c_uint32, _vp, _vp]),
     "sspsd_cascade_partials": (_i32, [_vp, C.POINTER(PartialsC)]),
     "sspsd_cascade_set_counts": (_i32, [_vp, C.POINTER(C.c_uint64), C.c_uint32]),
     "sspsd_cascade_seek": (_i32, [_vp, C.c_uint64]),
@@ -157,6 +174,8 @@ PROTOTYPES = {
                                         C.POINTER(DecodeInfoC)]),
     "sspsd_csd_process_frames": (_i32, [_vp, _vp, C.c_uint32, C.c_uint32, _vp, _sz, _sz, _sz, _i32, C.POINTER(LossC),
                                         C.POINTER(DecodeInfoC)]),
+    "sspsd_zoom_process_frames": (_i32, [_vp, _vp, C.POINTER(C.c_uint32), _vp, _sz, _sz, _sz, _i32,
+                                         C.POINTER(LossC), C.POINTER(DecodeInfoC)]),
     "sspsd_loss_update": (None, [C.POINTER(LossC), C.c_uint32, C.c_uint8]),
     "sspsd_loss_ratio": (C.c_float, [C.POINTER(LossC)]),
     "sspsd_var_eval": (C.c_float, [C.POINTER(VarC), _vp, _vp, _sz, C.c_float]),
@@ -200,6 +219,8 @@ PROTOTYPES = {
                                        C.POINTER(DecodeInfoC)]),
     "sspsd_receiver_pump_csd": (_i32, [_vp, _vp, _vp, C.c_uint32, C.c_uint32, C.c_uint32, _i32, C.POINTER(LossC),
                                        C.POINTER(DecodeInfoC)]),
+    "sspsd_receiver_pump_zoom": (_i32, [_vp, _vp, _vp, C.POINTER(C.c_uint32), C.c_uint32, _i32, C.POINTER(LossC),
+                                        C.POINTER(DecodeInfoC)]),
 }
 
 _lib = None

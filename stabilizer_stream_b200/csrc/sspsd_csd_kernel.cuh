@@ -2,6 +2,8 @@
 // two-channel cascade (XCascade).  For every segment s of the launch it adds, per bin k = 0 .. N/2,
 //   Sxx[k] += w_s |X_s[k]|^2,  Syy[k] += w_s |Y_s[k]|^2,  Sxy[k] += w_s conj(X_s[k]) Y_s[k]
 // (scipy.signal.csd's convention: H = Sxy / Sxx for y = h * x), with the PSD kernel's weights w_s.
+// iq_stage_kernel shares the body (pair_stage) up to the per-bin epilogue and adds instead the two sides of the
+// spectrum of z = x + i y itself: P+[k] += w_s |Z_s[k]|^2, P-[k] += w_s |Z_s[N-k]|^2 (DESIGN.md 3c).
 //
 // Two-for-one transform: z[n] = x~[n] + i y~[n] (both channels detrended on their own, same window) is
 // transformed by ONE N-point complex FFT, and
@@ -11,7 +13,7 @@
 //
 // Structure as psd_stage_kernel: a persistent CTA walks a contiguous range of tiles; a tile holds T
 // consecutive hops (+ overlap) of BOTH channels, each brought in by TMA bulk copies from its own StreamSrc
-// (one mbarrier per buffer with two arrivals, one per channel); the four rows accumulate in registers over
+// (one mbarrier per buffer with two arrivals, one per channel); the epilogue's rows accumulate in registers over
 // the CTA's whole range and are flushed with one atomicAdd (or one partial-row store) per value.
 #pragma once
 #include "sspsd_stage_kernel.cuh"
@@ -169,9 +171,34 @@ __device__ __forceinline__ void pair_flush(const float (&acc)[5][ROWS], int j, i
     }
 }
 
-template <int LOG2N>
-__global__ void __launch_bounds__(Plan<LOG2N + 1>::NT, Plan<LOG2N + 1>::NT <= 256 ? 2 : 1)
-csd_stage_kernel(const XStageParams p)
+// The per-bin epilogues of pair_stage: what one owned bin's Z[k] and Z[N-k] add to the thread's ROWS accumulators.
+// CsdEpi: the two-for-one split into Sxx, Syy, Re Sxy, Im Sxy (csd_stage_kernel).
+struct CsdEpi {
+    static constexpr int ROWS = CSD_ROWS;
+    static __device__ __forceinline__ void bin(float2 zk, float2 zm, float wseg, float (&a)[ROWS])
+    {
+        csd_bin(zk, zm, wseg, a);
+    }
+};
+
+// IqEpi: the two sides of the spectrum of z itself, P+ = |Z[k]|^2 and P- = |Z[N-k]|^2 (iq_stage_kernel).  wseg
+// carries ewma_weight's 0.25 of the split, which has no place here: 4 wseg is the weight, exactly (a power of two).
+enum { IQ_ROWS = 2 };
+struct IqEpi {
+    static constexpr int ROWS = IQ_ROWS;
+    static __device__ __forceinline__ void bin(float2 zk, float2 zm, float wseg, float (&a)[ROWS])
+    {
+        const float w = 4.0f * wseg;
+        a[0] = fmaf(w, fmaf(zk.y, zk.y, zk.x * zk.x), a[0]);
+        a[1] = fmaf(w, fmaf(zm.y, zm.y, zm.x * zm.x), a[1]);
+    }
+};
+
+// The body of both pair kernels: tiles of both channels, two-for-one transform of z = x + i y, EPI per owned bin,
+// flush of EPI::ROWS rows.  tid is threadIdx.x read in the kernel, where the compiler knows its range from the launch
+// bounds (csd_stage_kernel then compiles exactly as it did before the body was shared).
+template <int LOG2N, class EPI>
+__device__ __forceinline__ void pair_stage(const XStageParams& p, const int tid)
 {
     using PL = Plan<LOG2N + 1>;
     constexpr int N = PL::M, TPS = PL::TPS, NT = PL::NT, G = PL::G, K = PL::K, WS = PL::WS;
@@ -183,7 +210,6 @@ csd_stage_kernel(const XStageParams p)
     float* red = wgt + ((p.T + 3) & ~3);
     uint64_t* bars = reinterpret_cast<uint64_t*>(red + ((2 * G * WPG + 1) & ~1));
 
-    const int tid = threadIdx.x;
     const int group = tid / TPS;
     const int j = tid % TPS;
     const int hop = p.hop;
@@ -226,11 +252,11 @@ csd_stage_kernel(const XStageParams p)
 
     float* wre = wsb + group * 2 * WS;
     float* wim = wre + WS;
-    float acc[5][4];  // [owned_bins][Sxx, Syy, Re Sxy, Im Sxy]
+    float acc[5][EPI::ROWS];  // [owned_bins][EPI's rows]
 #pragma unroll
     for (int b = 0; b < 5; ++b)
 #pragma unroll
-        for (int r = 0; r < 4; ++r) acc[b][r] = 0.f;
+        for (int r = 0; r < EPI::ROWS; ++r) acc[b][r] = 0.f;
 
     for (int tl = tile0; tl < tile1; ++tl) {
     const int buf = (tl - tile0) & 1;
@@ -256,7 +282,7 @@ csd_stage_kernel(const XStageParams p)
 
         mid_passes<LOG2N + 1, 1>(wre, wim, j, group, tw);
 
-        // ---- last pass (radix 4 on contiguous points) + two-for-one split + cross products ----
+        // ---- last pass (radix 4 on contiguous points) + the epilogue of the owned bins ----
         float4 ar = *reinterpret_cast<const float4*>(wre + posA);
         float4 ai = *reinterpret_cast<const float4*>(wim + posA);
         float4 br = *reinterpret_cast<const float4*>(wre + posB);
@@ -268,16 +294,16 @@ csd_stage_kernel(const XStageParams p)
         dft4_planes(ar, ai, za);  // Z[kA + K t]
         dft4_planes(br, bi, zb);  // Z[N - kA - K (3 - t)]  (j == 0: Z[K/2 + K t])
         if (j != 0) {
-            csd_bin(za[0], zb[3], wseg, acc[0]);  // bin kA
-            csd_bin(za[1], zb[2], wseg, acc[1]);  // bin kA + K
-            csd_bin(zb[1], za[2], wseg, acc[2]);  // bin 2K - kA
-            csd_bin(zb[0], za[3], wseg, acc[3]);  // bin K - kA
+            EPI::bin(za[0], zb[3], wseg, acc[0]);  // bin kA
+            EPI::bin(za[1], zb[2], wseg, acc[1]);  // bin kA + K
+            EPI::bin(zb[1], za[2], wseg, acc[2]);  // bin 2K - kA
+            EPI::bin(zb[0], za[3], wseg, acc[3]);  // bin K - kA
         } else {
-            csd_bin(za[0], za[0], wseg, acc[0]);  // bin 0
-            csd_bin(za[1], za[3], wseg, acc[1]);  // bin K
-            csd_bin(za[2], za[2], wseg, acc[2]);  // bin 2K = N/2
-            csd_bin(zb[0], zb[3], wseg, acc[3]);  // bin K/2
-            csd_bin(zb[1], zb[2], wseg, acc[4]);  // bin 3K/2
+            EPI::bin(za[0], za[0], wseg, acc[0]);  // bin 0
+            EPI::bin(za[1], za[3], wseg, acc[1]);  // bin K
+            EPI::bin(za[2], za[2], wseg, acc[2]);  // bin 2K = N/2
+            EPI::bin(zb[0], zb[3], wseg, acc[3]);  // bin K/2
+            EPI::bin(zb[1], zb[2], wseg, acc[4]);  // bin 3K/2
         }
     }
 
@@ -286,6 +312,22 @@ csd_stage_kernel(const XStageParams p)
     }  // tiles
 
     pair_flush<LOG2N>(acc, j, kA, acc_sink(nullptr, p.acc, p.part, p.part_stride, blockIdx.x * G + group), p.stride);
+}
+
+template <int LOG2N>
+__global__ void __launch_bounds__(Plan<LOG2N + 1>::NT, Plan<LOG2N + 1>::NT <= 256 ? 2 : 1)
+csd_stage_kernel(const XStageParams p)
+{
+    pair_stage<LOG2N, CsdEpi>(p, threadIdx.x);
+}
+
+// The two-sided spectrum of z = x + i y (XCascade's I/Q kind): P+[k] += w |Z[k]|^2, P-[k] += w |Z[N-k]|^2 for
+// k = 0 .. N/2, csd_stage_kernel's transform, tiles, launch shape and shared memory (csd_smem_bytes).
+template <int LOG2N>
+__global__ void __launch_bounds__(Plan<LOG2N + 1>::NT, Plan<LOG2N + 1>::NT <= 256 ? 2 : 1)
+iq_stage_kernel(const XStageParams p)
+{
+    pair_stage<LOG2N, IqEpi>(p, threadIdx.x);
 }
 
 // shared memory (bytes) of csd_stage_kernel<LOG2N> for tiles of T segments

@@ -241,4 +241,18 @@ int32_t sspsd_receiver_pump_csd(sspsd_receiver* h, sspsd_decoder* d, sspsd_csd* 
                                     info);
 }
 
+int32_t sspsd_receiver_pump_zoom(sspsd_receiver* h, sspsd_decoder* d, sspsd_zoom* z, const uint32_t* traces,
+                                 uint32_t max_frames, int32_t timeout_ms, sspsd_loss* loss, sspsd_decode_info* info)
+{
+    if (!h) return SSPSD_EINVAL;
+    if (info) std::memset(info, 0, sizeof(*info));
+    int rc = sspsd_zoom_process_frames(d, z, traces, nullptr, 0, 0, 0, SSPSD_MEM_HOST, nullptr, nullptr);
+    if (rc) return rc;
+    const uint8_t* frames = nullptr;
+    size_t n = 0, len = 0;
+    rc = h->r.recv(max_frames, timeout_ms, &frames, &n, &len);
+    if (rc || n == 0) return rc;
+    return sspsd_zoom_process_frames(d, z, traces, frames, n, len, h->r.slot_bytes(), SSPSD_MEM_HOST, loss, info);
+}
+
 }  // extern "C"

@@ -1,5 +1,6 @@
 // sspsd_xcascade.cu -- XCascade: the cascaded cross-spectral density of two streams (sspsd_csd_* of
-// include/sspsd.h) and the cross-spectral matrix of K = 2 .. 4 streams (sspsd_csm_*).
+// include/sspsd.h), the cross-spectral matrix of K = 2 .. 4 streams (sspsd_csm_*) and the two-sided spectrum of
+// z = i + i q (ZoomCascade, sspsd_zoom_*: I/Q streams, or a real stream mixed down around a carrier).
 //
 // K Cascades, one per channel, are driven in lockstep.  Their bookkeeping (segments, decimation, deferral,
 // EWMA counts) does not depend on the data, so all run exactly the same stages over the same segment ranges;
@@ -14,7 +15,8 @@
 // is csd_stage_kernel's four rows; the off-diagonal block (K >= 3) is csm_cross_kernel's eight.  A stage's
 // accumulator block is [pair (0,1): Sxx Syy ReSxy ImSxy][pair (2,3): the same][cross: 8 rows], so K = 2 (the
 // CSD) has exactly the first four rows.  K = 3 runs pair (2,3)'s csd_stage_kernel with channel 2 in both slots:
-// its rows 1..3 are S22 again and are never read.
+// its rows 1..3 are S22 again and are never read.  The two-sided kind (K = 2, DESIGN.md 3c) runs iq_stage_kernel
+// instead: a block of two rows, P+ and P-.
 #include "sspsd_cascade.cuh"
 
 #include <algorithm>
@@ -24,12 +26,13 @@
 #include <vector>
 
 #include "sspsd_csm_kernel.cuh"
+#include "sspsd_mix_kernel.cuh"
 
 namespace sspsd {
 
 namespace {
 
-// One of the two block kernels at one N, its rows and its shared-memory budget per CTA
+// One of the block kernels at one N, its rows and its shared-memory budget per CTA
 struct BlockKernel {
     void (*fn)(XStageParams);
     size_t (*smem)(int T, int hop);  // bytes for tiles of T segments
@@ -37,10 +40,10 @@ struct BlockKernel {
     int rows;
     const char* what;
 };
-enum { DIAG = 0, CROSS = 1 };
+enum { DIAG = 0, CROSS = 1, IQ = 2 };
 struct BlockKernels {
-    BlockKernel k[2];  // [DIAG]: csd_stage_kernel, [CROSS]: csm_cross_kernel
-    int nt, groups;    // threads per CTA, segments in flight per CTA (both kernels)
+    BlockKernel k[3];  // [DIAG]: csd_stage_kernel, [CROSS]: csm_cross_kernel, [IQ]: iq_stage_kernel
+    int nt, groups;    // threads per CTA, segments in flight per CTA (all kernels)
 };
 
 template <int LOG2N>
@@ -53,7 +56,9 @@ BlockKernels block_kernels_t()
     return {{{csd_stage_kernel<LOG2N>, csd_smem_bytes<LOG2N>, two ? 100 * 1024 : 200 * 1024, CSD_ROWS,
               "csd_stage_kernel launch"},
              {csm_cross_kernel<LOG2N>, csm_smem_bytes<LOG2N>, two ? 110 * 1024 : 220 * 1024, CSM_XROWS,
-              "csm_cross_kernel launch"}},
+              "csm_cross_kernel launch"},
+             {iq_stage_kernel<LOG2N>, csd_smem_bytes<LOG2N>, two ? 100 * 1024 : 200 * 1024, IQ_ROWS,
+              "iq_stage_kernel launch"}},
             PL::NT,
             PL::G};
 }
@@ -111,7 +116,7 @@ class XCascade : public StageHook {
 public:
     XCascade() = default;
     ~XCascade();
-    int init(const sspsd_config& cfg, int k);
+    int init(const sspsd_config& cfg, int k, bool two_sided = false);
     int clone_from(XCascade& o);
     int reset();
     int process(const float* const* x, size_t n, int mem);
@@ -122,6 +127,8 @@ public:
     int read(const sspsd_merge_opts& o, float* pxx, float* pyy, float* pxy, size_t* p_len, sspsd_break* b,
              size_t* b_len);
     int read_matrix(const sspsd_merge_opts& o, float* s, size_t* p_len, sspsd_break* b, size_t* b_len);
+    int read_two_sided(const sspsd_merge_opts& o, float* p_pos, float* p_neg, size_t* p_len, sspsd_break* b,
+                       size_t* b_len);
     int num_stages(uint32_t* n);
     int channels() const { return k_; }
     int device() const { return cfg_.device; }
@@ -130,12 +137,12 @@ public:
     int stage_psd(Cascade& c, size_t i, const StreamSrc& src, uint64_t k0, uint64_t nseg, const EwmaPlan& e) override;
 
 private:
-    int setup(const sspsd_config& cfg, int k);
+    int setup(const sspsd_config& cfg, int k, bool two_sided);
     sspsd_config channel_cfg() const;
     int feed_chunk(const float* const* x, size_t n, bool device);
     int flush_staged();
     int flush_all();
-    size_t block_rows() const { return k_ == 2 ? CSD_ROWS : 2 * CSD_ROWS + CSM_XROWS; }
+    size_t block_rows() const { return two_sided_ ? IQ_ROWS : k_ == 2 ? CSD_ROWS : 2 * CSD_ROWS + CSM_XROWS; }
     size_t acc_floats() const { return (size_t)SSPSD_MAX_STAGES * block_rows() * stride_; }
     int ensure_part(float** part, size_t* cap, size_t need);
     int launch_block(int kind, XStageParams p, uint64_t nseg, float* acc, float** part, size_t* part_cap);
@@ -155,12 +162,13 @@ private:
     } own_;
     Cascade ch_[4];  // channel 0 launches the block kernels; 1 .. k_-1 leave their sources
     int k_ = 2;
+    bool two_sided_ = false;  // K = 2: iq_stage_kernel's rows P+, P- instead of the CSD's four
     sspsd_config cfg_{};
     cudaStream_t stream_ = nullptr;
     uint32_t n_ = 0, log2n_ = 0;
     int num_sms_ = 148;
     BlockKernels kern_{};
-    int tmax_[2] = {1, 1};  // largest tile of each block kernel
+    int tmax_[3] = {1, 1, 1};  // largest tile of each block kernel
     uint32_t stride_ = 0;  // floats per row; a stage's block is block_rows() rows
     float* d_win_ = nullptr;
     float2* d_tw_ = nullptr;
@@ -198,9 +206,9 @@ sspsd_config XCascade::channel_cfg() const
 }
 
 // everything but the channels: the stream, the window and twiddle tables, the accumulator blocks
-int XCascade::setup(const sspsd_config& cfg, int k)
+int XCascade::setup(const sspsd_config& cfg, int k, bool two_sided)
 {
-    if (k < 2 || k > 4) {
+    if (k < 2 || k > 4 || (two_sided && k != 2)) {
         set_error("CsmCascade supports 2 .. 4 channels");
         return SSPSD_EINVAL;
     }
@@ -226,6 +234,7 @@ int XCascade::setup(const sspsd_config& cfg, int k)
     if (!g.ok) return SSPSD_ECUDA;
     cfg_ = cfg;
     k_ = k;
+    two_sided_ = two_sided;
     if (cfg.stream) {
         stream_ = (cudaStream_t)cfg.stream;
     } else {
@@ -238,7 +247,11 @@ int XCascade::setup(const sspsd_config& cfg, int k)
     const int hop = cfg.window == SSPSD_WINDOW_HANN ? (int)n / 2 : (int)n;
     int rc = block_kernels((int)log2n_, &kern_);
     if (rc) return rc;
-    for (int kind = DIAG; kind <= (k_ > 2 ? CROSS : DIAG); ++kind) {
+    if (two_sided_) {
+        rc = prepare_block(kern_.k[IQ], hop, &tmax_[IQ]);
+        if (rc) return rc;
+    }
+    for (int kind = DIAG; !two_sided_ && kind <= (k_ > 2 ? CROSS : DIAG); ++kind) {
         rc = prepare_block(kern_.k[kind], hop, &tmax_[kind]);
         if (rc) return rc;
     }
@@ -276,9 +289,9 @@ int XCascade::setup(const sspsd_config& cfg, int k)
     return SSPSD_OK;
 }
 
-int XCascade::init(const sspsd_config& cfg, int k)
+int XCascade::init(const sspsd_config& cfg, int k, bool two_sided)
 {
-    int rc = setup(cfg, k);
+    int rc = setup(cfg, k, two_sided);
     if (rc) return rc;
     const sspsd_config c = channel_cfg();
     for (int i = 0; i < k_; ++i) {
@@ -292,7 +305,7 @@ int XCascade::clone_from(XCascade& o)
 {
     int rc = o.sync();
     if (rc) return rc;
-    rc = setup(o.cfg_, o.k_);  // the caller's stream (cfg.stream) is shared by the copy, a private one is not
+    rc = setup(o.cfg_, o.k_, o.two_sided_);  // the caller's stream (cfg.stream) is shared by the copy, a private one is not
     if (rc) return rc;
     const sspsd_config c = channel_cfg();
     for (int i = 0; i < k_; ++i) {
@@ -400,6 +413,7 @@ int XCascade::stage_psd(Cascade& c, size_t i, const StreamSrc& src, uint64_t k0,
         scale_kernel<<<(nblock + 255) / 256, 256, 0, stream_>>>(acc, nblock, e.total);
         SSPSD_CUDA(cudaGetLastError());
     }
+    if (two_sided_) return launch_block(IQ, p, nseg, acc, &d_part_, &part_cap_);
     // diagonal blocks: csd_stage_kernel over pair (0, 1), then (2, 3)
     int rc = launch_block(DIAG, p, nseg, acc, &d_part_, &part_cap_);
     if (rc || k_ == 2) return rc;
@@ -658,6 +672,28 @@ int XCascade::read(const sspsd_merge_opts& o, float* pxx, float* pyy, float* pxy
     return SSPSD_OK;
 }
 
+// The two-sided kind: P+ and P- merged as read() merges its rows, then halved (exact): the two-sided density, so a
+// real x fed as (x, 0) reads back psd(x) / 2 on each side.
+int XCascade::read_two_sided(const sspsd_merge_opts& o, float* p_pos, float* p_neg, size_t* p_len, sspsd_break* b,
+                             size_t* b_len)
+{
+    uint64_t book[4 * SSPSD_MAX_STAGES + 2];
+    size_t pl, ns;
+    int rc = read_rows(o, p_pos && p_neg, p_len, b, b_len, book, &pl, &ns);
+    if (rc || ns == 0) return rc;
+    const size_t block = block_rows() * stride_;
+    float* outs[IQ_ROWS] = {p_pos, p_neg};
+    for (int r = 0; r < IQ_ROWS; ++r) {
+        size_t pr = pl, br = ns;
+        rc = Cascade::merge_host(ch_[0].cfg_, book, h_acc_ + (size_t)r * stride_, block, o, outs[r], &pr, b, &br);
+        if (rc) return rc;
+        for (size_t k = 0; k < pl; ++k) outs[r][k] *= 0.5f;
+    }
+    *p_len = pl;
+    *b_len = ns;
+    return SSPSD_OK;
+}
+
 // The whole K x K matrix, s[2 ((i K + j) p_len + k) + {0, 1}]: every stored row merged as read() merges its rows,
 // the diagonal real (imaginary part 0), the lower triangle the conjugate of the upper.
 int XCascade::read_matrix(const sspsd_merge_opts& o, float* s, size_t* p_len, sspsd_break* b, size_t* b_len)
@@ -715,6 +751,250 @@ int XCascade::read_matrix(const sspsd_merge_opts& o, float* s, size_t* p_len, ss
     return SSPSD_OK;
 }
 
+
+// ZoomCascade: the two-sided XCascade over z = i + i q, fed either I/Q streams as they are (SSPSD_ZOOM_IQ) or one real
+// stream mixed down by the carrier ftw / 2^32 (SSPSD_ZOOM_HETERODYNE, DESIGN.md 3c).  The mixer runs on the
+// XCascade's one stream into buffers owned here, which the XCascade then reads in place (SSPSD_MEM_DEVICE): stream
+// order alone makes their reuse by the next mixer launch safe.  Host input is collected in pinned staging buffers,
+// as Cascade::process_host collects small calls, and goes to the device by cudaMemcpyAsync on the same stream.
+class ZoomCascade {
+public:
+    ~ZoomCascade();
+    int init(const sspsd_config& cfg, int mode, uint32_t ftw);
+    int clone_from(ZoomCascade& o);
+    int reset();
+    int process_iq(const float* i, const float* q, size_t n, int mem);
+    int process(const float* x, size_t n, int mem);
+    int process_device_mixed(const float* x, size_t n);  // x: device memory valid in stream order
+    int set_avg(sspsd_avg_opts a);
+    int set_detrend(int d);
+    int flush();
+    int sync();
+    int read(const sspsd_merge_opts& o, float* p_pos, float* p_neg, size_t* p_len, sspsd_break* b, size_t* b_len);
+    int num_stages(uint32_t* n);
+    int mode() const { return mode_; }
+    uint32_t ftw() const { return ftw_; }
+    XCascade& x() { return x_; }
+    const XCascade& x() const { return x_; }
+
+private:
+    int ensure_mix();
+    int flush_host();
+    int mix_and_feed(const float* d_x, size_t n);
+
+    XCascade x_;
+    int mode_ = SSPSD_ZOOM_IQ;
+    uint32_t ftw_ = 0;
+    uint64_t pos_ = 0;  // absolute index of the next sample mixed: phi_n = (n ftw) mod 2^32
+    size_t mix_cap_ = 0;  // samples per mixer launch (a multiple of 4) and of d_i_, d_q_
+    float* d_i_ = nullptr;
+    float* d_q_ = nullptr;
+    size_t stage_cap_ = 0;  // host staging, cfg.host_stage rounded to a multiple of 4: pinned h_stage_[2], d_x_
+    float* h_stage_[2] = {nullptr, nullptr};
+    float* d_x_ = nullptr;
+    cudaEvent_t ev_stage_[2] = {nullptr, nullptr};  // the H2D copy of h_stage_[b] has completed
+    bool stage_pending_[2] = {false, false};
+    int stage_buf_ = 0;
+    size_t staged_ = 0;
+};
+
+ZoomCascade::~ZoomCascade()
+{
+    if (!d_i_ && !h_stage_[0]) return;
+    DeviceGuard g(x_.device());
+    cudaStreamSynchronize(x_.stream());
+    cudaFree(d_i_);
+    cudaFree(d_q_);
+    cudaFree(d_x_);
+    for (int b = 0; b < 2; ++b) {
+        if (h_stage_[b]) cudaFreeHost(h_stage_[b]);
+        if (ev_stage_[b]) cudaEventDestroy(ev_stage_[b]);
+    }
+}
+
+int ZoomCascade::init(const sspsd_config& cfg, int mode, uint32_t ftw)
+{
+    if (mode != SSPSD_ZOOM_IQ && mode != SSPSD_ZOOM_HETERODYNE) {
+        set_error("unknown zoom mode");
+        return SSPSD_EINVAL;
+    }
+    if (mode == SSPSD_ZOOM_IQ && ftw != 0) {
+        set_error("I/Q mode has no carrier: ftw must be 0");
+        return SSPSD_EINVAL;
+    }
+    mode_ = mode;
+    ftw_ = ftw;
+    stage_cap_ = std::max<size_t>(4096, (cfg.host_stage ? (size_t)cfg.host_stage : (size_t)1 << 22) & ~(size_t)3);
+    return x_.init(cfg, 2, true);
+}
+
+int ZoomCascade::clone_from(ZoomCascade& o)
+{
+    int rc = o.flush_host();  // XCascade::clone_from then syncs the source's stream
+    if (rc) return rc;
+    rc = x_.clone_from(o.x_);
+    if (rc) return rc;
+    mode_ = o.mode_;
+    ftw_ = o.ftw_;
+    pos_ = o.pos_;
+    stage_cap_ = o.stage_cap_;
+    return SSPSD_OK;
+}
+
+int ZoomCascade::reset()
+{
+    int rc = x_.reset();
+    if (rc) return rc;
+    pos_ = 0;
+    staged_ = 0;
+    return SSPSD_OK;
+}
+
+int ZoomCascade::ensure_mix()
+{
+    if (d_i_) return SSPSD_OK;
+    mix_cap_ = (size_t)1 << 23;  // as Cascade::host_chunk()
+    SSPSD_CUDA(cudaMalloc(&d_i_, mix_cap_ * sizeof(float)));
+    SSPSD_CUDA(cudaMalloc(&d_q_, mix_cap_ * sizeof(float)));
+    return SSPSD_OK;
+}
+
+// Mixer launches of at most mix_cap_ samples (a multiple of 4, so that a stream position that is a multiple of 4
+// stays one and stage 0 reads the mix buffers in place), each followed by the XCascade's launches over them.
+int ZoomCascade::mix_and_feed(const float* d_x, size_t n)
+{
+    int rc = ensure_mix();
+    if (rc) return rc;
+    for (size_t off = 0; off < n; off += mix_cap_) {
+        const size_t m = std::min(mix_cap_, n - off);
+        const int grid = (int)std::min<size_t>((m + 255) / 256, 148 * 16);
+        heterodyne_kernel<<<grid, 256, 0, x_.stream()>>>(d_x + off, m, pos_, ftw_, d_i_, d_q_);
+        SSPSD_CUDA(cudaGetLastError());
+        const float* xs[2] = {d_i_, d_q_};
+        rc = x_.process(xs, m, SSPSD_MEM_DEVICE);
+        if (rc) return rc;
+        pos_ += m;
+    }
+    return SSPSD_OK;
+}
+
+// the staged host samples: H2D copy, mixer, cascade, all on the stream; the other pinned buffer becomes current
+int ZoomCascade::flush_host()
+{
+    if (staged_ == 0) return SSPSD_OK;
+    DeviceGuard g(x_.device());
+    if (!g.ok) return SSPSD_ECUDA;
+    const int b = stage_buf_;
+    SSPSD_CUDA(cudaMemcpyAsync(d_x_, h_stage_[b], staged_ * sizeof(float), cudaMemcpyHostToDevice, x_.stream()));
+    SSPSD_CUDA(cudaEventRecord(ev_stage_[b], x_.stream()));
+    stage_pending_[b] = true;
+    const size_t n = staged_;
+    staged_ = 0;
+    stage_buf_ ^= 1;
+    return mix_and_feed(d_x_, n);
+}
+
+int ZoomCascade::process_iq(const float* i, const float* q, size_t n, int mem)
+{
+    if (mode_ != SSPSD_ZOOM_IQ) {
+        set_error("heterodyne mode takes one real stream (sspsd_zoom_process_f32)");
+        return SSPSD_EINVAL;
+    }
+    if (n && (!i || !q)) {
+        set_error("null input");
+        return SSPSD_EINVAL;
+    }
+    const float* xs[2] = {i, q};
+    return x_.process(xs, n, mem);
+}
+
+int ZoomCascade::process_device_mixed(const float* x, size_t n)
+{
+    int rc = flush_host();
+    if (rc) return rc;
+    return mix_and_feed(x, n);
+}
+
+int ZoomCascade::process(const float* x, size_t n, int mem)
+{
+    if (mode_ != SSPSD_ZOOM_HETERODYNE) {
+        set_error("I/Q mode takes two streams (sspsd_zoom_process_iq_f32)");
+        return SSPSD_EINVAL;
+    }
+    if (n == 0) return SSPSD_OK;
+    if (!x) {
+        set_error("null input");
+        return SSPSD_EINVAL;
+    }
+    if (mem != SSPSD_MEM_HOST && mem != SSPSD_MEM_DEVICE) {
+        set_error("bad mem kind");
+        return SSPSD_EINVAL;
+    }
+    DeviceGuard g(x_.device());
+    if (!g.ok) return SSPSD_ECUDA;
+    if (mem == SSPSD_MEM_DEVICE) return process_device_mixed(x, n);
+    if (!h_stage_[0]) {
+        for (int b = 0; b < 2; ++b) {
+            SSPSD_CUDA(cudaMallocHost(&h_stage_[b], stage_cap_ * sizeof(float)));
+            SSPSD_CUDA(cudaEventCreateWithFlags(&ev_stage_[b], cudaEventDisableTiming));
+        }
+        SSPSD_CUDA(cudaMalloc(&d_x_, stage_cap_ * sizeof(float)));
+    }
+    for (size_t pos = 0; pos < n;) {
+        const int b = stage_buf_;
+        if (stage_pending_[b]) {  // its previous H2D copy still reads it
+            SSPSD_CUDA(cudaEventSynchronize(ev_stage_[b]));
+            stage_pending_[b] = false;
+        }
+        const size_t take = std::min(n - pos, stage_cap_ - staged_);
+        std::memcpy(h_stage_[b] + staged_, x + pos, take * sizeof(float));
+        staged_ += take;
+        pos += take;
+        if (staged_ == stage_cap_) {
+            int rc = flush_host();
+            if (rc) return rc;
+        }
+    }
+    return SSPSD_OK;
+}
+
+int ZoomCascade::set_avg(sspsd_avg_opts a)
+{
+    int rc = flush_host();
+    return rc ? rc : x_.set_avg(a);
+}
+
+int ZoomCascade::set_detrend(int d)
+{
+    int rc = flush_host();
+    return rc ? rc : x_.set_detrend(d);
+}
+
+int ZoomCascade::flush()
+{
+    int rc = flush_host();
+    return rc ? rc : x_.flush();
+}
+
+int ZoomCascade::sync()
+{
+    int rc = flush_host();
+    return rc ? rc : x_.sync();
+}
+
+int ZoomCascade::read(const sspsd_merge_opts& o, float* p_pos, float* p_neg, size_t* p_len, sspsd_break* b,
+                      size_t* b_len)
+{
+    int rc = flush_host();
+    return rc ? rc : x_.read_two_sided(o, p_pos, p_neg, p_len, b, b_len);
+}
+
+int ZoomCascade::num_stages(uint32_t* n)
+{
+    int rc = flush_host();
+    return rc ? rc : x_.num_stages(n);
+}
+
 }  // namespace sspsd
 
 struct sspsd_csd {
@@ -723,6 +1003,10 @@ struct sspsd_csd {
 
 struct sspsd_csm {
     sspsd::XCascade c;
+};
+
+struct sspsd_zoom {
+    sspsd::ZoomCascade z;
 };
 
 using sspsd::set_error;
@@ -809,6 +1093,39 @@ struct XSink : sspsd::FrameSink {
     }
 };
 
+// Heterodyne mode: trace map[0] of every decoded sub-chunk, mixed and fed on the handle's one stream (the mixer reads
+// the decoder's trace buffer in stream order, so the consumption event recorded after it covers that read).
+struct MixSink : sspsd::FrameSink {
+    sspsd::ZoomCascade& z;
+    uint32_t trace;
+    MixSink(sspsd::ZoomCascade& z_, uint32_t t) : z(z_), trace(t) {}
+    int check_device(int device) override
+    {
+        if (z.x().device() != device) {
+            set_error("zoom handle and decoder live on different devices");
+            return SSPSD_EINVAL;
+        }
+        return SSPSD_OK;
+    }
+    int accept(unsigned int fmt) override
+    {
+        const uint32_t ntr = fmt == SSPSD_FORMAT_MPLL ? 3 : 4;
+        if (trace >= ntr) {
+            set_error("trace index " + std::to_string(trace) + " past the " + std::to_string(ntr) +
+                      " traces of the frames' format");
+            return SSPSD_EINVAL;
+        }
+        return SSPSD_OK;
+    }
+    int consume(sspsd_decoder* d, float* const* tr, uint32_t, size_t ns, cudaEvent_t ready) override
+    {
+        const cudaStream_t s = z.x().stream();
+        if (ready) SSPSD_CUDA(cudaStreamWaitEvent(s, ready, 0));
+        int rc = z.process_device_mixed(tr[trace], ns);
+        return rc ? rc : sspsd::trace_consumed(d, (int)trace, s);
+    }
+};
+
 // sspsd_csd / sspsd_csm_process_frames; traces: one index per channel, NULL for 0 .. K-1
 template <class H>
 int32_t x_process_frames(sspsd_decoder* d, H* h, const uint32_t* traces, const uint8_t* frames, size_t n_frames,
@@ -831,6 +1148,19 @@ int32_t x_process_frames(sspsd_decoder* d, H* h, const uint32_t* traces, const u
     }
     XSink sink(h->c, map);
     return sspsd::process_frames(d, sink, frames, n_frames, frame_len, frame_stride, frames_mem, loss, info);
+}
+
+// the trace map of a zoom handle: I/Q mode two indices (i, q), heterodyne mode one; NULL for 0 (.. 1)
+int check_traces(const uint32_t* traces, int n, uint32_t* map)
+{
+    for (int i = 0; i < n; ++i) {
+        map[i] = traces ? traces[i] : (uint32_t)i;
+        if (map[i] >= SSPSD_MAX_TRACES) {
+            set_error("trace index " + std::to_string(map[i]) + " out of range (frames carry at most 4 traces)");
+            return SSPSD_EINVAL;
+        }
+    }
+    return SSPSD_OK;
 }
 
 }  // namespace
@@ -961,3 +1291,130 @@ int32_t sspsd_csm_stream(const sspsd_csm* h, void** stream)
 
 int32_t sspsd_csm_flush(sspsd_csm* h) { return h ? h->c.flush() : SSPSD_EINVAL; }
 int32_t sspsd_csm_sync(sspsd_csm* h) { return h ? h->c.sync() : SSPSD_EINVAL; }
+
+int32_t sspsd_zoom_create(const sspsd_config* cfg, int32_t mode, uint32_t ftw, sspsd_zoom** out)
+{
+    if (!cfg || !out) {
+        set_error("null argument");
+        return SSPSD_EINVAL;
+    }
+    *out = nullptr;
+    sspsd_zoom* h = new (std::nothrow) sspsd_zoom();
+    if (!h) return SSPSD_ENOMEM;
+    int rc = h->z.init(*cfg, mode, ftw);
+    if (rc) {
+        delete h;
+        return rc;
+    }
+    *out = h;
+    return SSPSD_OK;
+}
+
+void sspsd_zoom_destroy(sspsd_zoom* h) { delete h; }
+
+int32_t sspsd_zoom_clone(sspsd_zoom* h, sspsd_zoom** out)
+{
+    if (!h || !out) {
+        set_error("null argument");
+        return SSPSD_EINVAL;
+    }
+    *out = nullptr;
+    sspsd_zoom* n = new (std::nothrow) sspsd_zoom();
+    if (!n) return SSPSD_ENOMEM;
+    int rc = n->z.clone_from(h->z);
+    if (rc) {
+        delete n;
+        return rc;
+    }
+    *out = n;
+    return SSPSD_OK;
+}
+
+int32_t sspsd_zoom_reset(sspsd_zoom* h) { return h ? h->z.reset() : SSPSD_EINVAL; }
+
+int32_t sspsd_zoom_process_iq_f32(sspsd_zoom* h, const float* i, const float* q, size_t n, int32_t mem)
+{
+    return h ? h->z.process_iq(i, q, n, mem) : SSPSD_EINVAL;
+}
+
+int32_t sspsd_zoom_process_f32(sspsd_zoom* h, const float* x, size_t n, int32_t mem)
+{
+    return h ? h->z.process(x, n, mem) : SSPSD_EINVAL;
+}
+
+int32_t sspsd_zoom_process_frames(sspsd_decoder* d, sspsd_zoom* z, const uint32_t* traces, const uint8_t* frames,
+                                  size_t n_frames, size_t frame_len, size_t frame_stride, int32_t frames_mem,
+                                  sspsd_loss* loss, sspsd_decode_info* info)
+{
+    if (!d || !z || (n_frames && !frames) || frame_stride < frame_len) {
+        set_error("bad argument");
+        return SSPSD_EINVAL;
+    }
+    uint32_t map[2];
+    const bool iq = z->z.mode() == SSPSD_ZOOM_IQ;
+    int rc = check_traces(traces, iq ? 2 : 1, map);
+    if (rc) return rc;
+    if (iq) {
+        XSink sink(z->z.x(), map);
+        return sspsd::process_frames(d, sink, frames, n_frames, frame_len, frame_stride, frames_mem, loss, info);
+    }
+    MixSink sink(z->z, map[0]);
+    return sspsd::process_frames(d, sink, frames, n_frames, frame_len, frame_stride, frames_mem, loss, info);
+}
+
+int32_t sspsd_zoom_set_avg(sspsd_zoom* h, sspsd_avg_opts avg) { return h ? h->z.set_avg(avg) : SSPSD_EINVAL; }
+
+int32_t sspsd_zoom_set_detrend(sspsd_zoom* h, int32_t d) { return h ? h->z.set_detrend(d) : SSPSD_EINVAL; }
+
+int32_t sspsd_zoom_rbw(const sspsd_zoom* h, float* rbw)
+{
+    if (!h || !rbw) return SSPSD_EINVAL;
+    *rbw = h->z.x().rbw();
+    return SSPSD_OK;
+}
+
+int32_t sspsd_zoom_read(sspsd_zoom* h, const sspsd_merge_opts* opts, float* p_pos, float* p_neg, size_t* p_len,
+                        sspsd_break* b, size_t* b_len)
+{
+    if (!h) return SSPSD_EINVAL;
+    sspsd_merge_opts o{0, 1, 0};  // MergeOpts::default(), psd.rs:350-358
+    if (opts) o = *opts;
+    return h->z.read(o, p_pos, p_neg, p_len, b, b_len);
+}
+
+int32_t sspsd_zoom_carrier(const sspsd_zoom* h, int32_t* mode, uint32_t* ftw)
+{
+    if (!h || !mode || !ftw) return SSPSD_EINVAL;
+    *mode = h->z.mode();
+    *ftw = h->z.ftw();
+    return SSPSD_OK;
+}
+
+int32_t sspsd_zoom_num_stages(sspsd_zoom* h, uint32_t* n)
+{
+    if (!h || !n) return SSPSD_EINVAL;
+    return h->z.num_stages(n);
+}
+
+int32_t sspsd_zoom_stream(const sspsd_zoom* h, void** stream)
+{
+    if (!h || !stream) return SSPSD_EINVAL;
+    *stream = (void*)h->z.x().stream();
+    return SSPSD_OK;
+}
+
+int32_t sspsd_zoom_flush(sspsd_zoom* h) { return h ? h->z.flush() : SSPSD_EINVAL; }
+int32_t sspsd_zoom_sync(sspsd_zoom* h) { return h ? h->z.sync() : SSPSD_EINVAL; }
+
+int32_t sspsd_heterodyne_f32(void* stream, const float* x, size_t n, uint64_t pos0, uint32_t ftw, float* i_out,
+                             float* q_out)
+{
+    if (n == 0) return SSPSD_OK;
+    if (!x || !i_out || !q_out) {
+        set_error("null argument");
+        return SSPSD_EINVAL;
+    }
+    const int grid = (int)std::min<size_t>((n + 255) / 256, 148 * 16);
+    sspsd::heterodyne_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(x, n, pos0, ftw, i_out, q_out);
+    return sspsd::cuda_ok(cudaGetLastError(), "heterodyne_kernel launch") ? SSPSD_OK : SSPSD_ECUDA;
+}

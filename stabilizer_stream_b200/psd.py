@@ -550,6 +550,139 @@ class CsmCascade(_StreamOrdered):
             self._h = None
 
 
+class ZoomCascade(_StreamOrdered):
+    """Two-sided cascaded spectrum of a complex stream z (include/sspsd.h, sspsd_zoom_*), in one of two modes:
+    ZoomCascade.iq(n): z = i + i q of two real streams (a lock-in's BI / BQ); ZoomCascade.heterodyne(n, ftw):
+    z = x exp(-2 pi i phi_n / 2^32), phi_n = (n ftw) mod 2^32, one real stream mixed down by the carrier
+    f0 = ftw / 2^32 (units of the sample rate) on the device, so the cascade's fine low-frequency resolution lands
+    around f0.  spectrum() returns both sides, p_pos at f0 + f and p_neg at f0 - f, with PsdCascade.psd's breaks and
+    the two-sided density's scale (a real x fed as (x, 0) reads back psd(x) / 2 per side).  n = 64 .. 4096."""
+
+    def __init__(self, n=512, mode=L.ZOOM_IQ, ftw=0, window=Window.HANN, device=0, hbf=Hbf.TAPS_140, stream=None,
+                 max_batch=0, host_stage=0, deep_defer=0, deterministic=False, _handle=None):
+        self.n = n
+        self.mode = int(mode)
+        self.ftw = int(ftw)
+        self.device = int(device)
+        if _handle is not None:
+            self._h = _handle
+            return
+        cfg = _config(n, window, hbf, device, stream, max_batch, host_stage, deep_defer, deterministic)
+        h = C.c_void_p()
+        L.check(L.lib().sspsd_zoom_create(C.byref(cfg), self.mode, self.ftw, C.byref(h)))
+        self._h = h
+
+    @classmethod
+    def iq(cls, n=512, **kw):
+        """I/Q mode: process(i, q)"""
+        return cls(n, L.ZOOM_IQ, 0, **kw)
+
+    @classmethod
+    def heterodyne(cls, n, ftw, **kw):
+        """heterodyne mode around the carrier ftw / 2^32 (ftw: a 32-bit frequency tuning word, see ftw_of): process(x)"""
+        if not 0 <= int(ftw) < 2 ** 32:
+            raise ValueError("ftw must be a 32-bit frequency tuning word, got %d" % ftw)
+        return cls(n, L.ZOOM_HETERODYNE, ftw, **kw)
+
+    @staticmethod
+    def ftw_of(f0):
+        """the tuning word of the carrier f0 (units of the sample rate, any sign): round(f0 2^32) mod 2^32"""
+        return int(round(float(f0) * 2.0 ** 32)) % 2 ** 32
+
+    def clone(self):
+        h = C.c_void_p()
+        L.check(L.lib().sspsd_zoom_clone(self._h, C.byref(h)))
+        return ZoomCascade(self.n, self.mode, self.ftw, device=self.device, _handle=h)
+
+    def _stream_ptr(self):
+        s = C.c_void_p()
+        L.check(L.lib().sspsd_zoom_stream(self._h, C.byref(s)))
+        return s.value or 0
+
+    def reset(self):
+        L.check(L.lib().sspsd_zoom_reset(self._h))
+
+    def rbw(self):
+        r = C.c_float()
+        L.check(L.lib().sspsd_zoom_rbw(self._h, C.byref(r)))
+        return r.value
+
+    def carrier(self):
+        """-> (mode, ftw) of the handle"""
+        m, f = C.c_int32(), C.c_uint32()
+        L.check(L.lib().sspsd_zoom_carrier(self._h, C.byref(m), C.byref(f)))
+        return m.value, f.value
+
+    def set_avg(self, avg: AvgOpts):
+        L.check(L.lib().sspsd_zoom_set_avg(self._h, L.AvgOptsC(avg.limit, avg.count)))
+
+    def set_detrend(self, d: Detrend):
+        L.check(L.lib().sspsd_zoom_set_detrend(self._h, int(d)))
+
+    def process(self, x, q=None):
+        """the next samples: process(x) in heterodyne mode, process(i, q) in I/Q mode; float32 numpy arrays or CUDA
+        tensors (both of a pair alike)"""
+        if (q is None) != (self.mode == L.ZOOM_HETERODYNE):
+            raise ValueError("heterodyne mode takes process(x), I/Q mode process(i, q)")
+        px, n, mem, kx = _as_buffer(x)
+        if q is None:
+            if mem == L.MEM_DEVICE:
+                self._order_device_input(kx)
+            L.check(L.lib().sspsd_zoom_process_f32(self._h, px, n, mem))
+        else:
+            pq, nq, memq, kq = _as_buffer(q)
+            if n != nq:
+                raise ValueError("i and q must have the same length (%d != %d)" % (n, nq))
+            if mem != memq:
+                raise ValueError("i and q must both be host arrays or both be CUDA tensors")
+            if mem == L.MEM_DEVICE:
+                self._order_device_input(kx)
+                self._order_device_input(kq)
+            L.check(L.lib().sspsd_zoom_process_iq_f32(self._h, px, pq, n, mem))
+        if mem == L.MEM_DEVICE:
+            self._release_device_input(kx)
+
+    def flush(self):
+        L.check(L.lib().sspsd_zoom_flush(self._h))
+
+    def sync(self):
+        L.check(L.lib().sspsd_zoom_sync(self._h))
+
+    def num_stages(self):
+        n = C.c_uint32()
+        L.check(L.lib().sspsd_zoom_num_stages(self._h, C.byref(n)))
+        return n.value
+
+    def spectrum(self, opts: MergeOpts = None):
+        """-> (p_pos, p_neg, breaks): the densities at f0 + f and f0 - f, f = Break.frequencies(breaks) >= 0"""
+        opts = opts or MergeOpts()
+        o = L.MergeOptsC(int(opts.keep_overlap), opts.min_count, int(opts.keep_transition_band))
+        cap = L.MAX_STAGES * (self.n // 2 + 1)
+        pp, pn = np.zeros(cap, np.float32), np.zeros(cap, np.float32)
+        b = (L.BreakC * L.MAX_STAGES)()
+        pl, bl = C.c_size_t(cap), C.c_size_t(L.MAX_STAGES)
+        L.check(L.lib().sspsd_zoom_read(self._h, C.byref(o), pp.ctypes.data, pn.ctypes.data, C.byref(pl), b,
+                                        C.byref(bl)))
+        n = pl.value
+        return pp[:n].copy(), pn[:n].copy(), [Break._from_c(b[i]) for i in range(bl.value)]
+
+    @staticmethod
+    def two_sided(p_pos, p_neg, breaks, ftw=0):
+        """-> (f, p) in ascending absolute frequency f = f0 -+ f_j (units of the sample rate, f0 = ftw / 2^32), the
+        DC (f_j = 0) and Nyquist (f_j = 1/2) bins once: they are the same bin on both sides"""
+        f = Break.frequencies(breaks).astype(np.float64)
+        p_pos, p_neg = np.asarray(p_pos), np.asarray(p_neg)
+        neg = (f > 0) & (f < 0.5)
+        f0 = int(ftw) / 2.0 ** 32
+        return (np.concatenate([f0 - f[neg][::-1], f0 + f]), np.concatenate([p_neg[neg][::-1], p_pos]))
+
+    def __del__(self):
+        h = getattr(self, "_h", None)
+        if h and L is not None and getattr(L, "_lib", None) is not None:
+            L._lib.sspsd_zoom_destroy(h)
+            self._h = None
+
+
 class Psd(_StreamOrdered):
     """Psd<N> + trait PsdStage, src/psd.rs:119-288 (one stage, decimated output exposed)."""
 
@@ -662,13 +795,17 @@ class Loss:
 
 
 def _trace_map(target, traces):
-    """The trace indices a CsdCascade / CsmCascade target of process_frames / pump reads, one per channel (default
-    0 .. K-1); None for a list of PsdCascades, which take trace t into target[t]."""
-    if not isinstance(target, (CsdCascade, CsmCascade)):
+    """The trace indices a CsdCascade / CsmCascade / ZoomCascade target of process_frames / pump reads, one per channel
+    (default 0 .. K-1; a heterodyne ZoomCascade reads one trace); None for a list of PsdCascades, which take trace t
+    into target[t]."""
+    if not isinstance(target, (CsdCascade, CsmCascade, ZoomCascade)):
         if traces is not None:
-            raise ValueError("traces= applies to a CsdCascade or CsmCascade target")
+            raise ValueError("traces= applies to a CsdCascade, CsmCascade or ZoomCascade target")
         return None
-    k = 2 if isinstance(target, CsdCascade) else target.channels
+    if isinstance(target, ZoomCascade):
+        k = 1 if target.mode == L.ZOOM_HETERODYNE else 2
+    else:
+        k = 2 if isinstance(target, CsdCascade) else target.channels
     tmap = list(range(k)) if traces is None else [int(t) for t in traces]
     if len(tmap) != k:
         raise ValueError("expected %d trace indices (one per channel), got %d" % (k, len(tmap)))
@@ -753,8 +890,9 @@ class FrameDecoder(_StreamOrdered):
     def process_frames(self, target, frames, frame_len, loss: Loss = None, frame_stride=None, n_frames=None,
                        traces=None):
         """Fused decode -> spectra.  `target` is a list of PsdCascades (trace t -> target[t], None drops a trace;
-        src/bin/psd.rs:174-182), a CsdCascade (x, y <- traces, default (0, 1)) or a CsmCascade (channel i <-
-        traces[i], default range(K)).  Raises DecodeError on a malformed frame after having consumed the frames
+        src/bin/psd.rs:174-182), a CsdCascade (x, y <- traces, default (0, 1)), a CsmCascade (channel i <-
+        traces[i], default range(K)) or a ZoomCascade (I/Q: i, q <- traces, default (0, 1), e.g. (2, 3) for Fls BI /
+        BQ; heterodyne: x <- traces[0], default 0, mixed on the device).  Raises DecodeError on a malformed frame after having consumed the frames
         before it."""
         tmap = _trace_map(target, traces)
         frame_stride = frame_stride or frame_len
@@ -766,6 +904,9 @@ class FrameDecoder(_StreamOrdered):
         if isinstance(target, CsmCascade):
             st = L.lib().sspsd_csm_process_frames(self._h, target._h, (C.c_uint32 * len(tmap))(*tmap), ptr, n_frames,
                                                   frame_len, frame_stride, mem, lp, C.byref(info))
+        elif isinstance(target, ZoomCascade):
+            st = L.lib().sspsd_zoom_process_frames(self._h, target._h, (C.c_uint32 * len(tmap))(*tmap), ptr, n_frames,
+                                                   frame_len, frame_stride, mem, lp, C.byref(info))
         elif isinstance(target, CsdCascade):
             st = L.lib().sspsd_csd_process_frames(self._h, target._h, tmap[0], tmap[1], ptr, n_frames, frame_len,
                                                   frame_stride, mem, lp, C.byref(info))
@@ -931,6 +1072,9 @@ class Receiver:
         if isinstance(target, CsmCascade):
             st = L.lib().sspsd_receiver_pump_csm(self._h, decoder._h, target._h, (C.c_uint32 * len(tmap))(*tmap),
                                                  max_frames, timeout_ms, lp, C.byref(info))
+        elif isinstance(target, ZoomCascade):
+            st = L.lib().sspsd_receiver_pump_zoom(self._h, decoder._h, target._h, (C.c_uint32 * len(tmap))(*tmap),
+                                                  max_frames, timeout_ms, lp, C.byref(info))
         elif isinstance(target, CsdCascade):
             st = L.lib().sspsd_receiver_pump_csd(self._h, decoder._h, target._h, tmap[0], tmap[1], max_frames,
                                                  timeout_ms, lp, C.byref(info))

@@ -16,6 +16,12 @@ Host reads go through a pinned double buffer, so the H2D copy of block b+1 overl
 --csm TRACES (with --file or --udp), e.g. 0,2 or 0,1,2,3: feed the listed traces of the frames to one CsmCascade
 instead of one PsdCascade per trace, and report the diagonal PSD of --trace (one of TRACES, default the first) plus
 the median coherence of every pair; --save FILE.npz writes the matrix S [K, K, bins], the frequencies and the breaks.
+
+--iq I,Q (with --file or --udp), e.g. 2,3 for the BI / BQ of Fls frames: feed the two traces as z = I + i Q to a
+ZoomCascade and report its two-sided spectrum.  --zoom FTW (with --file or --udp): mix trace --trace down by the
+carrier FTW / 2^32 of the sample rate on the device (ZoomCascade.heterodyne) and report the two-sided spectrum around
+it.  With either, --save FILE.npz writes p_pos, p_neg, the frequencies f >= 0 (p_pos at f0 + f, p_neg at f0 - f), the
+absolute two-sided axis and spectrum, and the breaks.
 """
 import argparse
 import json
@@ -28,7 +34,7 @@ import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
 from stabilizer_stream_b200 import (Break, CsmCascade, Detrend, FrameDecoder, Loss, MergeOpts, PsdCascade, Receiver,
-                                    Source, Var)  # noqa: E402
+                                    Source, Var, ZoomCascade)  # noqa: E402
 
 BREAK_FIELDS = ("start", "include", "count", "avg", "bins_start", "bins_end", "fft_size", "decimation", "pending",
                 "processed")
@@ -42,8 +48,8 @@ def break_row(k):
 def parse_csm(ap, a):
     """--csm / --trace / --save checks, before any device work: -> the trace list or None"""
     if a.csm is None:
-        if a.save:
-            ap.error("--save needs --csm")
+        if a.save and a.iq is None and a.zoom is None:
+            ap.error("--save needs --csm, --iq or --zoom")
         return None
     try:
         traces = [int(t) for t in a.csm.split(",")]
@@ -57,6 +63,32 @@ def parse_csm(ap, a):
         ap.error("--csm needs --file or --udp (frames carry the traces)")
     if a.trace is not None and a.trace not in traces:
         ap.error("--trace must be one of the --csm traces")
+    return traces
+
+
+def parse_zoom(ap, a):
+    """--iq / --zoom checks, before any device work: -> the trace map of the ZoomCascade or None"""
+    if sum(v is not None for v in (a.csm, a.iq, a.zoom)) > 1:
+        ap.error("use one of --csm, --iq, --zoom")
+    if a.iq is None and a.zoom is None:
+        return None
+    if not (a.file or a.udp):
+        ap.error("--iq / --zoom need --file or --udp (frames carry the traces)")
+    if a.iq is not None:
+        try:
+            traces = [int(t) for t in a.iq.split(",")]
+        except ValueError:
+            traces = []
+        if len(traces) != 2:
+            ap.error("--iq takes two trace indices I,Q, e.g. 2,3")
+        if a.trace is not None:
+            ap.error("--trace does not apply to --iq (the spectrum is of I + i Q)")
+    else:
+        if not 0 <= a.zoom < 2 ** 32:
+            ap.error("--zoom takes a 32-bit frequency tuning word")
+        traces = [0 if a.trace is None else a.trace]
+    if any(not 0 <= t < 4 for t in traces):
+        ap.error("--iq / --trace indices are 0 .. 3")
     return traces
 
 
@@ -74,11 +106,17 @@ def main():
     ap.add_argument("--detrend", default="midpoint", choices=["none", "midpoint", "span", "mean"])
     ap.add_argument("--trace", type=int, default=None, help="trace to report (default 0; with --csm the first of TRACES)")
     ap.add_argument("--csm", metavar="TRACES", help="comma-separated traces (2 to 4) into one CsmCascade")
-    ap.add_argument("--save", metavar="FILE.npz", help="with --csm: write S, the frequencies and the breaks")
+    ap.add_argument("--iq", metavar="I,Q", help="two traces into one ZoomCascade as I + i Q (two-sided spectrum)")
+    ap.add_argument("--zoom", metavar="FTW", type=int,
+                    help="mix --trace down by the carrier FTW / 2^32 of the sample rate (two-sided spectrum around it)")
+    ap.add_argument("--save", metavar="FILE.npz", help="with --csm, --iq or --zoom: write the spectra, frequencies and breaks")
     ap.add_argument("--block", type=int, default=1 << 24, help="items (or frames*64) read per block")
     ap.add_argument("--json", action="store_true")
     a = ap.parse_args()
     csm_traces = parse_csm(ap, a)
+    zoom_traces = parse_zoom(ap, a)
+    if zoom_traces:
+        csm_traces = None
     if a.trace is None:
         a.trace = csm_traces[0] if csm_traces else 0
     dev = torch.device("cuda", 0)
@@ -89,6 +127,12 @@ def main():
     t0 = time.perf_counter()
 
     def cascades(n):
+        if zoom_traces:
+            if not cas:
+                z = ZoomCascade.iq(a.fft) if a.iq is not None else ZoomCascade.heterodyne(a.fft, a.zoom)
+                z.set_detrend(det)
+                cas.append(z)
+            return
         if csm_traces:
             if not cas:
                 m = CsmCascade(a.fft, len(csm_traces))
@@ -101,7 +145,9 @@ def main():
             cas.append(c)
 
     def target():
-        return cas[0] if csm_traces else cas
+        return cas[0] if (csm_traces or zoom_traces) else cas
+
+    tmap = zoom_traces or csm_traces
 
     if a.noise is not None or a.dsm is not None:
         cascades(1)
@@ -148,7 +194,7 @@ def main():
                         continue
                     break
                 cascades(4)
-                info = dec.process_frames(target(), data[:nfr * a.frame_size], a.frame_size, loss, traces=csm_traces)
+                info = dec.process_frames(target(), data[:nfr * a.frame_size], a.frame_size, loss, traces=tmap)
                 if not names:
                     from stabilizer_stream_b200.psd import TRACE_NAMES, Format
                     names = list(TRACE_NAMES[Format(info.format)])
@@ -161,7 +207,7 @@ def main():
         dec = FrameDecoder()
         cascades(4)
         while True:
-            info = rx.pump(dec, target(), loss, max_frames=1024, timeout_ms=1000, traces=csm_traces)
+            info = rx.pump(dec, target(), loss, max_frames=1024, timeout_ms=1000, traces=tmap)
             if info.frames_ok == 0:
                 break
             if not names:
@@ -174,7 +220,22 @@ def main():
         ap.error("one of --raw, --file, --udp, --noise, --dsm is required")
 
     coherence = []
-    if csm_traces:
+    zoom = None
+    if zoom_traces:
+        pp, pn, b = cas[0].spectrum(MergeOpts())
+        dt = time.perf_counter() - t0
+        ftw = a.zoom or 0
+        fa, pa = ZoomCascade.two_sided(pp, pn, b, ftw)
+        y = (pp + pn).astype(np.float32)  # both sides folded: what fdev of a real trace would see
+        zoom = {"mode": "iq" if a.iq is not None else "heterodyne", "traces": zoom_traces, "ftw": ftw,
+                "f0": ftw / 2.0 ** 32, "bins": int(pa.size),
+                "peak": {"f": float(fa[np.argmax(pa)]), "p": float(np.max(pa))} if pa.size else None}
+        if a.save:
+            np.savez(a.save, p_pos=pp, p_neg=pn, frequencies=Break.frequencies(b), f_abs=fa, p_abs=pa,
+                     traces=np.array(zoom_traces), ftw=np.uint32(ftw),
+                     breaks=np.array([break_row(k_) for k_ in b], np.uint64).reshape(-1, len(BREAK_FIELDS)),
+                     break_fields=np.array(BREAK_FIELDS))
+    elif csm_traces:
         S, b = cas[0].csm(MergeOpts())
         dt = time.perf_counter() - t0
         y = np.real(S[csm_traces.index(a.trace), csm_traces.index(a.trace)]).astype(np.float32)
@@ -208,12 +269,17 @@ def main():
            "fdev": fdev[:8], "loss": {"received": loss.received, "dropped": loss.dropped}}
     if csm_traces:
         out["csm"] = {"traces": csm_traces, "coherence": coherence}
+    if zoom:
+        out["zoom"] = zoom
     if a.json:
         print(json.dumps(out))
     else:
         print("breaks:", out["breaks"])
         print("psd: %d bins, median %.6g" % (out["psd_bins"], out["psd_median"] or 0))
         print("fdev:", out["fdev"])
+        if zoom and zoom["peak"]:
+            print("two-sided: %d bins around f0 = %.9g, peak %.6g at %.9g" % (zoom["bins"], zoom["f0"], zoom["peak"]["p"],
+                                                                          zoom["peak"]["f"]))
         for c_ in coherence:
             i, j = c_["traces"]
             print("coherence %s / %s: median %.4g over %d bins" % (names[i] if names else i, names[j] if names else j,
