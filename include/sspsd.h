@@ -176,7 +176,8 @@ int32_t sspsd_cascade_sync(sspsd_cascade *h);
  * readout has the breaks of sspsd_cascade_psd and the same 1/(gain_i 8^i) scale on every row: pxx is what
  * a cascade fed x alone returns.  n_fft = 64 .. 4096 (8192 returns SSPSD_EINVAL: the two-for-one transform
  * is an N-point complex FFT).  SSPSD_MEM_DEVICE input follows the rule of sspsd_cascade_process_f32 for
- * BOTH x and y, on the handle's stream (sspsd_csd_stream).  Multi-GPU groups are not supported.
+ * BOTH x and y, on the handle's stream (sspsd_csd_stream).  One long capture can be spread over GPUs in time
+ * chunks: a group of kind SSPSD_GROUP_CSD (sspsd_group_create_kind).
  * --------------------------------------------------------------------------------------------- */
 typedef struct sspsd_csd sspsd_csd;
 int32_t sspsd_csd_create(const sspsd_config *cfg, sspsd_csd **out);
@@ -205,7 +206,8 @@ int32_t sspsd_csd_sync(sspsd_csd *h);
  * (sspsd_csd_*'s convention: S[0,1] is pxy of a sspsd_csd fed (x0, x1)), with sspsd_csd_*'s limits
  * (n_fft = 64 .. 4096, Hann or rectangular, Linear detrend SSPSD_EUNIMPLEMENTED).  Every transform is
  * shared by all pairs, so the matrix costs k decimations and k FFTs per segment, where k (k - 1) / 2
- * sspsd_csd handles cost k (k - 1) of each.  k = 2 computes exactly what sspsd_csd_* computes.
+ * sspsd_csd handles cost k (k - 1) of each.  k = 2 computes exactly what sspsd_csd_* computes.  Time-chunked
+ * multi-GPU groups: kind SSPSD_GROUP_CSM (sspsd_group_create_kind).
  * --------------------------------------------------------------------------------------------- */
 typedef struct sspsd_csm sspsd_csm;
 /* k not in {2, 3, 4}: SSPSD_EINVAL */
@@ -244,7 +246,8 @@ int32_t sspsd_csm_sync(sspsd_csm *h);
  * p_pos[j] is the density at f0 + f_j and p_neg[j] at f0 - f_j, f_j of sspsd_break_frequencies (f0 = 0 in I/Q
  * mode).  Limits as sspsd_csd_*: n_fft = 64 .. 4096 (else SSPSD_EINVAL), Hann or rectangular window, Linear
  * detrend SSPSD_EUNIMPLEMENTED.  SSPSD_MEM_DEVICE input follows the rule of sspsd_cascade_process_f32, on the
- * handle's stream (sspsd_zoom_stream).
+ * handle's stream (sspsd_zoom_stream).  Time-chunked multi-GPU groups: kind SSPSD_GROUP_ZOOM
+ * (sspsd_group_create_kind); every rank's mixer starts at the absolute index of its first sample.
  * --------------------------------------------------------------------------------------------- */
 typedef struct sspsd_zoom sspsd_zoom;
 enum { SSPSD_ZOOM_IQ = 0, SSPSD_ZOOM_HETERODYNE = 1 };
@@ -401,6 +404,47 @@ int32_t sspsd_group_time_process_all_f32(sspsd_group *g, const float *x, size_t 
 int32_t sspsd_group_time_process_noise(sspsd_group *g, int64_t exponent, uint64_t seed);
 /* the exchange (collective in a multi-process group): ONE reduction to rank 0, which then runs the deep stages */
 int32_t sspsd_group_time_finish(sspsd_group *g);
+
+/* ---- group kinds: time chunks of the cross-spectral handles ----
+ * A group made by sspsd_group_create / _create_rank is of kind SSPSD_GROUP_PSD.  The other kinds spread one capture of
+ * several streams over GPUs as the PSD kind spreads one stream: the same planner (sspsd_time_plan, sspsd_time_chunk),
+ * every rank a sspsd_csd / sspsd_csm / sspsd_zoom handle positioned and windowed on all its channels alike, and ONE
+ * reduction of [accumulator rows | counts | every channel's tail slices] to rank 0, which runs the deep stages.  Cross
+ * kinds are SSPSD_SHARD_TIME only (SSPSD_SHARD_CHANNELS: SSPSD_EINVAL, the channels of a cross-spectrum share every
+ * transform) and take the limits of their handles (n_fft = 64 .. 4096, else SSPSD_EINVAL).  In heterodyne mode every
+ * rank's mixer starts at its feed_lo, so phi_n = (n ftw) mod 2^32 runs over the absolute index of the whole stream.
+ *   kind       SSPSD_GROUP_*
+ *   channels   CSM: k = 2 .. 4; CSD and zoom: 2 (0 = that); PSD: 1 (0 = that)
+ *   zoom_mode  SSPSD_ZOOM_IQ / SSPSD_ZOOM_HETERODYNE (zoom only, else 0); ftw: the carrier (heterodyne only, else 0)
+ * On a group of another kind, sspsd_group_psd, sspsd_group_time_process_f32 / _all_f32 / _noise of a cross kind and the
+ * cross readouts return SSPSD_EINVAL with nothing consumed. */
+enum { SSPSD_GROUP_PSD = 0, SSPSD_GROUP_CSD = 1, SSPSD_GROUP_CSM = 2, SSPSD_GROUP_ZOOM = 3 };
+typedef struct {
+    int32_t kind;
+    int32_t channels;
+    int32_t zoom_mode;
+    uint32_t ftw;
+} sspsd_group_kind;
+int32_t sspsd_group_create_kind(const sspsd_config *cfg, const sspsd_group_kind *kind, const int32_t *devices,
+                                uint32_t n_devices, int32_t shard_mode, sspsd_group **out);
+int32_t sspsd_group_create_kind_rank(const sspsd_config *cfg, const sspsd_group_kind *kind,
+                                     const uint8_t id[SSPSD_GROUP_ID_BYTES], uint32_t rank, uint32_t n_ranks,
+                                     int32_t shard_mode, sspsd_group **out);
+/* the kind of a group, channels filled in */
+int32_t sspsd_group_kind_of(const sspsd_group *g, sspsd_group_kind *out);
+/* x: one pointer per input stream of the kind, in the order of the handle's process call (PSD 1, CSD 2 (x, y),
+ * CSM k, zoom I/Q 2 (i, q), zoom heterodyne 1), all in the same memory kind; otherwise as sspsd_group_time_process_f32 */
+int32_t sspsd_group_time_process_multi_f32(sspsd_group *g, uint32_t rank, const float *const *x, size_t n, int32_t mem);
+/* single-process groups: x[i] = the whole of stream i in host memory, the library feeds every rank its range */
+int32_t sspsd_group_time_process_all_multi_f32(sspsd_group *g, const float *const *x, size_t n);
+/* rank 0's result after sspsd_group_time_finish, with the layouts and SSPSD_ESHORT rules of sspsd_csd_read /
+ * sspsd_csm_read / sspsd_zoom_read (lengths 0 on the processes that do not hold rank 0) */
+int32_t sspsd_group_csd_read(sspsd_group *g, const sspsd_merge_opts *opts, float *pxx, float *pyy, float *pxy,
+                             size_t *p_len, sspsd_break *b, size_t *b_len);
+int32_t sspsd_group_csm_read(sspsd_group *g, const sspsd_merge_opts *opts, float *s, size_t *p_len, sspsd_break *b,
+                             size_t *b_len);
+int32_t sspsd_group_zoom_read(sspsd_group *g, const sspsd_merge_opts *opts, float *p_pos, float *p_neg, size_t *p_len,
+                              sspsd_break *b, size_t *b_len);
 
 /* ---- measurement hooks (no reference analogue) ----
  * With profiling enabled every kernel launch of the handle is bracketed by CUDA events on the

@@ -12,6 +12,7 @@
 #pragma once
 #include <cstddef>
 #include <cstdint>
+#include <initializer_list>
 #include <limits>
 #include <stdexcept>
 #include <string>
@@ -762,6 +763,34 @@ public:
         cfg.hbf = hbf;
         check(sspsd_group_create(&cfg, devices.data(), (uint32_t)devices.size(), (int32_t)mode, &g_));
     }
+    /// What a group computes (sspsd_group_kind): Group(devices, Group::kind_csm(4)) time-chunks one capture of four streams
+    static sspsd_group_kind kind_psd() { return {SSPSD_GROUP_PSD, 1, 0, 0}; }
+    static sspsd_group_kind kind_csd() { return {SSPSD_GROUP_CSD, 2, 0, 0}; }
+    static sspsd_group_kind kind_csm(int32_t k) { return {SSPSD_GROUP_CSM, k, 0, 0}; }
+    static sspsd_group_kind kind_zoom_iq() { return {SSPSD_GROUP_ZOOM, 2, SSPSD_ZOOM_IQ, 0}; }
+    static sspsd_group_kind kind_zoom_heterodyne(uint32_t ftw) { return {SSPSD_GROUP_ZOOM, 2, SSPSD_ZOOM_HETERODYNE, ftw}; }
+    Group(const std::vector<int32_t>& devices, const sspsd_group_kind& kind, Shard mode = Shard::Time,
+          int32_t hbf = SSPSD_HBF_140, Window w = Window::Hann)
+    {
+        sspsd_config cfg;
+        check(sspsd_config_default((uint32_t)N, &cfg));
+        cfg.hbf = hbf;
+        cfg.window = (int32_t)w;
+        check(sspsd_group_create_kind(&cfg, &kind, devices.data(), (uint32_t)devices.size(), (int32_t)mode, &g_));
+    }
+    sspsd_group_kind kind() const
+    {
+        sspsd_group_kind k;
+        check(sspsd_group_kind_of(g_, &k));
+        return k;
+    }
+    /// input streams of time_process: PSD 1, CSD 2, CSM k, zoom I/Q 2, zoom heterodyne 1
+    size_t inputs() const
+    {
+        const sspsd_group_kind k = kind();
+        if (k.kind == SSPSD_GROUP_ZOOM) return k.zoom_mode == SSPSD_ZOOM_IQ ? 2 : 1;
+        return (size_t)k.channels;
+    }
     Group(const Group&) = delete;
     Group& operator=(const Group&) = delete;
     ~Group() { sspsd_group_destroy(g_); }
@@ -800,11 +829,98 @@ public:
     {
         check(sspsd_group_time_process_f32(g_, rank, x, n, (int32_t)mem));
     }
+    /// x: one pointer per input stream of the kind, in the order of the matching handle's process
+    void time_process(uint32_t rank, std::initializer_list<const float*> x, size_t n, Mem mem = Mem::Host)
+    {
+        process_streams(rank, x.begin(), x.size(), n, mem);
+    }
+    template <size_t M>
+    void time_process(uint32_t rank, const std::array<const float*, M>& x, size_t n, Mem mem = Mem::Host)
+    {
+        process_streams(rank, x.data(), M, n, mem);
+    }
     void time_process_all(const std::vector<float>& x) { check(sspsd_group_time_process_all_f32(g_, x.data(), x.size())); }
+    /// the whole capture, one vector per input stream (single-process groups)
+    void time_process_all(const std::vector<std::vector<float>>& x)
+    {
+        const float* p[4];
+        check_streams(x.size());
+        for (size_t i = 0; i < x.size(); ++i) {
+            if (x[i].size() != x[0].size()) throw Error(SSPSD_EINVAL, "streams must have the same length");
+            p[i] = x[i].data();
+        }
+        check(sspsd_group_time_process_all_multi_f32(g_, p, x[0].size()));
+    }
     void time_finish() { check(sspsd_group_time_finish(g_)); }
     void sync() { check(sspsd_group_sync(g_)); }
+    /// readouts of rank 0 after time_finish, shaped as CsdCascade<N>::csd, CsmCascade<N>::csm, ZoomCascade<N>::spectrum
+    typename CsdCascade<N>::Spectra csd(const MergeOpts& o = MergeOpts()) const
+    {
+        sspsd_merge_opts mo{o.keep_overlap, o.min_count, o.keep_transition_band};
+        typename CsdCascade<N>::Spectra s;
+        const size_t cap = SSPSD_MAX_STAGES * (N / 2 + 1);
+        s.pxx.resize(cap);
+        s.pyy.resize(cap);
+        std::vector<float> xy(2 * cap);
+        sspsd_break cb[SSPSD_MAX_STAGES];
+        size_t pl = cap, bl = SSPSD_MAX_STAGES;
+        check(sspsd_group_csd_read(g_, &mo, s.pxx.data(), s.pyy.data(), xy.data(), &pl, cb, &bl));
+        s.pxx.resize(pl);
+        s.pyy.resize(pl);
+        for (size_t k = 0; k < pl; ++k) s.pxy.emplace_back(xy[2 * k], xy[2 * k + 1]);
+        s.breaks = breaks_of(cb, bl);
+        return s;
+    }
+    typename CsmCascade<N>::Matrix csm(const MergeOpts& o = MergeOpts()) const
+    {
+        sspsd_merge_opts mo{o.keep_overlap, o.min_count, o.keep_transition_band};
+        const size_t k = (size_t)kind().channels, cap = SSPSD_MAX_STAGES * (N / 2 + 1);
+        std::vector<float> s(2 * k * k * cap);
+        sspsd_break cb[SSPSD_MAX_STAGES];
+        size_t pl = cap, bl = SSPSD_MAX_STAGES;
+        check(sspsd_group_csm_read(g_, &mo, s.data(), &pl, cb, &bl));
+        typename CsmCascade<N>::Matrix m;
+        m.k = k;
+        m.bins = pl;
+        for (size_t r = 0; r < k * k * pl; ++r) m.s.emplace_back(s[2 * r], s[2 * r + 1]);
+        m.breaks = breaks_of(cb, bl);
+        return m;
+    }
+    typename ZoomCascade<N>::Spectra spectrum(const MergeOpts& o = MergeOpts()) const
+    {
+        sspsd_merge_opts mo{o.keep_overlap, o.min_count, o.keep_transition_band};
+        typename ZoomCascade<N>::Spectra s;
+        const size_t cap = SSPSD_MAX_STAGES * (N / 2 + 1);
+        s.p_pos.resize(cap);
+        s.p_neg.resize(cap);
+        sspsd_break cb[SSPSD_MAX_STAGES];
+        size_t pl = cap, bl = SSPSD_MAX_STAGES;
+        check(sspsd_group_zoom_read(g_, &mo, s.p_pos.data(), s.p_neg.data(), &pl, cb, &bl));
+        s.p_pos.resize(pl);
+        s.p_neg.resize(pl);
+        s.breaks = breaks_of(cb, bl);
+        return s;
+    }
 
 private:
+    void check_streams(size_t m) const
+    {
+        if (m != inputs()) throw Error(SSPSD_EINVAL, "one input stream per input of the group's kind");
+    }
+    void process_streams(uint32_t rank, const float* const* x, size_t m, size_t n, Mem mem)
+    {
+        check_streams(m);
+        check(sspsd_group_time_process_multi_f32(g_, rank, x, n, (int32_t)mem));
+    }
+    static std::vector<Break> breaks_of(const sspsd_break* cb, size_t bl)
+    {
+        std::vector<Break> b;
+        for (size_t i = 0; i < bl; ++i)
+            b.push_back(Break{(size_t)cb[i].start, cb[i].include != 0, cb[i].count, cb[i].avg,
+                              {(size_t)cb[i].bins_start, (size_t)cb[i].bins_end}, (size_t)cb[i].fft_size,
+                              (size_t)cb[i].decimation, (size_t)cb[i].pending, (size_t)cb[i].processed});
+        return b;
+    }
     sspsd_group* g_ = nullptr;
 };
 

@@ -6,8 +6,8 @@ works without a GPU, creating any handle does not.
 """
 from .psd import (DEPTH, HBF_PASSBAND, AvgOpts, Break, CsdCascade, CsmCascade, DecodeError, Detrend, Format, FrameDecoder, Hbf, Loss,
                   MergeOpts, Psd, PsdCascade, Receiver, ShardMode, Source, SourceKind, TimeChunk, Trace, Var, Window,
-                  ZoomCascade, Group, time_plan)
+                  ZoomCascade, Group, GroupKind, time_plan)
 
 __all__ = ["DEPTH", "HBF_PASSBAND", "AvgOpts", "Break", "CsdCascade", "CsmCascade", "DecodeError", "Detrend", "Format", "FrameDecoder", "Hbf",
            "Loss", "MergeOpts", "Psd", "PsdCascade", "Receiver", "ShardMode", "Source", "SourceKind", "TimeChunk", "Trace",
-           "Var", "Window", "ZoomCascade", "Group", "time_plan"]
+           "Var", "Window", "ZoomCascade", "Group", "GroupKind", "time_plan"]

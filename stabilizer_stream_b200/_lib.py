@@ -14,6 +14,7 @@ LIB_PATH = os.environ.get("SSPSD_LIB") or os.path.join(_HERE, "libsspsd.so")
 OK, EINVAL, EUNIMPLEMENTED, ECUDA, ENOMEM, EHEADER, EFORMAT, ESIZE, EBATCHES, ESHORT, ENCCL, EIO = range(12)
 MEM_HOST, MEM_DEVICE = 0, 1
 ZOOM_IQ, ZOOM_HETERODYNE = 0, 1
+GROUP_PSD, GROUP_CSD, GROUP_CSM, GROUP_ZOOM = 0, 1, 2, 3
 FLAG_DETERMINISTIC = 1
 MAX_STAGES = 16
 MAX_TRACES = 4
@@ -70,6 +71,10 @@ class PlotOptsC(C.Structure):
 class TimeChunkC(C.Structure):
     _fields_ = [("own_lo", C.c_uint64), ("own_hi", C.c_uint64), ("feed_lo", C.c_uint64), ("feed_hi", C.c_uint64),
                 ("tail_lo", C.c_uint64), ("tail_hi", C.c_uint64), ("n_local", C.c_uint32), ("_pad", C.c_uint32)]
+
+
+class GroupKindC(C.Structure):
+    _fields_ = [("kind", C.c_int32), ("channels", C.c_int32), ("zoom_mode", C.c_int32), ("ftw", C.c_uint32)]
 
 
 class VarC(C.Structure):
@@ -209,6 +214,16 @@ PROTOTYPES = {
     "sspsd_group_time_process_all_f32": (_i32, [_vp, _vp, _sz]),
     "sspsd_group_time_process_noise": (_i32, [_vp, C.c_int64, C.c_uint64]),
     "sspsd_group_time_finish": (_i32, [_vp]),
+    "sspsd_group_create_kind": (_i32, [C.POINTER(Config), C.POINTER(GroupKindC), C.POINTER(_i32), C.c_uint32, _i32,
+                                       C.POINTER(_vp)]),
+    "sspsd_group_create_kind_rank": (_i32, [C.POINTER(Config), C.POINTER(GroupKindC), _vp, C.c_uint32, C.c_uint32, _i32,
+                                            C.POINTER(_vp)]),
+    "sspsd_group_kind_of": (_i32, [_vp, C.POINTER(GroupKindC)]),
+    "sspsd_group_time_process_multi_f32": (_i32, [_vp, C.c_uint32, _vp, _sz, _i32]),
+    "sspsd_group_time_process_all_multi_f32": (_i32, [_vp, _vp, _sz]),
+    "sspsd_group_csd_read": (_i32, [_vp, C.POINTER(MergeOptsC), _vp, _vp, _vp, _psz, C.POINTER(BreakC), _psz]),
+    "sspsd_group_csm_read": (_i32, [_vp, C.POINTER(MergeOptsC), _vp, _psz, C.POINTER(BreakC), _psz]),
+    "sspsd_group_zoom_read": (_i32, [_vp, C.POINTER(MergeOptsC), _vp, _vp, _psz, C.POINTER(BreakC), _psz]),
     "sspsd_receiver_create": (_i32, [C.c_char_p, C.c_uint16, C.c_uint32, C.c_uint32, _i32, C.POINTER(_vp)]),
     "sspsd_receiver_destroy": (None, [_vp]),
     "sspsd_receiver_info": (_i32, [_vp, C.POINTER(C.c_uint16), _psz, C.POINTER(C.c_uint64)]),

@@ -8,6 +8,9 @@
 //     stages < K locally from a FIR warm-up halo (Cascade::seek / set_window), and at readout ONE sum-reduction
 //     combines [K accumulator rows | K segment counts | the ranks' slices of the stage-K input stream]; rank 0
 //     then runs the deep stages (<= 0.2 % of the work) on the gathered stream.
+// The time-chunked mode also serves the cross-spectral kinds (sspsd_group_create_kind): a rank then holds an XCascade
+// (CSD, CSM) or a ZoomCascade, whose K channels are windowed alike; the reduction carries R accumulator rows per stage
+// and C tail streams (DESIGN.md 5, "Cross kinds").
 // A group is either all ranks in ONE process (sspsd_group_create: one handle per device, ncclCommInitAll, or
 // direct peer loads over NVLink) or one rank of a multi-process job (sspsd_group_create_rank: torchrun / MPI,
 // ncclCommInitRank with an id made by sspsd_group_unique_id on rank 0).  NCCL is loaded with dlopen at the first
@@ -26,9 +29,11 @@
 #include <new>
 #include <vector>
 
-#include "sspsd_cascade.cuh"
+#include "sspsd_xcascade.cuh"
 
 using sspsd::Cascade;
+using sspsd::XCascade;
+using sspsd::ZoomCascade;
 using sspsd::set_error;
 
 extern "C" int32_t sspsd_source_seek(sspsd_source* s, uint64_t pos);
@@ -238,43 +243,49 @@ uint32_t auto_n_local(uint64_t total, uint32_t world, const Geo& g)
 // ---------------------------------------------------------------------------------------------
 // device helpers of the exchange
 // ---------------------------------------------------------------------------------------------
-// buf[0 .. n_local*stride) = acc rows * factor[stage]; buf[tail_off .. +tail_len) = tail; the rest of buf zero
+// buf[0 .. n_local*R*stride) = acc rows * factor[stage] (R rows of `stride` per stage); tail stream c (tail + c * pitch)
+// at buf[tail_off + c * gap ..][0 .. tail_len); the rest of buf zero
 __global__ void pack_exchange_kernel(double* __restrict__ buf, size_t size, const float* __restrict__ acc, uint32_t n_local,
-                                     size_t stride, const double* __restrict__ factor, const float* __restrict__ tail,
-                                     size_t tail_off, size_t tail_len)
+                                     uint32_t R, size_t stride, const double* __restrict__ factor,
+                                     const float* __restrict__ tail, uint32_t C, size_t pitch, size_t tail_off, size_t gap,
+                                     size_t tail_len)
 {
-    const size_t nacc = (size_t)n_local * stride;
+    const size_t per_stage = (size_t)R * stride, nacc = (size_t)n_local * per_stage;
     for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < size; i += (size_t)gridDim.x * blockDim.x) {
         double v = 0.0;
-        if (i < nacc)
-            v = (double)acc[i] * factor[i / stride];
-        else if (i >= tail_off && i < tail_off + tail_len)
-            v = (double)tail[i - tail_off];
+        if (i < nacc) {
+            v = (double)acc[i] * factor[i / per_stage];
+        } else if (i >= tail_off) {
+            const size_t c = (i - tail_off) / gap, j = (i - tail_off) % gap;
+            if (c < C && j < tail_len) v = (double)tail[c * pitch + j];
+        }
         buf[i] = v;
     }
 }
 
-// rows: buf[0 .. nacc) -> acc (float); gathered tail slices -> one contiguous float stream
+// rows: buf[0 .. nacc) -> acc (float); the gathered tail slices of stream c -> tail_out[c * len ..][0 .. len), one
+// contiguous float stream each (len = out_off[n_ranks]); stream c's slot of rank r is at slot_off[r] + c * gap
 struct UnpackArgs {
     const double* buf;
     float* acc;
     size_t nacc;
     float* tail_out;
-    uint32_t n_ranks;
-    size_t slot_off[SSPSD_GROUP_MAX_RANKS];  // offset of rank r's slot in buf
+    uint32_t n_ranks, C;
+    size_t gap;
+    size_t slot_off[SSPSD_GROUP_MAX_RANKS];  // offset of rank r's slot of stream 0 in buf
     size_t out_off[SSPSD_GROUP_MAX_RANKS + 1];  // prefix sums of the slice lengths
 };
 __global__ void unpack_exchange_kernel(const UnpackArgs a)
 {
-    const size_t total = a.nacc + a.out_off[a.n_ranks];
+    const size_t len = a.out_off[a.n_ranks], total = a.nacc + a.C * len;
     for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total; i += (size_t)gridDim.x * blockDim.x) {
         if (i < a.nacc) {
             a.acc[i] = (float)a.buf[i];
         } else {
-            const size_t j = i - a.nacc;
+            const size_t c = (i - a.nacc) / len, j = (i - a.nacc) % len;
             uint32_t r = 0;
             while (r + 1 < a.n_ranks && j >= a.out_off[r + 1]) ++r;
-            a.tail_out[j] = (float)a.buf[a.slot_off[r] + (j - a.out_off[r])];
+            a.tail_out[c * len + j] = (float)a.buf[a.slot_off[r] + c * a.gap + (j - a.out_off[r])];
         }
     }
 }
@@ -285,15 +296,15 @@ __global__ void unpack_exchange_kernel(const UnpackArgs a)
 struct PeerRows {
     const float* acc[SSPSD_GROUP_MAX_RANKS];
     double factor[SSPSD_GROUP_MAX_RANKS][SSPSD_MAX_STAGES];
-    uint32_t n_ranks, n_local;
+    uint32_t n_ranks, n_local, R;  // R rows of `stride` floats per stage
     size_t stride;
     float* out;
 };
 __global__ void peer_reduce_rows_kernel(const PeerRows a)
 {
-    const size_t n = (size_t)a.n_local * a.stride;
+    const size_t per_stage = (size_t)a.R * a.stride, n = (size_t)a.n_local * per_stage;
     for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (size_t)gridDim.x * blockDim.x) {
-        const uint32_t st = (uint32_t)(i / a.stride);
+        const uint32_t st = (uint32_t)(i / per_stage);
         double s = 0.0;
         for (uint32_t r = 0; r < a.n_ranks; ++r) s += (double)a.acc[r][i] * a.factor[r][st];
         a.out[i] = (float)s;
@@ -317,8 +328,13 @@ struct sspsd_group {
     int32_t reduce = SSPSD_REDUCE_NCCL;
     // channels: cascade of channel c (nullptr if another process owns it)
     std::vector<sspsd_cascade*> chan;
-    // time chunks: one cascade per local rank
+    // what the group computes: SSPSD_GROUP_PSD (cascades) or a cross kind (time chunks only)
+    sspsd_group_kind kind{SSPSD_GROUP_PSD, 1, 0, 0};
+    // time chunks: one cascade per local rank (kind PSD) ...
     std::vector<sspsd_cascade*> tc;
+    // ... or one XCascade (CSD, CSM: owned; zoom: the ZoomCascade's) and, for the zoom kind, its ZoomCascade
+    std::vector<XCascade*> xc;
+    std::vector<ZoomCascade*> zc;
     std::vector<sspsd_time_chunk> plan;  // per GLOBAL rank
     uint64_t total = 0;
     uint32_t n_local_stages = 0;
@@ -349,6 +365,13 @@ struct sspsd_group {
     uint64_t noise_seed = 0;
 
     uint32_t n_local() const { return (uint32_t)devices.size(); }
+    bool cross() const { return kind.kind != SSPSD_GROUP_PSD; }
+    // streams a rank is fed: PSD 1, CSD 2, CSM k, zoom I/Q 2, zoom heterodyne 1
+    uint32_t n_inputs() const
+    {
+        if (kind.kind == SSPSD_GROUP_ZOOM) return kind.zoom_mode == SSPSD_ZOOM_IQ ? 2 : 1;
+        return (uint32_t)kind.channels;
+    }
     bool is_root() const { return first_rank == 0; }
     int local_of(uint32_t rank) const
     {
@@ -403,20 +426,65 @@ int make_cascade(sspsd_group* g, int device, sspsd_cascade** out)
     return rc;
 }
 
+// the handle of a cross kind on `device`: *x its XCascade, *z its ZoomCascade (zoom kind) or nullptr
+int make_xrank(sspsd_group* g, int device, XCascade** x, ZoomCascade** z)
+{
+    sspsd_config c = g->cfg;
+    c.device = device;
+    *x = nullptr;
+    *z = nullptr;
+    int rc;
+    if (g->kind.kind == SSPSD_GROUP_ZOOM) {
+        *z = new (std::nothrow) ZoomCascade();
+        if (!*z) return SSPSD_ENOMEM;
+        rc = (*z)->init(c, g->kind.zoom_mode, g->kind.ftw);
+        *x = &(*z)->x();
+    } else {
+        *x = new (std::nothrow) XCascade();
+        if (!*x) return SSPSD_ENOMEM;
+        rc = (*x)->init(c, g->kind.channels);
+    }
+    if (!rc && g->avg_set) rc = (*x)->set_avg(g->avg);
+    if (!rc && g->detrend) rc = (*x)->set_detrend(g->detrend);
+    return rc;
+}
+
+void destroy_xrank(XCascade* x, ZoomCascade* z)
+{
+    if (z)
+        delete z;
+    else
+        delete x;
+}
+
 int ensure_time_cascades(sspsd_group* g)
 {
-    if (!g->tc.empty()) return SSPSD_OK;
+    if (!g->tc.empty() || !g->xc.empty()) return SSPSD_OK;
     const uint32_t nl = g->n_local();
-    std::vector<sspsd_cascade*> tc(nl, nullptr);
-    for (uint32_t l = 0; l < nl; ++l) {
-        int rc = make_cascade(g, g->devices[l], &tc[l]);
-        if (rc) {
-            // all or nothing: a half-built set would pass the "already made" test above on the next call
-            for (auto* c : tc) sspsd_cascade_destroy(c);
-            return rc;
+    if (g->cross()) {
+        std::vector<XCascade*> xc(nl, nullptr);
+        std::vector<ZoomCascade*> zc(nl, nullptr);
+        for (uint32_t l = 0; l < nl; ++l) {
+            int rc = make_xrank(g, g->devices[l], &xc[l], &zc[l]);
+            if (rc) {
+                for (uint32_t m = 0; m <= l; ++m) destroy_xrank(xc[m], zc[m]);  // all or nothing, as below
+                return rc;
+            }
         }
+        g->xc = xc;
+        if (g->kind.kind == SSPSD_GROUP_ZOOM) g->zc = zc;
+    } else {
+        std::vector<sspsd_cascade*> tc(nl, nullptr);
+        for (uint32_t l = 0; l < nl; ++l) {
+            int rc = make_cascade(g, g->devices[l], &tc[l]);
+            if (rc) {
+                // all or nothing: a half-built set would pass the "already made" test above on the next call
+                for (auto* c : tc) sspsd_cascade_destroy(c);
+                return rc;
+            }
+        }
+        g->tc = tc;
     }
-    g->tc = tc;
     g->fed.assign(nl, 0);
     g->d_buf.assign(nl, nullptr);
     g->d_tail.assign(nl, nullptr);
@@ -424,6 +492,82 @@ int ensure_time_cascades(sspsd_group* g)
     g->buf_cap.assign(nl, 0);
     g->tail_cap.assign(nl, 0);
     return SSPSD_OK;
+}
+
+// a kind is valid for a group of shard mode `mode` and FFT size n: *out is the kind with its channel count filled in
+int check_kind(const sspsd_group_kind* k, int32_t mode, uint32_t n, sspsd_group_kind* out)
+{
+    if (!k) {
+        set_error("null argument");
+        return SSPSD_EINVAL;
+    }
+    sspsd_group_kind v = *k;
+    switch (v.kind) {
+    case SSPSD_GROUP_PSD:
+        if (v.channels == 0) v.channels = 1;
+        if (v.channels != 1 || v.zoom_mode || v.ftw) {
+            set_error("a PSD group has one channel and no carrier");
+            return SSPSD_EINVAL;
+        }
+        break;
+    case SSPSD_GROUP_CSD:
+    case SSPSD_GROUP_ZOOM:
+        if (v.channels == 0) v.channels = 2;
+        if (v.channels != 2) {
+            set_error("CSD and zoom groups have two channels");
+            return SSPSD_EINVAL;
+        }
+        if (v.kind == SSPSD_GROUP_CSD && (v.zoom_mode || v.ftw)) {
+            set_error("a CSD group has no carrier");
+            return SSPSD_EINVAL;
+        }
+        if (v.kind == SSPSD_GROUP_ZOOM && v.zoom_mode != SSPSD_ZOOM_IQ && v.zoom_mode != SSPSD_ZOOM_HETERODYNE) {
+            set_error("unknown zoom mode");
+            return SSPSD_EINVAL;
+        }
+        if (v.kind == SSPSD_GROUP_ZOOM && v.zoom_mode == SSPSD_ZOOM_IQ && v.ftw) {
+            set_error("I/Q mode has no carrier: ftw must be 0");
+            return SSPSD_EINVAL;
+        }
+        break;
+    case SSPSD_GROUP_CSM:
+        if (v.channels < 2 || v.channels > 4 || v.zoom_mode || v.ftw) {
+            set_error("a CSM group has 2 .. 4 channels and no carrier");
+            return SSPSD_EINVAL;
+        }
+        break;
+    default:
+        set_error("unknown group kind");
+        return SSPSD_EINVAL;
+    }
+    if (v.kind != SSPSD_GROUP_PSD) {
+        if (mode != SSPSD_SHARD_TIME) {
+            // every transform of a cross-spectrum is shared by its channels: they cannot live on different GPUs
+            set_error("cross-spectral groups are time-chunked only (SSPSD_SHARD_TIME)");
+            return SSPSD_EINVAL;
+        }
+        if (n < 64 || n > 4096 || (n & (n - 1))) {
+            set_error("cross-spectral groups support n_fft = 64 .. 4096");
+            return SSPSD_EINVAL;
+        }
+    }
+    *out = v;
+    return SSPSD_OK;
+}
+
+// the zoom handle of a local rank takes the rank's input in its own mode; the others take all streams at once
+int process_rank(sspsd_group* g, uint32_t l, const float* const* x, size_t n, int32_t mem)
+{
+    if (g->kind.kind == SSPSD_GROUP_PSD) return g->tc[l]->c.process(x[0], n, mem);
+    if (g->kind.kind != SSPSD_GROUP_ZOOM) return g->xc[l]->process(x, n, mem);
+    if (g->kind.zoom_mode == SSPSD_ZOOM_IQ) return g->zc[l]->process_iq(x[0], x[1], n, mem);
+    return g->zc[l]->process(x[0], n, mem);
+}
+
+int wrong_kind(const char* what)
+{
+    set_error(what);
+    return SSPSD_EINVAL;
 }
 
 }  // namespace
@@ -590,6 +734,48 @@ int32_t sspsd_group_create_rank(const sspsd_config* cfg, const uint8_t id[SSPSD_
     return SSPSD_OK;
 }
 
+int32_t sspsd_group_create_kind(const sspsd_config* cfg, const sspsd_group_kind* kind, const int32_t* devices,
+                                uint32_t n_devices, int32_t shard_mode, sspsd_group** out)
+{
+    if (out) *out = nullptr;
+    sspsd_group_kind k{};
+    if (!cfg || !out) {
+        set_error("null argument");
+        return SSPSD_EINVAL;
+    }
+    int rc = check_kind(kind, shard_mode, cfg->n_fft, &k);
+    if (rc) return rc;
+    rc = sspsd_group_create(cfg, devices, n_devices, shard_mode, out);
+    if (rc) return rc;
+    (*out)->kind = k;
+    return SSPSD_OK;
+}
+
+int32_t sspsd_group_create_kind_rank(const sspsd_config* cfg, const sspsd_group_kind* kind,
+                                     const uint8_t id[SSPSD_GROUP_ID_BYTES], uint32_t rank, uint32_t n_ranks,
+                                     int32_t shard_mode, sspsd_group** out)
+{
+    if (out) *out = nullptr;
+    sspsd_group_kind k{};
+    if (!cfg || !out) {
+        set_error("null argument");
+        return SSPSD_EINVAL;
+    }
+    int rc = check_kind(kind, shard_mode, cfg->n_fft, &k);
+    if (rc) return rc;
+    rc = sspsd_group_create_rank(cfg, id, rank, n_ranks, shard_mode, out);
+    if (rc) return rc;
+    (*out)->kind = k;
+    return SSPSD_OK;
+}
+
+int32_t sspsd_group_kind_of(const sspsd_group* g, sspsd_group_kind* out)
+{
+    if (!g || !out) return SSPSD_EINVAL;
+    *out = g->kind;
+    return SSPSD_OK;
+}
+
 void sspsd_group_destroy(sspsd_group* g)
 {
     if (!g) return;
@@ -600,6 +786,7 @@ void sspsd_group_destroy(sspsd_group* g)
     for (auto* s : g->noise_src) sspsd_source_destroy(s);
     for (auto* c : g->chan) sspsd_cascade_destroy(c);
     for (auto* c : g->tc) sspsd_cascade_destroy(c);
+    for (size_t l = 0; l < g->xc.size(); ++l) destroy_xrank(g->xc[l], g->zc.empty() ? nullptr : g->zc[l]);
     for (uint32_t l = 0; l < g->d_buf.size(); ++l) {
         DevGuard dg(g->devices[l]);
         cudaFree(g->d_buf[l]);
@@ -652,6 +839,14 @@ int32_t sspsd_group_set_avg(sspsd_group* g, sspsd_avg_opts avg)
             int rc = g->tc[l]->c.set_avg(avg);
             if (rc) return rc;
         }
+    for (size_t l = 0; l < g->xc.size(); ++l) {
+        if (g->total && g->fed[l]) {
+            set_error("time-chunked mode: options must be set before the first sample");
+            return SSPSD_EINVAL;
+        }
+        int rc = g->xc[l]->set_avg(avg);
+        if (rc) return rc;
+    }
     return SSPSD_OK;
 }
 
@@ -677,6 +872,10 @@ int32_t sspsd_group_set_detrend(sspsd_group* g, int32_t d)
             int rc = c->c.set_detrend(d);
             if (rc) return rc;
         }
+    for (auto* x : g->xc) {
+        int rc = x->set_detrend(d);
+        if (rc) return rc;
+    }
     return SSPSD_OK;
 }
 
@@ -738,6 +937,10 @@ int32_t sspsd_group_sync(sspsd_group* g)
             int rc = c->c.sync();
             if (rc) return rc;
         }
+    for (size_t l = 0; l < g->xc.size(); ++l) {
+        int rc = g->zc.empty() ? g->xc[l]->sync() : g->zc[l]->sync();
+        if (rc) return rc;
+    }
     return SSPSD_OK;
 }
 
@@ -745,6 +948,7 @@ int32_t sspsd_group_psd(sspsd_group* g, uint32_t channel, const sspsd_merge_opts
                         sspsd_break* b, size_t* b_len)
 {
     if (!g || !p_len || !b_len) return SSPSD_EINVAL;
+    if (g->cross()) return wrong_kind("a cross-spectral group reads out with sspsd_group_csd_read / _csm_read / _zoom_read");
     sspsd_merge_opts o{0, 1, 0};
     if (opts) o = *opts;
     if (g->mode == SSPSD_SHARD_TIME) {
@@ -921,6 +1125,10 @@ int32_t sspsd_group_time_plan(sspsd_group* g, uint64_t total, uint32_t n_local_s
         rc = c->c.reset();
         if (rc) return rc;
     }
+    for (size_t l = 0; l < g->xc.size(); ++l) {
+        rc = g->zc.empty() ? g->xc[l]->reset() : g->zc[l]->reset();
+        if (rc) return rc;
+    }
     g->total = total;
     g->n_local_stages = n_local_stages;
     g->finished = false;
@@ -928,10 +1136,17 @@ int32_t sspsd_group_time_plan(sspsd_group* g, uint64_t total, uint32_t n_local_s
     for (uint32_t r = 0; r < g->n_ranks; ++r) plan_rank(total, g->n_ranks, r, geo, n_local_stages, &g->plan[r]);
     for (uint32_t l = 0; l < g->n_local(); ++l) {
         const sspsd_time_chunk& pl = g->plan[g->first_rank + l];
-        Cascade& c = g->tc[l]->c;
-        rc = c.seek(pl.feed_lo);
-        if (rc) return rc;
-        rc = c.set_window(pl.own_lo, pl.own_hi, n_local_stages);
+        if (g->cross()) {
+            // the zoom kind's mixer starts at the rank's absolute position: phi_n = (n ftw) mod 2^32 of the whole stream
+            rc = g->zc.empty() ? g->xc[l]->seek(pl.feed_lo) : g->zc[l]->seek(pl.feed_lo);
+            if (rc) return rc;
+            rc = g->xc[l]->set_window(pl.own_lo, pl.own_hi, n_local_stages);
+        } else {
+            Cascade& c = g->tc[l]->c;
+            rc = c.seek(pl.feed_lo);
+            if (rc) return rc;
+            rc = c.set_window(pl.own_lo, pl.own_hi, n_local_stages);
+        }
         if (rc) return rc;
         g->fed[l] = 0;
     }
@@ -948,7 +1163,7 @@ int32_t sspsd_group_time_chunk(const sspsd_group* g, uint32_t rank, sspsd_time_c
     return SSPSD_OK;
 }
 
-int32_t sspsd_group_time_process_f32(sspsd_group* g, uint32_t rank, const float* x, size_t n, int32_t mem)
+int32_t sspsd_group_time_process_multi_f32(sspsd_group* g, uint32_t rank, const float* const* x, size_t n, int32_t mem)
 {
     if (!g || g->mode != SSPSD_SHARD_TIME || g->plan.empty()) {
         set_error("no plan (call sspsd_group_time_plan first)");
@@ -961,14 +1176,55 @@ int32_t sspsd_group_time_process_f32(sspsd_group* g, uint32_t rank, const float*
         set_error("more samples than the rank's range [feed_lo, feed_hi)");
         return SSPSD_EINVAL;
     }
-    int rc = g->tc[l]->c.process(x, n, mem);
+    if (n && !x) {
+        set_error("null input");
+        return SSPSD_EINVAL;
+    }
+    for (uint32_t i = 0; n && i < g->n_inputs(); ++i)
+        if (!x[i]) {
+            set_error("null input");
+            return SSPSD_EINVAL;
+        }
+    int rc = n ? process_rank(g, (uint32_t)l, x, n, mem) : SSPSD_OK;
     if (rc) return rc;
     g->fed[l] += n;
     return SSPSD_OK;
 }
 
+int32_t sspsd_group_time_process_f32(sspsd_group* g, uint32_t rank, const float* x, size_t n, int32_t mem)
+{
+    if (g && g->cross()) return wrong_kind("a cross-spectral group takes sspsd_group_time_process_multi_f32");
+    return sspsd_group_time_process_multi_f32(g, rank, &x, n, mem);
+}
+
+int32_t sspsd_group_time_process_all_multi_f32(sspsd_group* g, const float* const* x, size_t n)
+{
+    if (!g || g->mode != SSPSD_SHARD_TIME || g->plan.empty() || g->multi_process) {
+        set_error("needs a planned single-process time-chunked group");
+        return SSPSD_EINVAL;
+    }
+    if (n != g->total || !x) {
+        set_error("x must hold the whole planned stream");
+        return SSPSD_EINVAL;
+    }
+    for (uint32_t i = 0; i < g->n_inputs(); ++i)
+        if (!x[i]) {
+            set_error("null input");
+            return SSPSD_EINVAL;
+        }
+    for (uint32_t r = 0; r < g->n_ranks; ++r) {
+        const sspsd_time_chunk& pl = g->plan[r];
+        const float* xs[4];
+        for (uint32_t i = 0; i < g->n_inputs(); ++i) xs[i] = x[i] + pl.feed_lo;
+        int rc = sspsd_group_time_process_multi_f32(g, r, xs, (size_t)(pl.feed_hi - pl.feed_lo), SSPSD_MEM_HOST);
+        if (rc) return rc;
+    }
+    return SSPSD_OK;
+}
+
 int32_t sspsd_group_time_process_all_f32(sspsd_group* g, const float* x, size_t n)
 {
+    if (g && g->cross()) return wrong_kind("a cross-spectral group takes sspsd_group_time_process_all_multi_f32");
     if (!g || g->mode != SSPSD_SHARD_TIME || g->plan.empty() || g->multi_process) {
         set_error("needs a planned single-process time-chunked group");
         return SSPSD_EINVAL;
@@ -987,6 +1243,7 @@ int32_t sspsd_group_time_process_all_f32(sspsd_group* g, const float* x, size_t 
 
 int32_t sspsd_group_time_process_noise(sspsd_group* g, int64_t exponent, uint64_t seed)
 {
+    if (g && g->cross()) return wrong_kind("device-generated noise feeds PSD groups only");
     if (!g || g->mode != SSPSD_SHARD_TIME || g->plan.empty()) {
         set_error("no plan (call sspsd_group_time_plan first)");
         return SSPSD_EINVAL;
@@ -1027,8 +1284,11 @@ int32_t sspsd_group_time_finish(sspsd_group* g)
     const uint32_t K = g->n_local_stages, W = g->n_ranks, NL = g->n_local();
     const std::vector<StreamSt> st = stream_state(g->total, geo);
     const size_t stride = ((size_t)g->cfg.n_fft / 2 + 1 + 63) & ~(size_t)63;
+    // R accumulator rows per stage, C tail streams (PSD: 1 and 1; CSD 4 and 2, CSM k >= 3 16 and k, zoom 2 and 2)
+    const uint32_t R = g->cross() ? (uint32_t)g->xc[0]->block_rows() : 1;
+    const uint32_t C = g->cross() ? (uint32_t)g->xc[0]->channels() : 1;
     // layout of the single reduction buffer (float64 words):
-    // [K accumulator rows of `stride`] [W tail slots of `slot`] [K counts] [W x (first, length)]
+    // [K stages x R accumulator rows of `stride`] [C tail streams x W slots of `slot`] [K counts] [W x (first, length)]
     const uint64_t tail_total = st.size() > K ? st[K].L : 0;
     // slot = the longest slice any rank owns (the ownership boundaries are cut in stage-0 samples, so the slices
     // differ by a few samples; every rank derives the same number from the plan)
@@ -1037,13 +1297,13 @@ int32_t sspsd_group_time_finish(sspsd_group* g)
         const uint64_t hi = std::min<uint64_t>(g->plan[r].tail_hi, tail_total), lo = std::min<uint64_t>(g->plan[r].tail_lo, hi);
         slot = std::max<size_t>(slot, (size_t)(hi - lo) + 64);
     }
-    const size_t nacc = (size_t)K * stride, meta = nacc + (size_t)W * slot, size = meta + K + 2 * (size_t)W;
+    const size_t nacc = (size_t)K * R * stride, gap = (size_t)W * slot, meta = nacc + C * gap, size = meta + K + 2 * (size_t)W;
     for (uint32_t l = 0; l < NL; ++l)
         if (g->fed[l] != g->plan[g->first_rank + l].feed_hi - g->plan[g->first_rank + l].feed_lo) {
             set_error("a rank has not been fed its whole range yet");
             return SSPSD_EINVAL;
         }
-    // ---- per local rank: wait, export the tail slice, weight the rows for what follows the rank's chunk ----
+    // ---- per local rank: wait, export the tail slices, weight the rows for what follows the rank's chunk ----
     std::vector<std::vector<double>> factor(NL, std::vector<double>(SSPSD_MAX_STAGES, 1.0));
     std::vector<std::vector<double>> book(NL, std::vector<double>(K + 2 * (size_t)W, 0.0));
     std::vector<sspsd_partials> parts(NL);
@@ -1052,22 +1312,35 @@ int32_t sspsd_group_time_finish(sspsd_group* g)
     for (uint32_t l = 0; l < NL; ++l) {
         const uint32_t r = g->first_rank + l;
         const sspsd_time_chunk& pl = g->plan[r];
-        Cascade& c = g->tc[l]->c;
         DevGuard dg(g->devices[l]);
         if (!dg.ok) return SSPSD_ECUDA;
-        if (slot > g->tail_cap[l]) {
+        if (C * slot > g->tail_cap[l]) {
             cudaFree(g->d_tail[l]);
             g->d_tail[l] = nullptr;
-            SSPSD_CUDA(cudaMalloc(&g->d_tail[l], slot * sizeof(float)));
-            g->tail_cap[l] = slot;
+            SSPSD_CUDA(cudaMalloc(&g->d_tail[l], C * slot * sizeof(float)));
+            g->tail_cap[l] = C * slot;
         }
         if (!g->d_factor[l]) SSPSD_CUDA(cudaMalloc(&g->d_factor[l], SSPSD_MAX_STAGES * sizeof(double)));
         size_t n = slot;
-        int rc = c.take_tail(pl.tail_lo, pl.tail_hi, g->d_tail[l], &n, &tfirst[l], SSPSD_MEM_DEVICE);  // (synchronises)
+        int rc;
+        if (g->cross()) {
+            if (!g->zc.empty()) {
+                rc = g->zc[l]->flush();  // the zoom handle's staged host input
+                if (rc) return rc;
+            }
+            float* outs[4];
+            for (uint32_t c = 0; c < C; ++c) outs[c] = g->d_tail[l] + c * slot;
+            rc = g->xc[l]->take_tail(pl.tail_lo, pl.tail_hi, outs, &n, &tfirst[l]);  // (synchronises)
+            if (rc) return rc;
+            rc = g->xc[l]->partials(&parts[l]);
+        } else {
+            Cascade& c = g->tc[l]->c;
+            rc = c.take_tail(pl.tail_lo, pl.tail_hi, g->d_tail[l], &n, &tfirst[l], SSPSD_MEM_DEVICE);  // (synchronises)
+            if (rc) return rc;
+            rc = c.partials(&parts[l]);
+        }
         if (rc) return rc;
         tlen[l] = n;
-        rc = c.partials(&parts[l]);
-        if (rc) return rc;
         // EWMA (psd.rs:218-225) follows the GLOBAL segment order: a rank's row is normalised as if the stream
         // ended after its last owned segment b; every later segment j rescales by g = avg/(avg+1) iff j >= avg+1
         for (uint32_t i = 0; i < K; ++i) {
@@ -1084,9 +1357,9 @@ int32_t sspsd_group_time_finish(sspsd_group* g)
         book[l][K + 2 * r] = (double)tfirst[l];
         book[l][K + 2 * r + 1] = (double)tlen[l];
     }
+    auto rank_stream = [&](uint32_t l) { return g->cross() ? g->xc[l]->stream() : g->tc[l]->c.stream(); };
     // ---- combine: rows and counts are summed, the slices land in disjoint slots ----
     std::vector<double> red_book(K + 2 * (size_t)W, 0.0);
-    Cascade& root = g->tc[0]->c;
     const bool have_root = g->is_root();
     if (!g->comms.empty()) {
         for (uint32_t l = 0; l < NL; ++l) {
@@ -1097,28 +1370,28 @@ int32_t sspsd_group_time_finish(sspsd_group* g)
                 SSPSD_CUDA(cudaMalloc(&g->d_buf[l], size * sizeof(double)));
                 g->buf_cap[l] = size;
             }
-            cudaStream_t s = g->tc[l]->c.stream();
+            cudaStream_t s = rank_stream(l);
             SSPSD_CUDA(cudaMemcpyAsync(g->d_factor[l], factor[l].data(), SSPSD_MAX_STAGES * sizeof(double), cudaMemcpyHostToDevice, s));
             const uint32_t r = g->first_rank + l;
-            pack_exchange_kernel<<<296, 256, 0, s>>>(g->d_buf[l], meta, parts[l].acc, K, stride, g->d_factor[l], g->d_tail[l],
-                                                     nacc + (size_t)r * slot, tlen[l]);
+            pack_exchange_kernel<<<296, 256, 0, s>>>(g->d_buf[l], meta, parts[l].acc, K, R, stride, g->d_factor[l], g->d_tail[l],
+                                                     C, slot, nacc + (size_t)r * slot, gap, tlen[l]);
             SSPSD_CUDA(cudaGetLastError());
             SSPSD_CUDA(cudaMemcpyAsync(g->d_buf[l] + meta, book[l].data(), book[l].size() * sizeof(double), cudaMemcpyHostToDevice, s));
         }
         SSPSD_NCCL(nccl().GroupStart());
         for (uint32_t l = 0; l < NL; ++l) {
             DevGuard dg(g->devices[l]);
-            SSPSD_NCCL(nccl().Reduce(g->d_buf[l], g->d_buf[l], size, ncclFloat64, ncclSum, 0, g->comms[l], g->tc[l]->c.stream()));
+            SSPSD_NCCL(nccl().Reduce(g->d_buf[l], g->d_buf[l], size, ncclFloat64, ncclSum, 0, g->comms[l], rank_stream(l)));
         }
         SSPSD_NCCL(nccl().GroupEnd());
         if (have_root) {
             DevGuard dg(g->devices[0]);
             SSPSD_CUDA(cudaMemcpyAsync(red_book.data(), g->d_buf[0] + meta, red_book.size() * sizeof(double), cudaMemcpyDeviceToHost,
-                                       root.stream()));
+                                       rank_stream(0)));
         }
         for (uint32_t l = 0; l < NL; ++l) {
             DevGuard dg(g->devices[l]);
-            SSPSD_CUDA(cudaStreamSynchronize(g->tc[l]->c.stream()));
+            SSPSD_CUDA(cudaStreamSynchronize(rank_stream(l)));
         }
     } else {
         // all ranks in this process: the root kernel reads the peers' rows in place (fixed order, f64)
@@ -1129,13 +1402,15 @@ int32_t sspsd_group_time_finish(sspsd_group* g)
         g->finished = true;
         return SSPSD_OK;
     }
-    // ---- root: install rows + bookkeeping, gather the slices into one stream, run the deep stages ----
+    // ---- root: install rows + bookkeeping, gather the slices into one stream per channel, run the deep stages ----
     DevGuard dg(g->devices[0]);
     if (!dg.ok) return SSPSD_ECUDA;
     std::vector<uint64_t> first(W), len(W);
     uint64_t pos = 0;
     UnpackArgs ua{};
     ua.n_ranks = W;
+    ua.C = C;
+    ua.gap = gap;
     ua.nacc = nacc;
     for (uint32_t r = 0; r < W; ++r) {
         first[r] = (uint64_t)std::llround(red_book[K + 2 * r]);
@@ -1158,16 +1433,17 @@ int32_t sspsd_group_time_finish(sspsd_group* g)
             set_error("internal: reduced segment count differs from the closed form");
             return SSPSD_EINVAL;
         }
-    if (pos > g->tail_all_cap) {
+    // the gathered stream of channel c at d_tail_all + c * pos
+    if (C * pos > g->tail_all_cap) {
         cudaFree(g->d_tail_all);
         g->d_tail_all = nullptr;
-        SSPSD_CUDA(cudaMalloc(&g->d_tail_all, (pos + 64) * sizeof(float)));
-        g->tail_all_cap = pos;
+        SSPSD_CUDA(cudaMalloc(&g->d_tail_all, (C * pos + 64) * sizeof(float)));
+        g->tail_all_cap = C * pos;
     }
     sspsd_partials pr;
-    int rc = root.partials(&pr);
+    int rc = g->cross() ? g->xc[0]->partials(&pr) : g->tc[0]->c.partials(&pr);
     if (rc) return rc;
-    cudaStream_t rs = root.stream();
+    cudaStream_t rs = rank_stream(0);
     if (!g->comms.empty()) {
         ua.buf = g->d_buf[0];
         ua.acc = pr.acc;
@@ -1178,6 +1454,7 @@ int32_t sspsd_group_time_finish(sspsd_group* g)
         PeerRows a{};
         a.n_ranks = NL;
         a.n_local = K;
+        a.R = R;
         a.stride = stride;
         a.out = pr.acc;
         for (uint32_t l = 0; l < NL; ++l) {
@@ -1187,29 +1464,92 @@ int32_t sspsd_group_time_finish(sspsd_group* g)
         peer_reduce_rows_kernel<<<148, 256, 0, rs>>>(a);
         SSPSD_CUDA(cudaGetLastError());
         for (uint32_t l = 0; l < NL; ++l)
-            if (tlen[l]) {
+            for (uint32_t c = 0; c < C && tlen[l]; ++c) {
+                float* dst = g->d_tail_all + c * pos + ua.out_off[l];
+                const float* src = g->d_tail[l] + c * slot;
                 if (g->devices[l] == g->devices[0])
-                    SSPSD_CUDA(cudaMemcpyAsync(g->d_tail_all + ua.out_off[l], g->d_tail[l], tlen[l] * sizeof(float),
-                                               cudaMemcpyDeviceToDevice, rs));
+                    SSPSD_CUDA(cudaMemcpyAsync(dst, src, tlen[l] * sizeof(float), cudaMemcpyDeviceToDevice, rs));
                 else
-                    SSPSD_CUDA(cudaMemcpyPeerAsync(g->d_tail_all + ua.out_off[l], g->devices[0], g->d_tail[l], g->devices[l],
-                                                   tlen[l] * sizeof(float), rs));
+                    SSPSD_CUDA(cudaMemcpyPeerAsync(dst, g->devices[0], src, g->devices[l], tlen[l] * sizeof(float), rs));
             }
     }
     for (uint32_t i = 0; i < K && i < st.size(); ++i) {
         const uint32_t a = stage_avg_of(g->avg, i);
-        rc = root.set_stream_state(i, st[i].L, a == 0xffffffffu ? st[i].craw : std::min<uint64_t>(st[i].craw, (uint64_t)a + 1));
+        const uint64_t segs = a == 0xffffffffu ? st[i].craw : std::min<uint64_t>(st[i].craw, (uint64_t)a + 1);
+        rc = g->cross() ? g->xc[0]->set_stream_state(i, st[i].L, segs) : g->tc[0]->c.set_stream_state(i, st[i].L, segs);
         if (rc) return rc;
     }
     SSPSD_CUDA(cudaStreamSynchronize(rs));  // process_stage copies on the stage's own stream
     if (pos) {
-        rc = root.process_stage(K, g->d_tail_all, (size_t)pos, SSPSD_MEM_DEVICE);
+        if (g->cross()) {
+            // the zoom kind's tails are the mixed I and Q: the deep stages take them as they are
+            const float* xs[4];
+            for (uint32_t c = 0; c < C; ++c) xs[c] = g->d_tail_all + c * pos;
+            rc = g->xc[0]->process_stage(K, xs, (size_t)pos);
+        } else {
+            rc = g->tc[0]->c.process_stage(K, g->d_tail_all, (size_t)pos, SSPSD_MEM_DEVICE);
+        }
         if (rc) return rc;
     }
-    rc = root.sync();
+    rc = g->cross() ? g->xc[0]->sync() : g->tc[0]->c.sync();
     if (rc) return rc;
     g->finished = true;
     return SSPSD_OK;
+}
+
+// ---------------------------------------------------------------------------------------------
+// readouts of the cross kinds: rank 0's handle after sspsd_group_time_finish (lengths 0 on the other processes)
+// ---------------------------------------------------------------------------------------------
+namespace {
+int cross_ready(sspsd_group* g, int32_t kind, size_t* p_len, size_t* b_len, bool* empty)
+{
+    *empty = false;
+    if (!g || !p_len || !b_len) return SSPSD_EINVAL;
+    if (g->kind.kind != kind) return wrong_kind("the readout does not match the group's kind");
+    if (!g->finished) {
+        set_error("time-chunked group: call sspsd_group_time_finish first");
+        return SSPSD_EINVAL;
+    }
+    if (!g->is_root()) {
+        *p_len = 0;
+        *b_len = 0;
+        *empty = true;
+    }
+    return SSPSD_OK;
+}
+}  // namespace
+
+int32_t sspsd_group_csd_read(sspsd_group* g, const sspsd_merge_opts* opts, float* pxx, float* pyy, float* pxy,
+                             size_t* p_len, sspsd_break* b, size_t* b_len)
+{
+    bool empty;
+    int rc = cross_ready(g, SSPSD_GROUP_CSD, p_len, b_len, &empty);
+    if (rc || empty) return rc;
+    sspsd_merge_opts o{0, 1, 0};
+    if (opts) o = *opts;
+    return g->xc[0]->read(o, pxx, pyy, pxy, p_len, b, b_len);
+}
+
+int32_t sspsd_group_csm_read(sspsd_group* g, const sspsd_merge_opts* opts, float* s, size_t* p_len, sspsd_break* b,
+                             size_t* b_len)
+{
+    bool empty;
+    int rc = cross_ready(g, SSPSD_GROUP_CSM, p_len, b_len, &empty);
+    if (rc || empty) return rc;
+    sspsd_merge_opts o{0, 1, 0};
+    if (opts) o = *opts;
+    return g->xc[0]->read_matrix(o, s, p_len, b, b_len);
+}
+
+int32_t sspsd_group_zoom_read(sspsd_group* g, const sspsd_merge_opts* opts, float* p_pos, float* p_neg, size_t* p_len,
+                              sspsd_break* b, size_t* b_len)
+{
+    bool empty;
+    int rc = cross_ready(g, SSPSD_GROUP_ZOOM, p_len, b_len, &empty);
+    if (rc || empty) return rc;
+    sspsd_merge_opts o{0, 1, 0};
+    if (opts) o = *opts;
+    return g->zc[0]->read(o, p_pos, p_neg, p_len, b, b_len);
 }
 
 }  // extern "C"

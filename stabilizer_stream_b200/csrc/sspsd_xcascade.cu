@@ -17,7 +17,7 @@
 // CSD) has exactly the first four rows.  K = 3 runs pair (2,3)'s csd_stage_kernel with channel 2 in both slots:
 // its rows 1..3 are S22 again and are never read.  The two-sided kind (K = 2, DESIGN.md 3c) runs iq_stage_kernel
 // instead: a block of two rows, P+ and P-.
-#include "sspsd_cascade.cuh"
+#include "sspsd_xcascade.cuh"
 
 #include <algorithm>
 #include <cmath>
@@ -32,19 +32,7 @@ namespace sspsd {
 
 namespace {
 
-// One of the block kernels at one N, its rows and its shared-memory budget per CTA
-struct BlockKernel {
-    void (*fn)(XStageParams);
-    size_t (*smem)(int T, int hop);  // bytes for tiles of T segments
-    long long budget;
-    int rows;
-    const char* what;
-};
-enum { DIAG = 0, CROSS = 1, IQ = 2 };
-struct BlockKernels {
-    BlockKernel k[3];  // [DIAG]: csd_stage_kernel, [CROSS]: csm_cross_kernel, [IQ]: iq_stage_kernel
-    int nt, groups;    // threads per CTA, segments in flight per CTA (all kernels)
-};
+enum { DIAG = 0, CROSS = 1, IQ = 2 };  // BlockKernels::k
 
 template <int LOG2N>
 BlockKernels block_kernels_t()
@@ -112,78 +100,7 @@ TiledLaunch tiled_launch(uint64_t nseg, int groups, int tmax, int hop, int n, in
 
 }  // namespace
 
-class XCascade : public StageHook {
-public:
-    XCascade() = default;
-    ~XCascade();
-    int init(const sspsd_config& cfg, int k, bool two_sided = false);
-    int clone_from(XCascade& o);
-    int reset();
-    int process(const float* const* x, size_t n, int mem);
-    int set_avg(sspsd_avg_opts a);
-    int set_detrend(int d);
-    int flush();
-    int sync();
-    int read(const sspsd_merge_opts& o, float* pxx, float* pyy, float* pxy, size_t* p_len, sspsd_break* b,
-             size_t* b_len);
-    int read_matrix(const sspsd_merge_opts& o, float* s, size_t* p_len, sspsd_break* b, size_t* b_len);
-    int read_two_sided(const sspsd_merge_opts& o, float* p_pos, float* p_neg, size_t* p_len, sspsd_break* b,
-                       size_t* b_len);
-    int num_stages(uint32_t* n);
-    int channels() const { return k_; }
-    int device() const { return cfg_.device; }
-    float rbw() const { return ch_[0].rbw(); }
-    cudaStream_t stream() const { return stream_; }
-    int stage_psd(Cascade& c, size_t i, const StreamSrc& src, uint64_t k0, uint64_t nseg, const EwmaPlan& e) override;
-
-private:
-    int setup(const sspsd_config& cfg, int k, bool two_sided);
-    sspsd_config channel_cfg() const;
-    int feed_chunk(const float* const* x, size_t n, bool device);
-    int flush_staged();
-    int flush_all();
-    size_t block_rows() const { return two_sided_ ? IQ_ROWS : k_ == 2 ? CSD_ROWS : 2 * CSD_ROWS + CSM_XROWS; }
-    size_t acc_floats() const { return (size_t)SSPSD_MAX_STAGES * block_rows() * stride_; }
-    int ensure_part(float** part, size_t* cap, size_t need);
-    int launch_block(int kind, XStageParams p, uint64_t nseg, float* acc, float** part, size_t* part_cap);
-    int read_rows(const sspsd_merge_opts& o, bool outs, size_t* p_len, sspsd_break* b, size_t* b_len,
-                  uint64_t (&book)[4 * SSPSD_MAX_STAGES + 2], size_t* pl, size_t* ns);
-
-    // destroyed after the channels, whose destructors still synchronise the stream
-    struct OwnedStream {
-        cudaStream_t s = nullptr;
-        int device = 0;
-        ~OwnedStream()
-        {
-            if (!s) return;
-            DeviceGuard g(device);
-            cudaStreamDestroy(s);
-        }
-    } own_;
-    Cascade ch_[4];  // channel 0 launches the block kernels; 1 .. k_-1 leave their sources
-    int k_ = 2;
-    bool two_sided_ = false;  // K = 2: iq_stage_kernel's rows P+, P- instead of the CSD's four
-    sspsd_config cfg_{};
-    cudaStream_t stream_ = nullptr;
-    uint32_t n_ = 0, log2n_ = 0;
-    int num_sms_ = 148;
-    BlockKernels kern_{};
-    int tmax_[3] = {1, 1, 1};  // largest tile of each block kernel
-    uint32_t stride_ = 0;  // floats per row; a stage's block is block_rows() rows
-    float* d_win_ = nullptr;
-    float2* d_tw_ = nullptr;
-    float* d_acc_ = nullptr;  // [SSPSD_MAX_STAGES][block_rows()][stride_]
-    float* h_acc_ = nullptr;
-    float* d_part_ = nullptr;   // deterministic mode: csd_stage_kernel's partial blocks
-    size_t part_cap_ = 0;
-    float* d_xpart_ = nullptr;  // and csm_cross_kernel's (another row layout: its padding must stay zero too)
-    size_t xpart_cap_ = 0;
-    struct Source {
-        StreamSrc src;
-        uint64_t k0, nseg;
-        bool valid;
-    } srcs_[4][SSPSD_MAX_STAGES] = {};
-};
+size_t XCascade::block_rows() const { return two_sided_ ? IQ_ROWS : k_ == 2 ? CSD_ROWS : 2 * CSD_ROWS + CSM_XROWS; }
 
 XCascade::~XCascade()
 {
@@ -610,6 +527,80 @@ int XCascade::num_stages(uint32_t* n)
     return SSPSD_OK;
 }
 
+// Time-chunk mode: the channels' bookkeeping stays identical, so windowed channels still run the same stages over the
+// same (owned) segment ranges and channel 0's hook launches the block kernels over exactly the segments the rank owns.
+int XCascade::seek(uint64_t pos)
+{
+    for (int c = 0; c < k_; ++c) {
+        int rc = ch_[c].seek(pos);
+        if (rc) return rc;
+    }
+    return SSPSD_OK;
+}
+
+int XCascade::set_window(uint64_t own_lo, uint64_t own_hi, uint32_t n_local)
+{
+    for (int c = 0; c < k_; ++c) {
+        int rc = ch_[c].set_window(own_lo, own_hi, n_local);
+        if (rc) return rc;
+    }
+    return SSPSD_OK;
+}
+
+int XCascade::take_tail(uint64_t j_lo, uint64_t j_hi, float* const* out, size_t* len, uint64_t* first)
+{
+    int rc = sync();  // staged input in lockstep first: the channels' own sync() then finds nothing to run
+    if (rc) return rc;
+    const size_t cap = *len;
+    for (int c = 0; c < k_; ++c) {
+        *len = cap;
+        rc = ch_[c].take_tail(j_lo, j_hi, out[c], len, first, SSPSD_MEM_DEVICE);
+        if (rc) return rc;
+    }
+    return SSPSD_OK;
+}
+
+// feed_chunk's order for a deep stage: per chunk, channels k_-1 .. 1 leave their sources, then channel 0 launches
+int XCascade::process_stage(uint32_t stage, const float* const* x, size_t n)
+{
+    DeviceGuard g(cfg_.device);
+    if (!g.ok) return SSPSD_ECUDA;
+    int rc = flush_all();
+    if (rc) return rc;
+    const size_t chunk = (size_t)ch_[0].cfg_.max_batch;
+    for (size_t pos = 0; pos < n; pos += chunk) {
+        const size_t m = std::min(chunk, n - pos);
+        for (int c = k_ - 1; c >= 0; --c) {
+            rc = ch_[c].process_stage(stage, x[c] + pos, m, SSPSD_MEM_DEVICE);
+            if (rc) return rc;
+        }
+    }
+    return SSPSD_OK;
+}
+
+int XCascade::set_stream_state(uint32_t stage, uint64_t samples, uint64_t segments)
+{
+    for (int c = 0; c < k_; ++c) {
+        int rc = ch_[c].set_stream_state(stage, samples, segments);
+        if (rc) return rc;
+    }
+    return SSPSD_OK;
+}
+
+int XCascade::partials(sspsd_partials* out)
+{
+    if (!out) return SSPSD_EINVAL;
+    DeviceGuard g(cfg_.device);
+    if (!g.ok) return SSPSD_ECUDA;
+    int rc = flush_all();
+    if (rc) return rc;
+    rc = ch_[0].partials(out);  // the counts (every channel has the same)
+    if (rc) return rc;
+    out->acc = d_acc_;
+    out->acc_stride = stride_;
+    return SSPSD_OK;
+}
+
 // The common start of read() and read_matrix(): flush, export the book, size the readout (*pl bins, *ns breaks) and
 // check the caller's capacity (outs: the output pointers are non-null), then copy every stage's block to h_acc_.
 // With nothing to merge (*ns == 0) or too little room, *p_len and *b_len are set here and the caller returns rc.
@@ -752,52 +743,6 @@ int XCascade::read_matrix(const sspsd_merge_opts& o, float* s, size_t* p_len, ss
 }
 
 
-// ZoomCascade: the two-sided XCascade over z = i + i q, fed either I/Q streams as they are (SSPSD_ZOOM_IQ) or one real
-// stream mixed down by the carrier ftw / 2^32 (SSPSD_ZOOM_HETERODYNE, DESIGN.md 3c).  The mixer runs on the
-// XCascade's one stream into buffers owned here, which the XCascade then reads in place (SSPSD_MEM_DEVICE): stream
-// order alone makes their reuse by the next mixer launch safe.  Host input is collected in pinned staging buffers,
-// as Cascade::process_host collects small calls, and goes to the device by cudaMemcpyAsync on the same stream.
-class ZoomCascade {
-public:
-    ~ZoomCascade();
-    int init(const sspsd_config& cfg, int mode, uint32_t ftw);
-    int clone_from(ZoomCascade& o);
-    int reset();
-    int process_iq(const float* i, const float* q, size_t n, int mem);
-    int process(const float* x, size_t n, int mem);
-    int process_device_mixed(const float* x, size_t n);  // x: device memory valid in stream order
-    int set_avg(sspsd_avg_opts a);
-    int set_detrend(int d);
-    int flush();
-    int sync();
-    int read(const sspsd_merge_opts& o, float* p_pos, float* p_neg, size_t* p_len, sspsd_break* b, size_t* b_len);
-    int num_stages(uint32_t* n);
-    int mode() const { return mode_; }
-    uint32_t ftw() const { return ftw_; }
-    XCascade& x() { return x_; }
-    const XCascade& x() const { return x_; }
-
-private:
-    int ensure_mix();
-    int flush_host();
-    int mix_and_feed(const float* d_x, size_t n);
-
-    XCascade x_;
-    int mode_ = SSPSD_ZOOM_IQ;
-    uint32_t ftw_ = 0;
-    uint64_t pos_ = 0;  // absolute index of the next sample mixed: phi_n = (n ftw) mod 2^32
-    size_t mix_cap_ = 0;  // samples per mixer launch (a multiple of 4) and of d_i_, d_q_
-    float* d_i_ = nullptr;
-    float* d_q_ = nullptr;
-    size_t stage_cap_ = 0;  // host staging, cfg.host_stage rounded to a multiple of 4: pinned h_stage_[2], d_x_
-    float* h_stage_[2] = {nullptr, nullptr};
-    float* d_x_ = nullptr;
-    cudaEvent_t ev_stage_[2] = {nullptr, nullptr};  // the H2D copy of h_stage_[b] has completed
-    bool stage_pending_[2] = {false, false};
-    int stage_buf_ = 0;
-    size_t staged_ = 0;
-};
-
 ZoomCascade::~ZoomCascade()
 {
     if (!d_i_ && !h_stage_[0]) return;
@@ -847,6 +792,18 @@ int ZoomCascade::reset()
     if (rc) return rc;
     pos_ = 0;
     staged_ = 0;
+    return SSPSD_OK;
+}
+
+int ZoomCascade::seek(uint64_t pos)
+{
+    if (staged_) {
+        set_error("seek() needs a fresh cascade");
+        return SSPSD_EINVAL;
+    }
+    int rc = x_.seek(pos);
+    if (rc) return rc;
+    pos_ = pos;
     return SSPSD_OK;
 }
 
@@ -996,18 +953,6 @@ int ZoomCascade::num_stages(uint32_t* n)
 }
 
 }  // namespace sspsd
-
-struct sspsd_csd {
-    sspsd::XCascade c;
-};
-
-struct sspsd_csm {
-    sspsd::XCascade c;
-};
-
-struct sspsd_zoom {
-    sspsd::ZoomCascade z;
-};
 
 using sspsd::set_error;
 

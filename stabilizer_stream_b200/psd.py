@@ -183,6 +183,49 @@ def _config(n, window, hbf, device, stream, max_batch, host_stage, deep_defer=0,
     return cfg
 
 
+def _merge_opts(opts):
+    opts = opts or MergeOpts()
+    return L.MergeOptsC(int(opts.keep_overlap), opts.min_count, int(opts.keep_transition_band))
+
+
+def _read_csd(read, h, n, opts):
+    """sspsd_csd_read or sspsd_group_csd_read -> (pxx, pyy, pxy (complex64), breaks)"""
+    o = _merge_opts(opts)
+    cap = L.MAX_STAGES * (n // 2 + 1)
+    pxx, pyy = np.zeros(cap, np.float32), np.zeros(cap, np.float32)
+    pxy = np.zeros(2 * cap, np.float32)
+    b = (L.BreakC * L.MAX_STAGES)()
+    pl, bl = C.c_size_t(cap), C.c_size_t(L.MAX_STAGES)
+    L.check(read(h, C.byref(o), pxx.ctypes.data, pyy.ctypes.data, pxy.ctypes.data, C.byref(pl), b, C.byref(bl)))
+    m = pl.value
+    return (pxx[:m].copy(), pyy[:m].copy(), pxy[:2 * m].view(np.complex64).copy(),
+            [Break._from_c(b[i]) for i in range(bl.value)])
+
+
+def _read_csm(read, h, n, k, opts):
+    """sspsd_csm_read or sspsd_group_csm_read -> (S complex64 [K, K, bins], breaks)"""
+    o = _merge_opts(opts)
+    cap = L.MAX_STAGES * (n // 2 + 1)
+    s = np.zeros(2 * k * k * cap, np.float32)
+    b = (L.BreakC * L.MAX_STAGES)()
+    pl, bl = C.c_size_t(cap), C.c_size_t(L.MAX_STAGES)
+    L.check(read(h, C.byref(o), s.ctypes.data, C.byref(pl), b, C.byref(bl)))
+    m = pl.value
+    return s[:2 * k * k * m].view(np.complex64).reshape(k, k, m).copy(), [Break._from_c(b[i]) for i in range(bl.value)]
+
+
+def _read_zoom(read, h, n, opts):
+    """sspsd_zoom_read or sspsd_group_zoom_read -> (p_pos, p_neg, breaks)"""
+    o = _merge_opts(opts)
+    cap = L.MAX_STAGES * (n // 2 + 1)
+    pp, pn = np.zeros(cap, np.float32), np.zeros(cap, np.float32)
+    b = (L.BreakC * L.MAX_STAGES)()
+    pl, bl = C.c_size_t(cap), C.c_size_t(L.MAX_STAGES)
+    L.check(read(h, C.byref(o), pp.ctypes.data, pn.ctypes.data, C.byref(pl), b, C.byref(bl)))
+    m = pl.value
+    return pp[:m].copy(), pn[:m].copy(), [Break._from_c(b[i]) for i in range(bl.value)]
+
+
 class PsdCascade(_StreamOrdered):
     """PsdCascade<N>, src/psd.rs:399-544.  `PsdCascade(n)` is `PsdCascade::<N>::default()`."""
 
@@ -396,18 +439,7 @@ class CsdCascade(_StreamOrdered):
 
     def csd(self, opts: MergeOpts = None):
         """-> (pxx, pyy, pxy (complex64), breaks), merged like PsdCascade.psd"""
-        opts = opts or MergeOpts()
-        o = L.MergeOptsC(int(opts.keep_overlap), opts.min_count, int(opts.keep_transition_band))
-        cap = L.MAX_STAGES * (self.n // 2 + 1)
-        pxx, pyy = np.zeros(cap, np.float32), np.zeros(cap, np.float32)
-        pxy = np.zeros(2 * cap, np.float32)
-        b = (L.BreakC * L.MAX_STAGES)()
-        pl, bl = C.c_size_t(cap), C.c_size_t(L.MAX_STAGES)
-        L.check(L.lib().sspsd_csd_read(self._h, C.byref(o), pxx.ctypes.data, pyy.ctypes.data, pxy.ctypes.data,
-                                       C.byref(pl), b, C.byref(bl)))
-        n = pl.value
-        return (pxx[:n].copy(), pyy[:n].copy(), pxy[:2 * n].view(np.complex64).copy(),
-                [Break._from_c(b[i]) for i in range(bl.value)])
+        return _read_csd(L.lib().sspsd_csd_read, self._h, self.n, opts)
 
     @staticmethod
     def coherence(pxx, pyy, pxy):
@@ -505,17 +537,7 @@ class CsmCascade(_StreamOrdered):
 
     def csm(self, opts: MergeOpts = None):
         """-> (S complex64 [K, K, bins], breaks), every entry merged like PsdCascade.psd"""
-        opts = opts or MergeOpts()
-        o = L.MergeOptsC(int(opts.keep_overlap), opts.min_count, int(opts.keep_transition_band))
-        k = self.channels
-        cap = L.MAX_STAGES * (self.n // 2 + 1)
-        s = np.zeros(2 * k * k * cap, np.float32)
-        b = (L.BreakC * L.MAX_STAGES)()
-        pl, bl = C.c_size_t(cap), C.c_size_t(L.MAX_STAGES)
-        L.check(L.lib().sspsd_csm_read(self._h, C.byref(o), s.ctypes.data, C.byref(pl), b, C.byref(bl)))
-        n = pl.value
-        m = s[:2 * k * k * n].view(np.complex64).reshape(k, k, n).copy()
-        return m, [Break._from_c(b[i]) for i in range(bl.value)]
+        return _read_csm(L.lib().sspsd_csm_read, self._h, self.n, self.channels, opts)
 
     @staticmethod
     def coherence(S):
@@ -655,16 +677,7 @@ class ZoomCascade(_StreamOrdered):
 
     def spectrum(self, opts: MergeOpts = None):
         """-> (p_pos, p_neg, breaks): the densities at f0 + f and f0 - f, f = Break.frequencies(breaks) >= 0"""
-        opts = opts or MergeOpts()
-        o = L.MergeOptsC(int(opts.keep_overlap), opts.min_count, int(opts.keep_transition_band))
-        cap = L.MAX_STAGES * (self.n // 2 + 1)
-        pp, pn = np.zeros(cap, np.float32), np.zeros(cap, np.float32)
-        b = (L.BreakC * L.MAX_STAGES)()
-        pl, bl = C.c_size_t(cap), C.c_size_t(L.MAX_STAGES)
-        L.check(L.lib().sspsd_zoom_read(self._h, C.byref(o), pp.ctypes.data, pn.ctypes.data, C.byref(pl), b,
-                                        C.byref(bl)))
-        n = pl.value
-        return pp[:n].copy(), pn[:n].copy(), [Break._from_c(b[i]) for i in range(bl.value)]
+        return _read_zoom(L.lib().sspsd_zoom_read, self._h, self.n, opts)
 
     @staticmethod
     def two_sided(p_pos, p_neg, breaks, ftw=0):
@@ -1107,6 +1120,14 @@ class ShardMode(enum.IntEnum):
     TIME = 1
 
 
+class GroupKind(enum.IntEnum):
+    """what a Group computes: PsdCascade.psd, or (time chunks only) CsdCascade.csd, CsmCascade.csm, ZoomCascade.spectrum"""
+    PSD = L.GROUP_PSD
+    CSD = L.GROUP_CSD
+    CSM = L.GROUP_CSM
+    ZOOM = L.GROUP_ZOOM
+
+
 @dataclass
 class TimeChunk:
     """sspsd_time_chunk: what one rank of a time-chunked group owns and is fed"""
@@ -1138,25 +1159,39 @@ class Group:
 
     Group(n, devices=[0, 1, ...])            all ranks in this process (ncclCommInitAll / peer loads)
     Group(n, rank=r, n_ranks=w, unique_id=b) one rank of a multi-process job (torchrun): unique_id from
-                                             Group.unique_id() on rank 0, broadcast by the caller"""
+                                             Group.unique_id() on rank 0, broadcast by the caller
+
+    kind=GroupKind.CSD / CSM (channels=k) / ZOOM (zoom_mode=, ftw=) time-chunks one capture of several streams
+    (mode=ShardMode.TIME only): time_process(rank, *xs) / time_process_all(*xs) take the streams in the order of the
+    matching handle's process, and csd() / csm() / spectrum() return what that handle returns."""
 
     def __init__(self, n=512, devices=None, mode=ShardMode.CHANNELS, rank=None, n_ranks=None, unique_id=None, device=0,
-                 hbf=Hbf.TAPS_140, max_batch=0, host_stage=0, stream=None):
+                 hbf=Hbf.TAPS_140, max_batch=0, host_stage=0, stream=None, kind=GroupKind.PSD, channels=0,
+                 zoom_mode=L.ZOOM_IQ, ftw=0, window=Window.HANN, deterministic=False):
         self.n = n
-        cfg = _config(n, Window.HANN, hbf, device, 0, max_batch, host_stage)
+        self.kind = GroupKind(kind)
+        cfg = _config(n, window, hbf, device, 0, max_batch, host_stage, deterministic=deterministic)
         cfg.stream = stream  # one-rank-per-process groups only; None = private streams
         h = C.c_void_p()
+        k = L.GroupKindC(int(kind), int(channels), int(zoom_mode) if self.kind == GroupKind.ZOOM else 0, int(ftw))
         if rank is None:
             devices = list(devices if devices is not None else [0])
             arr = (C.c_int32 * len(devices))(*devices)
-            L.check(L.lib().sspsd_group_create(C.byref(cfg), arr, len(devices), int(mode), C.byref(h)))
-            self.n_ranks, self.rank = len(devices), 0
+            L.check(L.lib().sspsd_group_create_kind(C.byref(cfg), C.byref(k), arr, len(devices), int(mode), C.byref(h)))
+            self.n_ranks, self.rank, self.devices = len(devices), 0, devices
         else:
             buf = (C.c_uint8 * 128).from_buffer_copy(bytes(unique_id)) if unique_id is not None else None
-            L.check(L.lib().sspsd_group_create_rank(C.byref(cfg), buf, rank, n_ranks, int(mode), C.byref(h)))
-            self.n_ranks, self.rank = n_ranks, rank
+            L.check(L.lib().sspsd_group_create_kind_rank(C.byref(cfg), C.byref(k), buf, rank, n_ranks, int(mode),
+                                                         C.byref(h)))
+            self.n_ranks, self.rank, self.devices = n_ranks, rank, [int(device)]
         self._h = h
         self.mode = ShardMode(mode)
+        got = L.GroupKindC()
+        L.check(L.lib().sspsd_group_kind_of(h, C.byref(got)))
+        self.channels, self.zoom_mode, self.ftw = got.channels, got.zoom_mode, got.ftw
+        # input streams of time_process: PSD 1, CSD 2, CSM k, zoom I/Q 2, zoom heterodyne 1
+        self.n_inputs = (1 if self.kind == GroupKind.ZOOM and self.zoom_mode == L.ZOOM_HETERODYNE
+                         else 2 if self.kind == GroupKind.ZOOM else self.channels)
 
     @staticmethod
     def unique_id():
@@ -1242,25 +1277,69 @@ class Group:
         L.check(L.lib().sspsd_group_time_chunk(self._h, rank, C.byref(out)))
         return TimeChunk._from_c(out)
 
-    def time_process(self, rank, x):
-        ptr, n, mem, keep = _as_buffer(x)
+    def _streams(self, xs):
+        if len(xs) != self.n_inputs:
+            raise ValueError("a %s group takes %d input streams, got %d" % (self.kind.name, self.n_inputs, len(xs)))
+        bufs = [_as_buffer(x) for x in xs]
+        if any(b[1] != bufs[0][1] for b in bufs):
+            raise ValueError("all streams must have the same length (%s)" % [b[1] for b in bufs])
+        if any(b[2] != bufs[0][2] for b in bufs):
+            raise ValueError("streams must all be host arrays or all be CUDA tensors")
+        return bufs
+
+    def time_process(self, rank, *xs):
+        """the next samples of rank `rank`'s range: one stream per input of the kind (PSD: x; CSD: x, y; CSM: k
+        streams; zoom: i, q or x), float32 numpy arrays or CUDA tensors"""
+        bufs = self._streams(xs)
+        n, mem = bufs[0][1], bufs[0][2]
         if mem == L.MEM_DEVICE:
             import torch
-            torch.cuda.current_stream(keep.device).synchronize()
-        L.check(L.lib().sspsd_group_time_process_f32(self._h, rank, ptr, n, mem))
+            for b in bufs:
+                torch.cuda.current_stream(b[3].device).synchronize()
+        if self.kind == GroupKind.PSD:
+            L.check(L.lib().sspsd_group_time_process_f32(self._h, rank, bufs[0][0], n, mem))
+        else:
+            ptrs = (C.c_void_p * len(bufs))(*[b[0] for b in bufs])
+            L.check(L.lib().sspsd_group_time_process_multi_f32(self._h, rank, ptrs, n, mem))
         if mem == L.MEM_DEVICE:
             self.sync()
-        del keep
+        del bufs
 
-    def time_process_all(self, x):
-        a = np.ascontiguousarray(x, dtype=np.float32)
-        L.check(L.lib().sspsd_group_time_process_all_f32(self._h, a.ctypes.data, a.size))
+    def time_process_all(self, *xs):
+        """the whole planned capture (single-process groups): host arrays go through one library call, CUDA tensors
+        rank by rank, each rank's range copied to the rank's device where it lives elsewhere"""
+        bufs = self._streams(xs)
+        if bufs[0][2] == L.MEM_DEVICE:
+            for r in range(self.n_ranks):
+                c = self.time_chunk(r)
+                dev = self.devices[r]
+                self.time_process(r, *[x[c.feed_lo:c.feed_hi].to("cuda:%d" % dev) for x in xs])
+            return
+        if self.kind == GroupKind.PSD:
+            L.check(L.lib().sspsd_group_time_process_all_f32(self._h, bufs[0][0], bufs[0][1]))
+        else:
+            ptrs = (C.c_void_p * len(bufs))(*[b[0] for b in bufs])
+            L.check(L.lib().sspsd_group_time_process_all_multi_f32(self._h, ptrs, bufs[0][1]))
+        del bufs
 
     def time_process_noise(self, exponent=0, seed=Source.SEED):
         L.check(L.lib().sspsd_group_time_process_noise(self._h, exponent, seed))
 
     def time_finish(self):
         L.check(L.lib().sspsd_group_time_finish(self._h))
+
+    def csd(self, opts: MergeOpts = None):
+        """CSD groups after time_finish: CsdCascade.csd of the whole capture (empty on processes without rank 0)"""
+        return _read_csd(L.lib().sspsd_group_csd_read, self._h, self.n, opts)
+
+    def csm(self, opts: MergeOpts = None):
+        """CSM groups after time_finish: CsmCascade.csm of the whole capture (empty on processes without rank 0)"""
+        return _read_csm(L.lib().sspsd_group_csm_read, self._h, self.n, max(self.channels, 1), opts)
+
+    def spectrum(self, opts: MergeOpts = None):
+        """zoom groups after time_finish: ZoomCascade.spectrum of the whole capture (empty on processes without
+        rank 0)"""
+        return _read_zoom(L.lib().sspsd_group_zoom_read, self._h, self.n, opts)
 
     def __del__(self):
         h, self._h = getattr(self, "_h", None), None

@@ -3,6 +3,10 @@
 the group's result against the sequential cascade on rank 0 and prints one JSON line.
 
     torchrun --nproc-per-node N tools/group_rank.py --mode time|time_preset|channels [--total 6e6] [--n 512]
+                                                    [--kind psd|csd|csm|zoom]
+
+--kind csd / csm / zoom time-chunks one capture of 2 / 4 streams (zoom: one stream mixed down around a carrier) and
+checks rank 0's readout against the matching sequential handle.
 """
 import argparse
 import json
@@ -17,11 +21,59 @@ import torch  # noqa: E402
 import torch.distributed as dist  # noqa: E402
 
 
+FTW = 0x9E3779B9
+
+
+def cross_kind(sp, kind, n, total, rank, world, local, uid):
+    """every process makes the same streams; each feeds its own rank's range; rank 0 checks the readout"""
+    rng = np.random.default_rng(4321)
+    x = (rng.random(total, dtype=np.float32) - np.float32(0.5)).astype(np.float32)
+    xs = [x]
+    if kind != "zoom":
+        for c in range(1, 2 if kind == "csd" else 4):
+            y = np.convolve(x, [0.5, -0.25 * c, 0.1])[:total] + 0.3 * (rng.random(total, dtype=np.float32) - 0.5)
+            xs.append(y.astype(np.float32))
+    args = {"csd": dict(kind=sp.GroupKind.CSD), "csm": dict(kind=sp.GroupKind.CSM, channels=4),
+            "zoom": dict(kind=sp.GroupKind.ZOOM, zoom_mode=1, ftw=FTW)}[kind]
+    g = sp.Group(n, rank=rank, n_ranks=world, unique_id=uid, device=local, mode=sp.ShardMode.TIME, **args)
+    g.set_detrend(sp.Detrend.MEAN)
+    g.set_avg(sp.AvgOpts(999, 2 ** 32 - 2))
+    g.time_plan(total)
+    c = g.time_chunk(rank)
+    g.time_process(rank, *[v[c.feed_lo:c.feed_hi] for v in xs])
+    g.time_finish()
+    read = {"csd": lambda o: o.csd(), "csm": lambda o: o.csm(), "zoom": lambda o: o.spectrum()}[kind]
+    got = read(g)
+    if rank != 0:
+        assert got[0].size == 0 and got[-1] == []
+        return {}
+    seq = {"csd": lambda: sp.CsdCascade(n, device=local), "csm": lambda: sp.CsmCascade(n, 4, device=local),
+           "zoom": lambda: sp.ZoomCascade.heterodyne(n, FTW, device=local)}[kind]()
+    seq.set_detrend(sp.Detrend.MEAN)
+    seq.set_avg(sp.AvgOpts(999, 2 ** 32 - 2))
+    seq.process(xs) if kind == "csm" else seq.process(*xs)
+    want = read(seq)
+    same = [(k.count, k.pending, k.processed, k.bins) for k in got[-1]] == \
+        [(k.count, k.pending, k.processed, k.bins) for k in want[-1]]
+    # every part of the readout relative to the largest diagonal entry of its bin (cross terms pass through zero)
+    a = [np.asarray(v, np.complex128) for v in got[:-1]]
+    b = [np.asarray(v, np.complex128) for v in want[:-1]]
+    if kind == "csm":
+        scale = np.max(np.abs(np.einsum("iib->ib", b[0])), axis=0)
+    else:
+        scale = np.max(np.abs(np.stack(b[:2])), axis=0)
+    rel = max(float(np.max(np.abs(u - v)[..., 2:] / scale[2:])) for u, v in zip(a, b)) if a[0].shape == b[0].shape \
+        else float("inf")
+    return dict(breaks_equal=same, max_rel_diff_vs_sequential=rel, ok=bool(same and rel < 5e-5),
+                reduce=g.info()["reduce"], n_local=c.n_local)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--mode", default="time")
     ap.add_argument("--total", type=float, default=6e6)
     ap.add_argument("--n", type=int, default=512)
+    ap.add_argument("--kind", choices=["psd", "csd", "csm", "zoom"], default="psd")
     args = ap.parse_args()
     import stabilizer_stream_b200 as sp
     rank, world, local = int(os.environ["RANK"]), int(os.environ["WORLD_SIZE"]), int(os.environ.get("LOCAL_RANK", "0"))
@@ -31,8 +83,10 @@ def main():
     dist.broadcast_object_list(ids, src=0)
     n, total = args.n, int(args.total)
     preset = args.mode == "time_preset"
-    out = {"world": world, "mode": args.mode}
-    if args.mode.startswith("time"):
+    out = {"world": world, "mode": args.mode, "kind": args.kind}
+    if args.kind != "psd":
+        out.update(cross_kind(sp, args.kind, n, total, rank, world, local, ids[0]))
+    elif args.mode.startswith("time"):
         g = sp.Group(n, rank=rank, n_ranks=world, unique_id=ids[0], device=local, mode=sp.ShardMode.TIME)
         if preset:
             g.set_detrend(sp.Detrend.MEAN)
