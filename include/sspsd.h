@@ -603,6 +603,61 @@ int32_t sspsd_source_seek(sspsd_source *s, uint64_t pos);
 int32_t sspsd_cascade_process_source(sspsd_cascade *c, sspsd_source *s, size_t n);
 
 /* ---------------------------------------------------------------------------------------------
+ * Plants (DESIGN.md 3d): seeded multi-channel test signals generated on the device, with a cross-spectral matrix
+ * known in closed form.  A plant has m = 1 .. 4 independent inputs and k = 1 .. 4 outputs, each an FIR mix of all
+ * the inputs with taps h[k][m][taps_len], taps_len = 1 .. 32:
+ *   y_i[n] = round_f32( sum_{m'} sum_{t} h[i][m'][t] u_m'[n - t] ),   u[n] = 0 for n < 0,
+ * the sum formed in f64, m' ascending then t ascending, rounded to f32 once; n is the absolute position since
+ * create, reset or seek, so the outputs do not depend on how they are cut into calls.  Inputs:
+ *   SSPSD_PLANT_NOISE  param = exponent e (0 .. 8), seed: exactly the stream of sspsd_source_create(SSPSD_SOURCE_NOISE,
+ *                      e, seed) from position 0 (negative exponents carry state: SSPSD_EUNIMPLEMENTED, as
+ *                      sspsd_source_seek; e > 8 likewise)
+ *   SSPSD_PLANT_TONE   param = ftw (u32), amplitude a: u[n] = a c(phi_n), phi_n = (n ftw) mod 2^32, c the cosine
+ *                      factor of the heterodyne mixer (sspsd_heterodyne_f32), rounded to f32; seed unused
+ * A plant with k = m = taps_len = 1, tap 1.0 and a NOISE(e, seed) input reproduces sspsd_source NOISE(e, seed) bit for
+ * bit.  The spec is copied at create.  Bad counts, lengths, kinds or tuning words: SSPSD_EINVAL.
+ * --------------------------------------------------------------------------------------------- */
+enum { SSPSD_PLANT_NOISE = 0, SSPSD_PLANT_TONE = 1 };
+typedef struct {
+    int32_t kind;
+    int32_t _pad;
+    int64_t param;   /* NOISE: exponent; TONE: ftw */
+    uint64_t seed;   /* NOISE: Philox key */
+    float amplitude; /* TONE */
+    uint32_t _pad2;
+} sspsd_plant_input;
+typedef struct {
+    uint32_t k, m, taps_len, _pad;
+    const float *taps;                /* [k][m][taps_len] */
+    const sspsd_plant_input *inputs;  /* m of them */
+} sspsd_plant_spec;
+typedef struct sspsd_plant sspsd_plant;
+/* stream: as in sspsd_config (NULL = private stream, (void*)1 = legacy default stream) */
+int32_t sspsd_plant_create(const sspsd_plant_spec *spec, int32_t device, void *stream, sspsd_plant **out);
+void sspsd_plant_destroy(sspsd_plant *p);
+/* back to position 0 */
+int32_t sspsd_plant_reset(sspsd_plant *p);
+/* continue at position pos (every input is counter-based) */
+int32_t sspsd_plant_seek(sspsd_plant *p, uint64_t pos);
+int32_t sspsd_plant_position(const sspsd_plant *p, uint64_t *pos);
+/* the next n positions of all k outputs into the device buffers d_out[0 .. k-1], asynchronously on the plant's stream */
+int32_t sspsd_plant_generate(sspsd_plant *p, float *const *d_out, size_t n);
+/* Generate the next n positions straight into a handle, in bounded slices into scratch buffers the plant owns, on the
+ * handle's stream (no host memory is touched).  k must equal the handle's input streams: PSD 1, CSD 2 (x, y), CSM the
+ * handle's k, zoom I/Q 2 (i, q), zoom heterodyne 1 (mixed by the handle's own mixer).  A k mismatch, or a plant and a
+ * handle on different devices: SSPSD_EINVAL with nothing consumed. */
+int32_t sspsd_cascade_process_plant(sspsd_cascade *c, sspsd_plant *p, size_t n);
+int32_t sspsd_csd_process_plant(sspsd_csd *c, sspsd_plant *p, size_t n);
+int32_t sspsd_csm_process_plant(sspsd_csm *c, sspsd_plant *p, size_t n);
+int32_t sspsd_zoom_process_plant(sspsd_zoom *z, sspsd_plant *p, size_t n);
+/* Time-chunked groups (any kind): every local rank builds its own plant from `spec` on its device and stream, seeks
+ * it to the rank's next unfed position (feed_lo + samples fed so far) and feeds the rest of its range; spec->k must
+ * equal the kind's input streams.  The plants are cached on the group while the spec stays the same.  Nothing is
+ * waited for on the host.  A k mismatch: SSPSD_EINVAL; a spec sspsd_plant_create refuses: its code; both with nothing
+ * fed. */
+int32_t sspsd_group_time_process_plant(sspsd_group *g, const sspsd_plant_spec *spec);
+
+/* ---------------------------------------------------------------------------------------------
  * UDP ingest: the Data::Udp source of src/source.rs:81-93 (socket set-up: 1 MiB receive buffer,
  * reuse-address, multicast join, bind) and 159-165 (one `socket.read` + Frame::from_bytes +
  * loss.update + traces per datagram).  Here datagrams are collected with recvmmsg into a ring of

@@ -651,6 +651,64 @@ private:
     sspsd_source* h_ = nullptr;
 };
 
+/// A plant (sspsd_plant_*, DESIGN.md 3d): K outputs, each an FIR mix of M independent seekable inputs, generated on
+/// the device.  taps: [k][m][taps_len], copied at construction.
+class Plant {
+public:
+    struct Input {
+        int32_t kind;
+        int64_t param;
+        uint64_t seed;
+        float amplitude;
+    };
+    /// white noise differenced `exponent` times (the stream of Source::noise(exponent, seed))
+    static Input noise(int32_t exponent = 0, uint64_t seed = Source::SEED) { return {SSPSD_PLANT_NOISE, exponent, seed, 0.f}; }
+    /// amplitude * cos(2 pi (n ftw mod 2^32) / 2^32)
+    static Input tone(uint32_t ftw, float amplitude = 1.f) { return {SSPSD_PLANT_TONE, (int64_t)ftw, 0, amplitude}; }
+
+    Plant(uint32_t k, uint32_t m, uint32_t taps_len, const std::vector<float>& taps, const std::vector<Input>& inputs,
+          int device = 0, void* stream = nullptr)
+        : k_(k)
+    {
+        if (taps.size() != (size_t)k * m * taps_len || inputs.size() != m)
+            throw Error(SSPSD_EINVAL, "taps must hold k * m * taps_len values and inputs m");
+        std::vector<sspsd_plant_input> in(m);
+        for (uint32_t i = 0; i < m; ++i) in[i] = sspsd_plant_input{inputs[i].kind, 0, inputs[i].param, inputs[i].seed,
+                                                                  inputs[i].amplitude, 0};
+        const sspsd_plant_spec spec{k, m, taps_len, 0, taps.data(), in.data()};
+        check(sspsd_plant_create(&spec, device, stream, &h_));
+    }
+    Plant(const Plant&) = delete;
+    Plant& operator=(const Plant&) = delete;
+    Plant(Plant&& o) noexcept : h_(o.h_), k_(o.k_) { o.h_ = nullptr; }
+    ~Plant() { sspsd_plant_destroy(h_); }
+    uint32_t k() const { return k_; }
+    void reset() { check(sspsd_plant_reset(h_)); }
+    void seek(uint64_t pos) { check(sspsd_plant_seek(h_, pos)); }
+    uint64_t position() const
+    {
+        uint64_t p;
+        check(sspsd_plant_position(h_, &p));
+        return p;
+    }
+    /// the next n positions of output i into d_out[i] (device memory), on the plant's stream
+    void generate(float* const* d_out, size_t n) { check(sspsd_plant_generate(h_, d_out, n)); }
+    /// the next n positions straight into a handle whose input streams are the plant's k
+    template <size_t N>
+    void feed(PsdCascade<N>& c, size_t n) { check(sspsd_cascade_process_plant(c.handle(), h_, n)); }
+    template <size_t N>
+    void feed(CsdCascade<N>& c, size_t n) { check(sspsd_csd_process_plant(c.handle(), h_, n)); }
+    template <size_t N>
+    void feed(CsmCascade<N>& c, size_t n) { check(sspsd_csm_process_plant(c.handle(), h_, n)); }
+    template <size_t N>
+    void feed(ZoomCascade<N>& z, size_t n) { check(sspsd_zoom_process_plant(z.handle(), h_, n)); }
+    sspsd_plant* handle() const { return h_; }
+
+private:
+    sspsd_plant* h_ = nullptr;
+    uint32_t k_ = 1;
+};
+
 /// Data::Udp of src/source.rs:81-93, 159-165: recvmmsg into page-locked slots, decoded per batch.
 class Receiver {
 public:
@@ -850,6 +908,18 @@ public:
             p[i] = x[i].data();
         }
         check(sspsd_group_time_process_all_multi_f32(g_, p, x[0].size()));
+    }
+    /// every local rank generates its own range of the plant described by the arguments of Plant's constructor
+    void time_process_plant(uint32_t k, uint32_t m, uint32_t taps_len, const std::vector<float>& taps,
+                            const std::vector<Plant::Input>& inputs)
+    {
+        if (taps.size() != (size_t)k * m * taps_len || inputs.size() != m)
+            throw Error(SSPSD_EINVAL, "taps must hold k * m * taps_len values and inputs m");
+        std::vector<sspsd_plant_input> in(m);
+        for (uint32_t i = 0; i < m; ++i) in[i] = sspsd_plant_input{inputs[i].kind, 0, inputs[i].param, inputs[i].seed,
+                                                                  inputs[i].amplitude, 0};
+        const sspsd_plant_spec spec{k, m, taps_len, 0, taps.data(), in.data()};
+        check(sspsd_group_time_process_plant(g_, &spec));
     }
     void time_finish() { check(sspsd_group_time_finish(g_)); }
     void sync() { check(sspsd_group_sync(g_)); }

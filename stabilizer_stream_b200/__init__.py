@@ -5,9 +5,9 @@ C ABI in include/sspsd.h.  The CUDA library is the only implementation: importin
 works without a GPU, creating any handle does not.
 """
 from .psd import (DEPTH, HBF_PASSBAND, AvgOpts, Break, CsdCascade, CsmCascade, DecodeError, Detrend, Format, FrameDecoder, Hbf, Loss,
-                  MergeOpts, Psd, PsdCascade, Receiver, ShardMode, Source, SourceKind, TimeChunk, Trace, Var, Window,
+                  MergeOpts, Plant, PlantInput, PlantSpec, Psd, PsdCascade, Receiver, ShardMode, Source, SourceKind, TimeChunk, Trace, Var, Window,
                   ZoomCascade, Group, GroupKind, time_plan)
 
 __all__ = ["DEPTH", "HBF_PASSBAND", "AvgOpts", "Break", "CsdCascade", "CsmCascade", "DecodeError", "Detrend", "Format", "FrameDecoder", "Hbf",
-           "Loss", "MergeOpts", "Psd", "PsdCascade", "Receiver", "ShardMode", "Source", "SourceKind", "TimeChunk", "Trace",
+           "Loss", "MergeOpts", "Plant", "PlantInput", "PlantSpec", "Psd", "PsdCascade", "Receiver", "ShardMode", "Source", "SourceKind", "TimeChunk", "Trace",
            "Var", "Window", "ZoomCascade", "Group", "GroupKind", "time_plan"]

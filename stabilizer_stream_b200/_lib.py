@@ -15,6 +15,7 @@ OK, EINVAL, EUNIMPLEMENTED, ECUDA, ENOMEM, EHEADER, EFORMAT, ESIZE, EBATCHES, ES
 MEM_HOST, MEM_DEVICE = 0, 1
 ZOOM_IQ, ZOOM_HETERODYNE = 0, 1
 GROUP_PSD, GROUP_CSD, GROUP_CSM, GROUP_ZOOM = 0, 1, 2, 3
+PLANT_NOISE, PLANT_TONE = 0, 1
 FLAG_DETERMINISTIC = 1
 MAX_STAGES = 16
 MAX_TRACES = 4
@@ -75,6 +76,16 @@ class TimeChunkC(C.Structure):
 
 class GroupKindC(C.Structure):
     _fields_ = [("kind", C.c_int32), ("channels", C.c_int32), ("zoom_mode", C.c_int32), ("ftw", C.c_uint32)]
+
+
+class PlantInputC(C.Structure):
+    _fields_ = [("kind", C.c_int32), ("_pad", C.c_int32), ("param", C.c_int64), ("seed", C.c_uint64),
+                ("amplitude", C.c_float), ("_pad2", C.c_uint32)]
+
+
+class PlantSpecC(C.Structure):
+    _fields_ = [("k", C.c_uint32), ("m", C.c_uint32), ("taps_len", C.c_uint32), ("_pad", C.c_uint32),
+                ("taps", C.POINTER(C.c_float)), ("inputs", C.POINTER(PlantInputC))]
 
 
 class VarC(C.Structure):
@@ -192,6 +203,17 @@ PROTOTYPES = {
     "sspsd_source_position": (_i32, [_vp, C.POINTER(C.c_uint64)]),
     "sspsd_cascade_process_source": (_i32, [_vp, _vp, _sz]),
     "sspsd_source_seek": (_i32, [_vp, C.c_uint64]),
+    "sspsd_plant_create": (_i32, [C.POINTER(PlantSpecC), _i32, _vp, C.POINTER(_vp)]),
+    "sspsd_plant_destroy": (None, [_vp]),
+    "sspsd_plant_reset": (_i32, [_vp]),
+    "sspsd_plant_seek": (_i32, [_vp, C.c_uint64]),
+    "sspsd_plant_position": (_i32, [_vp, C.POINTER(C.c_uint64)]),
+    "sspsd_plant_generate": (_i32, [_vp, _vp, _sz]),
+    "sspsd_cascade_process_plant": (_i32, [_vp, _vp, _sz]),
+    "sspsd_csd_process_plant": (_i32, [_vp, _vp, _sz]),
+    "sspsd_csm_process_plant": (_i32, [_vp, _vp, _sz]),
+    "sspsd_zoom_process_plant": (_i32, [_vp, _vp, _sz]),
+    "sspsd_group_time_process_plant": (_i32, [_vp, C.POINTER(PlantSpecC)]),
     "sspsd_group_create": (_i32, [C.POINTER(Config), C.POINTER(_i32), C.c_uint32, _i32, C.POINTER(_vp)]),
     "sspsd_group_unique_id": (_i32, [_vp]),
     "sspsd_group_create_rank": (_i32, [C.POINTER(Config), _vp, C.c_uint32, C.c_uint32, _i32, C.POINTER(_vp)]),

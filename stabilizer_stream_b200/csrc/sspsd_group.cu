@@ -29,7 +29,7 @@
 #include <new>
 #include <vector>
 
-#include "sspsd_xcascade.cuh"
+#include "sspsd_plant.cuh"
 
 using sspsd::Cascade;
 using sspsd::XCascade;
@@ -363,6 +363,8 @@ struct sspsd_group {
     std::vector<sspsd_source*> noise_src;  // per local rank, for sspsd_group_time_process_noise
     int64_t noise_exp = 0;
     uint64_t noise_seed = 0;
+    std::vector<sspsd_plant*> plants;  // per local rank, for sspsd_group_time_process_plant
+    std::vector<uint8_t> plant_key;    // the spec they were made from (k, m, taps_len, taps, inputs)
 
     uint32_t n_local() const { return (uint32_t)devices.size(); }
     bool cross() const { return kind.kind != SSPSD_GROUP_PSD; }
@@ -784,6 +786,7 @@ void sspsd_group_destroy(sspsd_group* g)
                 g->first_rank, (unsigned long long)g->n_readouts, 1e6 * g->t_wait / g->n_readouts, 1e6 * g->t_pack / g->n_readouts,
                 1e6 * g->t_gather / g->n_readouts, 1e6 * g->t_d2h / g->n_readouts, 1e6 * g->t_merge / g->n_readouts);
     for (auto* s : g->noise_src) sspsd_source_destroy(s);
+    for (auto* p : g->plants) sspsd_plant_destroy(p);
     for (auto* c : g->chan) sspsd_cascade_destroy(c);
     for (auto* c : g->tc) sspsd_cascade_destroy(c);
     for (size_t l = 0; l < g->xc.size(); ++l) destroy_xrank(g->xc[l], g->zc.empty() ? nullptr : g->zc[l]);
@@ -1267,6 +1270,61 @@ int32_t sspsd_group_time_process_noise(sspsd_group* g, int64_t exponent, uint64_
         if (rc) return rc;
         const uint64_t n = pl.feed_hi - pl.feed_lo - g->fed[l];
         rc = sspsd_cascade_process_source(g->tc[l], g->noise_src[l], (size_t)n);
+        if (rc) return rc;
+        g->fed[l] += n;
+    }
+    return SSPSD_OK;
+}
+
+int32_t sspsd_group_time_process_plant(sspsd_group* g, const sspsd_plant_spec* spec)
+{
+    if (!g || g->mode != SSPSD_SHARD_TIME || g->plan.empty()) {
+        set_error("no plan (call sspsd_group_time_plan first)");
+        return SSPSD_EINVAL;
+    }
+    int rc = sspsd::plant_check(spec);
+    if (rc) return rc;
+    if (spec->k != g->n_inputs()) {
+        set_error("the plant's outputs must match the group's input streams");
+        return SSPSD_EINVAL;
+    }
+    // as sspsd_group_time_process_noise: every local rank generates its own range on its device and stream, and
+    // nothing is waited for here; the plants live with the group while the spec stays the same
+    std::vector<uint8_t> key(4 * sizeof(uint32_t));
+    const uint32_t dims[4] = {spec->k, spec->m, spec->taps_len, 0};
+    std::memcpy(key.data(), dims, sizeof(dims));
+    const uint8_t* taps = reinterpret_cast<const uint8_t*>(spec->taps);
+    key.insert(key.end(), taps, taps + sizeof(float) * spec->k * spec->m * spec->taps_len);
+    for (uint32_t m = 0; m < spec->m; ++m) {
+        const sspsd_plant_input& in = spec->inputs[m];
+        uint32_t amp;
+        std::memcpy(&amp, &in.amplitude, sizeof(amp));
+        const int64_t f[4] = {in.kind, in.param, (int64_t)in.seed, amp};
+        const uint8_t* b = reinterpret_cast<const uint8_t*>(f);
+        key.insert(key.end(), b, b + sizeof(f));
+    }
+    if (g->plants.size() != g->n_local() || g->plant_key != key) {
+        for (auto* p : g->plants) sspsd_plant_destroy(p);
+        g->plants.assign(g->n_local(), nullptr);
+        g->plant_key.clear();
+        for (uint32_t l = 0; l < g->n_local(); ++l) {
+            void* s = g->cross() ? (void*)g->xc[l]->stream() : (void*)g->tc[l]->c.stream();
+            rc = sspsd_plant_create(spec, g->devices[l], s, &g->plants[l]);
+            if (rc) return rc;
+        }
+        g->plant_key = key;
+    }
+    for (uint32_t l = 0; l < g->n_local(); ++l) {
+        const sspsd_time_chunk& pl = g->plan[g->first_rank + l];
+        rc = sspsd_plant_seek(g->plants[l], pl.feed_lo + g->fed[l]);
+        if (rc) return rc;
+        const size_t n = (size_t)(pl.feed_hi - pl.feed_lo - g->fed[l]);
+        if (g->kind.kind == SSPSD_GROUP_PSD)
+            rc = sspsd::plant_feed(g->plants[l], g->tc[l]->c, n);
+        else if (g->kind.kind == SSPSD_GROUP_ZOOM)
+            rc = sspsd::plant_feed(g->plants[l], *g->zc[l], n);
+        else
+            rc = sspsd::plant_feed(g->plants[l], *g->xc[l], n);
         if (rc) return rc;
         g->fed[l] += n;
     }

@@ -96,7 +96,7 @@ __device__ __forceinline__ uint32_t dsm_input(unsigned long long i, uint32_t ftw
 // ---------------------------------------------------------------------------------------------
 // White noise and differentiated noise: one Philox block (4 samples) per thread
 // ---------------------------------------------------------------------------------------------
-__global__ void __launch_bounds__(256) source_diff_kernel(SourceParams p)
+static __global__ void __launch_bounds__(256) source_diff_kernel(SourceParams p)
 {
     const long long q0 = (long long)(p.pos >> 2);
     const long long nq = (long long)((p.pos + p.n + 3) >> 2) - q0;

@@ -282,6 +282,10 @@ class PsdCascade(_StreamOrdered):
         the loop of bin/stream_test.rs:52-58 with `--noise` / `--dsm`."""
         L.check(L.lib().sspsd_cascade_process_source(self._h, source._h, n))
 
+    def process_plant(self, plant, n):
+        """Feed the next n positions of a one-output Plant, generated on the device on the cascade's stream"""
+        L.check(L.lib().sspsd_cascade_process_plant(self._h, plant._h, n))
+
     def flush(self):
         L.check(L.lib().sspsd_cascade_flush(self._h))
 
@@ -426,6 +430,10 @@ class CsdCascade(_StreamOrdered):
             self._release_device_input(kx)
         del kx, ky
 
+    def process_plant(self, plant, n):
+        """Feed the next n positions of a two-output Plant (x, y), generated on the device on the handle's stream"""
+        L.check(L.lib().sspsd_csd_process_plant(self._h, plant._h, n))
+
     def flush(self):
         L.check(L.lib().sspsd_csd_flush(self._h))
 
@@ -523,6 +531,10 @@ class CsmCascade(_StreamOrdered):
         if mem == L.MEM_DEVICE:
             self._release_device_input(bufs[0][3])
         del bufs
+
+    def process_plant(self, plant, n):
+        """Feed the next n positions of a K-output Plant, generated on the device on the handle's stream"""
+        L.check(L.lib().sspsd_csm_process_plant(self._h, plant._h, n))
 
     def flush(self):
         L.check(L.lib().sspsd_csm_flush(self._h))
@@ -663,6 +675,11 @@ class ZoomCascade(_StreamOrdered):
             L.check(L.lib().sspsd_zoom_process_iq_f32(self._h, px, pq, n, mem))
         if mem == L.MEM_DEVICE:
             self._release_device_input(kx)
+
+    def process_plant(self, plant, n):
+        """Feed the next n positions of a Plant generated on the device on the handle's stream: two outputs (i, q) in
+        I/Q mode, one output x in heterodyne mode (mixed by the handle's mixer)"""
+        L.check(L.lib().sspsd_zoom_process_plant(self._h, plant._h, n))
 
     def flush(self):
         L.check(L.lib().sspsd_zoom_flush(self._h))
@@ -1036,6 +1053,136 @@ class Source:
             L._lib.sspsd_source_destroy(h)
 
 
+@dataclass(frozen=True)
+class PlantInput:
+    """one input of a Plant: Plant.noise(...) or Plant.tone(...)"""
+    kind: int
+    param: int
+    seed: int = 0
+    amplitude: float = 0.0
+
+
+class PlantSpec:
+    """the C description of a plant (sspsd_plant_spec): what Plant and Group.time_process_plant pass to the library.
+    Holds the arrays the struct points at."""
+
+    def __init__(self, taps, inputs):
+        taps = np.ascontiguousarray(np.asarray(taps, np.float32))
+        if taps.ndim != 3:
+            raise ValueError("taps must be a [K, M, L] array, got shape %s" % (taps.shape,))
+        inputs = list(inputs)
+        if taps.shape[1] != len(inputs):
+            raise ValueError("taps have %d inputs, %d given" % (taps.shape[1], len(inputs)))
+        for u in inputs:
+            if not isinstance(u, PlantInput):
+                raise TypeError("inputs must be Plant.noise(...) / Plant.tone(...)")
+        self.taps, self.inputs = taps, inputs
+        self.k, self.m, self.taps_len = taps.shape
+        self._in = (L.PlantInputC * max(len(inputs), 1))(
+            *[L.PlantInputC(u.kind, 0, u.param, u.seed & (2 ** 64 - 1), u.amplitude, 0) for u in inputs])
+        self.c = L.PlantSpecC(self.k, self.m, self.taps_len, 0, taps.ctypes.data_as(C.POINTER(C.c_float)), self._in)
+
+
+class Plant:
+    """A seeded multi-channel test signal generated on the device (include/sspsd.h, sspsd_plant_*): K outputs, each
+    an FIR mix of M independent inputs,
+        y_i[n] = round_f32( sum_m sum_t taps[i, m, t] u_m[n - t] )   (f64 sum, m then t ascending; u[n < 0] = 0)
+    with Plant.noise(e, seed) (the stream of Source.noise(e, seed), e = 0 .. 8) and Plant.tone(ftw, amplitude)
+    (amplitude * cos(2 pi (n ftw mod 2^32) / 2^32), the heterodyne mixer's cosine) inputs.  Its cross-spectral
+    matrix is known in closed form (expected_csm), so it checks CsdCascade / CsmCascade / ZoomCascade end to end.
+    Fed with process_plant of a handle or Group.time_process_plant."""
+
+    def __init__(self, taps, inputs, device=0, stream=None):
+        self._spec = PlantSpec(taps, inputs)
+        if stream is None:
+            stream = _default_stream(device)
+        h = C.c_void_p()
+        L.check(L.lib().sspsd_plant_create(C.byref(self._spec.c), int(device), stream, C.byref(h)))
+        self._h = h
+        self._stream = stream
+        self.device = int(device)
+        self.k = self._spec.k
+
+    @staticmethod
+    def noise(exponent=0, seed=Source.SEED):
+        """white noise differenced `exponent` times (PSD ~ f^exponent at low f), zero mean, unit RMS before differencing"""
+        return PlantInput(L.PLANT_NOISE, int(exponent), int(seed))
+
+    @staticmethod
+    def tone(ftw, amplitude=1.0):
+        """amplitude * cos(2 pi phi_n / 2^32), phi_n = (n ftw) mod 2^32 (ZoomCascade.ftw_of gives ftw)"""
+        return PlantInput(L.PLANT_TONE, int(ftw), 0, float(amplitude))
+
+    @property
+    def taps(self):
+        return self._spec.taps
+
+    @property
+    def inputs(self):
+        return list(self._spec.inputs)
+
+    def spec(self):
+        """the plant's description, for Group.time_process_plant"""
+        return self._spec
+
+    def reset(self):
+        L.check(L.lib().sspsd_plant_reset(self._h))
+
+    def seek(self, pos):
+        L.check(L.lib().sspsd_plant_seek(self._h, int(pos)))
+
+    def position(self):
+        p = C.c_uint64()
+        L.check(L.lib().sspsd_plant_position(self._h, C.byref(p)))
+        return p.value
+
+    def generate(self, n, out=None):
+        """the next n positions of every output as a (K, n) float32 tensor on the plant's device.  Generated on
+        the plant's stream, which torch's current stream then waits for."""
+        import torch
+        if out is None:
+            out = torch.empty((self.k, n), dtype=torch.float32, device="cuda:%d" % self.device)
+        if not (out.is_cuda and out.dtype == torch.float32 and out.dim() == 2 and out.shape[0] == self.k
+                and out.shape[1] >= n and out.stride(1) == 1):
+            raise ValueError("out must be a (K, >= n) float32 CUDA tensor with contiguous rows")
+        ptrs = (C.c_void_p * self.k)(*[out[i].data_ptr() for i in range(self.k)])
+        cur = torch.cuda.current_stream(out.device)
+        mine = (cur.cuda_stream or 1) == (self._stream or 1)
+        if not mine:
+            hs = (torch.cuda.default_stream(out.device) if self._stream in (0, 1)
+                  else torch.cuda.ExternalStream(self._stream, device=out.device))
+            hs.wait_stream(cur)
+        L.check(L.lib().sspsd_plant_generate(self._h, ptrs, n))
+        if not mine:
+            cur.wait_stream(hs)
+        return out[:, :n]
+
+    def expected_csm(self, f):
+        """The closed-form one-sided cross-spectral matrix of the outputs [K, K, len(f)] (complex128), in the density
+        convention of CsmCascade.csm (S_ij = <conj(X_i) X_j>, a unit-RMS white stream reads 2), for f in cycles per
+        stage-0 sample:
+            S_ij(f) = 2 sum_m (2 sin pi f)^(2 e_m) conj(H_im(f)) H_jm(f),  H_im(f) = sum_t taps[i, m, t] e^(-2 pi i f t)
+        over the NOISE inputs (each unit RMS before its e_m differences).  Tones are spectral lines, not densities:
+        they are left out."""
+        f = np.asarray(f, np.float64)
+        taps = self.taps.astype(np.float64)
+        t = np.arange(taps.shape[2])
+        e = np.exp(-2j * np.pi * f[None, :] * t[:, None])              # [L, F]
+        H = np.einsum("kmt,tf->kmf", taps, e)                           # [K, M, F]
+        S = np.zeros((self.k, self.k, f.size), np.complex128)
+        for m, u in enumerate(self._spec.inputs):
+            if u.kind != L.PLANT_NOISE:
+                continue
+            g = 2.0 * (2.0 * np.sin(np.pi * f)) ** (2 * u.param)
+            S += g[None, None, :] * np.conj(H[:, None, m, :]) * H[None, :, m, :]
+        return S
+
+    def __del__(self):
+        h, self._h = getattr(self, "_h", None), None
+        if h and L is not None and getattr(L, "_lib", None) is not None:
+            L._lib.sspsd_plant_destroy(h)
+
+
 class Receiver:
     """Data::Udp of src/source.rs:81-93, 159-165: datagrams collected with recvmmsg into page-locked
     slots and handed on as runs of equally sized frames.
@@ -1324,6 +1471,12 @@ class Group:
 
     def time_process_noise(self, exponent=0, seed=Source.SEED):
         L.check(L.lib().sspsd_group_time_process_noise(self._h, exponent, seed))
+
+    def time_process_plant(self, plant):
+        """every local rank generates its own range of a Plant (or PlantSpec, Plant.spec()) on its device and feeds
+        it; the plant's K must be the kind's input streams"""
+        spec = plant.spec() if isinstance(plant, Plant) else plant
+        L.check(L.lib().sspsd_group_time_process_plant(self._h, C.byref(spec.c)))
 
     def time_finish(self):
         L.check(L.lib().sspsd_group_time_finish(self._h))

@@ -10,6 +10,10 @@ Sources (reference src/source.rs:16-48, 102-167):
   --udp IP:PORT       live Stabilizer stream (source.rs:81-93, 159-165): recvmmsg batches into page-locked slots;
                       ends after --samples items per trace or 1 s without traffic
   --dsm FTW           MASH-1-1-1 modulated sine marker generated on the device (source.rs:119-130)
+  --plant SPEC.json   a seeded multi-channel test signal generated on the device (Plant): {"taps": [K][M][L],
+                      "inputs": [{"noise": e, "seed": s} or {"tone": ftw, "amplitude": a}, ...], "samples": n}.
+                      K = 1 feeds the PsdCascade (or, with --zoom FTW, the mixer), K = 2 .. 4 feed --csm (K indices
+                      naming the outputs in order) and K = 2 --iq (the outputs as I, Q)
 --repeat wraps files around; the run ends after --samples items per trace (files: at EOF without --repeat).
 Host reads go through a pinned double buffer, so the H2D copy of block b+1 overlaps the kernels of block b.
 
@@ -33,8 +37,8 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np  # noqa: E402
 import torch  # noqa: E402
 
-from stabilizer_stream_b200 import (Break, CsmCascade, Detrend, FrameDecoder, Loss, MergeOpts, PsdCascade, Receiver,
-                                    Source, Var, ZoomCascade)  # noqa: E402
+from stabilizer_stream_b200 import (Break, CsmCascade, Detrend, FrameDecoder, Loss, MergeOpts, Plant, PsdCascade,
+                                    Receiver, Source, Var, ZoomCascade)  # noqa: E402
 
 BREAK_FIELDS = ("start", "include", "count", "avg", "bins_start", "bins_end", "fft_size", "decimation", "pending",
                 "processed")
@@ -59,8 +63,8 @@ def parse_csm(ap, a):
         ap.error("--csm takes 2 to 4 trace indices (a CsmCascade has at most 4 channels)")
     if any(not 0 <= t < 4 for t in traces):
         ap.error("--csm trace indices are 0 .. 3")
-    if not (a.file or a.udp):
-        ap.error("--csm needs --file or --udp (frames carry the traces)")
+    if not (a.file or a.udp or a.plant):
+        ap.error("--csm needs --file or --udp (frames carry the traces), or --plant")
     if a.trace is not None and a.trace not in traces:
         ap.error("--trace must be one of the --csm traces")
     return traces
@@ -72,8 +76,8 @@ def parse_zoom(ap, a):
         ap.error("use one of --csm, --iq, --zoom")
     if a.iq is None and a.zoom is None:
         return None
-    if not (a.file or a.udp):
-        ap.error("--iq / --zoom need --file or --udp (frames carry the traces)")
+    if not (a.file or a.udp or a.plant):
+        ap.error("--iq / --zoom need --file or --udp (frames carry the traces), or --plant")
     if a.iq is not None:
         try:
             traces = [int(t) for t in a.iq.split(",")]
@@ -92,6 +96,51 @@ def parse_zoom(ap, a):
     return traces
 
 
+def parse_plant(ap, a):
+    """--plant checks, before any device work: -> (taps [K, M, L], inputs, samples) or None"""
+    if a.plant is None:
+        return None
+    if sum(v is not None for v in (a.raw, a.file, a.udp, a.noise, a.dsm)):
+        ap.error("use one of --raw, --file, --udp, --noise, --dsm, --plant")
+    try:
+        with open(a.plant) as f:
+            spec = json.load(f)
+    except (OSError, ValueError) as e:
+        ap.error("--plant: cannot read the JSON spec (%s)" % e)
+    if not isinstance(spec, dict) or "taps" not in spec or "inputs" not in spec:
+        ap.error("--plant: the spec needs taps [K][M][L] and inputs")
+    if not isinstance(spec.get("samples"), (int, float)) or spec["samples"] <= 0:
+        ap.error("--plant: the spec needs a positive sample count (samples)")
+    inputs = []
+    for u in spec["inputs"]:
+        if isinstance(u, dict) and "noise" in u:
+            inputs.append(Plant.noise(int(u["noise"]), int(u.get("seed", Source.SEED))))
+        elif isinstance(u, dict) and "tone" in u:
+            inputs.append(Plant.tone(int(u["tone"]), float(u.get("amplitude", 1.0))))
+        else:
+            ap.error("--plant: every input is {\"noise\": e, \"seed\": s} or {\"tone\": ftw, \"amplitude\": a}")
+    try:
+        taps = np.asarray(spec["taps"], np.float32)
+    except (TypeError, ValueError):
+        taps = np.zeros(0, np.float32)
+    if taps.ndim != 3 or taps.shape[1] != len(inputs) or not (1 <= taps.shape[0] <= 4 and 1 <= taps.shape[1] <= 4
+                                                             and 1 <= taps.shape[2] <= 32):
+        ap.error("--plant: taps must be [K, M, L] with K, M = 1 .. 4, L = 1 .. 32 and M the number of inputs")
+    k = taps.shape[0]
+    if a.csm is not None:
+        if len(a.csm.split(",")) != k:
+            ap.error("--plant: --csm must name the plant's %d outputs" % k)
+    elif a.iq is not None:
+        if k != 2:
+            ap.error("--plant: --iq takes a plant with 2 outputs, this one has %d" % k)
+    elif a.zoom is not None:
+        if k != 1:
+            ap.error("--plant: --zoom mixes one stream, this plant has %d outputs" % k)
+    elif k != 1:
+        ap.error("--plant: a plant with %d outputs feeds --csm, --iq or --zoom" % k)
+    return taps, inputs, int(spec["samples"])
+
+
 def main():
     ap = argparse.ArgumentParser(description=__doc__, formatter_class=argparse.RawDescriptionHelpFormatter)
     ap.add_argument("--raw")
@@ -100,6 +149,7 @@ def main():
     ap.add_argument("--noise", type=int)
     ap.add_argument("--dsm", type=int)
     ap.add_argument("--udp")
+    ap.add_argument("--plant", metavar="SPEC.json", help="a Plant generated on the device (see above)")
     ap.add_argument("--repeat", action="store_true")
     ap.add_argument("--samples", type=float, default=0, help="stop after this many items per trace (0: until EOF)")
     ap.add_argument("--fft", type=int, default=512, help="FFT size N (the reference binaries use 512)")
@@ -113,6 +163,7 @@ def main():
     ap.add_argument("--block", type=int, default=1 << 24, help="items (or frames*64) read per block")
     ap.add_argument("--json", action="store_true")
     a = ap.parse_args()
+    plant = parse_plant(ap, a)
     csm_traces = parse_csm(ap, a)
     zoom_traces = parse_zoom(ap, a)
     if zoom_traces:
@@ -149,7 +200,17 @@ def main():
 
     tmap = zoom_traces or csm_traces
 
-    if a.noise is not None or a.dsm is not None:
+    if plant is not None:
+        cascades(1)
+        taps, inputs, limit = plant
+        names = ["plant%d" % i for i in range(taps.shape[0])]
+        p = Plant(taps, inputs)
+        while total < limit:
+            n = min(a.block, limit - total)
+            target_ = target()
+            (target_[0] if isinstance(target_, list) else target_).process_plant(p, n)  # generated and consumed on the device
+            total += n
+    elif a.noise is not None or a.dsm is not None:
         cascades(1)
         names = ["noise" if a.dsm is None else "dsm"]
         src = Source.noise(a.noise) if a.dsm is None else Source.dsm(a.dsm)
