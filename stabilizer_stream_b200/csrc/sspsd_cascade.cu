@@ -135,7 +135,7 @@ int launch_decim_t(const DecimParams& p, int grid, cudaStream_t s)
     return cuda_ok(cudaGetLastError(), "decim8_kernel launch") ? SSPSD_OK : SSPSD_ECUDA;
 }
 
-// persistent TMA-staged decimator (default; SSPSD_K3=tiled selects the first-generation kernel)
+// persistent TMA-staged decimator with the de-interleaving round trip (SSPSD_K3=tma960: the reference of the default)
 template <int MA, int MB, int MC, int PRESET, int OB, int CTAS>
 int launch_decim_tma_t(const DecimParams& p, long long n_out, int num_sms, cudaStream_t s)
 {
@@ -143,6 +143,16 @@ int launch_decim_tma_t(const DecimParams& p, long long n_out, int num_sms, cudaS
     const int grid = std::min(ntiles, num_sms * CTAS);
     decim8_tma_kernel<MA, MB, MC, PRESET, OB, CTAS><<<grid, DEC_NT, decim_tma_smem_bytes<MA, MB, MC, OB>(), s>>>(p, ntiles);
     return cuda_ok(cudaGetLastError(), "decim8_tma_kernel launch") ? SSPSD_OK : SSPSD_ECUDA;
+}
+
+// persistent decimator whose stage A reads the TMA-staged tile directly (default)
+template <int MA, int MB, int MC, int PRESET, int OB, int CTAS>
+int launch_decim_direct_t(const DecimParams& p, long long n_out, int num_sms, cudaStream_t s)
+{
+    const int ntiles = (int)((n_out + OB - 1) / OB);
+    const int grid = std::min(ntiles, num_sms * CTAS);
+    decim8_direct_kernel<MA, MB, MC, PRESET, OB, CTAS><<<grid, DEC_NT, decim_direct_smem_bytes<MA, MB, MC, OB>(), s>>>(p, ntiles);
+    return cuda_ok(cudaGetLastError(), "decim8_direct_kernel launch") ? SSPSD_OK : SSPSD_ECUDA;
 }
 
 template <int MA, int MB, int MC, int PRESET, int OB, int CTAS>
@@ -195,6 +205,10 @@ int upload_taps_once(int device)
                                     (int)(DecGeom<5, 10, 23>::SMEM_FLOATS * sizeof(float))));
     SSPSD_CUDA(cudaFuncSetAttribute(decim8_kernel<3, 6, 15, SSPSD_HBF_98>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                     (int)(DecGeom<3, 6, 15>::SMEM_FLOATS * sizeof(float))));
+    SSPSD_CUDA(cudaFuncSetAttribute(decim8_direct_kernel<5, 10, 23, SSPSD_HBF_140, 960, 2>,
+                                    cudaFuncAttributeMaxDynamicSharedMemorySize, (int)decim_direct_smem_bytes<5, 10, 23, 960>()));
+    SSPSD_CUDA(cudaFuncSetAttribute(decim8_direct_kernel<3, 6, 15, SSPSD_HBF_98, 960, 2>,
+                                    cudaFuncAttributeMaxDynamicSharedMemorySize, (int)decim_direct_smem_bytes<3, 6, 15, 960>()));
     SSPSD_CUDA(cudaFuncSetAttribute(decim8_async_kernel<5, 10, 23, SSPSD_HBF_140, 960, 2>,
                                     cudaFuncAttributeMaxDynamicSharedMemorySize, (int)decim_async_smem_bytes<5, 10, 23, 960>()));
     SSPSD_CUDA(cudaFuncSetAttribute(decim8_async_kernel<5, 10, 23, SSPSD_HBF_140, 640, 3>,
@@ -406,11 +420,12 @@ int Cascade::init(const sspsd_config& cfg, uint32_t max_stages)
     if (const char* e = getenv("SSPSD_DEFER")) defer_ = strtoull(e, nullptr, 0);
     k2_variant_ = k2_variant_from_env();
     {
-        // K3 variant (A/B switch): SSPSD_K3 = tiled | tma960 | tma640 | async960 | async640
+        // K3 variant (A/B switch): unset = direct stage A (default), SSPSD_K3 = tiled | tma960 | tma768 | tma640 |
+        // async960 | async640 | pf960 | pf640
         const char* e = getenv("SSPSD_K3");
-        std::string m = e ? e : "tma960";
-        k3_variant_ = m == "tiled" ? 0 : m == "tma960" ? 1 : m == "tma640" ? 2 : m == "async640" ? 4 : m == "pf960" ? 5 :
-                      m == "pf640" ? 6 : m == "tma768" ? 7 : 3;
+        std::string m = e ? e : "";
+        k3_variant_ = m.empty() ? 8 : m == "tiled" ? 0 : m == "tma960" ? 1 : m == "tma640" ? 2 : m == "async640" ? 4 :
+                      m == "pf960" ? 5 : m == "pf640" ? 6 : m == "tma768" ? 7 : 3;
     }
     rc = prepare_stage((int)log2n_, k2_variant_ >= 1, (int)hop_, &tmax_, &nt_);
     if (rc) return rc;
@@ -694,13 +709,16 @@ int Cascade::launch_decim(size_t i, const StreamSrc& src, uint64_t m0, uint64_t 
     int grid = (int)((p.m1 - lo + DEC_OB - 1) / DEC_OB);
     cudaStream_t ss = stage_stream(i);
     static const bool fuse_carry = !getenv("SSPSD_CARRY_KERNEL");  // A/B switch: keep the separate carry_copy_kernel launch
-    if (cc_valid_ && fuse_carry && (k3_variant_ == 1 || k3_variant_ == 2 || k3_variant_ == 7)) {
+    if (cc_valid_ && fuse_carry && (k3_variant_ == 1 || k3_variant_ == 2 || k3_variant_ == 7 || k3_variant_ == 8)) {
         p.cc = cc_pending_;  // the TMA-staged kernels build the stage's next carry buffer themselves
         cc_valid_ = false;
     }
     prof_begin(i == 0 ? SSPSD_PROF_DECIM_STAGE0 : SSPSD_PROF_DECIM_DEEP, (uint64_t)(p.m1 - lo) * 8, ss);
     int rc;
-    if (k3_variant_ == 0) {
+    if (k3_variant_ == 8) {
+        rc = cfg_.hbf == SSPSD_HBF_98 ? launch_decim_direct_t<3, 6, 15, SSPSD_HBF_98, 960, 2>(p, p.m1 - lo, num_sms_, ss)
+                                      : launch_decim_direct_t<5, 10, 23, SSPSD_HBF_140, 960, 2>(p, p.m1 - lo, num_sms_, ss);
+    } else if (k3_variant_ == 0) {
         rc = cfg_.hbf == SSPSD_HBF_98 ? launch_decim_t<3, 6, 15, SSPSD_HBF_98>(p, grid, ss)
                                       : launch_decim_t<5, 10, 23, SSPSD_HBF_140>(p, grid, ss);
     } else if (k3_variant_ == 1) {

@@ -201,7 +201,7 @@ private:
     uint64_t defer_window_ = 0;    // threshold in force for the stage that has just received samples
     CarryJob cc_pending_{};    // carry copy of the stage being run, until a decimator launch (or the fallback kernel) takes it
     bool cc_valid_ = false;
-    int k3_variant_ = 1;       // SSPSD_K3 at creation: 0 = tiled, 1 = persistent TMA (960 outputs/tile), 2 = (640)
+    int k3_variant_ = 8;       // SSPSD_K3 at creation: 8 = direct stage A (default), 0 = tiled, 1 = persistent TMA (960 outputs/tile), 2 = (640)
     int k2_variant_ = 2;       // SSPSD_K2 at creation: 0 = radix-8 tiled, 1 = radix-16 tiled, 2 = TMA ring (N = 4096)
     bool single_stage_avg_set_ = false;
     uint32_t single_stage_avg_ = 0xffffffffu;

@@ -77,6 +77,40 @@ struct DecimParams {
     int preset;
 };
 
+// The P consecutive outputs q of one run, starting at an even output: y[q] = centre(q) + a_q, where a_q is the tap
+// sum over the run's odd-phase window win[0 .. 2M + P - 2] (output q reads win[q .. q + 2M - 1]), held as aligned
+// register pairs wp[m] = (win[2m], win[2m+1]).  Every decimator kernel computes its outputs with this one expression,
+// which is what makes them bit-identical.
+template <int M, int P, int PRESET, int SET, class Centre>
+__device__ __forceinline__ void hbf_outputs(const float2 (&wp)[M + P / 2], Centre centre, float (&y)[P])
+{
+    static_assert(P % 2 == 0, "runs start and end on an output pair");
+    // Taps are paired so that both window operands of a packed add are aligned pairs: for even q the
+    // pairs (0,1), (2,3), ..., for odd q the pairs (1,2), (3,4), ...; tap i multiplies
+    // win[q+i] + win[q+2M-1-i], and the mirrored operand of a pair is the swapped pair (free swizzle).
+    // The two halves of the packed accumulator hold the even- and the odd-tap partial sums.
+    const float2* __restrict__ tp0 = reinterpret_cast<const float2*>(&c_hbf_taps[PRESET][SET][0]);
+    const float2* __restrict__ tp1 = reinterpret_cast<const float2*>(&c_hbf_taps_sh[PRESET][SET][0]);
+#pragma unroll
+    for (int q = 0; q < P; ++q) {
+        float2 acc = make_float2(0.f, 0.f);
+        const int i0 = q & 1;  // first paired tap
+#pragma unroll
+        for (int i = i0; i + 1 < M; i += 2) {
+            const float2 l = wp[(q + i) >> 1];
+            const float2 r = wp[(q + 2 * M - 2 - i) >> 1];
+            const float2 sum = __fadd2_rn(l, make_float2(r.y, r.x));
+            acc = __ffma2_rn(sum, (q & 1) ? tp1[(i - 1) >> 1] : tp0[i >> 1], acc);
+        }
+        float a = acc.x + acc.y;
+        auto winv = [&](int k) { return (k & 1) ? wp[k >> 1].y : wp[k >> 1].x; };
+        if (q & 1) a = fmaf(winv(q) + winv(q + 2 * M - 1), c_hbf_taps[PRESET][SET][0], a);  // tap 0
+        // the last tap is unpaired when the paired range [i0, M) has odd length
+        if (((M - i0) & 1) != 0) a = fmaf(winv(q + M - 1) + winv(q + M), c_hbf_taps[PRESET][SET][M - 1], a);
+        y[q] = centre(q) + a;
+    }
+}
+
 template <int M, int SI, int SO, int REL0, bool FINAL, int PRESET, int SET>
 __device__ __forceinline__ void hbf_stage(const float* __restrict__ ine, const float* __restrict__ ino,
                                           int n_out, float* __restrict__ oute,
@@ -98,34 +132,11 @@ __device__ __forceinline__ void hbf_stage(const float* __restrict__ ine, const f
             const float x = ino[(c & (P - 1)) * SI + (c >> LP) + w];
             if (i & 1) wp[i >> 1].y = x; else wp[i >> 1].x = x;
         }
-        // Taps are paired so that both window operands of a packed add are aligned pairs: for even q the
-        // pairs (0,1), (2,3), ..., for odd q the pairs (1,2), (3,4), ...; tap i multiplies
-        // win[q+i] + win[q+2M-1-i], and the mirrored operand of a pair is the swapped pair (free swizzle).
-        // The two halves of the packed accumulator hold the even- and the odd-tap partial sums.
-        const float2* __restrict__ tp0 = reinterpret_cast<const float2*>(&c_hbf_taps[PRESET][SET][0]);
-        const float2* __restrict__ tp1 = reinterpret_cast<const float2*>(&c_hbf_taps_sh[PRESET][SET][0]);
         float y[P];
-#pragma unroll
-        for (int q = 0; q < P; ++q) {
-            float2 acc = make_float2(0.f, 0.f);
-            constexpr int dummy = 0;
-            (void)dummy;
-            const int i0 = q & 1;  // first paired tap
-#pragma unroll
-            for (int i = i0; i + 1 < M; i += 2) {
-                const float2 l = wp[(q + i) >> 1];
-                const float2 r = wp[(q + 2 * M - 2 - i) >> 1];
-                const float2 sum = __fadd2_rn(l, make_float2(r.y, r.x));
-                acc = __ffma2_rn(sum, (q & 1) ? tp1[(i - 1) >> 1] : tp0[i >> 1], acc);
-            }
-            float a = acc.x + acc.y;
-            auto winv = [&](int k) { return (k & 1) ? wp[k >> 1].y : wp[k >> 1].x; };
-            if (q & 1) a = fmaf(winv(q) + winv(q + 2 * M - 1), c_hbf_taps[PRESET][SET][0], a);  // tap 0
-            // the last tap is unpaired when the paired range [i0, M) has odd length
-            if (((M - i0) & 1) != 0) a = fmaf(winv(q + M - 1) + winv(q + M), c_hbf_taps[PRESET][SET][M - 1], a);
+        hbf_outputs<M, P, PRESET, SET>(wp, [&](int q) {
             const int ce = REL0 + q - M + 1;
-            y[q] = ine[(ce & (P - 1)) * SI + (ce >> LP) + w] + a;
-        }
+            return ine[(ce & (P - 1)) * SI + (ce >> LP) + w];
+        }, y);
         if constexpr (FINAL) {
             // gout points at the block's first output; only [rel_lo, rel_hi) of the block is stored
 #pragma unroll
@@ -296,6 +307,146 @@ __global__ void __launch_bounds__(DEC_NT, CTAS) decim8_tma_kernel(const DecimPar
         // no barrier needed here: the next tile's de-interleave only writes xe/xo (last read before the
         // barrier after stage A), its stage A writes ae/ao (last read before the barrier after stage B), and
         // its stage B writes be/bo after two more barriers
+    }
+}
+
+// ---------------------------------------------------------------------------------------------
+// K3, fifth generation (default): persistent CTAs, stage A reads the contiguous TMA-staged tile itself.
+//
+// The TMA-staged kernel above spends 510 of its 1866 shared-memory wavefronts per 960-output tile (hbf140) on
+// reading the staging buffer back and de-interleaving it into polyphase planes, only so that stage A can read
+// unit-stride planes.  Here each thread computes DIR_P = 18 consecutive stage-A outputs from a window of the raw tile
+// read with LDS.128: run w starts at 16-byte chunk 9w of the staging buffer, so at every step the lanes of a quarter
+// warp sit on chunks 9w + k, whose bank groups (w + k) mod 8 are distinct -- an odd lane stride in chunks makes
+// lane-contiguous windows conflict-free with no padding and no swizzle.  The runs cover NRUN * 18 >= NA outputs; the
+// lowest D of them lie below the tile's stage-A range, are computed from samples that may not even have been copied
+// (below the carry buffer) and are not stored, so the tile geometry, its halo and the host's carry are those of
+// DecGeom.  Two staging buffers: tile t + gridDim.x is copied into the other one when tile t starts.  Stages B and C
+// are hbf_stage as everywhere, and every output is hbf_outputs' expression: bit-identical to the kernels above.
+// ---------------------------------------------------------------------------------------------
+constexpr int DIR_P = 18;  // stage-A outputs per run; P = 2 mod 4 makes the lane stride P/2 chunks odd
+
+__device__ __forceinline__ float4 lds128(const float4* p)
+{
+    float4 v;
+    asm volatile("ld.volatile.shared.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "r"(smem_u32(p)) : "memory");
+    return v;
+}
+
+constexpr int floor4(int v) { return v >= 0 ? v / 4 * 4 : -((3 - v) / 4 * 4); }
+
+template <int MA, int MB, int MC, int OB>
+struct DirectGeom {
+    using GE = DecGeom<MA, MB, MC, OB>;
+    static constexpr int P = DIR_P;
+    static constexpr int NRUN = (GE::NA + P - 1) / P;  // runs per tile (one per thread at most)
+    static constexpr int D = NRUN * P - GE::NA;        // outputs of run 0 below the tile's stage-A range: not stored
+    static constexpr int REL0 = GE::NX / 2 - GE::NA;   // as in hbf_stage: odd-plane index of output j is j + REL0
+    // Relative to the tile's x_base = 8 mhi - NX: run 0's first odd sample (output -D, window element 0) is at F; the
+    // staging buffer starts at the 16-byte chunk holding it and ends with the tile, NXS samples
+    static constexpr int F = 2 * (REL0 - 2 * MA + 1 - D) + 1;
+    static constexpr int XB = floor4(F);
+    static constexpr int NXS = GE::NX - XB;
+    static constexpr int NW = 2 * MA + P - 1;                         // odd samples per run window
+    static constexpr int W0 = F - XB;                                 // window element i = window sample W0 + 2i
+    static constexpr int C0 = 2 * (REL0 - MA + 1 - D) - XB;           // centre of output q = window sample C0 + 2q
+    static constexpr int WCH = (W0 + 2 * (NW - 1)) / 4 + 1;           // LDS.128 per run window
+    // stage-B input planes: polyphase by 8 like hbf_stage's, phase stride = 3 mod 32 (no stride makes the stage-A
+    // stores of lane-consecutive runs conflict-free; with this one about two thirds of them are 2-way)
+    static constexpr int SA = (GE::NA / 2 / DEC_P + 1 - 3 + 31) / 32 * 32 + 3;
+    static constexpr int SMEM_FLOATS = 2 * NXS + 2 * DEC_P * (SA + GE::SB);
+    static_assert(NXS % 4 == 0 && XB <= 0 && W0 >= 0 && C0 >= 0, "staging geometry");
+    static_assert((P / 2) * (NRUN - 1) + WCH <= NXS / 4, "the last run's window ends inside the staging buffer");
+    static_assert(C0 + 2 * (P - 1) < 4 * WCH, "centre samples inside the window");
+    static_assert(NRUN <= DEC_NT && D % 2 == 0 && D < P, "one run per thread; runs start at even outputs");
+    static_assert(SA >= (GE::NA / 2 + DEC_P - 1) / DEC_P, "stage-B planes hold NA / 2 samples each");
+};
+
+template <int MA, int MB, int MC, int OB>
+constexpr size_t decim_direct_smem_bytes()
+{
+    return (size_t)DirectGeom<MA, MB, MC, OB>::SMEM_FLOATS * sizeof(float) + 16;
+}
+
+template <int MA, int MB, int MC, int PRESET, int OB, int CTAS>
+__global__ void __launch_bounds__(DEC_NT, CTAS) decim8_direct_kernel(const DecimParams p, const int ntiles)
+{
+    using GE = DecGeom<MA, MB, MC, OB>;
+    using DG = DirectGeom<MA, MB, MC, OB>;
+    constexpr int P = DG::P;
+    extern __shared__ __align__(16) float smem[];
+    float* stg = smem;                      // two staging buffers of DG::NXS floats, 16-byte aligned
+    float* ae = stg + 2 * DG::NXS;
+    float* ao = ae + DEC_P * DG::SA;
+    float* be = ao + DEC_P * DG::SA;
+    float* bo = be + DEC_P * GE::SB;
+    uint64_t* bar = reinterpret_cast<uint64_t*>(bo + DEC_P * GE::SB);  // one per staging buffer (all counts above are even)
+
+    const int tid = threadIdx.x;
+    if (tid == 0) {
+        mbar_init(bar, 1);
+        mbar_init(bar + 1, 1);
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    }
+    __syncthreads();
+    // tiles as in decim8_tma_kernel; samples below the carry buffer are not copied (they only feed discarded outputs)
+    auto issue = [&](int t, int b) {
+        const long long g = 8 * (p.m1 - (long long)t * OB) - DG::NXS;
+        long long skip = p.src.carry_start - g;
+        skip = skip < 0 ? 0 : (skip > DG::NXS ? DG::NXS : skip);
+        ring_issue(p.src, g + skip, DG::NXS - (int)skip, stg + b * DG::NXS + skip, bar + b);
+    };
+    int tile = blockIdx.x;
+    if (tid == 0 && tile < ntiles) issue(tile, 0);
+    if (p.cc.n) carry_job(p.src, p.cc);  // while the first tile is in flight
+    const long long lo = p.m0 > p.drain ? p.m0 : p.drain;
+    for (unsigned it = 0; tile < ntiles; tile += gridDim.x, ++it) {
+        const long long mhi = p.m1 - (long long)tile * OB;
+        const long long c_base = mhi - OB;
+        const unsigned b = it & 1u;
+        // the other buffer was last read by stage A of the previous tile, two barriers ago
+        if (tid == 0 && tile + (int)gridDim.x < ntiles) issue(tile + (int)gridDim.x, (int)(b ^ 1u));
+        mbar_wait(bar + b, (it >> 1) & 1u);
+        // ---- stage A: run w = stage-A outputs j = P w - D + q, q < P, from the staged tile ----
+        for (int w = tid; w < DG::NRUN; w += DEC_NT) {
+            const float4* __restrict__ s4 = reinterpret_cast<const float4*>(stg + b * DG::NXS) + (P / 2) * w;
+            SSPSD_ASSERT((P / 2) * w + DG::WCH <= DG::NXS / 4);
+            // whole chunks even where only the odd samples are used: a scalar LDS at a lane stride of 36 floats would
+            // be a 4-way bank conflict, so the loads are kept as LDS.128 explicitly
+            float4 v[DG::WCH];
+#pragma unroll
+            for (int k = 0; k < DG::WCH; ++k) v[k] = lds128(s4 + k);
+            auto sample = [&](int s) {
+                const float4& c = v[s >> 2];
+                return (s & 3) == 0 ? c.x : (s & 3) == 1 ? c.y : (s & 3) == 2 ? c.z : c.w;
+            };
+            float2 wp[MA + P / 2];
+#pragma unroll
+            for (int i = 0; i < DG::NW; ++i) {
+                const float x = sample(DG::W0 + 2 * i);
+                if (i & 1) wp[i >> 1].y = x; else wp[i >> 1].x = x;
+            }
+            float y[P];
+            hbf_outputs<MA, P, PRESET, 2>(wp, [&](int q) { return sample(DG::C0 + 2 * q); }, y);
+            // output j (even: plane ae, odd: ao) has plane index j >> 1 = (P/2) w + (q - D) >> 1
+#pragma unroll
+            for (int q = 0; q < P; ++q) {
+                if (q >= DG::D || w > 0) {
+                    const int r = (P / 2) * w + ((q - DG::D) >> 1);
+                    SSPSD_ASSERT(r >= 0 && r < GE::NA / 2);
+                    ((q & 1) ? ao : ae)[(r & (DEC_P - 1)) * DG::SA + (r >> DEC_LP)] = y[q];
+                }
+            }
+        }
+        __syncthreads();
+        hbf_stage<MB, DG::SA, GE::SB, GE::NA / 2 - GE::NB, false, PRESET, 1>(ae, ao, GE::NB, be, bo, nullptr, 0, 0);
+        __syncthreads();
+        const int rel_lo = lo > c_base ? (int)(lo - c_base) : 0;
+        hbf_stage<MC, GE::SB, GE::SB, GE::NB / 2 - OB, true, PRESET, 0>(be, bo, OB, nullptr, nullptr,
+                                                                        p.out_fresh + (c_base - p.drain - p.out_split),
+                                                                        rel_lo, OB, c_base - p.drain - p.out_split, p.out_cap);
+        // no barrier needed here: the next tile's stage A writes ae/ao (last read by stage B, before the barrier
+        // after it) and its stage B writes be/bo after the barrier that follows stage A
     }
 }
 
